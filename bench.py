@@ -9,6 +9,7 @@ env-step, Env(0, tick 1, step 1_000_000).  One bench "step" = one full pass of t
 global env id; no per-step collective, one NCCL all-gather of the statistics at the end.
 
     python bench.py --gpus 1 --steps 5 --warmup 3
+    python bench.py --gpus 1 --steps 5 --warmup 3 --dump-outputs DIR   # + the last timed pass's outputs, DIR/*.npy
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference        # the reference's CPU algorithm (oracle) on the host cores
 """
@@ -148,6 +149,36 @@ def run_reference(args):
     return 0
 
 
+DUMP_HISTORY_BYTES = 8 << 20   # per workload; with the row caps below, c3 + c4 + c5 stay under 64 MB in all
+DUMP_LOG_ENVS, DUMP_LOG_ROWS = 2, 32768
+TRADE_COLS = ("t", "side", "price", "vol", "active", "passive")
+ORDER_COLS = ("side", "status", "arr_time", "end_time", "vol", "start_vol", "price", "trader")
+
+
+def dump_outputs(env, out_dir: str, prefix: str):
+    """Writes what a caller of the timed path holds after its last pass, for a fixed (seed 0) sample of the envs, as
+    float64 .npy files (every field is an integer below 2**53, so float64 holds it exactly):
+      <prefix>_envs      sampled env indices (local to this rank)
+      <prefix>_history   [env, step, word] observation history of the sampled envs
+      <prefix>_trades    [row] env, trade index, then t, side, price, vol, active id, passive id  (first DUMP_LOG_ENVS envs)
+      <prefix>_orders    [row] env, order id, then side, status, arr_time, end_time, vol, start_vol, price, trader  (same envs)
+    Trade and order tables longer than DUMP_LOG_ROWS are sampled (seed 0) to that many rows."""
+    rng = np.random.default_rng(0)
+    row_bytes = max(1, env.n_steps(0)) * env.obs_words * 8
+    envs = np.sort(rng.choice(env.n_envs, min(env.n_envs, 256, max(1, DUMP_HISTORY_BYTES // row_bytes)), replace=False))
+    out = {"envs": envs, "history": np.stack([env.history(int(e)) for e in envs])}
+    for name, cols, read in (("trades", TRADE_COLS, env.trades_arrays), ("orders", ORDER_COLS, env.orders_arrays)):
+        rows = []
+        for e in envs[:DUMP_LOG_ENVS]:
+            c = read(int(e))
+            n = len(c[cols[0]])
+            idx = np.arange(n) if n <= DUMP_LOG_ROWS else np.sort(rng.choice(n, DUMP_LOG_ROWS, replace=False))
+            rows.append(np.stack([np.full(len(idx), e), idx] + [c[k][idx] for k in cols], axis=1).astype(np.float64))
+        out[name] = np.concatenate(rows)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{prefix}_{name}.npy"), np.asarray(a, dtype=np.float64))
+
+
 def workload_config(n_gpus: int, sample: str | None = None) -> dict:
     c = {"workload": "C3: 4096 envs/GPU x (50+50) RandomAgents x 1000 env-steps, level-1 obs per env-step, "
                      "Env(start 0, tick 1, step 1_000_000), agents tick_size 2 (crates/step_sim/examples/random_agents/main.rs)",
@@ -218,6 +249,8 @@ def run_gpu(args):
     stats = env.stats()
     if stats["error_envs"]:
         raise SystemExit(f"device flagged errors in {stats['error_envs']} envs: {np.unique(env.env_errors())}")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(env, args.dump_outputs, "c3")
     total_ms = sum(step_ms)
 
     # ---- end-to-end through the public API with HOST buffers: agent table up, full obs history + stats down
@@ -247,7 +280,7 @@ def run_gpu(args):
         cap_t, cap_o = int(n_tr.max()) + 1024, int(n_or.max()) + 1024
         tr_host = torch.empty((n_envs, cap_t, 32), dtype=torch.uint8, pin_memory=True).numpy().view(abi.TRADE_REC_DTYPE).reshape(n_envs, cap_t)
         or_host = torch.empty((n_envs, cap_o, 64), dtype=torch.uint8, pin_memory=True).numpy().view(abi.ORDER_REC_DTYPE).reshape(n_envs, cap_o)
-        n_log = 2
+        n_log = args.steps
         for i in range(n_log + 1):
             if i == 1:
                 barrier()
@@ -310,9 +343,9 @@ def run_gpu(args):
         env.close()
         del hist_host
         torch.cuda.empty_cache()
-        c4 = measure_c4(ctx, 8192, N_SIM_STEPS, 3, 3, args.max_orders, args.max_trades, False)
+        c4 = measure_c4(ctx, 8192, N_SIM_STEPS, args.steps, args.warmup, args.max_orders, args.max_trades, False, args.dump_outputs)
         c5_books = min(512, max(1, 1024 // world))
-        c5 = measure_c5(ctx, c5_books, 2, 3, "deep", 10, world == 1 and not args.no_cpu)
+        c5 = measure_c5(ctx, c5_books, args.steps, args.warmup, "deep", 10, world == 1 and not args.no_cpu, args.dump_outputs)
         c5["scaling"] = "strong (1024 books over the ranks)" if c5_books * world == 1024 else f"{c5_books * world} of the 1024 books (one GPU holds at most 512)"
         secondary = {"c4": c4, "c5": c5}
     if rank == 0:
@@ -502,7 +535,8 @@ def roofline_block(alg_bytes: float, k_ms: float, kernel: str, traffic=None) -> 
             "kernel_ms": k_ms, "algorithmic_bytes_per_launch": alg_bytes, "peak_source": peak_src}
 
 
-def measure_c4(ctx: Ctx, per_gpu: int, n_steps: int, steps: int, warmup: int, max_orders: int, max_trades: int, with_cpu: bool) -> dict:
+def measure_c4(ctx: Ctx, per_gpu: int, n_steps: int, steps: int, warmup: int, max_orders: int, max_trades: int, with_cpu: bool,
+               dump_dir: str | None = None) -> dict:
     """BASELINE config C4, one GPU's shard per rank: `per_gpu` envs x (40+40 RandomAgents + 20-trader MomentumAgent) x
     n_steps env-steps, level-2 (45-word) record per env-step.  The general (paged) engine: whenever a book's ask side is
     swept empty the MomentumAgent's mid price is ~2^31 (orderbook.rs:272-276 with the empty-side sentinel) and its limit
@@ -532,6 +566,8 @@ def measure_c4(ctx: Ctx, per_gpu: int, n_steps: int, steps: int, warmup: int, ma
     stats = env.stats()
     if stats["error_envs"]:
         raise SystemExit(f"C4: device flagged errors in {stats['error_envs']} envs")
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(env, dump_dir, "c4")
     agg = gather_env_stats(env, sum(ms), ctx.comm)
     k_ms = sum(ms) / len(ms)
     out = {"workload": f"C4 shard: {per_gpu} envs/GPU x (40+40 RandomAgents + 20-trader MomentumAgent) x {n_steps} env-steps, "
@@ -554,7 +590,8 @@ def measure_c4(ctx: Ctx, per_gpu: int, n_steps: int, steps: int, warmup: int, ma
 C5_WINDOW, C5_CHUNKS = (7936, 12160), 98304
 
 
-def measure_c5(ctx: Ctx, per_gpu: int, steps: int, warmup: int, engine: str, pages_smem: int, with_cpu: bool) -> dict:
+def measure_c5(ctx: Ctx, per_gpu: int, steps: int, warmup: int, engine: str, pages_smem: int, with_cpu: bool,
+               dump_dir: str | None = None) -> dict:
     """BASELINE config C5, one GPU's shard per rank: `per_gpu` books x 1,000,000 resting orders (pre-loaded, untimed), then
     100 steps x 10,000 events per book with a 30% cancel/modify rate, replayed from device memory (timed)."""
     import torch
@@ -610,6 +647,8 @@ def measure_c5(ctx: Ctx, per_gpu: int, steps: int, warmup: int, engine: str, pag
     stats = env.stats()
     if stats["error_envs"]:
         raise SystemExit(f"C5: device flagged errors in {stats['error_envs']} envs")
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(env, dump_dir, "c5")
     # only the timed phase counts
     stats = {k: (stats[k] - pre_stats[k] if k in ("instructions", "orders_created", "trades", "traded_volume", "transitions", "env_steps") else stats[k]) for k in stats}
     stats["env_steps"] = n_envs * n_steps
@@ -680,14 +719,14 @@ def run_gpu_other(args):
     ev = ctx.events(args.steps)
     if args.workload == "c4":
         res = measure_c4(ctx, args.envs if args.envs != N_ENVS_PER_GPU else 8192, args.sim_steps, args.steps, args.warmup, args.max_orders,
-                         args.max_trades, world == 1 and not args.no_cpu)
+                         args.max_trades, world == 1 and not args.no_cpu, args.dump_outputs)
         if rank == 0:
             print(json.dumps(secondary_line(args, ctx, res)))
         ctx.finish()
         return 0
     if args.workload == "c5":
         res = measure_c5(ctx, args.envs if args.envs != N_ENVS_PER_GPU else 128, args.steps, args.warmup, args.engine, args.pages_smem,
-                         world == 1 and not args.no_cpu)
+                         world == 1 and not args.no_cpu, args.dump_outputs)
         if rank == 0:
             print(json.dumps(secondary_line(args, ctx, res)))
         ctx.finish()
@@ -826,7 +865,15 @@ def main():
                     help="default: dense for c3 / market (shallow books inside a known price window), paged for gym")
     ap.add_argument("--workload", default="c3", choices=["c1", "c2", "c3", "c4", "c5", "market", "gym"],
                     help="c3 = the headline line; the others are the secondary configs (market = the multi-asset example)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed pass computed (a seeded sample: observation history, "
+                         "trade log, order table) as DIR/<workload>_<name>.npy, float64, under 64 MB; c3 (with the c4 / c5 "
+                         "block), c4 and c5 only; rank 0's shard when --gpus > 1")
     args = ap.parse_args()
+    if args.dump_outputs:
+        if args.impl != "b200" or args.workload not in ("c3", "c4", "c5"):
+            ap.error("--dump-outputs covers the b200 c3, c4 and c5 workloads")
+        os.makedirs(args.dump_outputs, exist_ok=True)
     if args.engine is None:
         # c2: one CTA per book (k_deepw) while at most two books share an SM, the paged engine (one warp per book) beyond
         c2_deep = args.workload == "c2" and (args.envs == N_ENVS_PER_GPU or args.envs <= 296)
