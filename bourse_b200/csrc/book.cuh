@@ -213,6 +213,7 @@ struct Book {
     u32 free_top;          // dense engine: entries on the free-slot stack
     u32 ags;               // dense engine, k_sim: shared-space address of the agent -> slot table (u8, entry 0 unused)
     u64 tr_ptr;            // dense engine: address of the next trade record
+    u32 ev, jp, jend;      // dense k_sim, journaled (d_apply JRN): the event's queue entry, next / end of the trade journal
 };
 
 __device__ __forceinline__ u32 tag_addr(const Book& b, u32 i) { return b.sb + 128u + 4u * i; }

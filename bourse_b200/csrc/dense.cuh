@@ -101,12 +101,15 @@ template <class G> __device__ __forceinline__ void d_free_slot(Book& b, u32 slot
 // the loop body only runs while volume is left, so that is exactly "some fill brought the volume to zero".
 // STEPPED (k_sim): the per-launch transition / volume counters are settled once per env-step by the caller (from the
 // trade count and the step's trade_vol) instead of once per fill.
-template <bool STEPPED, class G> __device__ __forceinline__ u32 d_match(const G& g, Book& b, u32 side, u32 price, u32 vol, u32 id, u64 t) {
+// JRN: each fill leaves one trade-journal entry instead of its trade record, passive-record stores and counter updates
+// (see d_flush); the loop stops early, with volume left, when the journal is full.
+template <bool STEPPED, bool JRN, class G> __device__ __forceinline__ u32 d_match(const G& g, Book& b, u32 side, u32 price, u32 vol, u32 id, u64 t) {
     const u32 o = side ^ 1u;
     while (vol > 0u && has_best(b, o)) {
         const u32 bq = best_q(b, o);
         const u32 bprice = g.d_win_lo + bq;
         if (side ? (price < bprice) : (price > bprice)) break;
+        if (JRN && b.jp == b.jend) break;
         const u32 la = d_lv<G>(b, o, bq);
         const u64 lv = lds64(la);
         const u32 lvol = (u32)lv, hi = (u32)(lv >> 32);
@@ -115,8 +118,13 @@ template <bool STEPPED, class G> __device__ __forceinline__ u32 d_match(const G&
         const u32 pid = lds(sa + G::DL::OFF_ID), pvol = lds(sa + G::DL::OFF_SV);
         const u32 tv = min(vol, pvol);
         vol -= tv;
-        d_log_trade(g, b, t, o, bprice, tv, id, pid);
-        b.trade_vol += tv;
+        if (JRN) {
+            sts128(b.jp, make_uint4(b.ev | (bq << 20), pid, tv, pvol - tv));
+            b.jp += 16u;
+        } else {
+            d_log_trade(g, b, t, o, bprice, tv, id, pid);
+            b.trade_vol += tv;
+        }
         if (!STEPPED) {
             b.d_volume += tv;
             b.d_trans += 1;
@@ -124,9 +132,11 @@ template <bool STEPPED, class G> __device__ __forceinline__ u32 d_match(const G&
         add_side_vol(b, o, 0u - tv);
         const u64 pa = b.oh + (u64)pid * ORD_STRIDE;
         if (pvol == tv) {  // passive order Filled: leaves its slot and the head of its level
-            stg32(pa + OH_VOL, 0u);
-            stg32(pa + OH_META, ST_FILLED | (o ? META_BID : 0u));
-            stg64(pa + OC_END, t);
+            if (!JRN) {
+                stg32(pa + OH_VOL, 0u);
+                stg32(pa + OH_META, ST_FILLED | (o ? META_BID : 0u));
+                stg64(pa + OC_END, t);
+            }
             const u32 nxt = lds8(sa + G::DL::OFF_SL);
             d_free_slot<G>(b, head);
             if ((hi & 0xFFFFu) == 1u) {  // last order of the level (its `next` byte is stale by design)
@@ -139,7 +149,7 @@ template <bool STEPPED, class G> __device__ __forceinline__ u32 d_match(const G&
             }
         } else {
             sts(sa + G::DL::OFF_SV, pvol - tv);
-            stg32(pa + OH_VOL, pvol - tv);
+            if (!JRN) stg32(pa + OH_VOL, pvol - tv);
             sts(la, lvol - tv);  // side.remove_vol(price, tv)
         }
     }
@@ -152,8 +162,9 @@ template <bool STEPPED, class G> __device__ __forceinline__ u32 d_match(const G&
 // CHECK_TIME: the caller cannot guarantee that time moves strictly forward between resting inserts (replay mode).
 // CHECK_SLOTS: false when the caller has already made sure that a free slot exists (k_sim validates a whole env-step's
 // new orders against the free-slot count up front, so the event loop carries no per-insert test).
-template <bool CHECK_TIME, bool CHECK_SLOTS, class G> __device__ __forceinline__ u32 d_insert(const G& g, Book& b, u32 side, u32 price, u64 t,
-                                                                            u32 id, u32 vol) {
+// JRN: max_key_time is settled by d_flush.
+template <bool CHECK_TIME, bool CHECK_SLOTS, bool JRN, class G>
+__device__ __forceinline__ u32 d_insert(const G& g, Book& b, u32 side, u32 price, u64 t, u32 id, u32 vol) {
     u32 q = price - g.d_win_lo;
     if (q >= g.d_levels) {
         b.err |= ERR_CAP_PAGES;
@@ -193,7 +204,7 @@ template <bool CHECK_TIME, bool CHECK_SLOTS, class G> __device__ __forceinline__
     add_side_vol(b, side, vol);
     if (CHECK_TIME) {
         if (t > b.max_key_time) b.max_key_time = t;
-    } else {
+    } else if (!JRN) {
         b.max_key_time = t;  // time is strictly increasing by construction
     }
     return slot;
@@ -245,26 +256,38 @@ template <class G> __device__ __forceinline__ void d_remove(Book& b, u32 slot, u
 //   CANCEL hint = 1 + the slot the order was resting in when the agent looked: a mismatch of the slot's id means
 //          the order has left the book since (filled earlier in this step) and the cancel is a no-op
 // With HINT != 0 ids are trusted (generated in-kernel, capacity validated once per step by the caller).
-template <bool IS_NEW, bool CHECK_TIME, int HINT, class G>
-__device__ __forceinline__ void d_apply(const G& g, Book& b, u32 kind, u32 id, u32 side, u32 price, u32 vol, u32 trader, bool has_p,
-                                        bool has_v, u64 t, u32 hint) {
+// JRN (k_sim with RandomAgents only; HINT == 1, NEW and CANCEL only): no order record, trade record or trade counter is
+// written here.  The event leaves its outcome in its own queue entry at shared address Book::ev (NEW: the remaining
+// volume in the id word; CANCEL: 2 | side in the last word when it took effect, which the agents leave 0) and one
+// trade-journal entry per fill; d_flush turns them into the HBM writes.  `t` is unused.  Returns 0, or, when a fill
+// found the journal full, the NEW order's remaining volume: the event is then suspended before it rests, and the
+// caller flushes and runs it again with that volume.
+template <bool IS_NEW, bool CHECK_TIME, int HINT, bool JRN = false, class G>
+__device__ __forceinline__ u32 d_apply(const G& g, Book& b, u32 kind, u32 id, u32 side, u32 price, u32 vol, u32 trader, bool has_p,
+                                       bool has_v, u64 t, u32 hint) {
+    static_assert(!JRN || HINT == 1, "the journal derives order ids from the agents' hints");
     const u64 ra = b.oh + (u64)id * ORD_STRIDE;
     if (IS_NEW) {
         if (HINT == 0 && id >= g.max_orders) {
             b.err |= ERR_CAP_ORDERS;
-            return;
+            return 0u;
         }
         const bool trading = (b.flags & FL_TRADING) != 0u;
         u32 rem = vol;
-        if (trading) rem = d_match<HINT != 0>(g, b, side, price, vol, id, t);
+        if (trading) rem = d_match<HINT != 0, JRN>(g, b, side, price, vol, id, t);
+        if (JRN && rem != 0u && b.jp == b.jend) return rem;
         const bool filled = vol != 0u && rem == 0u;
         const bool market = side ? (price == 0xFFFFFFFFu) : (price == 0u);  // N3
         const bool ended = filled || market;
         // Filled, or an unfilled market order: Cancelled when trading, Rejected otherwise (orderbook.rs:517-531)
         const u32 status = filled ? ST_FILLED : market ? (trading ? ST_CANCELLED : ST_REJECTED) : ST_ACTIVE;
         if (!ended) {
-            const u32 slot = d_insert<CHECK_TIME, HINT == 0>(g, b, side, price, t, id, rem);
+            const u32 slot = d_insert<CHECK_TIME, HINT == 0, JRN>(g, b, side, price, t, id, rem);
             if (HINT == 1 || (HINT == 2 && hint)) sts8(b.ags + hint, slot);
+        }
+        if (JRN) {
+            sts(b.ev + 4u, rem);
+            return 0u;
         }
         // order record; the queue links of the HBM record are not used by this engine
         const u64 kt = ended ? 0ULL : t, end_time = ended ? t : ~0ULL;
@@ -279,26 +302,26 @@ __device__ __forceinline__ void d_apply(const G& g, Book& b, u32 kind, u32 id, u
         stg128(ra + OC_ARR, (u32)t, (u32)(t >> 32), (u32)end_time, (u32)(end_time >> 32));
         stg32(ra + OC_TRADER, trader);
         if (HINT == 0) b.d_trans += 1;
-        return;
+        return 0u;
     }
     if (HINT == 0 && (id >= b.n_orders || id >= g.max_orders)) {
         b.err |= ERR_BAD_ID;  // the reference panics (orderbook.rs:642, :749)
-        return;
+        return 0u;
     }
     u32 slot;
     if (HINT == 1 || (HINT == 2 && hint)) {
         slot = hint - 1u;
-        if (lds(b.sb + 4u * slot + G::DL::OFF_ID) != id) return;
+        if (lds(b.sb + 4u * slot + G::DL::OFF_ID) != id) return 0u;
     } else {
         slot = d_find<G>(b, id);
-        if (slot == D_NIL) return;  // not Active: cancel / modify are no-ops
+        if (slot == D_NIL) return 0u;  // not Active: cancel / modify are no-ops
     }
     const u32 sa = b.sb + 4u * slot;
     const u32 link = lds(sa + G::DL::OFF_SL), svol = lds(sa + G::DL::OFF_SV);
     const u32 next = link & 0xFFu, prev = (link >> 8) & 0xFFu, q = (link >> 16) & 0x7FFFu;
     side = link >> 31;
     if (kind == EV_MODIFY) {
-        if (!has_p && !has_v) return;
+        if (!has_p && !has_v) return 0u;
         if (!has_p && vol < svol) {  // reduce in place: priority kept (orderbook.rs:755-757)
             const u32 la = d_lv<G>(b, side, q);
             sts(sa + G::DL::OFF_SV, vol);
@@ -306,28 +329,111 @@ __device__ __forceinline__ void d_apply(const G& g, Book& b, u32 kind, u32 id, u
             add_side_vol(b, side, vol - svol);
             stg32(ra + OH_VOL, vol);
             b.d_trans += 1;
-            return;
+            return 0u;
         }
         if (!has_p) price = g.d_win_lo + q;
         if (!has_v) vol = svol;
     }
     d_remove<G>(b, slot, side, q, next, prev, svol);
     const u32 side_bit = side ? META_BID : 0u;
-    if (kind == EV_CANCEL) {
-        stg32(ra + OH_META, ST_CANCELLED | side_bit);
-        stg64(ra + OC_END, t);
+    if (JRN || kind == EV_CANCEL) {
+        if (JRN) {
+            sts(b.ev + 12u, 2u | side);
+        } else {
+            stg32(ra + OH_META, ST_CANCELLED | side_bit);
+            stg64(ra + OC_END, t);
+        }
         b.d_trans += 1;
-        return;
+        return 0u;
     }
     // replace_order (orderbook.rs:679-723): re-match, re-rest under key time t; never a market order (N4)
     u32 rem = vol;
-    if (b.flags & FL_TRADING) rem = d_match<HINT != 0>(g, b, side, price, vol, id, t);
+    if (b.flags & FL_TRADING) rem = d_match<HINT != 0, false>(g, b, side, price, vol, id, t);
     const bool filled = vol != 0u && rem == 0u;
-    if (!filled) d_insert<CHECK_TIME, HINT == 0>(g, b, side, price, t, id, rem);
+    if (!filled) d_insert<CHECK_TIME, HINT == 0, false>(g, b, side, price, t, id, rem);
     stg64v(ra + OH_PRICE, price, rem);
     stg32(ra + OH_META, (filled ? ST_FILLED : ST_ACTIVE) | side_bit);
     stg64(ra + (filled ? OC_END : OH_KEYT), t);
     b.d_trans += 1;
+    return 0u;
+}
+
+// Write-out of a journaled (JRN) stretch of an env-step, all lanes: the events at queue positions [e_lo, e_hi) — complete,
+// outcomes in place — and the `nj` trade-journal entries at `jb` (16 B each: queue-entry address | level << 20, passive
+// id, traded volume, passive volume left).  The stores, and the bytes they leave in the order table and the trade log,
+// are those of the write-through path: the write-out only moves them off lane 0's chain, where each record cost several
+// dependent instructions, to one store per lane.  Every record is written by at most one lane per instruction, and in
+// event order across instructions (a passive order's volume word keeps the value of its last fill); the __syncwarp
+// calls order the stores of different lanes to one record.  Settles the counters the event loop no longer keeps:
+// n_trades, trade_vol and max_key_time.  `agh`: the agents' held ids (a NEW event's id, by its hint).
+template <class G>
+__device__ __forceinline__ void d_flush(const G& g, Book& b, u32 qs, u32 agh, u64 start, u32 e_lo, u32 e_hi, u32 jb, u32 nj) {
+    const bool trading = (b.flags & FL_TRADING) != 0u;
+    u32 last_rest = 0;  // 1 + queue position of the last order that rested
+    for (u32 i = e_lo + b.lane; i < e_hi; i += 32u) {
+        const uint4 ev = lds128(qs + 16u * i);
+        const u64 t = start + i;
+        const u32 side_bit = (ev.x & 2u) ? META_BID : 0u;
+        if (ev.x & 1u) {
+            const u32 id = lds(agh + 4u * ((ev.x >> 2) & 0x7FFu) - 4u);
+            const u32 price = ev.z, vol = ev.w, rem = ev.y;
+            const bool filled = vol != 0u && rem == 0u;
+            const bool market = side_bit ? (price == 0xFFFFFFFFu) : (price == 0u);
+            const bool ended = filled || market;
+            const u32 status = filled ? ST_FILLED : market ? (trading ? ST_CANCELLED : ST_REJECTED) : ST_ACTIVE;
+            if (!ended) last_rest = i + 1u;
+            // 52 of the record's 64 bytes, as on the write-through path (see d_apply)
+            const u64 ra = b.oh + (u64)id * ORD_STRIDE;
+            const u64 kt = ended ? 0ULL : t, end_time = ended ? t : ~0ULL;
+            stg64v(ra + OH_PRICE, price, rem);
+            stg128(ra + OH_KEYT, (u32)kt, (u32)(kt >> 32), status | side_bit, vol);
+            stg128(ra + OC_ARR, (u32)t, (u32)(t >> 32), (u32)end_time, (u32)(end_time >> 32));
+            stg32(ra + OC_TRADER, ev.x >> 13);
+        } else if (ev.w) {
+            const u64 ra = b.oh + (u64)ev.y * ORD_STRIDE;
+            stg32(ra + OH_META, ST_CANCELLED | ((ev.w & 1u) ? META_BID : 0u));
+            stg64(ra + OC_END, t);
+        }
+    }
+    last_rest = __reduce_max_sync(BB_FULL, last_rest);
+    if (last_rest) b.max_key_time = start + (last_rest - 1u);
+    __syncwarp();
+    u32 err = 0, tv_sum = 0;
+    const u64 tr_env = g.tr_base + (u64)b.env * g.max_trades * 32u;
+    for (u32 k0 = 0; k0 < nj; k0 += 32u) {
+        const u32 k = k0 + b.lane;
+        const bool valid = k < nj;
+        const uint4 je = valid ? lds128(jb + 16u * k) : make_uint4(0u, BB_NIL, 0u, 0u);
+        const u32 same = __match_any_sync(BB_FULL, je.y);  // lanes of this chunk that fill the same passive order
+        if (valid) {
+            const u32 ea = je.x & 0xFFFFFu, pid = je.y, tv = je.z, left = je.w;
+            const u32 ax = lds(ea);  // the aggressor's queue entry
+            const u32 active = lds(agh + 4u * ((ax >> 2) & 0x7FFu) - 4u);
+            const u32 o = ((ax >> 1) & 1u) ^ 1u;
+            const u64 t = start + ((ea - qs) >> 4);
+            const u32 idx = b.n_trades + k;
+            if (idx < g.max_trades) {
+                const u64 ta = tr_env + (u64)idx * 32u;
+                stg128_cs(ta, (u32)t, (u32)(t >> 32), g.d_win_lo + (je.x >> 20), tv);
+                stg128_cs(ta + 16u, active, pid, o, 0u);
+            } else if (g.max_trades) {
+                err |= ERR_CAP_TRADES;
+            }
+            if ((same >> b.lane) == 1u) {  // the chunk's last fill of this passive order
+                const u64 pa = b.oh + (u64)pid * ORD_STRIDE;
+                stg32(pa + OH_VOL, left);
+                if (left == 0u) {
+                    stg32(pa + OH_META, ST_FILLED | (o ? META_BID : 0u));
+                    stg64(pa + OC_END, t);
+                }
+            }
+            tv_sum += tv;
+        }
+        __syncwarp();
+    }
+    b.trade_vol += __reduce_add_sync(BB_FULL, tv_sum);
+    b.n_trades += nj;
+    b.err |= __reduce_or_sync(BB_FULL, err);
 }
 
 // bb_load_book: put an Active order read from its HBM record back on its side (orderbook.rs:898-905)
@@ -336,7 +442,7 @@ template <class G> __device__ __forceinline__ void d_restore(const G& g, Book& b
     const uint4 a = ldg128(ra), c = ldg128(ra + 16u);
     if (order_id + 1u > b.n_orders) b.n_orders = order_id + 1u;
     if ((c.z & META_STATUS_MASK) == ST_ACTIVE)
-        d_insert<true, true>(g, b, (c.z & META_BID) ? 1u : 0u, a.x, ((u64)c.y << 32) | c.x, order_id, a.y);
+        d_insert<true, true, false>(g, b, (c.z & META_BID) ? 1u : 0u, a.x, ((u64)c.y << 32) | c.x, order_id, a.y);
 }
 
 // (vol, count) at an arbitrary price; per-lane (prices may differ between lanes)

@@ -452,11 +452,12 @@ __device__ __forceinline__ void random_agents_update_dense(const KParams& p, con
         const u32 side_bid = r.y >> 31;
         const u32 tick = ag.tick_lo + mulhi_range(r.z, ag.tick_hi - ag.tick_lo);
         const u32 vol = ag.vol_lo + mulhi_range(r.w, ag.vol_hi - ag.vol_lo);
-        // x: bit 0 NEW, bit 1 bid, bits 2..12 hint (NEW: 1 + agent index; CANCEL: 1 + slot), bits 13.. trader id
+        // x: bit 0 NEW, bit 1 bid, bits 2..12 hint (NEW: 1 + agent index; CANCEL: 1 + slot), bits 13.. trader id;
+        // w: a cancel's is 0 (the journaled event loop marks the cancels that take effect there)
         const u32 of = do_cancel ? ((hs + 1u) << 2) : (1u | (side_bid << 1) | ((ai + 1u) << 2) | (a << 13));
         const u32 pos = e.n + __popc(act_mask & below);
         if (active) {
-            if (pos < p.max_queue) sts128(qs + 16u * pos, make_uint4(of, do_cancel ? held : id, tick * ag.tick_size, vol));
+            if (pos < p.max_queue) sts128(qs + 16u * pos, make_uint4(of, do_cancel ? held : id, tick * ag.tick_size, do_cancel ? 0u : vol));
             sts(agh + 4u * ai, do_cancel ? BB_NIL : id);
         }
         e.n += __popc(act_mask);
@@ -870,7 +871,65 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                 __syncwarp();
             }
             // process in shuffled order at t = start + i
-            if constexpr (G::DENSE) {
+            if constexpr (G::DENSE && !MOM && !MKT) {
+                // Journaled: lane 0 runs the events alone (see below) and keeps only the book itself; the order records,
+                // the trade log and the trade counters are written by all lanes after it (d_flush).  The trade journal
+                // fills the queue entries past the step's events: when it is full, lane 0 stops, the warp flushes, and
+                // lane 0 goes on from the suspended event with the volume it had left.
+                const u32 nt0 = b.n_trades;
+                const u32 jb = qs + 16u * n, jend = qs + 16u * (p.max_queue + 2u);
+                u32 done = 0, rv = 0;  // events already written out; volume left of the suspended event `done`
+                for (;;) {
+                    u32 stop = n;
+                    if (lane == 0) {
+                        b.jp = jb;
+                        b.jend = jend;
+                        // two inlined handler copies on alternating prefetched quads, as on the write-through path
+                        auto handle = [&](const uint4& ev, u32 i) -> u32 {
+                            const u32 hint = (ev.x >> 2) & 0x7FFu;
+                            b.ev = qs + 16u * i;
+                            if (ev.x & 1u) {
+                                if (ev.x & 2u) return d_apply<true, false, 1, true>(g, b, EV_NEW, ev.y, 1u, ev.z, ev.w, 0u, false, false, 0ull, hint);
+                                return d_apply<true, false, 1, true>(g, b, EV_NEW, ev.y, 0u, ev.z, ev.w, 0u, false, false, 0ull, hint);
+                            }
+                            return d_apply<false, false, 1, true>(g, b, EV_CANCEL, ev.y, 0u, 0u, 0u, 0u, false, false, 0ull, hint);
+                        };
+                        uint4 e0 = lds128(qs + 16u * done);
+                        if (rv) e0.w = rv;
+                        for (u32 i = done; i < n; i += 2) {
+                            const uint4 e1 = lds128(qs + 16u * i + 16u);  // (the queue is padded by two entries)
+                            if ((rv = handle(e0, i))) {
+                                stop = i;
+                                break;
+                            }
+                            if (i + 1 >= n) break;
+                            e0 = lds128(qs + 16u * i + 32u);
+                            if ((rv = handle(e1, i + 1))) {
+                                stop = i + 1;
+                                break;
+                            }
+                        }
+                    }
+                    __syncwarp();
+                    stop = __shfl_sync(BB_FULL, stop, 0);
+                    rv = __shfl_sync(BB_FULL, rv, 0);
+                    const u32 nj = (__shfl_sync(BB_FULL, b.jp, 0) - jb) >> 4;
+                    b.vol_ask = __shfl_sync(BB_FULL, b.vol_ask, 0);
+                    b.vol_bid = __shfl_sync(BB_FULL, b.vol_bid, 0);
+                    b.bq_ask = __shfl_sync(BB_FULL, b.bq_ask, 0);
+                    b.bq_bid = __shfl_sync(BB_FULL, b.bq_bid, 0);
+                    b.flags = __shfl_sync(BB_FULL, b.flags, 0);
+                    b.d_trans = __shfl_sync(BB_FULL, b.d_trans, 0);
+                    b.free_top = __shfl_sync(BB_FULL, b.free_top, 0);
+                    b.err = __shfl_sync(BB_FULL, b.err, 0);
+                    d_flush(g, b, qs, agh, start, done, stop, jb, nj);
+                    done = stop;
+                    if (stop == n) break;
+                }
+                // transitions of the step: one per placed order and per fill (cancels counted theirs); traded volume
+                b.d_trans += (b.n_trades - nt0) + (n ? e.next_id - id0 : 0u);
+                b.d_volume += b.trade_vol;
+            } else if constexpr (G::DENSE) {
                 constexpr int H = MOM ? 2 : 1;  // RandomAgents always hint, MomentumAgent / NoiseAgent never do
                 // With every event hinted the matching path has no lane-parallel step left, so it runs on LANE 0 ALONE:
                 // a warp-uniform ld/st moves 32 copies of the same bytes through the L1 data pipe (4 wavefronts for a
