@@ -12,6 +12,7 @@ lockstep, with the same per-env semantics.
 from __future__ import annotations
 
 import ctypes as C
+import math
 import typing
 
 import numpy as np
@@ -59,14 +60,29 @@ class BatchedEnv:
     agents raise.
 
     `assets=A` (> 1) groups consecutive books into multi-asset markets with MarketEnv semantics
-    (crates/step_sim/src/market_env.rs:108-121); see `bourse_b200.market`."""
+    (crates/step_sim/src/market_env.rs:108-121); see `bourse_b200.market`.
 
-    def __init__(self, n_envs: int, seed: int, start_time: int, tick_size: int, step_size: int, trading: bool = True, *,
+    `tick_size` is one tick for every env, or a sequence of `n_envs` ticks, one per env (bb_set_tick_sizes): each book then
+    checks limit prices against its own tick and lays out its level-2 record at its own tick offsets.  Without an explicit
+    `price_granule` or `price_window` the ladder granule of a sequence is the gcd of its ticks.  On the paged engine a book
+    whose tick is k times the granule spreads its levels k times more thinly over the 32-price pages and may need a larger
+    `pages_total`; the dense and deep engines are unaffected."""
+
+    def __init__(self, n_envs: int, seed: int, start_time: int, tick_size: typing.Union[int, typing.Sequence[int]], step_size: int,
+                 trading: bool = True, *,
                  device: int = 0, env_id_base: int = 0, obs_words: int = abi.OBS_L2, max_orders: int = 1 << 16,
                  max_trades: int = 1 << 16, max_steps: int = 1 << 12, max_queue: int = 256, pages_smem: int = 0,
                  pages_total: int = 0, price_granule: int = 0, price_window: typing.Optional[typing.Tuple[int, int]] = None,
                  live_cap: int = 0, assets: int = 0, deep_chunks: int = 0):
         self._lib = abi.load()
+        ticks = None
+        if not isinstance(tick_size, (int, np.integer)):
+            ticks = [int(t) for t in tick_size]
+            if len(ticks) != n_envs:
+                raise ValueError(f"tick_size: one tick per env expected ({n_envs}), got {len(ticks)}")
+            if min(ticks) <= 0:
+                raise ValueError("tick sizes must be > 0")
+            tick_size = math.gcd(*ticks)   # the paged engine's ladder granule: every book's prices are multiples of it
         cfg = abi.Config()
         cfg.struct_size = C.sizeof(abi.Config)
         cfg.device, cfg.n_envs, cfg.env_id_base = device, n_envs, env_id_base
@@ -87,13 +103,21 @@ class BatchedEnv:
             raise ValueError("deep_chunks needs price_window=(lo, hi) (at most 8192 levels)")
         cfg.deep_chunks = deep_chunks
         self._h = C.c_void_p()
-        self.n_envs, self.obs_words, self.tick_size, self.device = n_envs, obs_words, tick_size, device
+        self.n_envs, self.obs_words, self.device = n_envs, obs_words, device
+        self.tick_size = int(tick_size)   # a sequence of ticks: their gcd (`tick_sizes` holds each env's)
+        self.tick_sizes = np.full(n_envs, tick_size, dtype=np.uint32)
         self.max_orders, self.max_trades, self.max_steps, self.max_queue = max_orders, max_trades, max_steps, max_queue
         rc = self._lib.bb_create(C.byref(cfg), C.byref(self._h))
         if rc != abi.BB_OK:
             msg = self._lib.bb_last_error(None)
             self._h = C.c_void_p()
             raise RuntimeError(f"bb_create failed ({rc}): {msg.decode() if msg else ''}")
+        if ticks is not None and any(t != tick_size for t in ticks):
+            try:
+                self.set_tick_sizes(ticks)
+            except Exception:
+                self.close()
+                raise
 
     def close(self):
         if getattr(self, "_h", None) and self._h.value:
@@ -140,6 +164,15 @@ class BatchedEnv:
     def clear_errors(self):
         """Zero every env's sticky error word (bb_clear_errors)."""
         self._ck(self._lib.bb_clear_errors(self._h))
+
+    def set_tick_sizes(self, ticks):
+        """Give each book its own tick (bb_set_tick_sizes; MarketEnv::new, market_env.rs:73-90): `n_envs` ticks, or on a
+        multi-asset handle `assets` ticks (asset a's tick for book a of every market).  ValueError, nothing changed, for a
+        tick of 0 or one that is not a multiple of the price granule, or while any env holds orders or queued transactions
+        (`reset()` first).  The ticks survive `reset()`."""
+        t = np.ascontiguousarray(ticks, dtype=np.uint32)
+        self._ck(self._lib.bb_set_tick_sizes(self._h, abi.ptr(t), len(t)))
+        self.tick_sizes = np.resize(t, self.n_envs) if len(t) != self.n_envs else t.copy()
 
     def reset(self): self._ck(self._lib.bb_reset(self._h))
     def synchronize(self): self._ck(self._lib.bb_synchronize(self._h))

@@ -139,6 +139,7 @@ __device__ __forceinline__ void stg128(u64 a, u32 x, u32 y, u32 z, u32 w) {
 
 // fire-and-forget pull of one 32-byte sector towards L2 (deep books: order records are DRAM-cold when first touched)
 __device__ __forceinline__ void prefetch_l2(u64 a) { asm volatile("prefetch.global.L2 [%0];" ::"l"(a)); }
+__device__ __forceinline__ void prefetch_l1(u64 a) { asm volatile("prefetch.global.L1 [%0];" ::"l"(a)); }
 
 // byte offsets inside records
 #define OH_PRICE 0u
@@ -165,13 +166,18 @@ __device__ __forceinline__ void prefetch_l2(u64 a) { asm volatile("prefetch.glob
 
 // Launch-invariant geometry (lives in the constant bank through the kernel parameter block).
 struct Geo {
-    u32 p_total, p_smem, granule, tick, max_orders, max_trades;
+    u32 p_total, p_smem, granule;
+    u32 pc_off;       // paged engine: offset (from the warp's shared-memory base) of the 128-entry page lookup cache
+    u32 max_orders, max_trades;
     u64 tr_base;      // trade slabs  [n_envs][max_trades] x 32 B
     u64 blobs_base;   // book blobs   [n_envs] x blob_stride
     u64 blob_stride;
+    // tick size of each env's book [n_envs] (bb_set_tick_sizes).  Read where it is used — once per level-2 record, row
+    // batch or agent update (k_deepw: once per launch, into a control word), never per event — so that it holds no
+    // register across the event loop.
+    const u32* ticks;
     // dense-window engine (dense.cuh): first price of the window, number of levels, number of order slots
     u32 d_win_lo, d_levels, d_live;
-    u32 pc_off;       // paged engine: offset (from the warp's shared-memory base) of the 128-entry page lookup cache
 };
 template <u32 LP_, u32 NWMAX_> struct DenseLayout;
 // Compile-time engine selection.
@@ -791,9 +797,11 @@ __device__ __forceinline__ void book_apply(const G& g, Book& b, u32 kind, u32 id
 // ---- observation emission ------------------------------------------------------------------------
 // Level-1 / level-2 record in the array layout of rust/src/step_sim_numpy.rs:300-368:
 // [trade_vol, bid_price, ask_price, ask_vol, bid_vol, then per level i: bid_vol_i, n_bid_i, ask_vol_i, n_ask_i]
-// Levels sit at FIXED tick offsets from the touch with wrapping arithmetic (orderbook.rs:229-264).
+// Levels sit at FIXED offsets of the env's tick from the touch with wrapping arithmetic (orderbook.rs:229-264).
 // Each lane returns the word(s) it owns: word index = lane (and lane + 32 for the 45-word record).
 template <class G> __device__ __forceinline__ void book_obs(const G& g, const Book& b, u32 n_words, u32* w0, u32* w1) {
+    // the tick is issued first so that its load overlaps the touch lookups (45-word records only)
+    const u32 tick = n_words > 9u ? __ldg(g.ticks + b.env) : 0u;
     const u32 bid = best_price(g, b, 1), ask = best_price(g, b, 0);
     u32 x = 0, y = 0;
     if (n_words <= 9u) {
@@ -812,8 +820,8 @@ template <class G> __device__ __forceinline__ void book_obs(const G& g, const Bo
             if (w >= 5u && w < 45u) {
                 const u32 i = (w - 5u) >> 2, f = (w - 5u) & 3u;
                 u32 v, n;
-                if (f < 2u) level_at_lane(g, b, 1, bid - i * g.tick, &v, &n);
-                else level_at_lane(g, b, 0, ask + i * g.tick, &v, &n);
+                if (f < 2u) level_at_lane(g, b, 1, bid - i * tick, &v, &n);
+                else level_at_lane(g, b, 0, ask + i * tick, &v, &n);
                 val = (f & 1u) ? n : v;
             } else if (w < 5u) {
                 val = w == 0 ? b.trade_vol : w == 1 ? bid : w == 2 ? ask : w == 3 ? b.vol_ask : b.vol_bid;

@@ -54,6 +54,8 @@ struct bb_handle {
     bb_instr* d_instrs = nullptr;
     size_t d_instrs_cap = 0;
     u32* d_snap = nullptr;  // [n_envs][45]
+    u32* d_tick = nullptr;  // [n_envs] tick size of each env's book (bb_set_tick_sizes); tick[] is its host mirror
+    std::vector<u32> tick;
     unsigned long long* d_stats = nullptr;
     u32* rslot = nullptr;
     MomState* mom = nullptr;
@@ -197,7 +199,7 @@ void fill_params(const bb_handle* h, const SmemLayout& l, KParams& p) {
     p.geo.p_total = h->p_total;
     p.geo.p_smem = h->p_smem;
     p.geo.granule = h->granule;
-    p.geo.tick = h->cfg.tick_size;
+    p.geo.ticks = h->d_tick;
     p.geo.max_orders = h->cfg.max_orders;
     p.geo.max_trades = h->cfg.max_trades;
     p.geo.tr_base = (u64)h->tr;
@@ -558,6 +560,9 @@ int bb_create(const bb_config* cfg, bb_handle** out) {
     TRY_ALLOC(cudaMalloc(&h->d_offsets, (ne + 1) * 8));
     TRY_ALLOC(cudaMalloc(&h->d_seeds, ne * 16));
     TRY_ALLOC(cudaMalloc(&h->d_snap, ne * 45 * 4));
+    TRY_ALLOC(cudaMalloc(&h->d_tick, ne * 4));
+    h->tick.assign(ne, cfg->tick_size);
+    TRY_ALLOC(cudaMemcpyAsync(h->d_tick, h->tick.data(), ne * 4, cudaMemcpyHostToDevice, h->stream));
     TRY_ALLOC(cudaMalloc(&h->d_stats, 8 * 8));
     TRY_ALLOC(cudaMallocHost(&h->h_offsets, (ne + 1) * 8));
     TRY_ALLOC(cudaMallocHost(&h->h_snap, ne * 45 * 4));
@@ -576,7 +581,7 @@ int bb_destroy(bb_handle* h) {
     if (h->stream) cudaStreamSynchronize(h->stream);
     if (h->copy_stream) cudaStreamSynchronize(h->copy_stream);
     cudaFree(h->blobs); cudaFree(h->ord); cudaFree(h->tr); cudaFree(h->hist); cudaFree(h->err_flag);
-    cudaFree(h->d_offsets); cudaFree(h->d_seeds); cudaFree(h->d_instrs); cudaFree(h->d_snap); cudaFree(h->d_stats);
+    cudaFree(h->d_offsets); cudaFree(h->d_seeds); cudaFree(h->d_instrs); cudaFree(h->d_snap); cudaFree(h->d_stats); cudaFree(h->d_tick);
     cudaFree(h->rslot); cudaFree(h->mom); cudaFree(h->scratch); cudaFree(h->d_ids); cudaFree(h->dp_pool);
     if (h->h_instrs) cudaFreeHost(h->h_instrs);
     if (h->h_offsets) cudaFreeHost(h->h_offsets);
@@ -592,6 +597,36 @@ int bb_reset(bb_handle* h) {
     CHECK_H(h);
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     return init_books(h);
+}
+
+int bb_set_tick_sizes(bb_handle* h, const uint32_t* ticks, uint32_t n) {
+    CHECK_H(h);
+    const u32 ne = h->cfg.n_envs;
+    if (!ticks) return fail(h, BB_EINVAL, "null tick array");
+    if (n != ne && !(h->assets > 1 && n == h->assets))
+        return fail(h, BB_EINVAL, "bb_set_tick_sizes: n must be n_envs (" + std::to_string(ne) + ")" +
+                                      (h->assets > 1 ? " or assets (" + std::to_string(h->assets) + ")" : std::string()));
+    for (u32 i = 0; i < n; ++i) {
+        if (ticks[i] == 0) return fail(h, BB_EINVAL, "bb_set_tick_sizes: tick " + std::to_string(i) + " is 0");
+        if (ticks[i] % h->granule != 0)
+            return fail(h, BB_EINVAL, "bb_set_tick_sizes: tick " + std::to_string(ticks[i]) + " is not a multiple of the price granule " +
+                                          std::to_string(h->granule));
+    }
+    // a reference book gets its tick at creation only (orderbook.rs:158-171): refuse while any book holds orders
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    std::vector<u32> n_ord(ne);
+    CUDA_TRY(h, cudaMemcpy2DAsync(n_ord.data(), 4, h->blobs + offsetof(BookHdr, n_orders), h->blob_stride, 4, ne,
+                                  cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    for (u32 e = 0; e < ne; ++e)
+        if (n_ord[e] || !h->queue[e].empty())
+            return fail(h, BB_EINVAL, "bb_set_tick_sizes: env " + std::to_string(e) + " has orders or queued transactions (bb_reset first)");
+    std::vector<u32> t(ne);
+    for (u32 e = 0; e < ne; ++e) t[e] = ticks[n == ne ? e : e % h->assets];  // market m's book a = env m * assets + a
+    CUDA_TRY(h, cudaMemcpyAsync(h->d_tick, t.data(), (size_t)ne * 4, cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    h->tick.swap(t);
+    return BB_OK;
 }
 
 int bb_set_stream(bb_handle* h, void* cuda_stream) {
@@ -626,10 +661,10 @@ int bb_submit(bb_handle* h, uint64_t n, const uint32_t* env, const uint32_t* act
             case BB_ACT_NEW: {
                 const bool market = flags && (f & BB_F_MARKET);
                 const u32 p = price ? price[r] : 0u;
-                if (!market && p % h->cfg.tick_size != 0) {  // create_order tick check, orderbook.rs:367-383
+                if (!market && p % h->tick[e] != 0) {  // create_order tick check against the env's tick, orderbook.rs:367-383
                     if (n_done) *n_done = r;
                     return fail(h, BB_EPRICE, "Price " + std::to_string(p) + " was not a multiple of tick-size " +
-                                                  std::to_string(h->cfg.tick_size));
+                                                  std::to_string(h->tick[e]));
                 }
                 if (h->n_orders_host[e] >= h->cfg.max_orders) {
                     if (n_done) *n_done = r;

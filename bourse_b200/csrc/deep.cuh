@@ -76,6 +76,7 @@ struct DeepOff {             // byte offsets from the CTA's shared-memory base, 
 #define RS_NTR 88u
 #define RS_RET_TAIL 92u
 #define RS_ERR 96u
+#define CT_TICK 100u        // the book's tick (level-2 records), written at set-up
 #define CT_WORDS 32u
 
 // retire entry kinds

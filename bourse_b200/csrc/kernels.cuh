@@ -46,7 +46,7 @@ struct KParams {
     u64 hist_env_stride;  // words
     u32 blob_smem_bytes;
     u32 n_envs, env_id_base;
-    Geo geo;  // p_total, p_smem, granule, tick, max_orders, max_trades
+    Geo geo;  // p_total, p_smem, granule, max_orders, max_trades, per-env ticks
     u32 max_steps, max_queue, obs_words;
     u32 warp_smem_bytes, off_perm, off_obs, off_instr, off_bar, off_q, off_ag;
     // k_apply
@@ -228,6 +228,7 @@ template <int MODE, int ENG> __global__ void __launch_bounds__(128, (ENG == ENG_
     for (u32 env = blockIdx.x * wpb + warp; env < p.n_envs; env += gridDim.x * wpb) {
         Book b;
         make_book(b, p, sb, env, lane);
+        if (lane == 0) prefetch_l1((u64)(g.ticks + env));  // the tick is read at the row checks and level-2 records
         if (!blob_load(p, sb, env, bar, ph_blob, lane)) {
             if (lane == 0) atomicOr(p.err_flag, 0x80000000u);
             return;
@@ -294,6 +295,7 @@ template <int MODE, int ENG> __global__ void __launch_bounds__(128, (ENG == ENG_
                     // is create_order's PriceError (orderbook.rs:367-383): nothing is created or queued, the env is flagged
                     u32 next = b.n_orders;
                     nv = 0;
+                    const u32 tick = __ldg(g.ticks + env);
                     for (u32 j0 = 0; j0 < mm; j0 += 32) {
                         const u32 j = j0 + lane;
                         u32 of = 0, price = 0;
@@ -302,7 +304,7 @@ template <int MODE, int ENG> __global__ void __launch_bounds__(128, (ENG == ENG_
                             price = ins[j].price;
                         }
                         const u32 op = of & BB_OP_MASK;
-                        const bool bad_tick = op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % g.tick != 0u);
+                        const bool bad_tick = op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % tick != 0u);
                         const bool is_new = op == BB_OP_NEW && !bad_tick;
                         const bool queued = is_new || op == BB_OP_CANCEL || op == BB_OP_MODIFY;
                         const u32 below = (1u << lane) - 1u;
@@ -487,9 +489,12 @@ __device__ __forceinline__ u32 round_price(double x, double tick, bool up) {
 struct MomOut {
     u32 n, next_id, err;
 };
-__device__ __noinline__ MomOut momentum_agent_update(const KParams& p, const bb_agent_group& ag, u64 oh, u32 lane, u32 bid,
+__device__ __noinline__ MomOut momentum_agent_update(const KParams& p, const bb_agent_group& ag, u64 oh, u32 book_tick, u32 bid,
                                                      u32 ask, uint4* q, u32 e_n, u32 e_next_id, MomState* ms, u32 env_g,
                                                      u32 step, u32 gi, u32 slot_base) {
+    // (`book_tick`, the tick of the book the group trades, takes the argument slot of the lane id, which is recomputed here:
+    // one more argument costs the momentum k_sim variants spill traffic)
+    const u32 lane = threadIdx.x & 31u;
     Emit e;
     e.n = e_n;
     e.next_id = e_next_id;
@@ -552,7 +557,7 @@ __device__ __noinline__ MomOut momentum_agent_update(const KParams& p, const bb_
             const double nrm = sqrt(-2.0 * log(u1)) * cos(6.283185307179586476925 * u2);
             const double dist = fabs(exp(ag.mu + ag.sigma * nrm));
             price = limit_bid ? round_price(mid - dist, tick, false) : round_price(mid + dist, tick, true);
-            if (price % p.geo.tick != 0) err |= ERR_GRANULE;  // the reference unwraps a PriceError here
+            if (price % book_tick != 0) err |= ERR_GRANULE;  // the reference unwraps a PriceError here
         }
         u32 total;
         const u32 cnt = (do_limit ? 1u : 0u) + (do_market ? 1u : 0u);
@@ -713,7 +718,7 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                     }
                 } else {
                     if (mine) {
-                        const MomOut mo = momentum_agent_update(p, ag, b.oh, lane, best_price(g, b, 1), best_price(g, b, 0), q, e.n,
+                        const MomOut mo = momentum_agent_update(p, ag, b.oh, __ldg(g.ticks + env), best_price(g, b, 1), best_price(g, b, 0), q, e.n,
                                                                 e.next_id, (MomState*)((char*)p.mom + ((size_t)env * p.mom_groups_per_env + mi) * p.mom_stride), env_g,
                                                                 step, gi, slot_base);
                         e.n = mo.n;
@@ -731,6 +736,7 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                 const u32 m = s == 0 ? (u32)(p.offsets[env + 1] - off) : 0u;  // the rows belong to the launch's first step
                 const bb_instr* ins = p.instrs + off;
                 u32 max_cancel = 0;  // 1 + largest id a cancel row names
+                const u32 tick = __ldg(g.ticks + env);
                 for (u32 j0 = 0; j0 < m; j0 += 32) {
                     const u32 j = j0 + lane;
                     u32 of = 0, price = 0, vol = 0, trader = 0, oid = 0;
@@ -741,7 +747,7 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                     const u32 op = of & BB_OP_MASK;
                     const bool bid = (of & BB_F_BID) != 0u;
                     // create_order's tick check (orderbook.rs:367-383): the row is dropped like the Err return
-                    const bool bad_tick = op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % g.tick != 0u);
+                    const bool bad_tick = op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % tick != 0u);
                     const bool is_new = op == BB_OP_NEW && !bad_tick, is_cancel = op == BB_OP_CANCEL;
                     const bool queued = is_new || is_cancel;
                     const u32 below = (1u << lane) - 1u;
@@ -1299,7 +1305,8 @@ __global__ void __launch_bounds__(128, ROOMY ? 2 : 4) k_deepw(const __grid_const
         for (u32 i = 0; i <= DW_RB; ++i) mbar_init_a(sb + o.bar + 8u * i, 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    for (u32 i = threadIdx.x; i < CT_WORDS; i += blockDim.x) sts(ctl + 4u * i, 0u);
+    // (CT_TICK: the book's tick, read by the level-2 records; loaded once here, off the record path)
+    for (u32 i = threadIdx.x; i < CT_WORDS; i += blockDim.x) sts(ctl + 4u * i, 4u * i == CT_TICK ? __ldg(p.geo.ticks + env) : 0u);
     for (u32 i = threadIdx.x; i < (ROOMY ? o.dirty_n : DW_DIRTY); i += blockDim.x) sts(sb + o.dirty + 4u * i, 0u);
     for (u32 i = threadIdx.x; i < (ROOMY ? o.swept_n : DW_SWEPT); i += blockDim.x) sts(sb + (ROOMY ? o.swept : o.scratch + SC_SWEPT) + 4u * i, 0u);
     fence_proxy_async();
@@ -1400,7 +1407,7 @@ __global__ void __launch_bounds__(128, ROOMY ? 2 : 4) k_deepw(const __grid_const
                     const u32 bid = (s.flags & FL_HAS_BID) ? r.win_lo + s.bq_bid : 0u;
                     const u32 ask = (s.flags & FL_HAS_ASK) ? r.win_lo + s.bq_ask : 0xFFFFFFFFu;
                     u32 w0, w1;
-                    bk_obs(r, p.geo.tick, lane, s.trade_vol, bid, ask, s.vol_ask, s.vol_bid, &w0, &w1);
+                    bk_obs(r, lds(r.ctl + CT_TICK), lane, s.trade_vol, bid, ask, s.vol_ask, s.vol_bid, &w0, &w1);
                     // (a level-1 record is the first 9 words of the level-2 one: words 5..8 are the touch level of each side)
                     const u32 nrec = lds(sb + HDR_NSTEPS);
                     __syncwarp();
@@ -1614,13 +1621,14 @@ __global__ void __launch_bounds__(128) k_snapshot_deep(const __grid_constant__ K
     };
     const u32 bid = h->has_best[1] ? lo + h->best_q[1] : 0u, ask = h->has_best[0] ? lo + h->best_q[0] : 0xFFFFFFFFu;
     if (out45) {
+        const u32 tick = __ldg(p.geo.ticks + env);
         for (u32 w = lane; w < words; w += 32u) {
             u32 val;
             if (w >= 5u) {
                 const u32 k = (w - 5u) >> 2, f = (w - 5u) & 3u;
                 u32 v, n;
-                if (f < 2u) level_at(1u, bid - k * p.geo.tick, &v, &n);
-                else level_at(0u, ask + k * p.geo.tick, &v, &n);
+                if (f < 2u) level_at(1u, bid - k * tick, &v, &n);
+                else level_at(0u, ask + k * tick, &v, &n);
                 val = (f & 1u) ? n : v;
             } else {
                 val = w == 0 ? h->trade_vol : w == 1 ? bid : w == 2 ? ask : w == 3 ? h->side_vol[0] : h->side_vol[1];

@@ -183,6 +183,8 @@ class VectorEnv:
     (step_sim_numpy.rs:256-267).  Semantics per env are exactly `submit_instructions` + `step`: ids in row order, the
     step's queue shuffled with the env's own Xoroshiro stream, event i at `t + i`.  A NEW row with an off-tick limit
     price creates nothing (the reference raises ValueError there); the env is flagged and `check_errors` raises.
+    `tick_size` may be a sequence of `n_envs` ticks, one per env (`core.BatchedEnv`): each env then checks its rows
+    against, and lays out its level-2 observation at, its own tick.
 
     Without background agents a step is ONE kernel launch on the env's stream (`env.set_stream(...)`) with no host
     synchronisation, so a loop of policy + `step` can be captured into a CUDA graph and replayed (tests/test_gpu_gym.py);
@@ -190,7 +192,7 @@ class VectorEnv:
     per-step history is a scratch ring for this class: `step` clears it (`bb_clear_history`) whenever `max_steps` records
     have accumulated; a caller replaying a captured step must do the same every `max_steps` replays."""
 
-    def __init__(self, n_envs: int, rows_per_env: int, seed: int, start_time: int, tick_size: int, step_size: int,
+    def __init__(self, n_envs: int, rows_per_env: int, seed: int, start_time: int, tick_size: typing.Union[int, typing.Sequence[int]], step_size: int,
                  trading: bool = True, *, level_1: bool = False, agents=None, agent_seed: int = 0, **kw):
         """`agents`: optional background population (a list of `core.random_group` / `momentum_group` / `noise_group`
         records).  With it every `step` is `{ agents.update(env); the action rows; env.step() }` in one launch

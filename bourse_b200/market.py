@@ -8,11 +8,14 @@ transaction queue per step.  The queue is shuffled as a whole and event i of the
 `(asset, id)` tuple.
 
 Books of one market are consecutive envs of a `BatchedEnv(assets=A)` handle, so `n_markets` independent markets
-advance in lockstep on one GPU exactly like plain envs do.  Limitation: one tick size per handle (the reference
-allows one per asset).
+advance in lockstep on one GPU exactly like plain envs do.  Each asset has its own tick size, as in the reference
+(market_env.rs:73-90): prices are checked against the asset's tick and its level-2 records step by that tick.  On the
+paged engine the ladder granule is the gcd of the ticks (unless `price_granule` is given), and an asset whose tick is
+k times the granule spreads its levels k times more thinly over the 32-price pages, so it may need a larger `pages_total`.
 """
 from __future__ import annotations
 
+import math
 import typing
 
 import numpy as np
@@ -84,13 +87,20 @@ class MarketEnv:
         ticks = [int(t) for t in tick_sizes]
         if not ticks:
             raise ValueError("at least one asset")
-        if any(t != ticks[0] for t in ticks):
-            raise NotImplementedError("bourse_b200 supports one tick size per handle: all assets must share it")
-        self.n_assets, self.n_markets, self.tick_size = len(ticks), n_markets, ticks[0]
+        if min(ticks) <= 0:
+            raise ValueError("tick sizes must be > 0")
+        self.n_assets, self.n_markets, self.tick_sizes = len(ticks), n_markets, ticks
+        self.tick_size = math.gcd(*ticks)   # the handle's tick: every asset's tick is a multiple of it
         kw.setdefault("max_steps", 1 << 10)
         # assets=1 would mean "plain envs" to the library; a one-asset market is the same thing as an Env
-        self._env = BatchedEnv(self.n_assets * n_markets, seed, start_time, ticks[0], step_size, trading,
+        self._env = BatchedEnv(self.n_assets * n_markets, seed, start_time, self.tick_size, step_size, trading,
                                assets=self.n_assets if self.n_assets > 1 else 0, obs_words=abi.OBS_L2, **kw)
+        if any(t != self.tick_size for t in ticks):   # (several assets: a one-asset market has one tick)
+            try:
+                self._env.set_tick_sizes(ticks)   # asset a's tick for book a of every market
+            except Exception:
+                self._env.close()
+                raise
 
     def _book(self, asset: int, market: int = 0) -> int:
         if not 0 <= asset < self.n_assets:

@@ -42,11 +42,11 @@ typedef enum {
 #define BB_ERR_CAP_PAGES  0x04u
 #define BB_ERR_CAP_QUEUE  0x08u
 #define BB_ERR_BAD_ID     0x10u
-#define BB_ERR_GRANULE    0x20u  /* a resting price was not a multiple of price_granule */
+#define BB_ERR_GRANULE    0x20u  /* a resting price was not a multiple of price_granule, or an agent's limit price not one of its book's tick */
 #define BB_ERR_CAP_STEPS  0x40u
 #define BB_ERR_CAP_LIVE   0x80u  /* MomentumAgent live-order list / dense engine's resting-order slots overflow */
 #define BB_ERR_TIME_ORDER 0x100u /* dense engine: a resting order arrived out of time order at its price level */
-#define BB_ERR_PRICE 0x200u      /* bb_step_device: a NEW row's limit price was not a multiple of tick_size (row dropped) */
+#define BB_ERR_PRICE 0x200u      /* bb_step_device: a NEW row's limit price was not a multiple of its env's tick (row dropped) */
 #define BB_ERR_ROW_OP 0x400u     /* bb_run_agents_with_rows: a MODIFY row or a trader id >= 2^19 (row dropped) */
 #define BB_ERR_LOCKED 0x800u     /* deep engine: both sides would rest at one price level (trading disabled) */
 
@@ -68,7 +68,7 @@ typedef struct {
     uint64_t start_time;    /* Nanos */
     uint64_t step_size;     /* Nanos advanced per Env::step */
     uint64_t seed;          /* env e shuffles with Xoroshiro128**(seed + env_id_base + e) (step_sim.rs:73) */
-    uint32_t tick_size;     /* > 0 */
+    uint32_t tick_size;     /* > 0; every book's tick until bb_set_tick_sizes gives books their own */
     uint32_t price_granule; /* ladder granularity; 0 => tick_size.  Every resting price must be a multiple */
     uint32_t trading;       /* initial trading flag */
     uint32_t obs_words;     /* BB_OBS_L1 or BB_OBS_L2: record written to the history each step */
@@ -199,6 +199,16 @@ int bb_reserve_queue(bb_handle* h, uint32_t max_queue);
  * order tables and trade logs are untouched.  For open-ended loops that consume each step's observation as it is produced
  * (bb_step_device / bb_run_agents_with_rows) and would otherwise run into max_steps.  Asynchronous. */
 int bb_clear_history(bb_handle* h);
+/* Per-book tick sizes (MarketEnv::new(start_time, tick_sizes, step_size, trading), crates/step_sim/src/market_env.rs:73-90,
+ * gives each asset's OrderBook its own tick).  n == n_envs: ticks[e] is env e's tick; on a multi-asset handle n == assets
+ * gives asset a's tick to book a of every market.  Each book then checks create_order prices against its own tick
+ * (bb_submit, bb_step_device, bb_run_agents_with_rows rows, MomentumAgent / NoiseAgent prices) and lays out its level-2
+ * record at its own tick offsets; until this is called every book has bb_config.tick_size.  Refused with BB_EINVAL, the
+ * handle unchanged, for a NULL array, a wrong n, a tick of 0 or one that is not a multiple of the price granule, and while
+ * any env holds orders or queued transactions (a reference book gets its tick at creation only; bb_reset first).  The ticks
+ * survive bb_reset.  On the paged engine a book whose tick is k x the granule spreads its levels k times more thinly over the
+ * 32-price pages and may need a larger pages_total; the dense and deep engines (granule 1) are unaffected.  Synchronous. */
+int bb_set_tick_sizes(bb_handle* h, const uint32_t* ticks, uint32_t n);
 const char* bb_last_error(const bb_handle* h /* may be NULL */);
 /* run on a caller-owned CUDA stream (cudaStream_t); NULL restores the handle's own stream */
 int bb_set_stream(bb_handle* h, void* cuda_stream);
