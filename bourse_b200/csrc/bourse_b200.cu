@@ -86,6 +86,7 @@ struct bb_handle {
     bool deep_serial = false;  // developer switch (BOURSE_B200_DEEP=serial): every event through k_deepw's serial path
     // agents
     std::vector<bb_agent_group> groups;
+    u32 rand_tick_mask = 0;  // KParams::rand_tick_mask, kept current by set_agents_impl and bb_set_tick_sizes
     std::vector<u32> group_asset;  // bb_set_agents_market: asset each group trades (empty: single-asset agents)
     u32 agents_per_env = 0, mom_groups = 0;
     u32 chip_agents = 0;  // on-chip agent table capacity of the dense engine (markets: the largest per-asset agent count)
@@ -599,6 +600,21 @@ int bb_reset(bb_handle* h) {
     return init_books(h);
 }
 
+// KParams::rand_tick_mask: bit gi for a RandomAgents group that trades some book whose tick does not divide its tick_size.
+// Only such groups can draw an off-tick limit price: a population with one runs on the k_sim variants that check the
+// queued prices (run_agents_impl), on-grid populations keep the RandomAgents-only kernels, which carry no check.
+static void update_rand_tick_mask(bb_handle* h) {
+    h->rand_tick_mask = 0;
+    for (size_t gi = 0; gi < h->groups.size(); ++gi) {
+        if (h->groups[gi].kind != BB_GROUP_RANDOM) continue;
+        for (u32 e = 0; e < h->cfg.n_envs; ++e)  // markets: env e is book e % assets of its market
+            if ((h->group_asset.empty() || e % h->assets == h->group_asset[gi]) && h->groups[gi].tick_size % h->tick[e] != 0) {
+                h->rand_tick_mask |= 1u << gi;
+                break;
+            }
+    }
+}
+
 int bb_set_tick_sizes(bb_handle* h, const uint32_t* ticks, uint32_t n) {
     CHECK_H(h);
     const u32 ne = h->cfg.n_envs;
@@ -626,6 +642,7 @@ int bb_set_tick_sizes(bb_handle* h, const uint32_t* ticks, uint32_t n) {
     CUDA_TRY(h, cudaMemcpyAsync(h->d_tick, t.data(), (size_t)ne * 4, cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     h->tick.swap(t);
+    update_rand_tick_mask(h);
     return BB_OK;
 }
 
@@ -778,6 +795,18 @@ int bb_replay(bb_handle* h, const bb_instr* instrs, const uint64_t* env_offsets)
     const u32 ne = h->cfg.n_envs;
     const size_t total = env_offsets[ne];
     if (total && !instrs) return fail(h, BB_EINVAL, "null instruction array");
+    // create_order's tick check (orderbook.rs:367-383) on every limit NEW, before anything is applied: a stream with an
+    // off-tick price changes no env (MODIFY prices are not checked, as in the reference).  A tick of 1 takes every price,
+    // so such an env's rows are not walked here (the pass would sit in front of the launch)
+    for (u32 e = 0; e < ne; ++e) {
+        if (h->tick[e] == 1) continue;
+        for (size_t i = env_offsets[e]; i < env_offsets[e + 1]; ++i) {
+            const bb_instr& x = instrs[i];
+            if ((x.op_flags & BB_OP_MASK) == BB_OP_NEW && !(x.op_flags & BB_F_MARKET) && x.price % h->tick[e] != 0)
+                return fail(h, BB_EPRICE, "bb_replay: env " + std::to_string(e) + " row " + std::to_string(i) + ": Price " +
+                                              std::to_string(x.price) + " was not a multiple of tick-size " + std::to_string(h->tick[e]));
+        }
+    }
     int rc = refresh_mirror(h);
     if (rc) return rc;
     if ((rc = ensure_instr_capacity(h, total + 1))) return rc;
@@ -864,6 +893,7 @@ static int set_agents_impl(bb_handle* h, const bb_agent_group* groups, const uin
         }
     }
     h->mom_groups = mom;
+    update_rand_tick_mask(h);
     h->lay_sim = make_layout(h, true, false, h->eng >= ENG_DENSE, asset != nullptr);  // the on-chip agent state depends on the population
     if (total) CUDA_TRY(h, cudaMemsetAsync(h->rslot, 0xFF, ne * total * 4, h->stream));
     if (mom) CUDA_TRY(h, cudaMemsetAsync(h->mom, 0, ne * mom * (size_t)h->mom_stride, h->stream));
@@ -1075,6 +1105,7 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
     p.seed_lo = (u32)seed;
     p.seed_hi = (u32)(seed >> 32);
     for (size_t i = 0; i < h->groups.size(); ++i) p.groups[i] = h->groups[i];
+    p.rand_tick_mask = h->rand_tick_mask;
     for (size_t i = 0; i < h->group_asset.size(); ++i) p.group_asset[i] = h->group_asset[i];
     if (ext) {
         p.instrs = ext->d_instrs;
@@ -1083,8 +1114,9 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
         p.obs_out = ext->d_obs_out;
     }
     int grid = 0, rc;
-    // external rows carry no slot hints: they run on the variants that also serve MomentumAgent / NoiseAgent events
-    const bool mom = h->mom_groups != 0 || ext != nullptr;
+    // external rows carry no slot hints: they run on the variants that also serve MomentumAgent / NoiseAgent events.  So
+    // does a RandomAgents group that can draw off its book's tick: only those variants check the queued prices
+    const bool mom = h->mom_groups != 0 || ext != nullptr || h->rand_tick_mask != 0;
     // markets: the A books of a market are A consecutive warps of one CTA (a CTA holds as many whole markets as fit in 4 warps)
     const u32 wpb = mkt ? (WPB / h->assets) * h->assets : wpb_for(h->lay_sim.warp_bytes);
     const size_t sim_smem = (size_t)h->lay_sim.warp_bytes * wpb;

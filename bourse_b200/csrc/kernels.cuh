@@ -77,6 +77,10 @@ struct KParams {
     unsigned char* dp_pool;
     u32 dp_chunks;
     u32 dp_fast;  // k_deepw: 1 = batch-parallel passes enabled (0: every event through the serial path; debugging)
+    // k_sim, bit gi: RandomAgents group gi trades a book whose tick does not divide the group's tick_size, so the queued
+    // prices are checked against the book's tick (the host derives it from the groups and the tick table).  Last, so that
+    // the other kernels' parameter offsets stay where they were
+    u32 rand_tick_mask;
 };
 
 // Values the optimiser would otherwise rematerialise at every use (S2R for the lane id, cvta + multiply
@@ -467,6 +471,23 @@ __device__ __forceinline__ void random_agents_update_dense(const KParams& p, con
     }
 }
 
+// create_order's tick check (orderbook.rs:367-383) on the step's queued agent NEWs, q[0, n): an off-tick limit price is
+// ERR_GRANULE, in the step at which the reference agent unwraps the PriceError.  It runs once per step over the queue,
+// after all groups' updates, not inside the RandomAgents draw loop.  A bid market order's price is the sentinel
+// 0xFFFFFFFF (types.rs:160-172) and is skipped; MomentumAgent / NoiseAgent limit prices were already checked at their
+// draw, so scanning them again flags nothing new.  The dense engine's queue is in shared memory at `qs`, the others' in
+// global scratch at `q`.
+template <bool DENSE>
+__device__ __forceinline__ void agent_tick_check(const uint4* q, u32 qs, u32 book_tick, u32 n, u32 lane, u32& err) {
+    __syncwarp();
+    bool bad = false;
+    for (u32 i = lane; i < n; i += 32) {
+        const u32 of = DENSE ? lds(qs + 16u * i) : q[i].x, price = DENSE ? lds(qs + 16u * i + 8u) : q[i].z;
+        bad |= (of & 1u) && price != 0xFFFFFFFFu && price % book_tick != 0u;
+    }
+    if (__any_sync(BB_FULL, bad)) err |= ERR_GRANULE;
+}
+
 __device__ __forceinline__ u32 warp_excl_scan(u32 v, u32 lane, u32* total) {
     u32 x = v;
 #pragma unroll
@@ -774,6 +795,12 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
             }
             if (e.n > p.max_queue) b.err |= ERR_CAP_QUEUE;
             u32 n = min(e.n, p.max_queue);
+            // a RandomAgents group in rand_tick_mask can draw off its book's tick: the host runs such a population on the MOM
+            // variants, so the hot RandomAgents-only kernels carry no check.  (The caller's rows are in the queue too: their
+            // off-tick limit NEWs were dropped above.)
+            if constexpr (MOM) {
+                if (p.rand_tick_mask) agent_tick_check<G::DENSE>(q, qs, __ldg(g.ticks + env), n, lane, b.err);
+            }
             b.n_orders = e.next_id;  // create_order at submission (env.rs:173)
             if constexpr (G::DENSE) {  // ids and slots are validated once per step (d_apply trusts hinted events)
                 if (e.next_id > g.max_orders) {

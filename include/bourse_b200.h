@@ -202,7 +202,8 @@ int bb_clear_history(bb_handle* h);
 /* Per-book tick sizes (MarketEnv::new(start_time, tick_sizes, step_size, trading), crates/step_sim/src/market_env.rs:73-90,
  * gives each asset's OrderBook its own tick).  n == n_envs: ticks[e] is env e's tick; on a multi-asset handle n == assets
  * gives asset a's tick to book a of every market.  Each book then checks create_order prices against its own tick
- * (bb_submit, bb_step_device, bb_run_agents_with_rows rows, MomentumAgent / NoiseAgent prices) and lays out its level-2
+ * (bb_submit, bb_replay, bb_step_device, bb_run_agents_with_rows rows, RandomAgents / MomentumAgent / NoiseAgent prices;
+ * not bb_replay_device) and lays out its level-2
  * record at its own tick offsets; until this is called every book has bb_config.tick_size.  Refused with BB_EINVAL, the
  * handle unchanged, for a NULL array, a wrong n, a tick of 0 or one that is not a multiple of the price granule, and while
  * any env holds orders or queued transactions (a reference book gets its tick at creation only; bb_reset first).  The ticks
@@ -253,9 +254,13 @@ int bb_memcpy(bb_handle* h, void* dst, const void* src, uint64_t bytes, int kind
 
 /* ---- immediate mode: OrderBook API / replayed streams (orderbook.rs:411-792) ------------------ */
 /* env_offsets[n_envs + 1] delimits each env's slice of `instrs`.  Every instruction executes at its
- * own `t`.  NEW rows get ids in stream order.  Rows flagged BB_F_EMIT append a level-2 record. */
+ * own `t`.  NEW rows get ids in stream order.  Rows flagged BB_F_EMIT append a level-2 record.  A limit NEW whose price
+ * is not a multiple of its env's tick (create_order's PriceError, orderbook.rs:367-383) refuses the whole call with
+ * BB_EPRICE before any env changes; bb_last_error() names the env, the row and the reference's message.  MODIFY prices
+ * are not checked, as in the reference. */
 int bb_replay(bb_handle* h, const bb_instr* instrs, const uint64_t* env_offsets);
-/* same with both arrays already resident in device memory (asynchronous on the handle's stream) */
+/* same with both arrays already resident in device memory (asynchronous on the handle's stream).  The stream never visits
+ * the host and is not tick-checked: the caller guarantees that every limit NEW is on its env's tick. */
 int bb_replay_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_env_offsets);
 
 /* ---- built-in agents: sim_runner (crates/step_sim/src/runner.rs:46-69) ------------------------ */

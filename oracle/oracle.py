@@ -100,9 +100,9 @@ def lib() -> C.CDLL:
     sig("orc_sim_n_steps", u64, vp)
     sig("orc_sim_history", None, vp, vp)
     sig("orc_sim_set_groups", None, vp, vp, u32)
-    sig("orc_sim_run", None, vp, i32, u64, u32, u64)
+    sig("orc_sim_run", i32, vp, i32, u64, u32, u64)
     sig("orc_sim_n_instructions", u64, vp)
-    sig("orc_sim_agents_update", None, vp, u64, u32)
+    sig("orc_sim_agents_update", i32, vp, u64, u32)
     sig("orc_sim_step_keyed", i32, vp, u64, u32)
     sig("orc_bench_agents", dbl, u32, u32, u64, u64, i32, u64, u32, u64, vp, u32, vp)
     sig("orc_bench_replay", dbl, u32, u32, u32, vp, u64, vp)
@@ -116,11 +116,12 @@ def lib() -> C.CDLL:
     sig("orc_market_n_steps", u64, vp, u32)
     sig("orc_market_history", None, vp, u32, vp)
     sig("orc_market_set_groups", None, vp, vp, vp, u32)
-    sig("orc_market_run", None, vp, i32, u64, u32, u64)
+    sig("orc_market_run", i32, vp, i32, u64, u32, u64)
     sig("orc_market_n_instructions", u64, vp)
     sig("orc_bench_market_agents", dbl, u32, u32, u64, u64, i32, u64, vp, u32, u64, vp, vp, u32, vp)
     sig("orc_bench_replay_suffix", dbl, u32, u32, vp, u64, u64, vp)
     sig("orc_bench_env_rows", dbl, u32, u32, u64, u32, vp, u32, u32, u64, u32, u64, vp)
+    sig("orc_last_error", C.c_char_p)
     sig("orc_philox", None, u32, u32, u32, u32, u32, u32, vp)
     sig("orc_xoroshiro", None, u64, u32, vp)
     sig("orc_xoroshiro_state", None, u64, u64, u32, vp, vp, vp, u32, vp)
@@ -132,6 +133,13 @@ def lib() -> C.CDLL:
 
 def _ptr(a: np.ndarray):
     return a.ctypes.data_as(C.c_void_p)
+
+
+def _check_agents(rc):
+    """An agent run returns -1 where a reference agent's create_order would raise PriceError and the agent's unwrap
+    panic: raised here as ValueError with the reference's message.  The steps completed before it keep their records."""
+    if rc:
+        raise ValueError(lib().orc_last_error().decode())
 
 
 def random_group(n_agents, tick_range, vol_range, tick_size, activity_rate):
@@ -343,11 +351,11 @@ class _EnvBase(_BookView):
         lib().orc_sim_set_groups(self._h, _ptr(arr), len(arr))
 
     def run_agents(self, n_steps, seed, env_id=0, keyed=True):
-        lib().orc_sim_run(self._h, int(keyed), seed, env_id, n_steps)
+        _check_agents(lib().orc_sim_run(self._h, int(keyed), seed, env_id, n_steps))
 
     def agents_update(self, seed, env_id=0):
         """First half of one keyed step: the built-in agents queue their instructions (Philox contract)."""
-        lib().orc_sim_agents_update(self._h, seed, env_id)
+        _check_agents(lib().orc_sim_agents_update(self._h, seed, env_id))
 
     def step_keyed(self, seed, env_id=0):
         """Second half: Env::step with the keyed shuffle over everything queued, the caller's own instructions included."""
@@ -544,7 +552,7 @@ class MarketEnv:
 
     def run_agents(self, n_steps, seed, market_id=0, keyed=True):
         """market_sim_runner (runner.rs:107-131); keyed=True uses the Philox contract keyed by market id."""
-        lib().orc_market_run(self._h, int(keyed), seed, market_id, n_steps)
+        _check_agents(lib().orc_market_run(self._h, int(keyed), seed, market_id, n_steps))
 
     def n_instructions(self): return lib().orc_market_n_instructions(self._h)
 

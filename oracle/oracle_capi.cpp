@@ -17,7 +17,12 @@
 
 using namespace oracle;
 
+// message of the last PriceError an agent run stopped at (orc_sim_run, orc_sim_agents_update, orc_market_run)
+static thread_local std::string last_error;
+
 extern "C" {
+
+const char* orc_last_error(void) { return last_error.c_str(); }
 
 struct orc_instr {  // 32 bytes, == bb_instr
     uint64_t t;
@@ -254,13 +259,30 @@ static void add_groups(Sim& sim, const orc_group* g, uint32_t n_groups) {
 }
 void orc_sim_set_groups(void* s, const orc_group* g, uint32_t n_groups) { add_groups(((SimHandle*)s)->sim, g, n_groups); }
 // keyed != 0: Philox contract (what the CUDA path mirrors);  keyed == 0: reference-style shared stream
-void orc_sim_run(void* s, int keyed, uint64_t seed, uint32_t env_id, uint64_t n_steps) {
+// 0, or -1 when an agent's limit price was off its book's tick: the reference agents unwrap create_order's PriceError
+// (orderbook.rs:367-383) and panic.  The env stays as it was at the throw (completed steps' records
+// readable, the failing step's instructions queued); orc_last_error() gives the reference's message.
+int orc_sim_run(void* s, int keyed, uint64_t seed, uint32_t env_id, uint64_t n_steps) {
     SimHandle* h = (SimHandle*)s;
-    if (keyed) h->sim.run_keyed(seed, env_id, n_steps); else h->sim.run_stream(seed, n_steps);
+    try {
+        if (keyed) h->sim.run_keyed(seed, env_id, n_steps); else h->sim.run_stream(seed, n_steps);
+    } catch (const PriceError& e) {
+        last_error = e.what();
+        return -1;
+    }
+    return 0;
 }
 uint64_t orc_sim_n_instructions(void* s) { return ((SimHandle*)s)->sim.n_instructions; }
 // the two halves of one keyed step (instructions queued in between take part in the step's shuffle)
-void orc_sim_agents_update(void* s, uint64_t seed, uint32_t env_id) { ((SimHandle*)s)->sim.agents_update_keyed(seed, env_id); }
+int orc_sim_agents_update(void* s, uint64_t seed, uint32_t env_id) {  // 0, or -1 as orc_sim_run
+    try {
+        ((SimHandle*)s)->sim.agents_update_keyed(seed, env_id);
+    } catch (const PriceError& e) {
+        last_error = e.what();
+        return -1;
+    }
+    return 0;
+}
 int orc_sim_step_keyed(void* s, uint64_t seed, uint32_t env_id) {
     try {
         ((SimHandle*)s)->sim.step_keyed(seed, env_id);
@@ -338,9 +360,16 @@ void orc_market_set_groups(void* m, const orc_group* g, const uint32_t* assets, 
     add_market_groups(((MarketHandle*)m)->sim, g, assets, n_groups);
 }
 // keyed != 0: Philox contract keyed by market id (what the CUDA path mirrors); keyed == 0: market_sim_runner's shared stream
-void orc_market_run(void* m, int keyed, uint64_t seed, uint32_t market_id, uint64_t n_steps) {
+// 0, or -1 as orc_sim_run
+int orc_market_run(void* m, int keyed, uint64_t seed, uint32_t market_id, uint64_t n_steps) {
     MarketHandle* h = (MarketHandle*)m;
-    if (keyed) h->sim.run_keyed(seed, market_id, n_steps); else h->sim.run_stream(seed, n_steps);
+    try {
+        if (keyed) h->sim.run_keyed(seed, market_id, n_steps); else h->sim.run_stream(seed, n_steps);
+    } catch (const PriceError& e) {
+        last_error = e.what();
+        return -1;
+    }
+    return 0;
 }
 uint64_t orc_market_n_instructions(void* m) { return ((MarketHandle*)m)->sim.n_instructions; }
 

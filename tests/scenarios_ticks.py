@@ -146,3 +146,35 @@ def apply_rows_oracle(o, rows):
             o.cancel_order(oid)
         else:
             o.modify_order(oid, price, vol)
+
+
+# ---- in-kernel agents off their book's tick (the reference agents unwrap create_order's PriceError and panic)
+# `m` is the oracle module or bourse_b200.core (same group records).  `u` is the handle's price granule: every group
+# tick is a multiple of it.  A main RandomAgents group on multiples of 4u keeps every book busy and on its grid; the
+# off-grid group quotes on multiples of u, so on books with tick 2u or 4u it draws an off-tick price now and then, at a
+# step that differs from env to env.  Noise traders quote around the mid price, which an empty side puts at ~2^31: no
+# dense price window holds that, so the dense populations leave them out (and momentum traders send market orders only).
+OFFGRID_POPS = ["random", "momentum", "noise"]
+SEED, STEP, N_STEPS = 17, 100_000, 40
+
+
+def offgrid_groups(m, pop, u, dense=False):
+    main = m.random_group(40, (40, 60), (10, 20), 4 * u, 0.7)
+    rare = m.random_group(2, (50, 54), (1, 5), u, 0.05)
+    if pop == "random":
+        return [main, rare]
+    if pop == "momentum":
+        return [main, rare, m.momentum_group(100, 12, 4 * u, 0.1, 10, 1.0, 5.0, 0.5, 0.0 if dense else 1.0, 0.0, 1.0)]
+    assert pop == "noise" and not dense
+    return [main, m.noise_group(200, 3, u, 0.05, 0.02, 0.2, 7, 0.5, 0.8)]
+
+
+def market_ticks(u):
+    return [u, 2 * u]
+
+
+def offgrid_market_groups(m, pop, u, dense=False):
+    """The same populations as market twins on ticks [u, 2u]: the main groups trade both assets, the off-grid one asset 1."""
+    single = offgrid_groups(m, pop, u, dense)
+    groups = [single[0], single[0]] + single[1:]
+    return groups, [0, 1] + [1] * (len(single) - 1)

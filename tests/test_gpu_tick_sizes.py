@@ -94,18 +94,28 @@ def test_market_agents_mixed_ticks_bit_exact(oracle, ticks, kw):
     assert n_tr > 500
 
 
-def test_momentum_off_its_books_tick_flags_that_asset_only():
+def test_momentum_off_its_books_tick_flags_that_asset_only(oracle):
     """A Momentum group with tick 3 trading a tick-2 asset: its limit prices are multiples of 3, so some are not on the
-    book's grid (the reference unwraps a PriceError): ERR_GRANULE on that asset's books, nothing on the other's."""
-    n_markets = 3
-    g = market.MarketEnv(0, 0, [1, 2], 100_000, n_markets=n_markets, max_orders=8192, max_trades=8192, max_queue=128,
+    book's grid (the reference unwraps a PriceError): ERR_GRANULE on that asset's books, nothing on the other's, and both
+    books of every market match the oracle up to the step at which it raised."""
+    n_markets, step = 3, 100_000
+    g = market.MarketEnv(0, 0, [1, 2], step, n_markets=n_markets, max_orders=8192, max_trades=8192, max_queue=128,
                          pages_smem=16, pages_total=64)
     agents = [market.RandomMarketAgents(0, 40, (40, 60), (10, 20), 1, 0.7), market.RandomMarketAgents(1, 40, (40, 60), (10, 20), 2, 0.7),
               market.MomentumMarketAgent(100, 12, 1, MOM._replace(tick_size=3))]
     market.market_sim_runner(g, agents, 5, 30)
     err = g.env_errors()
     assert (err[0::2] == 0).all(), err
-    assert ((err[1::2] & ERR_GRANULE) != 0).all(), err
+    assert (err[1::2] == ERR_GRANULE).all(), err
+    for mk in range(n_markets):
+        o = oracle.MarketEnv(0, 0, [1, 2], step)
+        o.set_groups([a.group for a in agents], [a.asset for a in agents])
+        with pytest.raises(ValueError, match="tick-size 2$"):
+            o.run_agents(30, 5, market_id=mk)
+        f = len(o.history(0))
+        for a in range(2):
+            assert np.array_equal(g.get_level_2_data_history(a, mk)[:f], o.history(a)), (mk, a)
+            assert [t for t in g.get_trades(a, mk) if t[0] < f * step] == o.get_trades(a), (mk, a)
 
 
 ENV_KW = [dict(pages_smem=32, pages_total=32), dict(price_window=(400, 800), live_cap=254)]
