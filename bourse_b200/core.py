@@ -220,6 +220,14 @@ class BatchedEnv:
                                           C.c_void_p(d_out_ids_ptr) if d_out_ids_ptr else None,
                                           C.c_void_p(d_obs_ptr) if d_obs_ptr else None))
 
+    def step_device_market(self, d_instrs_ptr: int, d_offsets_ptr: int, n_rows: int, d_out_ids_ptr: int = 0, d_obs_ptr: int = 0):
+        """One MarketEnv::step for every market of a multi-asset handle whose rows are already in device memory
+        (bb_step_device_market); asynchronous.  `d_offsets_ptr`: u64 [n_markets + 1] delimiting each market's rows; each
+        row's `aux` is its asset.  `d_out_ids_ptr` receives the per-book ids, `d_obs_ptr` [n_envs, obs_words] the records."""
+        self._ck(self._lib.bb_step_device_market(self._h, C.c_void_p(d_instrs_ptr), C.c_void_p(d_offsets_ptr), n_rows,
+                                                 C.c_void_p(d_out_ids_ptr) if d_out_ids_ptr else None,
+                                                 C.c_void_p(d_obs_ptr) if d_obs_ptr else None))
+
     def run_agents_with_rows(self, seed: int, d_instrs_ptr: int, d_offsets_ptr: int, n_rows: int, d_out_ids_ptr: int = 0,
                              d_obs_ptr: int = 0):
         """One env-step of { built-in agents update; the caller's device-resident rows; Env::step } (bb_run_agents_with_rows)."""

@@ -78,6 +78,7 @@ struct bb_handle {
     u32 dense_lp = 0, dense_nwmax = 0;  // DenseLayout parameters of the selected variant
     u64 hist_env_stride = 0;
     SmemLayout lay_apply{}, lay_sim{}, lay_snap{};
+    SmemLayout lay_apply_mkt{};  // k_apply<MODE_ENV_MKT>: the permutation holds a whole market's queue (assets * max_queue)
     // deep-book engine (deep.cuh): shared-memory offsets of k_deep, chunk pools [n_envs][dp_chunks] x 256 B
     DeepOff dp{};
     unsigned char* dp_pool = nullptr;
@@ -98,6 +99,9 @@ struct bb_handle {
     u32 assets = 1;
     std::vector<u32> market_seq;
     std::vector<u64> market_rng;  // Xoroshiro128** state, two words per market
+    // Which copy of the markets' shuffle streams is current: bb_step shuffles with market_rng on the host,
+    // bb_step_device_market on the device with a copy in the header (HDR_RNG0/1) of every book of the market
+    enum { RNG_SYNCED, RNG_HOST_AHEAD, RNG_DEVICE_AHEAD } market_rng_at = RNG_SYNCED;
     // bb_order_status: status column of one env, valid until the next launch that can change a status
     bool status_valid = false;
     u32 status_env = 0;
@@ -157,13 +161,16 @@ void seed_markets(bb_handle* h) {
     }
 }
 
-SmemLayout make_layout(const bb_handle* h, bool with_obs, bool with_instr, bool with_queue = false, bool market = false) {
+SmemLayout make_layout(const bb_handle* h, bool with_obs, bool with_instr, bool with_queue = false, bool market = false,
+                       bool market_rows = false) {
     SmemLayout l{};
     u32 off = align_up(h->blob_smem_bytes, 16);
     l.off_perm = off;
     // perm + jarr (u16 each) + slack for 8-byte jarr stores; the on-chip queue is shuffled in place and needs no perm.
-    // Markets with in-kernel agents: every book derives the permutation of the WHOLE market's queue (k_sim<.., MKT>)
+    // Markets with in-kernel agents: every book derives the permutation of the WHOLE market's queue (k_sim<.., MKT>).
+    // market_rows (k_apply<MODE_ENV_MKT>): every book shuffles the whole market's queue, u16 [assets * max_queue]
     if (market) off += 4u * align_up(h->assets * h->cfg.max_queue, 8) + 16u;
+    else if (market_rows) off += align_up(2u * h->assets * h->cfg.max_queue + 16u, 16);
     else off += align_up((with_queue ? 2u : 4u) * h->cfg.max_queue + 16u, 16);
     l.off_obs = off;
     if (with_obs) off += align_up((market ? 1u : 2u) * OBS_STAGE_STEPS(h->cfg.obs_words) * h->cfg.obs_words * 4u, 16);
@@ -277,7 +284,8 @@ int upload_seeds(bb_handle* h) {
     const bb_config& c = h->cfg;
     std::vector<u64> seeds(2 * (size_t)c.n_envs);
     for (u32 e = 0; e < c.n_envs; ++e) {  // Xoroshiro128StarStar::seed_from_u64 (rand_xoshiro 0.6.0)
-        u64 x = c.seed + c.env_id_base + e;
+        // every book of a market keeps a copy of the market's stream (seed_markets), which k_apply<MODE_ENV_MKT> shuffles with
+        u64 x = h->assets > 1 ? c.seed + c.env_id_base / h->assets + e / h->assets : c.seed + c.env_id_base + e;
         seeds[2 * e] = splitmix_next(x);
         seeds[2 * e + 1] = splitmix_next(x);
     }
@@ -310,7 +318,33 @@ int init_books(bb_handle* h) {
     std::fill(h->n_orders_host.begin(), h->n_orders_host.end(), 0);
     h->mirror_dirty = false;
     h->recorded_host = 0;
-    if (h->assets > 1) seed_markets(h);
+    if (h->assets > 1) {  // k_init rewrote the device copies of the markets' streams from the same seeds
+        seed_markets(h);
+        h->market_rng_at = bb_handle::RNG_SYNCED;
+    }
+    return BB_OK;
+}
+
+// The markets' shuffle streams, host mirror -> every book's header copy (bb_step_device_market after a bb_step) and back
+// (bb_step after a bb_step_device_market).  Synchronous; neither runs while the copies agree.
+int market_rng_to_device(bb_handle* h) {
+    const u32 ne = h->cfg.n_envs, A = h->assets;
+    std::vector<u64> s(2 * (size_t)ne);
+    for (u32 e = 0; e < ne; ++e) {
+        s[2 * e] = h->market_rng[2 * (e / A)];
+        s[2 * e + 1] = h->market_rng[2 * (e / A) + 1];
+    }
+    CUDA_TRY(h, cudaMemcpy2DAsync(h->blobs + HDR_RNG0, h->blob_stride, s.data(), 16, 16, ne, cudaMemcpyHostToDevice, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    h->market_rng_at = bb_handle::RNG_SYNCED;
+    return BB_OK;
+}
+int market_rng_to_host(bb_handle* h) {
+    static_assert(HDR_RNG1 == HDR_RNG0 + 8, "the two state words are adjacent");
+    CUDA_TRY(h, cudaMemcpy2DAsync(h->market_rng.data(), 16, h->blobs + HDR_RNG0, h->blob_stride * h->assets, 16, h->cfg.n_envs / h->assets,
+                                  cudaMemcpyDeviceToHost, h->stream));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    h->market_rng_at = bb_handle::RNG_SYNCED;
     return BB_OK;
 }
 
@@ -361,10 +395,25 @@ int ensure_instr_capacity(bb_handle* h, size_t n) {
     return BB_OK;
 }
 
+// bb_step_device*: the kernel keeps the ids between assignment and execution; without a caller buffer it uses the handle's
+int id_buffer(bb_handle* h, uint64_t n_rows, u64** d_out_ids) {
+    if (*d_out_ids) return BB_OK;
+    if (n_rows + 1 > h->d_ids_cap) {
+        CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+        cudaFree(h->d_ids);
+        h->d_ids = nullptr;
+        h->d_ids_cap = n_rows + n_rows / 2 + 1024;
+        CUDA_TRY(h, cudaMalloc(&h->d_ids, h->d_ids_cap * 8));
+    }
+    *d_out_ids = h->d_ids;
+    return BB_OK;
+}
+
 int launch_apply(bb_handle* h, int mode, const bb_instr* d_instrs, const u64* d_offsets, u32 n_steps, bool host_order = false,
                  u64* d_out_ids = nullptr, u32* d_obs_out = nullptr) {
     KParams p;
-    fill_params(h, h->lay_apply, p);
+    const SmemLayout& lay = mode == MODE_ENV_MKT ? h->lay_apply_mkt : h->lay_apply;
+    fill_params(h, lay, p);
     p.instrs = d_instrs;
     p.offsets = d_offsets;
     p.n_steps = n_steps;
@@ -388,11 +437,11 @@ int launch_apply(bb_handle* h, int mode, const bb_instr* d_instrs, const u64* d_
         return BB_OK;
     }
     int grid = 0, rc;
-    const u32 wpb = wpb_for(h->lay_apply.warp_bytes);
-    const size_t smem = (size_t)h->lay_apply.warp_bytes * wpb;
+    const u32 wpb = wpb_for(lay.warp_bytes);
+    const size_t smem = (size_t)lay.warp_bytes * wpb;
 #define LAUNCH_APPLY(M, E)                                                                            \
     do {                                                                                              \
-        if ((rc = grid_for(h, k_apply<M, E>, h->lay_apply, h->cfg.n_envs, &grid, wpb))) return rc;    \
+        if ((rc = grid_for(h, k_apply<M, E>, lay, h->cfg.n_envs, &grid, wpb))) return rc;             \
         k_apply<M, E><<<grid, wpb * 32, smem, h->stream>>>(p);                                        \
     } while (0)
     if (mode == MODE_REPLAY) {
@@ -401,6 +450,12 @@ int launch_apply(bb_handle* h, int mode, const bb_instr* d_instrs, const u64* d_
         else if (h->eng == ENG_FAST) LAUNCH_APPLY(MODE_REPLAY, ENG_FAST);
         else if (h->all_resident) LAUNCH_APPLY(MODE_REPLAY, ENG_PAGED_RES);
         else LAUNCH_APPLY(MODE_REPLAY, ENG_PAGED);
+    } else if (mode == MODE_ENV_MKT) {
+        if (h->eng == ENG_DENSE) LAUNCH_APPLY(MODE_ENV_MKT, ENG_DENSE);
+        else if (h->eng == ENG_DENSE_L) LAUNCH_APPLY(MODE_ENV_MKT, ENG_DENSE_L);
+        else if (h->eng == ENG_FAST) LAUNCH_APPLY(MODE_ENV_MKT, ENG_FAST);
+        else if (h->all_resident) LAUNCH_APPLY(MODE_ENV_MKT, ENG_PAGED_RES);
+        else LAUNCH_APPLY(MODE_ENV_MKT, ENG_PAGED);
     } else {
         if (h->eng == ENG_DENSE) LAUNCH_APPLY(MODE_ENV, ENG_DENSE);
         else if (h->eng == ENG_DENSE_L) LAUNCH_APPLY(MODE_ENV, ENG_DENSE_L);
@@ -414,7 +469,7 @@ int launch_apply(bb_handle* h, int mode, const bb_instr* d_instrs, const u64* d_
     // the host-side record count is unknown from here on and is re-read from the device when next needed
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     cudaStreamIsCapturing(h->stream, &cap);
-    if (mode == MODE_ENV && h->recorded_host >= 0 && cap == cudaStreamCaptureStatusNone) h->recorded_host += n_steps;
+    if (mode != MODE_REPLAY && h->recorded_host >= 0 && cap == cudaStreamCaptureStatusNone) h->recorded_host += n_steps;
     else h->recorded_host = -1;
     return BB_OK;
 }
@@ -534,6 +589,7 @@ int bb_create(const bb_config* cfg, bb_handle** out) {
     h->max_steps_padded = align_up(cfg->max_steps, 4);
     h->hist_env_stride = (u64)h->max_steps_padded * cfg->obs_words;
     h->lay_apply = make_layout(h, false, true);
+    h->lay_apply_mkt = make_layout(h, false, true, false, false, true);
     h->lay_sim = make_layout(h, true, false, h->eng >= ENG_DENSE);
     h->lay_snap = make_layout(h, false, false);
     h->queue.resize(cfg->n_envs);
@@ -745,6 +801,8 @@ int bb_step(bb_handle* h, uint32_t n_steps) {
         // event i of the shuffled queue runs at start + i.  Each book receives its events in that order with the
         // offset i in bb_instr::t (k_apply's host_order path).
         const u32 A = h->assets;
+        // the last shuffles ran on the device (bb_step_device_market): continue from its copy of the streams
+        if (h->market_rng_at == bb_handle::RNG_DEVICE_AHEAD && (rc = market_rng_to_host(h))) return rc;
         std::vector<bb_instr> all;
         std::vector<u32> book;
         std::vector<size_t> fill(A);
@@ -765,6 +823,7 @@ int bb_step(bb_handle* h, uint32_t n_steps) {
                     std::swap(all[i - 1], all[j]);
                     std::swap(book[i - 1], book[j]);
                 }
+                if (n > 1) h->market_rng_at = bb_handle::RNG_HOST_AHEAD;  // the books' header copies are behind now
                 for (u32 a = 0; a < A; ++a) fill[a] = h->h_offsets[m * A + a];
                 for (u32 i = 0; i < n; ++i) {
                     bb_instr x = all[i];
@@ -909,18 +968,39 @@ int bb_step_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_env
     for (auto& q : h->queue)
         if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    if (!d_out_ids) {  // the kernel needs somewhere to keep the ids between assignment and execution
-        if (n_rows + 1 > h->d_ids_cap) {
-            CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-            cudaFree(h->d_ids);
-            h->d_ids = nullptr;
-            h->d_ids_cap = n_rows + n_rows / 2 + 1024;
-            CUDA_TRY(h, cudaMalloc(&h->d_ids, h->d_ids_cap * 8));
-        }
-        d_out_ids = h->d_ids;
-    }
+    int rc = id_buffer(h, n_rows, &d_out_ids);
+    if (rc) return rc;
     h->mirror_dirty = true;  // ids were handed out on the device
     return launch_apply(h, MODE_ENV, d_instrs, d_env_offsets, 1, false, d_out_ids, d_obs_out);
+}
+
+int bb_step_device_market(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_market_offsets, uint64_t n_rows,
+                          uint64_t* d_out_ids, uint32_t* d_obs_out) {
+    CHECK_H(h);
+    if (!d_market_offsets || (n_rows && !d_instrs)) return fail(h, BB_EINVAL, "null argument");
+    if (h->assets < 2) return fail(h, BB_EINVAL, "bb_step_device_market drives multi-asset markets (single-asset envs: bb_step_device)");
+    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine replays instruction streams only");
+    if ((u64)h->assets * h->cfg.max_queue > 65535) return fail(h, BB_EINVAL, "assets * max_queue must stay below 65536");
+    for (auto& q : h->queue)
+        if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    if (h->market_rng_at == bb_handle::RNG_HOST_AHEAD) {
+        // bb_step shuffled on the host since the books' copies of the streams were last written: bring them up to date, but
+        // never inside a stream capture (the graph would replay a copy of the streams as they are now)
+        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+        cudaStreamIsCapturing(h->stream, &cap);
+        if (cap != cudaStreamCaptureStatusNone)
+            return fail(h, BB_EINVAL, "bb_step_device_market: the markets' shuffle streams last advanced in bb_step; call "
+                                      "bb_step_device_market once outside the capture (or bb_reset) before capturing it");
+        int rc = market_rng_to_device(h);
+        if (rc) return rc;
+    }
+    int rc = id_buffer(h, n_rows, &d_out_ids);
+    if (rc) return rc;
+    h->mirror_dirty = true;  // ids were handed out on the device
+    if ((rc = launch_apply(h, MODE_ENV_MKT, d_instrs, d_market_offsets, 1, false, d_out_ids, d_obs_out))) return rc;
+    h->market_rng_at = bb_handle::RNG_DEVICE_AHEAD;
+    return BB_OK;
 }
 
 int bb_level2_device(bb_handle* h, uint32_t* d_out) {
@@ -1027,6 +1107,7 @@ int bb_reserve_queue(bb_handle* h, uint32_t max_queue) {
         return fail(h, BB_ECAP, "max_queue does not fit in shared memory next to the book image");
     }
     h->lay_apply = la;
+    h->lay_apply_mkt = make_layout(h, false, true, false, false, true);
     h->lay_sim = make_layout(h, true, false, h->eng >= ENG_DENSE, !h->group_asset.empty());
     h->lay_snap = make_layout(h, false, false);
     cudaFree(h->scratch);  // k_sim's global-memory queues are sized by max_queue: reallocated at the next agent launch

@@ -4,6 +4,7 @@
 //   k_apply<MODE_REPLAY>  immediate-mode instruction streams (OrderBook API, config C2)
 //                         reference: orderbook.rs:411-421, 583-792 driven at explicit times
 //   k_apply<MODE_ENV>     Env::step over host-queued instructions (crates/step_sim/src/env.rs:116-135)
+//   k_apply<MODE_ENV_MKT> MarketEnv::step over device-resident rows, one slice per market (market_env.rs:108-121)
 //   k_sim                 persistent { agents.update; env.step } x n_steps (runner.rs:46-69) with the
 //                         built-in RandomAgents / MomentumAgent generated in-kernel
 //   k_snapshot            live level-1 / level-2 / touch data of every book (orderbook.rs:287-324)
@@ -18,6 +19,7 @@ namespace bb {
 
 #define MODE_REPLAY 0
 #define MODE_ENV 1
+#define MODE_ENV_MKT 2  // bb_step_device_market: MarketEnv::step over device-resident rows, one slice per market
 #define MAX_GROUPS 8
 #define LIVE_CAP 254  // default capacity of a MomentumAgent / NoiseAgent live-order list (per group per env)
 // env-steps of observation records staged in shared memory per bulk store: 8 level-1 records (288 B) or 4 level-2
@@ -238,8 +240,12 @@ template <int MODE, int ENG> __global__ void __launch_bounds__(128, (ENG == ENG_
             return;
         }
         book_from_header(g, b);
-        const u64 off = p.offsets[env];
-        const u32 n = (u32)(p.offsets[env + 1] - off);
+        // MODE_ENV_MKT: the offsets delimit markets; this book is asset mk_a of market env / assets
+        constexpr bool MK = MODE == MODE_ENV_MKT;
+        const u32 mk_a = MK ? env % p.assets : 0u;
+        const u32 slice = MK ? env / p.assets : env;
+        const u64 off = p.offsets[slice];
+        const u32 n = (u32)(p.offsets[slice + 1] - off);
         const bb_instr* ins = p.instrs + off;
 
         if (MODE == MODE_REPLAY) {
@@ -286,61 +292,114 @@ template <int MODE, int ENG> __global__ void __launch_bounds__(128, (ENG == ENG_
                 const u64 start = b.t;
                 b.trade_vol = 0;  // env.rs:117-118
                 const u32 m = (s == 0) ? n : 0u;
-                if (m > p.max_queue) b.err |= ERR_CAP_QUEUE;
-                if constexpr (G::DENSE) {  // the dense engine relies on t = start + i being new, increasing key times
-                    if (m > p.step_size || (start <= b.max_key_time && (b.flags & (FL_HAS_ASK | FL_HAS_BID)))) b.err |= ERR_TIME_ORDER;
-                }
-                const u32 mm = min(m, p.max_queue);
-                // (a) create_order happened at submission (env.rs:173): publish status New for the new ids
-                u32 nv = mm;  // transactions in the queue
-                if (p.assign_ids) {
-                    // device-submitted rows: what Env::place_order / cancel_order / modify_order would have done at
-                    // submission happens here, in row order — NEW rows take the next ids; a limit price off the tick grid
-                    // is create_order's PriceError (orderbook.rs:367-383): nothing is created or queued, the env is flagged
-                    u32 next = b.n_orders;
+                u32 nv;  // transactions in the queue
+                if constexpr (MK) {
+                    // device-submitted market rows: every book of the market walks the whole slice and does, in row order,
+                    // what MarketEnv::place_order / cancel_order / modify_order (market_env.rs:163-219) would have done for
+                    // the rows of its own asset (bb_instr::aux): NEW rows take the next ids of that asset's book
+                    // (market.rs:270-280), an off-tick limit price creates and queues nothing and flags that book.  Rows
+                    // naming no asset of the market queue nothing and flag book 0.  Each book writes the ids of its own
+                    // rows only (book 0 also those of the asset-less rows), and keeps the market-wide queue in `perm`
+                    const bool drop = m > p.assets * p.max_queue;  // the whole market's queue must fit the permutation
+                    if (drop) b.err |= ERR_CAP_QUEUE;
+                    const u32 book0 = env - mk_a;
+                    u32 next = b.n_orders, n_mine = 0;
                     nv = 0;
-                    const u32 tick = __ldg(g.ticks + env);
-                    for (u32 j0 = 0; j0 < mm; j0 += 32) {
+                    for (u32 j0 = 0; j0 < m; j0 += 32) {
                         const u32 j = j0 + lane;
-                        u32 of = 0, price = 0;
-                        if (j < mm) {
+                        u32 of = 0, price = 0, asset = 0;
+                        if (j < m) {
+                            const uint4 y = reinterpret_cast<const uint4*>(ins + j)[1];
                             of = ins[j].op_flags;
-                            price = ins[j].price;
+                            price = y.x;
+                            asset = y.w;
                         }
                         const u32 op = of & BB_OP_MASK;
-                        const bool bad_tick = op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % tick != 0u);
-                        const bool is_new = op == BB_OP_NEW && !bad_tick;
-                        const bool queued = is_new || op == BB_OP_CANCEL || op == BB_OP_MODIFY;
+                        const bool row_ok = j < m && !drop && asset < p.assets;
+                        const bool bad_tick = row_ok && op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % __ldg(g.ticks + book0 + asset) != 0u);
+                        const bool is_new = row_ok && op == BB_OP_NEW && !bad_tick;
+                        const bool queued = is_new || (row_ok && (op == BB_OP_CANCEL || op == BB_OP_MODIFY));
+                        const bool own = j < m && (asset < p.assets ? asset == mk_a : mk_a == 0u);
+                        const bool my_new = is_new && asset == mk_a;
                         const u32 below = (1u << lane) - 1u;
-                        const u32 nm = __ballot_sync(BB_FULL, is_new), qm = __ballot_sync(BB_FULL, queued);
+                        const u32 nm = __ballot_sync(BB_FULL, my_new), qm = __ballot_sync(BB_FULL, queued);
                         const u32 id = next + __popc(nm & below);
-                        if (j < mm) {
-                            p.out_ids[off + j] = is_new ? (u64)id : ~0ULL;
-                            if (is_new && id < g.max_orders)
+                        if (own) {
+                            p.out_ids[off + j] = my_new ? (u64)id : ~0ULL;
+                            if (my_new && id < g.max_orders)
                                 stg32(b.oh + (u64)id * ORD_STRIDE + OH_META, ST_NEW | ((of & BB_F_BID) ? META_BID : 0u));
                         }
                         if (queued) sts16(perm + 2u * (nv + __popc(qm & below)), j);
-                        if (__any_sync(BB_FULL, bad_tick)) b.err |= ERR_PRICE;
+                        if (__any_sync(BB_FULL, bad_tick && asset == mk_a)) b.err |= ERR_PRICE;
+                        if (__any_sync(BB_FULL, j < m && !drop && asset >= p.assets) && mk_a == 0u) b.err |= ERR_ROW_OP;
                         next += __popc(nm);
                         nv += __popc(qm);
+                        n_mine += __popc(__ballot_sync(BB_FULL, queued && asset == mk_a));
                     }
                     b.n_orders = next;
-                } else {
-                    u32 max_id = 0;
-                    for (u32 j = lane; j < mm; j += 32) {
-                        const u32 of = ins[j].op_flags, id = ins[j].order_id;
-                        if ((of & BB_OP_MASK) == BB_OP_NEW && id < g.max_orders) {
-                            stg32(b.oh + (u64)id * ORD_STRIDE + OH_META, ST_NEW | ((of & BB_F_BID) ? META_BID : 0u));
-                            max_id = max(max_id, id + 1);
-                        }
-                        sts16(perm + 2u * j, j);
+                    // the host-ordered path's rule, over this book's share of the queue
+                    if constexpr (G::DENSE) {
+                        if (n_mine > p.step_size || (start <= b.max_key_time && (b.flags & (FL_HAS_ASK | FL_HAS_BID)))) b.err |= ERR_TIME_ORDER;
                     }
-                    max_id = __reduce_max_sync(BB_FULL, max_id);
-                    if (max_id > b.n_orders) b.n_orders = max_id;
+                } else {
+                    if (m > p.max_queue) b.err |= ERR_CAP_QUEUE;
+                    if constexpr (G::DENSE) {  // the dense engine relies on t = start + i being new, increasing key times
+                        if (m > p.step_size || (start <= b.max_key_time && (b.flags & (FL_HAS_ASK | FL_HAS_BID)))) b.err |= ERR_TIME_ORDER;
+                    }
+                    const u32 mm = min(m, p.max_queue);
+                    // (a) create_order happened at submission (env.rs:173): publish status New for the new ids
+                    nv = mm;
+                    if (p.assign_ids) {
+                        // device-submitted rows: what Env::place_order / cancel_order / modify_order would have done at
+                        // submission happens here, in row order — NEW rows take the next ids; a limit price off the tick grid
+                        // is create_order's PriceError (orderbook.rs:367-383): nothing is created or queued, the env is flagged
+                        u32 next = b.n_orders;
+                        nv = 0;
+                        const u32 tick = __ldg(g.ticks + env);
+                        for (u32 j0 = 0; j0 < mm; j0 += 32) {
+                            const u32 j = j0 + lane;
+                            u32 of = 0, price = 0;
+                            if (j < mm) {
+                                of = ins[j].op_flags;
+                                price = ins[j].price;
+                            }
+                            const u32 op = of & BB_OP_MASK;
+                            const bool bad_tick = op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % tick != 0u);
+                            const bool is_new = op == BB_OP_NEW && !bad_tick;
+                            const bool queued = is_new || op == BB_OP_CANCEL || op == BB_OP_MODIFY;
+                            const u32 below = (1u << lane) - 1u;
+                            const u32 nm = __ballot_sync(BB_FULL, is_new), qm = __ballot_sync(BB_FULL, queued);
+                            const u32 id = next + __popc(nm & below);
+                            if (j < mm) {
+                                p.out_ids[off + j] = is_new ? (u64)id : ~0ULL;
+                                if (is_new && id < g.max_orders)
+                                    stg32(b.oh + (u64)id * ORD_STRIDE + OH_META, ST_NEW | ((of & BB_F_BID) ? META_BID : 0u));
+                            }
+                            if (queued) sts16(perm + 2u * (nv + __popc(qm & below)), j);
+                            if (__any_sync(BB_FULL, bad_tick)) b.err |= ERR_PRICE;
+                            next += __popc(nm);
+                            nv += __popc(qm);
+                        }
+                        b.n_orders = next;
+                    } else {
+                        u32 max_id = 0;
+                        for (u32 j = lane; j < mm; j += 32) {
+                            const u32 of = ins[j].op_flags, id = ins[j].order_id;
+                            if ((of & BB_OP_MASK) == BB_OP_NEW && id < g.max_orders) {
+                                stg32(b.oh + (u64)id * ORD_STRIDE + OH_META, ST_NEW | ((of & BB_F_BID) ? META_BID : 0u));
+                                max_id = max(max_id, id + 1);
+                            }
+                            sts16(perm + 2u * j, j);
+                        }
+                        max_id = __reduce_max_sync(BB_FULL, max_id);
+                        if (max_id > b.n_orders) b.n_orders = max_id;
+                    }
                 }
                 __syncwarp();
                 // (b) transactions.shuffle(rng) (env.rs:121): Fisher-Yates from the back.  Multi-asset markets shuffle
-                // one queue across their books (market_env.rs:114-115): the host did that, the slice is in order
+                // one queue across their books (market_env.rs:114-115): on the host-ordered path the host did that and the
+                // slice is in order; in MODE_ENV_MKT every book of the market shuffles the whole queue with its own copy
+                // of the market's Xoroshiro state (all copies advance alike)
                 if (!p.host_order && lane == 0u) {  // a serial chain: one lane applies it (see the swap loop of k_sim)
                     u64 s0 = lds64(b.sb + HDR_RNG0), s1 = lds64(b.sb + HDR_RNG1);
                     for (u32 i = nv; i > 1; --i) {
@@ -355,8 +414,30 @@ template <int MODE, int ENG> __global__ void __launch_bounds__(128, (ENG == ENG_
                 __syncwarp();
                 // (c) process in shuffled order at t = start + i (env.rs:123-127)
                 for (u32 i0 = 0; i0 < nv; i0 += 32) {
-                    const u32 cnt = min(32u, nv - i0);
-                    if (lane < cnt) {
+                    u32 cnt = min(32u, nv - i0);
+                    if constexpr (MK) {
+                        // this book's events of the batch, in queue order, each with its position in the shuffled market
+                        // queue (its time offset) in bb_instr::t; the NEW ids were written by this warp above
+                        bool mine = false;
+                        uint4 x0, x1;
+                        if (lane < cnt) {
+                            const u32 pj = lds16(perm + 2u * (i0 + lane));
+                            const uint4* src = reinterpret_cast<const uint4*>(ins + pj);
+                            x0 = src[0];
+                            x1 = src[1];
+                            mine = x1.w == mk_a;
+                            if (mine && (x0.z & BB_OP_MASK) == BB_OP_NEW) x0.w = (u32)p.out_ids[off + pj];
+                            x0.x = i0 + lane;
+                            x0.y = 0u;
+                        }
+                        const u32 mm = __ballot_sync(BB_FULL, mine);
+                        if (mine) {
+                            const u32 pos = __popc(mm & ((1u << lane) - 1u));
+                            sts128(chunk + 32u * pos, x0);
+                            sts128(chunk + 32u * pos + 16u, x1);
+                        }
+                        cnt = __popc(mm);
+                    } else if (lane < cnt) {
                         const u32 pj = lds16(perm + 2u * (i0 + lane));
                         const uint4* src = reinterpret_cast<const uint4*>(ins + pj);
                         uint4 x0 = src[0];
@@ -367,7 +448,7 @@ template <int MODE, int ENG> __global__ void __launch_bounds__(128, (ENG == ENG_
                     __syncwarp();
                     for (u32 k = 0; k < cnt; ++k) {
                         const uint4 x = lds128(chunk + 32u * k), y = lds128(chunk + 32u * k + 16u);
-                        const u64 t = start + (p.host_order ? (((u64)x.y << 32) | x.x) : (u64)(i0 + k));
+                        const u64 t = start + ((MK || p.host_order) ? (((u64)x.y << 32) | x.x) : (u64)(i0 + k));
                         b.t = t;
                         apply_instr<false>(g, b, x.z, x.w, y.x, y.y, y.z, t, false);
                     }

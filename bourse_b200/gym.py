@@ -10,10 +10,15 @@ Buffers are exchanged through DLPack (`__dlpack__` / `__dlpack_device__`: `torch
 `jax.dlpack`) and the CUDA array interface (`__cuda_array_interface__`, version 3), which torch, cupy and numba all
 speak, so this module needs none of them: both give zero-copy views, and a torch / cupy array (anything with `__dlpack__`
 or the CUDA array interface) can be passed to `step` directly.  numpy arrays are accepted too (copied host to device).
+
+`MarketVectorEnv` is the same loop for multi-asset markets (`MarketEnv` place / cancel / modify then `step`, one block of
+rows per market, each row naming its asset).  Use `VectorEnv` for independent single-asset envs, `MarketVectorEnv` when
+assets share a market's shuffled queue, and `market.MarketEnv` for host-driven, order-by-order market use.
 """
 from __future__ import annotations
 
 import ctypes as C
+import math
 import typing
 
 import numpy as np
@@ -147,10 +152,12 @@ def _device_ptr(x, nbytes: int) -> typing.Optional[int]:
     return int(cai["data"][0])
 
 
-def pack_actions(op, bid=None, vol=None, trader=None, price=None, order_id=None, market=None, has_price=None, has_vol=None) -> np.ndarray:
+def pack_actions(op, bid=None, vol=None, trader=None, price=None, order_id=None, market=None, has_price=None, has_vol=None,
+                 asset=None) -> np.ndarray:
     """Columns -> packed instruction rows (host numpy, any shape).  `op`: abi.OP_NOOP / OP_NEW / OP_CANCEL / OP_MODIFY.
     NEW rows: `market=True` is a market order (`price=None` in the reference).  MODIFY rows: `has_price` / `has_vol` say
-    which of `price` / `vol` is `Some` (default: both)."""
+    which of `price` / `vol` is `Some` (default: both).  `asset`: the row's asset for `MarketVectorEnv` (the `aux` column;
+    left 0 when not given)."""
     op = np.asarray(op, dtype=np.uint32)
     a = np.zeros(op.shape, dtype=ACTION_DTYPE)
 
@@ -167,10 +174,66 @@ def pack_actions(op, bid=None, vol=None, trader=None, price=None, order_id=None,
     oid = col(order_id).astype(np.uint64)
     a["order_id"] = np.where(oid > 0xFFFFFFFE, 0xFFFFFFFF, oid).astype(np.uint32)  # ids beyond u32 cannot exist: bad id
     a["price"], a["vol"], a["trader"] = col(price), col(vol), col(trader)
+    if asset is not None:
+        a["aux"] = col(asset)
     return a
 
 
-class VectorEnv:
+class _DeviceLoop:
+    """What `VectorEnv` and `MarketVectorEnv` share: the handle, the device buffers, host-action staging and the history ring."""
+
+    env: BatchedEnv
+    obs: DeviceArray
+    ids: DeviceArray
+    _what = "env"
+
+    def _buffers(self, obs_shape, rows_shape):
+        self.obs = DeviceArray(self.env, obs_shape, np.uint32)
+        self.ids = DeviceArray(self.env, rows_shape, np.uint64)
+        self._actions = DeviceArray(self.env, rows_shape, ACTION_DTYPE)  # staging for host-side actions
+        self._offsets = DeviceArray(self.env, (rows_shape[0] + 1,), np.uint64)
+        self._offsets.copy_from_host(np.arange(rows_shape[0] + 1, dtype=np.uint64) * np.uint64(rows_shape[1]))
+
+    def close(self):
+        for a in (self.obs, self.ids, self._actions, self._offsets):
+            a.free()
+        self.env.close()
+
+    def _observe(self) -> DeviceArray:
+        (self.env.level_1_data_device if self.obs_words == abi.OBS_L1 else self.env.level_2_data_device)(self.obs.ptr)
+        return self.obs
+
+    def reset(self) -> DeviceArray:
+        self._n_steps = 0
+        self.env.reset()   # (the agent population survives a reset; its state is cleared with the books)
+        return self._observe()
+
+    def _action_ptr(self, actions) -> int:
+        """Device address of the step's action block: the caller's device array, or the staging copy of a host array."""
+        shape = self._actions.shape
+        ptr = _device_ptr(actions, self._actions.nbytes)
+        if ptr is None:  # host array: one H2D copy
+            a = np.ascontiguousarray(actions, dtype=ACTION_DTYPE)
+            if a.shape != shape:
+                raise ValueError(f"actions must have shape {shape}")
+            self._actions.copy_from_host(a)
+            ptr = self._actions.ptr
+        # an open-ended loop consumes each observation as it is produced: the library's per-step history is a scratch ring here
+        self._n_steps += 1
+        if self._n_steps > self.env.max_steps:
+            self.env.clear_history()
+            self._n_steps = 1
+        return ptr
+
+    def check_errors(self):
+        """Raise if any env flagged an error (capacity, bad order id, off-tick price); synchronises."""
+        e = self.env.env_errors()
+        if e.any():
+            bad = np.flatnonzero(e)
+            raise RuntimeError(f"{len(bad)} {self._what}(s) flagged errors, first {self._what} {bad[0]}: 0x{int(e[bad[0]]):x}")
+
+
+class VectorEnv(_DeviceLoop):
     """`n_envs` lockstep `StepEnvNumpy(seed + env, start_time, tick_size, step_size, trading)` instances with a fixed action
     block of `rows_per_env` instruction rows per env and step (pad with OP_NOOP rows).
 
@@ -209,42 +272,12 @@ class VectorEnv:
         self.n_envs, self.rows = n_envs, rows_per_env
         self.env = BatchedEnv(n_envs, seed, start_time, tick_size, step_size, trading, obs_words=abi.OBS_L1 if level_1 else abi.OBS_L2, **kw)
         self.obs_words = abi.OBS_L1 if level_1 else abi.OBS_L2
-        self.obs = DeviceArray(self.env, (n_envs, self.obs_words), np.uint32)
-        self.ids = DeviceArray(self.env, (n_envs, rows_per_env), np.uint64)
-        self._actions = DeviceArray(self.env, (n_envs, rows_per_env), ACTION_DTYPE)  # staging for host-side actions
-        self._offsets = DeviceArray(self.env, (n_envs + 1,), np.uint64)
-        self._offsets.copy_from_host(np.arange(n_envs + 1, dtype=np.uint64) * np.uint64(rows_per_env))
+        self._buffers((n_envs, self.obs_words), (n_envs, rows_per_env))
         if agents:
             self.env.set_agents(agents)
 
-    def close(self):
-        for a in (self.obs, self.ids, self._actions, self._offsets):
-            a.free()
-        self.env.close()
-
-    def _observe(self) -> DeviceArray:
-        (self.env.level_1_data_device if self.obs_words == abi.OBS_L1 else self.env.level_2_data_device)(self.obs.ptr)
-        return self.obs
-
-    def reset(self) -> DeviceArray:
-        self._n_steps = 0
-        self.env.reset()   # (the agent population survives a reset; its state is cleared with the books)
-        return self._observe()
-
     def step(self, actions) -> typing.Tuple[DeviceArray, DeviceArray]:
-        nbytes = self.n_envs * self.rows * ACTION_DTYPE.itemsize
-        ptr = _device_ptr(actions, nbytes)
-        if ptr is None:  # host array: one H2D copy
-            a = np.ascontiguousarray(actions, dtype=ACTION_DTYPE)
-            if a.shape != (self.n_envs, self.rows):
-                raise ValueError(f"actions must have shape ({self.n_envs}, {self.rows})")
-            self._actions.copy_from_host(a)
-            ptr = self._actions.ptr
-        # an open-ended loop consumes each observation as it is produced: the library's per-step history is a scratch ring here
-        self._n_steps += 1
-        if self._n_steps > self.env.max_steps:
-            self.env.clear_history()
-            self._n_steps = 1
+        ptr = self._action_ptr(actions)
         # one launch: (background agents,) ids, Env::step and the observation records written straight into self.obs
         if self._agents:
             self.env.run_agents_with_rows(self._agent_seed, ptr, self._offsets.ptr, self.n_envs * self.rows, self.ids.ptr, self.obs.ptr)
@@ -252,9 +285,55 @@ class VectorEnv:
             self.env.step_device(ptr, self._offsets.ptr, self.n_envs * self.rows, self.ids.ptr, self.obs.ptr)
         return self.obs, self.ids
 
-    def check_errors(self):
-        """Raise if any env flagged an error (capacity, bad order id, off-tick price); synchronises."""
-        e = self.env.env_errors()
-        if e.any():
-            bad = np.flatnonzero(e)
-            raise RuntimeError(f"{len(bad)} env(s) flagged errors, first env {bad[0]}: 0x{int(e[bad[0]]):x}")
+
+class MarketVectorEnv(_DeviceLoop):
+    """`n_markets` lockstep `MarketEnv::new(start_time, tick_sizes, step_size, trading)` instances (market_env.rs:73-90),
+    market m shuffling with `Xoroshiro128StarStar::seed_from_u64(seed + m)`, driven by a fixed block of `rows_per_market`
+    instruction rows per market and step (pad with OP_NOOP rows; `pack_actions(..., asset=...)` sets each row's asset).
+
+        env = MarketVectorEnv(2048, rows_per_market=8, seed=0, start_time=0, tick_sizes=[1, 2, 5, 10], step_size=1000)
+        obs = env.reset()                       # DeviceArray [n_markets, assets, 45] u32
+        obs, ids = env.step(actions)            # actions: [n_markets, rows_per_market] packed rows, device or host
+
+    Per market, a step is exactly `MarketEnv::place_order / cancel_order / modify_order` for each row in row order, then
+    `MarketEnv::step(rng)` (bb_step_device_market): `ids[m, r]` is the id row r created in its asset's book (order ids are
+    per asset, `MarketOrderId = (asset, ids[m, r])`) or `abi.NO_ID`; CANCEL / MODIFY rows target `(asset, order_id)`.  An
+    off-tick limit price creates nothing and flags its asset's book (`check_errors` raises).  `obs[m, a]` is asset a's
+    end-of-step record.  A step is one kernel launch with no host synchronisation, so it can be captured into a CUDA graph;
+    the history is a scratch ring as in `VectorEnv`.  `tick_sizes` has one tick per asset, at least two assets (a
+    one-asset market is an Env: use `VectorEnv`).  Use this class for an RL-style loop over many markets; use
+    `market.MarketEnv` (`place_order` / `submit` + `step` on the host) for scripted, order-by-order use, and its
+    `run_agents` for markets of built-in agents."""
+
+    _what = "book"
+
+    def __init__(self, n_markets: int, rows_per_market: int, seed: int, start_time: int, tick_sizes: typing.Sequence[int],
+                 step_size: int, trading: bool = True, *, level_1: bool = False, **kw):
+        ticks = [int(t) for t in tick_sizes]
+        if len(ticks) < 2:
+            raise ValueError("MarketVectorEnv needs two or more assets; a one-asset market is an Env: use VectorEnv")
+        if min(ticks) <= 0:
+            raise ValueError("tick sizes must be > 0")
+        A = len(ticks)
+        kw.setdefault("max_queue", max(-(-rows_per_market // A), 16))   # a market's queue holds assets * max_queue rows
+        if rows_per_market > A * kw["max_queue"]:
+            raise ValueError("rows_per_market exceeds assets * max_queue")
+        self._n_steps = 0
+        self.n_markets, self.rows, self.n_assets, self.tick_sizes = n_markets, rows_per_market, A, ticks
+        self.obs_words = abi.OBS_L1 if level_1 else abi.OBS_L2
+        # as market.MarketEnv: the handle's tick is the gcd of the assets' ticks, each book then gets its asset's own
+        granule = math.gcd(*ticks)
+        self.env = BatchedEnv(A * n_markets, seed, start_time, granule, step_size, trading, assets=A, obs_words=self.obs_words, **kw)
+        try:
+            if any(t != granule for t in ticks):
+                self.env.set_tick_sizes(ticks)
+            self._buffers((n_markets, A, self.obs_words), (n_markets, rows_per_market))
+        except Exception:
+            self.env.close()
+            raise
+
+    def step(self, actions) -> typing.Tuple[DeviceArray, DeviceArray]:
+        ptr = self._action_ptr(actions)
+        # one launch: ids, the market-wide shuffle, MarketEnv::step and the observation records written straight into self.obs
+        self.env.step_device_market(ptr, self._offsets.ptr, self.n_markets * self.rows, self.ids.ptr, self.obs.ptr)
+        return self.obs, self.ids

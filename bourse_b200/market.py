@@ -80,7 +80,12 @@ class MarketEnv:
     """`MarketEnv::<ASSETS>::new(start_time, tick_sizes, step_size, trading)` (market_env.rs:73-90) plus the shuffle
     seed the reference passes to `step` as an RNG (`Xoroshiro128StarStar::seed_from_u64(seed)`).
 
-    `market` selects one of `n_markets` lockstep markets for the per-market calls (default 0)."""
+    `market` selects one of `n_markets` lockstep markets for the per-market calls (default 0).
+
+    Which path: this class submits on the host (`place_order` / `submit` return ids at once and raise on an off-tick
+    price; `step` synchronises), which suits scripted, order-by-order use and in-kernel agents (`run_agents`).  An
+    RL-style loop that produces a fixed block of rows per market and step on the GPU should use
+    `gym.MarketVectorEnv` instead: one launch per step, no host synchronisation, CUDA-graph capturable, same results."""
 
     def __init__(self, seed: int, start_time: int, tick_sizes: typing.Sequence[int], step_size: int, trading: bool = True, *,
                  n_markets: int = 1, **kw):

@@ -119,7 +119,8 @@ typedef struct {
     uint32_t price;    /* NEW: limit price; MODIFY: new price when BB_F_HAS_PRICE */
     uint32_t vol;      /* NEW: volume; MODIFY: new volume when BB_F_HAS_VOL; SET_TRADING: 0 / 1 */
     uint32_t trader;   /* NEW: trader id */
-    uint32_t aux;      /* reserved, 0 (the library keeps a market's submission order here while instructions are queued) */
+    uint32_t aux;      /* bb_step_device_market: the row's asset; elsewhere reserved, 0 (the library keeps a market's
+                          submission order here while instructions are queued) */
 } bb_instr;
 
 #define BB_OP_NOOP 0u
@@ -243,6 +244,28 @@ int bb_step(bb_handle* h, uint32_t n_steps);
  * CUDA graph together with the caller's own kernels (stream capture on the stream given to bb_set_stream). */
 int bb_step_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_env_offsets, uint64_t n_rows, uint64_t* d_out_ids,
                    uint32_t* d_obs_out);
+/* The same device-resident loop for multi-asset markets (bb_config.assets >= 2; no upper limit on assets here).  One call
+ * does, for every market m, what MarketEnv::place_order / cancel_order / modify_order for each of the market's rows, in row
+ * order, then one MarketEnv::step(rng) would do (crates/step_sim/src/market_env.rs:108-121, 163-219).
+ * d_market_offsets[n_markets + 1] (device) delimits market m's slice of d_instrs; bb_instr::t is ignored and bb_instr::aux
+ * is the row's asset (0 .. assets - 1).  BB_OP_NEW rows with an on-tick limit price or BB_F_MARKET create the next order id
+ * of their asset's book (ids are per book, MarketOrderId = (asset, id), market.rs:270-280) in d_out_ids[row];
+ * BB_OP_CANCEL / BB_OP_MODIFY rows target (aux, order_id); no-ops and unknown codes queue nothing.  A limit price off the
+ * asset's own tick creates and queues nothing and flags that asset's book BB_ERR_PRICE; a row with aux >= assets queues
+ * nothing and flags book 0 of its market BB_ERR_ROW_OP.  Every row that creates nothing gets BB_NO_ID.  The market's queue
+ * is shuffled as a whole with the same Xoroshiro128** stream bb_step uses for it (seed + env_id_base / assets + m), event i
+ * of the shuffled queue runs at start + i on its asset's book, and every book then advances by step_size and appends one
+ * record.  A market with more than assets * max_queue rows flags BB_ERR_CAP_QUEUE on each of its books, applies none of
+ * its rows and hands out no ids; its books still step.  On the dense engine BB_ERR_TIME_ORDER follows the rule of
+ * bb_step for the same queue.  d_obs_out ([n_envs][obs_words], may be NULL) receives every book's end-of-step record;
+ * book m * assets + a is asset a of market m.  In-kernel agents do not run.  bb_step and this call may be interleaved
+ * freely on one handle.  Asynchronous: one kernel launch, no host synchronisation, and it may be recorded into a CUDA graph
+ * on a freshly created or reset handle or after an earlier bb_step_device_market; right after a bb_step that shuffled,
+ * capture is refused with BB_EINVAL (call it once outside the capture first).  Refused with BB_EINVAL on a single-asset
+ * handle (use bb_step_device), on the deep engine, while host-queued instructions are pending, and for NULL arguments.
+ * n_rows sizes the internal id buffer when d_out_ids is NULL. */
+int bb_step_device_market(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_market_offsets, uint64_t n_rows,
+                          uint64_t* d_out_ids, uint32_t* d_obs_out);
 /* bb_level2 / bb_level1 into DEVICE memory: d_out[n_envs][45] / d_out[n_envs][9].  Asynchronous. */
 int bb_level2_device(bb_handle* h, uint32_t* d_out);
 int bb_level1_device(bb_handle* h, uint32_t* d_out);
