@@ -61,7 +61,7 @@ EXPORTS = [
     "bb_n_orders", "bb_n_trades", "bb_orders", "bb_trades", "bb_order_status", "bb_time", "bb_set_time",
     "bb_set_trading", "bb_env_errors", "bb_stats", "bb_history_device", "bb_order_keys", "bb_load_book",
     "bb_set_agents_market", "bb_step_device", "bb_level2_device", "bb_level1_device", "bb_device_alloc", "bb_device_free", "bb_memcpy", "bb_run_agents_with_rows", "bb_reserve", "bb_reserve_queue", "bb_clear_history", "bb_clear_errors",
-    "bb_orders_all", "bb_trades_all", "bb_set_tick_sizes", "bb_step_device_market", "bb_comm_unique_id", "bb_comm_init_rank", "bb_comm_init_all", "bb_comm_n_ranks", "bb_comm_destroy", "bb_comm_last_error", "bb_gather_stats",
+    "bb_orders_all", "bb_trades_all", "bb_set_tick_sizes", "bb_step_device_market", "bb_run_agents_with_rows_market", "bb_comm_unique_id", "bb_comm_init_rank", "bb_comm_init_all", "bb_comm_n_ranks", "bb_comm_destroy", "bb_comm_last_error", "bb_gather_stats",
 ]
 
 _lib = None
@@ -117,6 +117,7 @@ def load() -> C.CDLL:
     sig("bb_memcpy", i32, vp, vp, vp, u64, i32)
     sig("bb_run_agents", i32, vp, u64, u32)
     sig("bb_run_agents_with_rows", i32, vp, u64, vp, vp, u64, vp, vp)
+    sig("bb_run_agents_with_rows_market", i32, vp, u64, vp, vp, u64, vp, vp)
     sig("bb_run_agents_to_host", i32, vp, u64, u32, u32, vp)
     sig("bb_level1", i32, vp, vp)
     sig("bb_level2", i32, vp, vp)

@@ -235,6 +235,15 @@ class BatchedEnv:
                                                    C.c_void_p(d_out_ids_ptr) if d_out_ids_ptr else None,
                                                    C.c_void_p(d_obs_ptr) if d_obs_ptr else None))
 
+    def run_agents_with_rows_market(self, seed: int, d_instrs_ptr: int, d_offsets_ptr: int, n_rows: int, d_out_ids_ptr: int = 0,
+                                    d_obs_ptr: int = 0):
+        """One market step of { market agents update; the caller's device-resident rows; MarketEnv::step } for every market
+        of a multi-asset handle with market agents (bb_run_agents_with_rows_market); asynchronous.  Rows, offsets and ids
+        are laid out as for `step_device_market`."""
+        self._ck(self._lib.bb_run_agents_with_rows_market(self._h, seed, C.c_void_p(d_instrs_ptr), C.c_void_p(d_offsets_ptr), n_rows,
+                                                          C.c_void_p(d_out_ids_ptr) if d_out_ids_ptr else None,
+                                                          C.c_void_p(d_obs_ptr) if d_obs_ptr else None))
+
     def level_2_data_device(self, d_out_ptr: int): self._ck(self._lib.bb_level2_device(self._h, C.c_void_p(d_out_ptr)))
     def level_1_data_device(self, d_out_ptr: int): self._ck(self._lib.bb_level1_device(self._h, C.c_void_p(d_out_ptr)))
 

@@ -168,8 +168,10 @@ SmemLayout make_layout(const bb_handle* h, bool with_obs, bool with_instr, bool 
     l.off_perm = off;
     // perm + jarr (u16 each) + slack for 8-byte jarr stores; the on-chip queue is shuffled in place and needs no perm.
     // Markets with in-kernel agents: every book derives the permutation of the WHOLE market's queue (k_sim<.., MKT>).
-    // market_rows (k_apply<MODE_ENV_MKT>): every book shuffles the whole market's queue, u16 [assets * max_queue]
-    if (market) off += 4u * align_up(h->assets * h->cfg.max_queue, 8) + 16u;
+    // market_rows (k_apply<MODE_ENV_MKT>): every book shuffles the whole market's queue, u16 [assets * max_queue].
+    // Both (k_sim<.., MKT, EXT>, agents plus device rows): behind jarr, a bitmask over the market's queued rows and its
+    // per-word prefix counts, u32 [2][ceil(assets * max_queue / 32)], padded so that what follows stays 16-byte aligned
+    if (market) off += 4u * align_up(h->assets * h->cfg.max_queue, 8) + 16u + (market_rows ? align_up(8u * ((h->assets * h->cfg.max_queue + 31u) / 32u), 16) : 0u);
     else if (market_rows) off += align_up(2u * h->assets * h->cfg.max_queue + 16u, 16);
     else off += align_up((with_queue ? 2u : 4u) * h->cfg.max_queue + 16u, 16);
     l.off_obs = off;
@@ -1126,7 +1128,7 @@ int bb_set_agents_market(bb_handle* h, const bb_agent_group* groups, const uint3
 }
 
 namespace {
-struct ExtRows {  // bb_run_agents_with_rows: the caller's device-resident rows for the launch's first step
+struct ExtRows {  // bb_run_agents_with_rows(_market): the caller's device-resident rows for the launch's first step
     const bb_instr* d_instrs;
     const u64* d_offsets;
     u64* d_out_ids;
@@ -1143,6 +1145,16 @@ int bb_run_agents_with_rows(bb_handle* h, uint64_t seed, const bb_instr* d_instr
     if (!d_env_offsets || (n_rows && !d_instrs)) return fail(h, BB_EINVAL, "null argument");
     if (h->assets > 1) return fail(h, BB_EINVAL, "bb_run_agents_with_rows drives single-asset envs");
     const ExtRows ext{d_instrs, d_env_offsets, d_out_ids, d_obs_out};
+    return run_agents_impl(h, seed, 1, &ext);
+}
+
+int bb_run_agents_with_rows_market(bb_handle* h, uint64_t seed, const bb_instr* d_instrs, const uint64_t* d_market_offsets,
+                                   uint64_t n_rows, uint64_t* d_out_ids, uint32_t* d_obs_out) {
+    CHECK_H(h);
+    if (!d_market_offsets || (n_rows && !d_instrs)) return fail(h, BB_EINVAL, "null argument");
+    if (h->assets < 2) return fail(h, BB_EINVAL, "bb_run_agents_with_rows_market drives multi-asset markets (single-asset envs: use bb_run_agents_with_rows)");
+    if (h->group_asset.empty()) return fail(h, BB_EINVAL, "bb_set_agents_market has not been called");
+    const ExtRows ext{d_instrs, d_market_offsets, d_out_ids, d_obs_out};
     return run_agents_impl(h, seed, 1, &ext);
 }
 
@@ -1172,8 +1184,10 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
         h->recorded_host = *(u32*)h->h_offsets;
     }
     if ((u64)h->recorded_host + n_steps > h->max_steps_padded) return fail(h, BB_ECAP, "max_steps exceeded");
+    // agents plus market rows: the market variants' layout with the row mask behind the permutation (only that variant has it)
+    const SmemLayout lay = mkt && ext ? make_layout(h, true, false, h->eng >= ENG_DENSE, true, true) : h->lay_sim;
     KParams p;
-    fill_params(h, h->lay_sim, p);
+    fill_params(h, lay, p);
     p.n_steps = n_steps;
     p.n_groups = (u32)h->groups.size();
     p.agents_per_env = h->agents_per_env;
@@ -1199,13 +1213,14 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
     // does a RandomAgents group that can draw off its book's tick: only those variants check the queued prices
     const bool mom = h->mom_groups != 0 || ext != nullptr || h->rand_tick_mask != 0;
     // markets: the A books of a market are A consecutive warps of one CTA (a CTA holds as many whole markets as fit in 4 warps)
-    const u32 wpb = mkt ? (WPB / h->assets) * h->assets : wpb_for(h->lay_sim.warp_bytes);
-    const size_t sim_smem = (size_t)h->lay_sim.warp_bytes * wpb;
+    const u32 wpb = mkt ? (WPB / h->assets) * h->assets : wpb_for(lay.warp_bytes);
+    const size_t sim_smem = (size_t)lay.warp_bytes * wpb;
 #define SIM_CASE(E, M)                                                                                     \
     if (h->eng == E && mom == M) {                                                                         \
-        if (mkt) { if ((rc = grid_for(h, k_sim<E, M, true>, h->lay_sim, h->cfg.n_envs, &grid, wpb))) return rc; } \
-        else if (ext) { if ((rc = grid_for(h, k_sim<E, true, false, true>, h->lay_sim, h->cfg.n_envs, &grid, wpb))) return rc; } \
-        else if ((rc = grid_for(h, k_sim<E, M, false>, h->lay_sim, h->cfg.n_envs, &grid, wpb))) return rc;  \
+        if (mkt && ext) { if ((rc = grid_for(h, k_sim<E, true, true, true>, lay, h->cfg.n_envs, &grid, wpb))) return rc; } \
+        else if (mkt) { if ((rc = grid_for(h, k_sim<E, M, true>, lay, h->cfg.n_envs, &grid, wpb))) return rc; } \
+        else if (ext) { if ((rc = grid_for(h, k_sim<E, true, false, true>, lay, h->cfg.n_envs, &grid, wpb))) return rc; } \
+        else if ((rc = grid_for(h, k_sim<E, M, false>, lay, h->cfg.n_envs, &grid, wpb))) return rc;  \
     }
     SIM_CASE(ENG_FAST, false) SIM_CASE(ENG_FAST, true) SIM_CASE(ENG_PAGED, false) SIM_CASE(ENG_PAGED, true)
     SIM_CASE(ENG_DENSE, false) SIM_CASE(ENG_DENSE, true) SIM_CASE(ENG_DENSE_L, false) SIM_CASE(ENG_DENSE_L, true)
@@ -1220,7 +1235,8 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
     p.scratch = h->scratch;
 #define SIM_LAUNCH(E, M)                                                                       \
     if (h->eng == E && mom == M) {                                                             \
-        if (mkt) k_sim<E, M, true><<<grid, wpb * 32, sim_smem, h->stream>>>(p);                \
+        if (mkt && ext) k_sim<E, true, true, true><<<grid, wpb * 32, sim_smem, h->stream>>>(p); \
+        else if (mkt) k_sim<E, M, true><<<grid, wpb * 32, sim_smem, h->stream>>>(p);           \
         else if (ext) k_sim<E, true, false, true><<<grid, wpb * 32, sim_smem, h->stream>>>(p); \
         else k_sim<E, M, false><<<grid, wpb * 32, sim_smem, h->stream>>>(p);                   \
     }

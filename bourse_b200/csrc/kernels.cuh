@@ -718,13 +718,18 @@ __device__ __forceinline__ void market_bar_sync(u32 id, u32 n_threads) {
 // queue executing at start + i on its asset's book.  The warps exchange their per-group instruction counts through
 // shared memory (one named barrier per step), each then derives the same market-wide permutation from the market's
 // Philox key and pulls out its own events together with their positions in it.
-// EXT (bb_run_agents_with_rows; always with MOM, never with MKT): after the built-in agents' updates the caller's own
-// rows for the env — already in device memory, the action block of an RL-style loop — are submitted in row order, exactly
-// as `agents.update(env); env.place_order(..) / env.cancel_order(..); env.step()` would: NEW rows take the next ids, rows
+// EXT (bb_run_agents_with_rows; always with MOM): after the built-in agents' updates the caller's own rows for the env —
+// already in device memory, the action block of an RL-style loop — are submitted in row order, exactly as
+// `agents.update(env); env.place_order(..) / env.cancel_order(..); env.step()` would: NEW rows take the next ids, rows
 // that queue nothing are skipped, and everything takes part in the step's one shuffle.
+// MKT + EXT (bb_run_agents_with_rows_market): the rows are the market's slice, bb_instr::aux the row's asset.  Every book
+// walks the whole slice (as k_apply<MODE_ENV_MKT> does), so every warp knows the market's queued-row count and which of
+// those rows are its own: the queued rows follow all groups' instructions in the market's queue, and each book appends
+// its own after its agents' events.  A per-warp bitmask over the market's queued rows (with per-word prefix counts) maps a
+// shuffled position back to the book's own list; it sits behind jarr, in a layout only this variant uses.
 template <int ENG, bool MOM, bool MKT = false, bool EXT = false>
 __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __grid_constant__ KParams p) {
-    static_assert(!EXT || (MOM && !MKT), "external rows ride on the unhinted (MOM) single-asset variants");
+    static_assert(!EXT || MOM, "external rows ride on the unhinted (MOM) variants");
     typedef GeoT<ENG> G;
     extern __shared__ __align__(128) unsigned char smem[];
     const u32 lane = keep32(threadIdx.x & 31u), warp = threadIdx.x >> 5, wpb = blockDim.x >> 5;
@@ -737,6 +742,9 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
     const u32 mk_a = MKT ? warp % p.assets : 0u;                           // the asset this warp's book is
     const u32 mk_sb = MKT ? sb - mk_a * p.warp_smem_bytes + p.off_mkt : 0u;  // u32 [2][MAX_GROUPS] in the market's first warp
     const u32 mk_bar = MKT ? 1u + warp / p.assets : 0u;
+    // MKT + EXT: u32 [mk_words] mask of this book's rows among the market's queued rows, then u32 [mk_words] prefix counts
+    const u32 mk_words = MKT && EXT ? (p.assets * p.max_queue + 31u) >> 5 : 0u;
+    const u32 mk_rm = MKT && EXT ? perm + 4u * ((p.assets * p.max_queue + 7u) & ~7u) + 16u : 0u;
     u32 mk_phase = 0;
     // the step's transaction queue: L2-resident global scratch, or (dense engine) shared memory so that the event
     // loop fetches each instruction with one broadcast ld.shared.v4 instead of a gather + four shuffles
@@ -833,7 +841,8 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                 slot_base += ag.n_agents;
                 if (mine) chip_base += ag.n_agents;
             }
-            if constexpr (EXT) {
+            u32 mk_nr = 0;  // MKT + EXT: the market's queued rows (every book of the market counts the same)
+            if constexpr (EXT && !MKT) {
                 const u64 off = p.offsets[env];
                 const u32 m = s == 0 ? (u32)(p.offsets[env + 1] - off) : 0u;  // the rows belong to the launch's first step
                 const bb_instr* ins = p.instrs + off;
@@ -874,6 +883,74 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                 if (__reduce_max_sync(BB_FULL, max_cancel) > e.next_id) b.err |= ERR_BAD_ID;
                 __syncwarp();
             }
+            if constexpr (EXT && MKT) {
+                // MarketEnv::place_order / cancel_order (market_env.rs:163-219) for the market's rows in row order: every
+                // book walks the whole slice; NEW rows take the next ids of their asset's book, rows naming no asset of the
+                // market queue nothing and flag book 0, each row's id is written by its asset's book (book 0: asset-less rows)
+                const u64 off = p.offsets[env / p.assets];
+                const u32 m = s == 0 ? (u32)(p.offsets[env / p.assets + 1] - off) : 0u;
+                const bb_instr* ins = p.instrs + off;
+                const u32 book0 = env - mk_a;
+                const u32 cap = p.assets * p.max_queue;  // queued rows beyond it drop the market's step (below)
+                const u32 nw = min((m + 31u) >> 5, mk_words);  // mask words the slice can touch
+                for (u32 w = lane; w < nw; w += 32) sts(mk_rm + 4u * w, 0u);
+                __syncwarp();
+                u32 max_cancel = 0;  // 1 + largest id a cancel row of this book names
+                for (u32 j0 = 0; j0 < m; j0 += 32) {
+                    const u32 j = j0 + lane;
+                    u32 of = 0, price = 0, vol = 0, trader = 0, oid = 0, asset = 0;
+                    if (j < m) {
+                        const uint4 x = reinterpret_cast<const uint4*>(ins + j)[0], y = reinterpret_cast<const uint4*>(ins + j)[1];
+                        of = x.z; oid = x.w; price = y.x; vol = y.y; trader = y.z; asset = y.w;
+                    }
+                    const u32 op = of & BB_OP_MASK;
+                    const bool bid = (of & BB_F_BID) != 0u;
+                    const bool in_mkt = j < m && asset < p.assets;
+                    // create_order's tick check against the row's own asset (orderbook.rs:367-383); the in-kernel queue
+                    // carries NEW and CANCEL only, so a MODIFY row or a trader id beyond 19 bits is dropped and flagged
+                    const bool bad_tick = in_mkt && op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % __ldg(g.ticks + book0 + asset) != 0u);
+                    const bool bad_op = in_mkt && (op == BB_OP_MODIFY || (op == BB_OP_NEW && trader >= (1u << 19)));
+                    const bool is_new = in_mkt && op == BB_OP_NEW && !bad_tick && !bad_op;
+                    const bool is_cancel = in_mkt && op == BB_OP_CANCEL;
+                    const bool queued = is_new || is_cancel, mine = queued && asset == mk_a;
+                    const u32 below = (1u << lane) - 1u;
+                    const u32 nm = __ballot_sync(BB_FULL, is_new && asset == mk_a), qm = __ballot_sync(BB_FULL, queued);
+                    const u32 om = __ballot_sync(BB_FULL, mine);
+                    const u32 id = e.next_id + __popc(nm & below), pos = e.n + __popc(om & below);
+                    const u32 xq = mk_nr + __popc(qm & below);  // the row's index among the market's queued rows
+                    if (of & BB_F_MARKET) price = bid ? 0xFFFFFFFFu : 0u;  // types.rs:160-172, 213-225
+                    if (p.out_ids && (in_mkt ? asset == mk_a : (j < m && mk_a == 0u)))
+                        p.out_ids[off + j] = is_new ? (u64)id : ~0ULL;
+                    if (mine) {
+                        if (pos < p.max_queue) {
+                            const uint4 ev = make_uint4(is_new ? (1u | (bid ? 2u : 0u) | (trader << 13)) : 0u, is_new ? id : oid, price, vol);
+                            if constexpr (G::DENSE) sts128(qs + 16u * pos, ev);
+                            else q[pos] = ev;
+                        }
+                        if (xq < cap) asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(mk_rm + 4u * (xq >> 5)), "r"(1u << (xq & 31u)) : "memory");
+                    }
+                    if (is_cancel && asset == mk_a) max_cancel = max(max_cancel, oid == 0xFFFFFFFFu ? oid : oid + 1u);
+                    if (__any_sync(BB_FULL, bad_tick && asset == mk_a)) b.err |= ERR_PRICE;
+                    if (__any_sync(BB_FULL, bad_op && asset == mk_a)) b.err |= ERR_ROW_OP;
+                    if (__any_sync(BB_FULL, j < m && asset >= p.assets) && mk_a == 0u) b.err |= ERR_ROW_OP;
+                    e.next_id += __popc(nm);
+                    e.n += __popc(om);
+                    mk_nr += __popc(qm);
+                }
+                if (__reduce_max_sync(BB_FULL, max_cancel) > e.next_id) b.err |= ERR_BAD_ID;
+                __syncwarp();
+                // prefix counts: own queued rows in the words before each mask word
+                u32 run = 0;
+                for (u32 w0 = 0; w0 < nw; w0 += 32) {
+                    const u32 w = w0 + lane;
+                    u32 tot;
+                    const u32 c = w < nw ? __popc(lds(mk_rm + 4u * w)) : 0u;
+                    const u32 ex = warp_excl_scan(c, lane, &tot);
+                    if (w < nw) sts(mk_rm + 4u * (mk_words + w), run + ex);
+                    run += tot;
+                }
+                __syncwarp();
+            }
             if (e.n > p.max_queue) b.err |= ERR_CAP_QUEUE;
             u32 n = min(e.n, p.max_queue);
             // a RandomAgents group in rand_tick_mask can draw off its book's tick: the host runs such a population on the MOM
@@ -904,7 +981,7 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                 if (n > p.step_size || (start <= b.max_key_time && (b.flags & (FL_HAS_ASK | FL_HAS_BID)))) b.err |= ERR_TIME_ORDER;
             }
             // markets: exchange the per-group counts; `nq` is the length of the queue that gets shuffled
-            u32 nq = n, mk_off = 0, mk_loc = 0, mk_all = 0;
+            u32 nq = n, mk_off = 0, mk_loc = 0, mk_all = 0, mk_ag = 0, mk_ag_mine = 0;
             if constexpr (MKT) {
                 const u32 cb = mk_sb + 4u * MAX_GROUPS * (mk_phase & 1u);  // double-buffered: one barrier per step is enough
                 mk_phase += 1;
@@ -916,6 +993,11 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                 mk_off = warp_excl_scan(mk_all, lane, &total);            // first queue position of each group
                 mk_loc = warp_excl_scan(own ? mk_all : 0u, lane, &total_mine);  // ... and its first entry in this book's list
                 nq = total;
+                if constexpr (EXT) {  // the queued rows follow every group's instructions; this book's after its agents'
+                    mk_ag = total;
+                    mk_ag_mine = total_mine;
+                    nq = total + mk_nr;
+                }
                 if (nq > p.assets * p.max_queue) {  // some book overflowed its queue (flagged there): drop the step everywhere
                     b.err |= ERR_CAP_QUEUE;
                     nq = 0;
@@ -974,6 +1056,16 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                         if (gq - o < c && p.group_asset[k] == mk_a) {
                             is_mine = true;
                             li = lo + (gq - o);
+                        }
+                    }
+                    if constexpr (EXT) {
+                        const u32 x = gq - mk_ag;  // index among the market's queued rows
+                        if (gq < nq && gq >= mk_ag) {
+                            const u32 wd = lds(mk_rm + 4u * (x >> 5));
+                            if ((wd >> (x & 31u)) & 1u) {
+                                is_mine = true;
+                                li = mk_ag_mine + lds(mk_rm + 4u * (mk_words + (x >> 5))) + __popc(wd & ((1u << (x & 31u)) - 1u));
+                            }
                         }
                     }
                     const u32 m = __ballot_sync(BB_FULL, is_mine);

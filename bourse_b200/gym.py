@@ -301,23 +301,48 @@ class MarketVectorEnv(_DeviceLoop):
     off-tick limit price creates nothing and flags its asset's book (`check_errors` raises).  `obs[m, a]` is asset a's
     end-of-step record.  A step is one kernel launch with no host synchronisation, so it can be captured into a CUDA graph;
     the history is a scratch ring as in `VectorEnv`.  `tick_sizes` has one tick per asset, at least two assets (a
-    one-asset market is an Env: use `VectorEnv`).  Use this class for an RL-style loop over many markets; use
-    `market.MarketEnv` (`place_order` / `submit` + `step` on the host) for scripted, order-by-order use, and its
-    `run_agents` for markets of built-in agents."""
+    one-asset market is an Env: use `VectorEnv`).
+
+    With `agents` (the `market.RandomMarketAgents` / `MomentumMarketAgent` / `NoiseMarketAgent` objects that
+    `market.MarketEnv.set_agents` takes) every market is populated: a step is `agents.update(env)`, the rows, then
+    `MarketEnv::step` (bb_run_agents_with_rows_market), in one launch that refuses CUDA-graph capture.
+
+    Which class: this one for an RL-style loop over many markets, alone (no `agents`) or against built-in agents in the
+    same shuffled queue (`agents=`); `market.MarketEnv` (`place_order` / `submit` + `step` on the host) for scripted,
+    order-by-order use, and its `run_agents` for markets of built-in agents with no learner."""
 
     _what = "book"
 
     def __init__(self, n_markets: int, rows_per_market: int, seed: int, start_time: int, tick_sizes: typing.Sequence[int],
-                 step_size: int, trading: bool = True, *, level_1: bool = False, **kw):
+                 step_size: int, trading: bool = True, *, level_1: bool = False, agents=None, agent_seed: int = 0, **kw):
+        """`agents`: optional background population, a list of `market.RandomMarketAgents` / `MomentumMarketAgent` /
+        `NoiseMarketAgent`.  With it every `step` is `{ agents.update(env); the action rows; MarketEnv::step }` for every
+        market in one launch: the rows follow all groups' instructions in the market's one shuffled queue (Philox key
+        `agent_seed`), and each row's id in its asset's book comes after the ids the agents took.  Action rows may then be
+        NEW, CANCEL or no-op (MODIFY is refused).  At most 4 assets: a market's books are the warps of one CTA."""
         ticks = [int(t) for t in tick_sizes]
         if len(ticks) < 2:
             raise ValueError("MarketVectorEnv needs two or more assets; a one-asset market is an Env: use VectorEnv")
         if min(ticks) <= 0:
             raise ValueError("tick sizes must be > 0")
         A = len(ticks)
-        kw.setdefault("max_queue", max(-(-rows_per_market // A), 16))   # a market's queue holds assets * max_queue rows
+        if agents:
+            if A > 4:
+                raise ValueError("in-kernel market agents support at most 4 assets per market")
+            per_asset = [0] * A
+            for a in agents:
+                if not 0 <= a.asset < A:
+                    raise ValueError("agent group asset index out of range")
+                per_asset[a.asset] += int(a.group["n_agents"])
+            # each book's queue holds its agents' instructions and, at worst, every row of the market
+            kw.setdefault("max_queue", max(2 * max(per_asset) + rows_per_market, 16))
+        else:
+            kw.setdefault("max_queue", max(-(-rows_per_market // A), 16))   # a market's queue holds assets * max_queue rows
         if rows_per_market > A * kw["max_queue"]:
             raise ValueError("rows_per_market exceeds assets * max_queue")
+        if A * kw["max_queue"] > 65535:
+            raise ValueError("assets * max_queue must stay below 65536")
+        self._agents, self._agent_seed = agents, agent_seed
         self._n_steps = 0
         self.n_markets, self.rows, self.n_assets, self.tick_sizes = n_markets, rows_per_market, A, ticks
         self.obs_words = abi.OBS_L1 if level_1 else abi.OBS_L2
@@ -328,12 +353,19 @@ class MarketVectorEnv(_DeviceLoop):
             if any(t != granule for t in ticks):
                 self.env.set_tick_sizes(ticks)
             self._buffers((n_markets, A, self.obs_words), (n_markets, rows_per_market))
+            if agents:
+                self.env.set_agents([a.group for a in agents], assets=[a.asset for a in agents])
         except Exception:
             self.env.close()
             raise
 
     def step(self, actions) -> typing.Tuple[DeviceArray, DeviceArray]:
         ptr = self._action_ptr(actions)
-        # one launch: ids, the market-wide shuffle, MarketEnv::step and the observation records written straight into self.obs
-        self.env.step_device_market(ptr, self._offsets.ptr, self.n_markets * self.rows, self.ids.ptr, self.obs.ptr)
+        # one launch: (background agents,) ids, the market-wide shuffle, MarketEnv::step and the observation records written
+        # straight into self.obs
+        if self._agents:
+            self.env.run_agents_with_rows_market(self._agent_seed, ptr, self._offsets.ptr, self.n_markets * self.rows, self.ids.ptr,
+                                                 self.obs.ptr)
+        else:
+            self.env.step_device_market(ptr, self._offsets.ptr, self.n_markets * self.rows, self.ids.ptr, self.obs.ptr)
         return self.obs, self.ids

@@ -47,7 +47,7 @@ typedef enum {
 #define BB_ERR_CAP_LIVE   0x80u  /* MomentumAgent live-order list / dense engine's resting-order slots overflow */
 #define BB_ERR_TIME_ORDER 0x100u /* dense engine: a resting order arrived out of time order at its price level */
 #define BB_ERR_PRICE 0x200u      /* bb_step_device: a NEW row's limit price was not a multiple of its env's tick (row dropped) */
-#define BB_ERR_ROW_OP 0x400u     /* bb_run_agents_with_rows: a MODIFY row or a trader id >= 2^19 (row dropped) */
+#define BB_ERR_ROW_OP 0x400u     /* bb_run_agents_with_rows(_market): a MODIFY row or a trader id >= 2^19 (row dropped); markets: a row's aux names no asset */
 #define BB_ERR_LOCKED 0x800u     /* deep engine: both sides would rest at one price level (trading disabled) */
 
 #define BB_OBS_L1 9u   /* StepEnvNumpy.level_1_data layout, rust/src/step_sim_numpy.rs:300-318 */
@@ -266,6 +266,31 @@ int bb_step_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_env
  * n_rows sizes the internal id buffer when d_out_ids is NULL. */
 int bb_step_device_market(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_market_offsets, uint64_t n_rows,
                           uint64_t* d_out_ids, uint32_t* d_obs_out);
+/* The same market loop with the built-in market agents (bb_set_agents_market) trading in every market: ONE step of
+ * market_sim_runner (crates/step_sim/src/runner.rs:107-131) with the caller's calls between the agents' update and the
+ * step — `agents.update(&mut env, rng); env.place_order(..) / env.cancel_order(..) for each row; env.step(rng)`
+ * (market_env.rs:108-121, 163-219).  For every market m, in one launch:
+ *   1. all agent groups update in array order, each on its own asset's book, with bb_run_agents' Philox key (seed; global
+ *      market id (env_id_base + book) / assets, step, agent slot counted over all groups);
+ *   2. the market's rows (d_market_offsets and bb_instr::aux as for bb_step_device_market) are submitted in row order:
+ *      BB_OP_NEW with an on-tick limit price or BB_F_MARKET creates the next id of its asset's book (after the ids the
+ *      agents took) in d_out_ids[row] (may be NULL); BB_OP_CANCEL targets (aux, order_id); no-ops queue nothing; every
+ *      row that creates nothing gets BB_NO_ID;
+ *   3. the market's queue — every group's instructions in array order, then the queued rows in row order — is shuffled
+ *      as a whole with bb_run_agents' Philox-keyed Fisher-Yates, event i runs at start + i on its asset's book, and every
+ *      book advances by step_size and appends one record; d_obs_out ([n_envs][obs_words], may be NULL) receives it.
+ * Row errors are sticky per-book bits, and no row fails silently: a limit NEW off its asset's tick is dropped without
+ * taking an id (BB_ERR_PRICE on that asset's book); a row with aux >= assets queues nothing (BB_ERR_ROW_OP on book 0 of
+ * the market); a MODIFY row, or a NEW with a trader id >= 2^19, is dropped (the in-kernel queue carries NEW and CANCEL
+ * only; BB_ERR_ROW_OP on the row's book); a cancel of an id its book has not issued by the end of submission flags
+ * BB_ERR_BAD_ID on that book.  Queue capacity: a book whose own events (its groups' instructions plus its rows) exceed
+ * max_queue is flagged BB_ERR_CAP_QUEUE and its results are unspecified; a market whose whole queue exceeds
+ * assets * max_queue flags BB_ERR_CAP_QUEUE on every book and processes no event that step (ids are still taken and the
+ * books still step).  Refused with BB_EINVAL on a single-asset handle (use bb_run_agents_with_rows), before
+ * bb_set_agents_market, on the deep engine, while host-queued instructions are pending, for NULL arguments, and inside a
+ * stream capture (as every agent launch).  Asynchronous on the handle's stream. */
+int bb_run_agents_with_rows_market(bb_handle* h, uint64_t seed, const bb_instr* d_instrs, const uint64_t* d_market_offsets,
+                                   uint64_t n_rows, uint64_t* d_out_ids, uint32_t* d_obs_out);
 /* bb_level2 / bb_level1 into DEVICE memory: d_out[n_envs][45] / d_out[n_envs][9].  Asynchronous. */
 int bb_level2_device(bb_handle* h, uint32_t* d_out);
 int bb_level1_device(bb_handle* h, uint32_t* d_out);

@@ -7,7 +7,13 @@ book m * 4 + a receiving exactly the rows env m * 4 + a gets in the VectorEnv ru
 over --steps warmed steps, in windows of 100 steps that each start from reset books (nothing crosses PCIe inside a window); the host path with a host clock around steps that end in
 a synchronisation.  Prints the card and its power limit, then one JSON line.
 
+--bg-agents times the same two device loops with background agents instead: the C3 population (50 + 50 RandomAgents) on
+every book — as RandomMarketAgents on every asset of every market (bb_run_agents_with_rows_market), and as
+VectorEnv(agents=c3_groups()) on the 8192 single-asset books (bb_run_agents_with_rows) — with the rows repriced into the
+agents' range as `bench.py --workload gym --bg-agents` does.
+
     python scripts/bench_market_vector.py --steps 1000 --warmup 20
+    python scripts/bench_market_vector.py --bg-agents --steps 1000 --warmup 20
 """
 from __future__ import annotations
 
@@ -24,13 +30,16 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 
 from bench import gym_action_blocks  # noqa: E402
-from bourse_b200 import abi, gym, market  # noqa: E402
+from bourse_b200 import abi, gym, market, workloads  # noqa: E402
 
 N_MARKETS, ASSETS, ROWS_PER_BOOK = 2048, 4, 2
 N_BOOKS, ROWS = N_MARKETS * ASSETS, ASSETS * ROWS_PER_BOOK
 ENGINES = {"fast": dict(), "dense": dict(price_window=(960, 1056), live_cap=254)}
 KW = dict(max_orders=8192, max_trades=16384, max_steps=256)
 WINDOW = 100
+# background agents: the C3 population's prices are 20..178 (bench.py --workload gym --bg-agents)
+BG_ENGINES = {"fast": dict(), "dense": dict(price_window=(20, 180), live_cap=254)}
+BG_KW = dict(max_orders=8192, max_trades=16384, max_steps=256, max_queue=128)
 
 
 def card():
@@ -89,12 +98,15 @@ def main():
     ap.add_argument("--steps", type=int, default=1000)
     ap.add_argument("--warmup", type=int, default=20, help="untimed steps after each reset")
     ap.add_argument("--blocks", type=int, default=64, help="distinct action blocks, cycled")
+    ap.add_argument("--bg-agents", action="store_true", help="the C3 population trades in every book (see the module docstring)")
     args = ap.parse_args()
     import torch
 
     name, power = card()
     print(f"card: {name}, power limit: {power}", flush=True)
     blocks = gym_action_blocks(args.blocks, N_BOOKS, ROWS_PER_BOOK, seed=5)
+    if args.bg_agents:   # limit prices into the agents' range, as bench.py run_gym does
+        blocks["price"] = np.where((blocks["op_flags"] & abi.F_MARKET) != 0, blocks["price"], 2 * (40 + blocks["price"] % 21))
     mblocks = market_blocks(blocks)
     res = {"card": name, "power_limit": power, "markets": N_MARKETS, "assets": ASSETS, "rows_per_market": ROWS,
            "steps": args.steps, "warmup": args.warmup, "us_per_step": {}, "errors": {}}
@@ -104,6 +116,23 @@ def main():
 
     d_env, d_mkt = as_device(blocks), as_device(mblocks)
     torch.cuda.synchronize()
+    if args.bg_agents:
+        c3 = workloads.c3_groups()
+        res["agents"] = "C3 (50 + 50 RandomAgents) on every book"
+        agents = []
+        for a in range(ASSETS):
+            for g in c3:
+                agents.append(market.RandomMarketAgents(a, int(g["n_agents"]), (int(g["tick_lo"]), int(g["tick_hi"])),
+                                                        (int(g["vol_lo"]), int(g["vol_hi"])), int(g["tick_size"]), float(g["rate"])))
+        for eng, ekw in BG_ENGINES.items():
+            v = gym.MarketVectorEnv(N_MARKETS, ROWS, 0, 0, [1] * ASSETS, 1_000_000, agents=agents, agent_seed=5, **BG_KW, **ekw)
+            res["us_per_step"][f"market_vector_bg_{eng}"], res["errors"][f"market_vector_bg_{eng}"] = time_device(v, d_mkt, args.steps, args.warmup)
+            v.close()
+            ve = gym.VectorEnv(N_BOOKS, ROWS_PER_BOOK, 0, 0, 1, 1_000_000, agents=c3, agent_seed=5, **BG_KW, **ekw)
+            res["us_per_step"][f"vector_env_bg_{eng}"], res["errors"][f"vector_env_bg_{eng}"] = time_device(ve, d_env, args.steps, args.warmup)
+            ve.close()
+        print(json.dumps(res), flush=True)
+        return
     for eng, ekw in ENGINES.items():
         v = gym.MarketVectorEnv(N_MARKETS, ROWS, 0, 0, [1] * ASSETS, 1000, **KW, **ekw)
         res["us_per_step"][f"market_vector_{eng}"], res["errors"][f"market_vector_{eng}"] = time_device(v, d_mkt, args.steps, args.warmup)
