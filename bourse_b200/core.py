@@ -244,6 +244,24 @@ class BatchedEnv:
                                                           C.c_void_p(d_out_ids_ptr) if d_out_ids_ptr else None,
                                                           C.c_void_p(d_obs_ptr) if d_obs_ptr else None))
 
+    def orders_device(self, d_ids_ptr: int, d_assets_ptr: int, n_per_unit: int, side_is_bid: int = 0, status: int = 0,
+                      arr_time: int = 0, end_time: int = 0, vol: int = 0, start_vol: int = 0, price: int = 0, trader: int = 0):
+        """Order records of a [units, n_per_unit] block of device-resident ids (bb_orders_device); asynchronous.  A unit is an
+        env, or a market on a multi-asset handle, where `d_assets_ptr` ([units, n_per_unit] u32) names each query's asset
+        (0 on a single-asset handle).  The keyword arguments are device pointers of the [units, n_per_unit] output columns;
+        0 skips a column."""
+        p = C.c_void_p
+        self._ck(self._lib.bb_orders_device(self._h, p(d_ids_ptr), p(d_assets_ptr), n_per_unit, p(side_is_bid), p(status), p(arr_time),
+                                            p(end_time), p(vol), p(start_vol), p(price), p(trader)))
+
+    def trades_device(self, d_cursor_ptr: int, cap: int, count: int = 0, t: int = 0, side_is_bid: int = 0, price: int = 0,
+                      vol: int = 0, active_id: int = 0, passive_id: int = 0):
+        """Each book's trades since `d_cursor_ptr[book]` (u32 [n_envs], advanced) into [n_envs, cap] device columns
+        (bb_trades_device); asynchronous.  `count` (u32 [n_envs]) receives the number of trades each book had to report."""
+        p = C.c_void_p
+        self._ck(self._lib.bb_trades_device(self._h, p(d_cursor_ptr), cap, p(count), p(t), p(side_is_bid), p(price), p(vol),
+                                            p(active_id), p(passive_id)))
+
     def level_2_data_device(self, d_out_ptr: int): self._ck(self._lib.bb_level2_device(self._h, C.c_void_p(d_out_ptr)))
     def level_1_data_device(self, d_out_ptr: int): self._ck(self._lib.bb_level1_device(self._h, C.c_void_p(d_out_ptr)))
 

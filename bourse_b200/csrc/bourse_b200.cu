@@ -1019,6 +1019,42 @@ int bb_level1_device(bb_handle* h, uint32_t* d_out) {
     return snapshot(h, 0, h->cfg.n_envs, d_out, nullptr, 9u);
 }
 
+int bb_orders_device(bb_handle* h, const uint64_t* d_ids, const uint32_t* d_assets, uint64_t n_per_unit, uint8_t* d_side_is_bid,
+                     uint8_t* d_status, uint64_t* d_arr_time, uint64_t* d_end_time, uint32_t* d_vol, uint32_t* d_start_vol,
+                     uint32_t* d_price, uint32_t* d_trader) {
+    CHECK_H(h);
+    if (!d_ids) return fail(h, BB_EINVAL, "null argument");
+    if (h->assets > 1 && !d_assets) return fail(h, BB_EINVAL, "bb_orders_device: d_assets is required on a multi-asset handle");
+    if (h->assets == 1 && d_assets) return fail(h, BB_EINVAL, "bb_orders_device: d_assets must be NULL on a single-asset handle");
+    for (auto& q : h->queue)
+        if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
+    const u64 units = h->cfg.n_envs / h->assets, max_queries = 256ull * 0x7FFFFFFFull;  // (one launch: grid.x < 2^31)
+    if (n_per_unit > max_queries / units) return fail(h, BB_EINVAL, "bb_orders_device: too many queries for one launch");
+    const u64 n_queries = units * n_per_unit;
+    if (n_queries == 0) return BB_OK;
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    k_orders_gather<<<(unsigned)((n_queries + 255) / 256), 256, 0, h->stream>>>(
+        h->blobs, h->blob_stride, h->ord, h->cfg.max_orders, d_ids, d_assets, h->assets, n_per_unit, n_queries, d_side_is_bid, d_status,
+        d_arr_time, d_end_time, d_vol, d_start_vol, d_price, d_trader);
+    CUDA_TRY(h, cudaGetLastError());
+    return BB_OK;
+}
+
+int bb_trades_device(bb_handle* h, uint32_t* d_cursor, uint32_t cap, uint32_t* d_count, uint64_t* d_t, uint8_t* d_side_is_bid,
+                     uint32_t* d_price, uint32_t* d_vol, uint64_t* d_active_id, uint64_t* d_passive_id) {
+    CHECK_H(h);
+    if (!d_cursor) return fail(h, BB_EINVAL, "null argument");
+    if (h->cfg.max_trades == 0) return fail(h, BB_EINVAL, "bb_trades_device: the trade log is disabled (max_trades == 0)");
+    for (auto& q : h->queue)
+        if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    k_trades_window<<<(h->cfg.n_envs + 7) / 8, 256, 0, h->stream>>>(h->blobs, h->blob_stride, h->tr, h->cfg.max_trades, h->cfg.n_envs,
+                                                                     d_cursor, cap, d_count, d_t, d_side_is_bid, d_price, d_vol,
+                                                                     d_active_id, d_passive_id);
+    CUDA_TRY(h, cudaGetLastError());
+    return BB_OK;
+}
+
 int bb_device_alloc(bb_handle* h, uint64_t bytes, void** d_ptr) {
     CHECK_H(h);
     if (!d_ptr) return fail(h, BB_EINVAL, "null argument");

@@ -8,6 +8,8 @@
 //   k_sim                 persistent { agents.update; env.step } x n_steps (runner.rs:46-69) with the
 //                         built-in RandomAgents / MomentumAgent generated in-kernel
 //   k_snapshot            live level-1 / level-2 / touch data of every book (orderbook.rs:287-324)
+//   k_orders_gather       order records by id for a batch of queries (bb_orders_device)
+//   k_trades_window       each book's trades since a caller-owned cursor (bb_trades_device)
 #pragma once
 #include "../../include/bourse_b200.h"
 #include "book.cuh"
@@ -1842,6 +1844,95 @@ __global__ void __launch_bounds__(128) k_snapshot_deep(const __grid_constant__ K
         level_at(0u, ask, &av, &ac);
         out8[(size_t)i * 8u + lane] = lane == 0 ? bid : lane == 1 ? ask : lane == 2 ? h->side_vol[1] : lane == 3 ? h->side_vol[0]
                                       : lane == 4 ? bv : lane == 5 ? av : lane == 6 ? bc : ac;
+    }
+}
+
+// bb_orders_device: the records of order ids named by a [units][n_per_unit] query block (get_orders()[id] / order_status(id),
+// rust/src/step_sim_numpy.rs), one thread per query.  Query q of unit u reads book u, or book u * assets + asset[q] on a
+// multi-asset handle.  The first 32-byte sector of a record (price, vol, links, key time, meta, start_vol) is always read;
+// the second (arr_time, end_time, trader) only when one of its columns is requested.  A BB_NO_ID query, an id without a
+// record (ERR_BAD_ID on its book) and an asset outside the market (ERR_ROW_OP on the market's book 0) write "no order":
+// BB_STATUS_NONE and zeros.  Record and header layouts are shared by every engine, so one instantiation serves them all.
+__global__ void __launch_bounds__(256) k_orders_gather(unsigned char* blobs, u64 blob_stride, const OrderRec* ord, u32 max_orders,
+                                                       const u64* ids, const u32* asset, u32 assets, u64 n_per_unit, u64 n_queries,
+                                                       uint8_t* side_is_bid, uint8_t* status, u64* arr_time, u64* end_time, u32* vol,
+                                                       u32* start_vol, u32* price, u32* trader) {
+    const u64 q = (u64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= n_queries) return;
+    const u64 unit = q / n_per_unit, id = __ldg(ids + q);
+    uint4 s0 = make_uint4(0u, 0u, 0u, 0u), s1 = s0, c0 = s0, c1 = s0;  // the record's two sectors, 16 bytes at a time
+    u32 st = BB_STATUS_NONE;
+    if (id != BB_NO_ID) {
+        u64 book = unit;
+        u32 bad = 0u;
+        if (asset) {
+            const u32 a = __ldg(asset + q);
+            book = unit * assets + (a < assets ? a : 0u);
+            if (a >= assets) bad = ERR_ROW_OP;
+        }
+        BookHdr* h = reinterpret_cast<BookHdr*>(blobs + book * blob_stride);
+        if (!bad && (id >= __ldg(&h->n_orders) || id >= max_orders)) bad = ERR_BAD_ID;
+        if (bad) {
+            atomicOr(&h->err, bad);
+        } else {
+            const uint4* r = reinterpret_cast<const uint4*>(ord + book * max_orders + id);
+            s0 = __ldg(r);
+            s1 = __ldg(r + 1);
+            if (arr_time || end_time || trader) {
+                c0 = __ldg(r + 2);
+                c1 = __ldg(r + 3);
+            }
+            st = s1.z & META_STATUS_MASK;
+        }
+    }
+    if (side_is_bid) side_is_bid[q] = (s1.z & META_BID) ? 1u : 0u;
+    if (status) status[q] = (uint8_t)st;
+    if (arr_time) arr_time[q] = ((u64)c0.y << 32) | c0.x;
+    if (end_time) end_time[q] = ((u64)c0.w << 32) | c0.z;
+    if (vol) vol[q] = s0.y;
+    if (start_vol) start_vol[q] = s1.w;
+    if (price) price[q] = s0.x;
+    if (trader) trader[q] = c1.x;
+}
+
+// bb_trades_device: per book, the trades logged since the caller's cursor (get_trades(), rust/src/types.rs:4-17), one warp
+// per book.  Lanes copy consecutive 32-byte records of the log into row `book` of the [n_books][cap] columns and pad the
+// rest of the row with (0, 0, 0, 0, BB_NO_ID, BB_NO_ID); lane 0 writes the count and the advanced cursor.  Nothing at or
+// beyond min(n_trades, max_trades) is read.
+__global__ void __launch_bounds__(256) k_trades_window(const unsigned char* blobs, u64 blob_stride, const TradeRec* tr, u32 max_trades,
+                                                       u32 n_books, u32* cursor, u32 cap, u32* count, u64* t, uint8_t* side_is_bid,
+                                                       u32* price, u32* vol, u64* active_id, u64* passive_id) {
+    const u32 lane = threadIdx.x & 31u, book = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (book >= n_books) return;
+    u32 c = 0u, logged = 0u;
+    if (lane == 0u) {  // (one lane reads the cursor it alone writes back)
+        c = cursor[book];
+        logged = min(__ldg(&reinterpret_cast<const BookHdr*>(blobs + (u64)book * blob_stride)->n_trades), max_trades);
+    }
+    c = __shfl_sync(BB_FULL, c, 0);
+    logged = __shfl_sync(BB_FULL, logged, 0);
+    const u32 avail = c < logged ? logged - c : 0u, n = min(avail, cap);
+    const uint4* src = reinterpret_cast<const uint4*>(tr + (u64)book * max_trades + c);
+    const u64 row = (u64)book * cap;
+    for (u32 i = lane; i < cap; i += 32u) {
+        uint4 a = make_uint4(0u, 0u, 0u, 0u), b = a;
+        u64 act = BB_NO_ID, pas = BB_NO_ID;
+        if (i < n) {
+            a = __ldg(src + 2u * i);      // t, price, vol
+            b = __ldg(src + 2u * i + 1u);  // active, passive, side_bid
+            act = b.x;
+            pas = b.y;
+        }
+        if (t) t[row + i] = ((u64)a.y << 32) | a.x;
+        if (side_is_bid) side_is_bid[row + i] = (uint8_t)b.z;
+        if (price) price[row + i] = a.z;
+        if (vol) vol[row + i] = a.w;
+        if (active_id) active_id[row + i] = act;
+        if (passive_id) passive_id[row + i] = pas;
+    }
+    if (lane == 0u) {
+        if (count) count[book] = avail;
+        if (n) cursor[book] = c + n;
     }
 }
 

@@ -11,6 +11,10 @@ Buffers are exchanged through DLPack (`__dlpack__` / `__dlpack_device__`: `torch
 speak, so this module needs none of them: both give zero-copy views, and a torch / cupy array (anything with `__dlpack__`
 or the CUDA array interface) can be passed to `step` directly.  numpy arrays are accepted too (copied host to device).
 
+What happened to the learner's orders is read on the device as well: `orders(...)` returns the records of a block of order
+ids (the reference's `get_orders()[id]` / `order_status(id)`) and `trades(cap)` the trades every book logged since the last
+call (`get_trades()`), as device arrays, one launch each (bb_orders_device / bb_trades_device).
+
 `MarketVectorEnv` is the same loop for multi-asset markets (`MarketEnv` place / cancel / modify then `step`, one block of
 rows per market, each row naming its asset).  Use `VectorEnv` for independent single-asset envs, `MarketVectorEnv` when
 assets share a market's shuffled queue, and `market.MarketEnv` for host-driven, order-by-order market use.
@@ -27,7 +31,7 @@ from . import abi
 from .core import BatchedEnv
 
 # ---- DLPack (dlpack.h, v0.8 ABI: DLManagedTensor in a PyCapsule named "dltensor"), pure ctypes ---------------------------
-KDL_CUDA, KDL_UINT = 2, 1
+KDL_CUDA, KDL_INT, KDL_UINT = 2, 0, 1
 
 
 class _DLDevice(C.Structure):
@@ -63,8 +67,9 @@ def _dl_deleter(mt_ptr):   # called by the consumer when it drops the tensor: re
     _LIVE_EXPORTS.pop(C.addressof(mt_ptr.contents), None)
 
 
-def _dlpack_import(x) -> typing.Tuple[int, int, typing.Any]:
-    """(device pointer, byte size, keep-alive object) of anything that exports DLPack; C-contiguous CUDA tensors only."""
+def _dlpack_import(x) -> typing.Tuple[int, int, typing.Any, typing.Tuple[int, ...], typing.Tuple[int, int]]:
+    """(device pointer, byte size, keep-alive object, shape, (DLPack type code, bits)) of anything that exports DLPack;
+    C-contiguous CUDA tensors only."""
     capsule = x.__dlpack__()
     if not _api.PyCapsule_IsValid(capsule, _DLTENSOR):
         raise ValueError("not a DLPack capsule")
@@ -81,7 +86,7 @@ def _dlpack_import(x) -> typing.Tuple[int, int, typing.Any]:
             expect *= shape[i]
     nbytes = int(np.prod(shape)) * (t.dtype.bits * t.dtype.lanes // 8)
     # the capsule is kept (un-renamed) together with its producer: its own destructor releases the tensor when we drop it
-    return int(t.data) + int(t.byte_offset), nbytes, (capsule, x)
+    return int(t.data) + int(t.byte_offset), nbytes, (capsule, x), tuple(shape), (int(t.dtype.code), int(t.dtype.bits))
 
 ACTION_DTYPE = abi.INSTR_DTYPE  # one row = one instruction: (t ignored, op_flags, order_id, price, vol, trader, aux)
 
@@ -138,7 +143,7 @@ def _device_ptr(x, nbytes: int) -> typing.Optional[int]:
     cai = getattr(x, "__cuda_array_interface__", None)
     if cai is None:
         if hasattr(x, "__dlpack__") and not isinstance(x, np.ndarray):   # DLPack-only producers
-            ptr, n, keep = _dlpack_import(x)
+            ptr, n, keep, _, _ = _dlpack_import(x)
             if n != nbytes:
                 raise ValueError(f"device array holds {n} bytes, expected {nbytes}")
             _device_ptr.keep = keep   # alive until the next call: the launch that reads it is already enqueued by then
@@ -179,8 +184,16 @@ def pack_actions(op, bid=None, vol=None, trader=None, price=None, order_id=None,
     return a
 
 
+# bb_orders_device / bb_trades_device output columns (PyOrder / PyTrade fields, rust/src/types.rs:4-31)
+ORDER_COLUMNS = (("side_is_bid", np.uint8), ("status", np.uint8), ("arr_time", np.uint64), ("end_time", np.uint64), ("vol", np.uint32),
+                 ("start_vol", np.uint32), ("price", np.uint32), ("trader", np.uint32))
+TRADE_COLUMNS = (("t", np.uint64), ("side_is_bid", np.uint8), ("price", np.uint32), ("vol", np.uint32), ("active_id", np.uint64),
+                 ("passive_id", np.uint64))
+
+
 class _DeviceLoop:
-    """What `VectorEnv` and `MarketVectorEnv` share: the handle, the device buffers, host-action staging and the history ring."""
+    """What `VectorEnv` and `MarketVectorEnv` share: the handle, the device buffers, host-action staging, the history ring and
+    the order / trade reads."""
 
     env: BatchedEnv
     obs: DeviceArray
@@ -193,10 +206,17 @@ class _DeviceLoop:
         self._actions = DeviceArray(self.env, rows_shape, ACTION_DTYPE)  # staging for host-side actions
         self._offsets = DeviceArray(self.env, (rows_shape[0] + 1,), np.uint64)
         self._offsets.copy_from_host(np.arange(rows_shape[0] + 1, dtype=np.uint64) * np.uint64(rows_shape[1]))
+        self._units, self._book_shape = rows_shape[0], tuple(obs_shape[:-1])
+        self._cursor = DeviceArray(self.env, (self.env.n_envs,), np.uint32)  # trades(): each book's next unread trade
+        self._cursor.copy_from_host(np.zeros(self.env.n_envs, np.uint32))
+        self._reads: dict = {}   # orders() / trades() outputs and query staging, by kind and size: allocated once, then reused
 
     def close(self):
-        for a in (self.obs, self.ids, self._actions, self._offsets):
+        for a in (self.obs, self.ids, self._actions, self._offsets, self._cursor):
             a.free()
+        for bufs in self._reads.values():
+            for a in ((bufs,) if isinstance(bufs, DeviceArray) else bufs.values()):
+                a.free()
         self.env.close()
 
     def _observe(self) -> DeviceArray:
@@ -206,7 +226,68 @@ class _DeviceLoop:
     def reset(self) -> DeviceArray:
         self._n_steps = 0
         self.env.reset()   # (the agent population survives a reset; its state is cleared with the books)
+        self._cursor.copy_from_host(np.zeros(self.env.n_envs, np.uint32))
         return self._observe()
+
+    def _buffer(self, key, shape, dtype) -> DeviceArray:
+        if key not in self._reads:
+            self._reads[key] = DeviceArray(self.env, shape, dtype)
+        return self._reads[key]
+
+    def _columns(self, key, shape, columns) -> dict:
+        if key not in self._reads:
+            self._reads[key] = {name: DeviceArray(self.env, shape, dt) for name, dt in columns}
+        return self._reads[key]
+
+    def _query_block(self, x, dtype, name) -> typing.Tuple[int, int]:
+        """(device address, k) of a [units, k] query block: the caller's device array (CUDA array interface or DLPack, any
+        integer type of `dtype`'s size), or a staging copy of a host array."""
+        dtype, units = np.dtype(dtype), self._units
+        cai = getattr(x, "__cuda_array_interface__", None)
+        if cai is not None:
+            shape, typ = tuple(cai["shape"]), np.dtype(cai["typestr"])
+            if len(shape) != 2 or shape[0] != units or typ.kind not in "iu" or typ.itemsize != dtype.itemsize:
+                raise ValueError(f"{name} must be a [{units}, k] array of {dtype.itemsize}-byte integers")
+            return _device_ptr(x, units * shape[1] * dtype.itemsize), int(shape[1])
+        if hasattr(x, "__dlpack__") and not isinstance(x, np.ndarray):
+            ptr, _, keep, shape, (code, bits) = _dlpack_import(x)
+            if len(shape) != 2 or shape[0] != units or code not in (KDL_INT, KDL_UINT) or bits != 8 * dtype.itemsize:
+                raise ValueError(f"{name} must be a [{units}, k] array of {dtype.itemsize}-byte integers")
+            _device_ptr.keep = keep   # alive until the next call: the launch that reads it is already enqueued by then
+            return ptr, int(shape[1])
+        a = np.ascontiguousarray(x, dtype=dtype)
+        if a.ndim != 2 or a.shape[0] != units:
+            raise ValueError(f"{name} must have shape [{units}, k]")
+        buf = self._buffer((name, a.shape[1]), a.shape, dtype)
+        buf.copy_from_host(a)
+        return buf.ptr, a.shape[1]
+
+    def _orders(self, ids, assets) -> typing.Dict[str, DeviceArray]:
+        ids_ptr, k = self._query_block(ids, np.uint64, "ids")
+        assets_ptr = 0
+        if assets is not None:
+            assets_ptr, ka = self._query_block(assets, np.uint32, "assets")
+            if ka != k:
+                raise ValueError("ids and assets must have the same shape")
+        out = self._columns(("orders", k), (self._units, k), ORDER_COLUMNS)
+        if k:
+            self.env.orders_device(ids_ptr, assets_ptr, k, **{name: a.ptr for name, a in out.items()})
+        return out
+
+    def trades(self, cap: int) -> typing.Tuple[typing.Dict[str, DeviceArray], DeviceArray]:
+        """The trades every book logged since the last call (bb_trades_device): `(columns, count)`.  `columns` are `DeviceArray`s
+        keyed `t, side_is_bid, price, vol, active_id, passive_id` (the PyTrade fields, ids as u64), shaped `[n_envs, cap]` (a
+        `MarketVectorEnv`: `[n_markets, assets, cap]`); a book's first `min(count, cap)` slots hold its new trades in log
+        order, the rest `active_id = passive_id = abi.NO_ID` and zeros.  `count` (`[n_envs]` / `[n_markets, assets]`) is the
+        number of trades each book had to report; it may exceed `cap`, and the ones that did not fit come with the next call.
+        The env keeps the read position of every book (zeroed by `reset()`).  Trades a full log (`max_trades`) could not
+        hold are not reported; `check_errors` raises for them.  One launch on the env's stream, ordered after the steps
+        before it, with no host synchronisation; the outputs are allocated on the first call for a given `cap` and
+        overwritten by the next call with that `cap`.  Make that first call before capturing one into a CUDA graph."""
+        cols = self._columns(("trades", cap), self._book_shape + (cap,), TRADE_COLUMNS)
+        count = self._buffer(("count", cap), self._book_shape, np.uint32)
+        self.env.trades_device(self._cursor.ptr, cap, count.ptr, **{name: a.ptr for name, a in cols.items()})
+        return cols, count
 
     def _action_ptr(self, actions) -> int:
         """Device address of the step's action block: the caller's device array, or the staging copy of a host array."""
@@ -284,6 +365,18 @@ class VectorEnv(_DeviceLoop):
         else:
             self.env.step_device(ptr, self._offsets.ptr, self.n_envs * self.rows, self.ids.ptr, self.obs.ptr)
         return self.obs, self.ids
+
+    def orders(self, ids) -> typing.Dict[str, DeviceArray]:
+        """The records of the orders `ids` names (bb_orders_device; `get_orders()[id]` / `order_status(id)` of every env at
+        once).  `ids`: a `[n_envs, k]` block of 8-byte ids, row e naming orders of env e — a device array (CUDA array
+        interface / DLPack: `env.ids`, a torch tensor, the id columns of `trades`) or a numpy array (copied as `step` copies
+        actions).  Returns `DeviceArray` columns `[n_envs, k]` keyed `side_is_bid, status, arr_time, end_time, vol,
+        start_vol, price, trader` (the PyOrder fields).  An `abi.NO_ID` entry reads as status `abi.STATUS_NONE` with zeros
+        and is no error, so blocks may be padded; an id the env has not issued reads the same and flags the env
+        (`check_errors` raises).  One launch on the env's stream with no host synchronisation (device ids); the columns are
+        allocated on the first call for a given `k` and overwritten by the next call with that `k`.  Make that first call
+        before capturing one into a CUDA graph."""
+        return self._orders(ids, None)
 
 
 class MarketVectorEnv(_DeviceLoop):
@@ -369,3 +462,14 @@ class MarketVectorEnv(_DeviceLoop):
         else:
             self.env.step_device_market(ptr, self._offsets.ptr, self.n_markets * self.rows, self.ids.ptr, self.obs.ptr)
         return self.obs, self.ids
+
+    def orders(self, ids, assets) -> typing.Dict[str, DeviceArray]:
+        """The records of the orders `(assets, ids)` name (bb_orders_device; `MarketEnv.get_orders(asset)[id]` of every
+        market at once).  `ids` (8-byte integers) and `assets` (4-byte integers) are `[n_markets, k]` blocks: entry
+        `[m, j]` names order `ids[m, j]` of asset `assets[m, j]`'s book in market m, as `step`'s ids and action rows do.
+        Device arrays or numpy arrays, as in `VectorEnv.orders`; the returned `DeviceArray` columns are `[n_markets, k]`
+        with the same keys.  An `abi.NO_ID` entry reads as status `abi.STATUS_NONE` with zeros and is no error; an id the
+        book has not issued, or an asset outside the market, reads the same and flags a book (`check_errors` raises).  One
+        launch on the env's stream; outputs are allocated on the first call for a given `k`, overwritten by the next call
+        with that `k`."""
+        return self._orders(ids, assets)

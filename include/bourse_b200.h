@@ -294,6 +294,39 @@ int bb_run_agents_with_rows_market(bb_handle* h, uint64_t seed, const bb_instr* 
 /* bb_level2 / bb_level1 into DEVICE memory: d_out[n_envs][45] / d_out[n_envs][9].  Asynchronous. */
 int bb_level2_device(bb_handle* h, uint32_t* d_out);
 int bb_level1_device(bb_handle* h, uint32_t* d_out);
+/* Order records by id for a whole batch of device-resident queries: get_orders()[id] / order_status(id) of the reference
+ * (rust/src/step_sim_numpy.rs, rust/src/types.rs:19-31) for every env at once.  A unit is an env on a single-asset handle and
+ * a market on a multi-asset one; d_ids is [units][n_per_unit], the shape of the id block bb_step_device(_market) returns.
+ * Query q of unit u reads book u, or book u * assets + d_assets[q] on a multi-asset handle (d_assets [units][n_per_unit];
+ * it must be NULL on a single-asset handle and non-NULL on a multi-asset one).  Output q of every non-NULL column (each
+ * [units][n_per_unit], columns as in bb_orders) is that order's field.  A BB_NO_ID query writes BB_STATUS_NONE and zeros
+ * and flags nothing, so a padded block is legal input.  An id without a record (>= the book's order count, or >= max_orders
+ * after BB_ERR_CAP_ORDERS) writes the same and flags BB_ERR_BAD_ID on its book (the reference panics); an asset >= assets
+ * writes the same and flags BB_ERR_ROW_OP on book 0 of the market.  Those sticky bits are all the call changes.  Every
+ * engine, deep included.  Refused with BB_EINVAL for a NULL d_ids, for more than 2^39 - 256 queries, and while host-queued
+ * instructions are pending (their ids have no record yet).  Asynchronous on the handle's stream: one launch, no host synchronisation and no allocation,
+ * so the call may be recorded into a CUDA graph.  Outputs are ordered after every earlier launch on the stream. */
+#define BB_STATUS_NONE 0xFFu /* status written for a query that names no order */
+int bb_orders_device(bb_handle* h, const uint64_t* d_ids, const uint32_t* d_assets, uint64_t n_per_unit, uint8_t* d_side_is_bid,
+                     uint8_t* d_status, uint64_t* d_arr_time, uint64_t* d_end_time, uint32_t* d_vol, uint32_t* d_start_vol,
+                     uint32_t* d_price, uint32_t* d_trader);
+/* Per book, the trades logged since a caller-owned cursor: the entries get_trades() (rust/src/types.rs:4-17) gained since the
+ * last read, for every book at once.  d_cursor[n_envs] (device) is read and written.  For book b, with
+ * logged = min(trades, max_trades): d_count[b] = logged - d_cursor[b] (may exceed cap), the first min(count, cap) of those
+ * trades go to row b of the [n_envs][cap] columns in log order, and d_cursor[b] advances by the number written, so a small
+ * cap loses nothing: the rest come with the next call.  Unused slots of a row hold active_id = passive_id = BB_NO_ID and
+ * zeros elsewhere, so the id columns can be passed straight to bb_orders_device (book b of a market handle is asset
+ * b % assets of market b / assets).  A cursor at or past `logged` gives count 0 and is left as it is; after bb_reset the
+ * caller zeroes its cursors.  Trades the full log could not hold are not reported (the book's BB_ERR_CAP_TRADES says they
+ * happened); nothing past max_trades is read.  (A log that overflowed and was then grown with bb_reserve has no records in
+ * the slots between its old capacity and its trade count: they read as whatever the slab holds there, as with bb_trades;
+ * bb_reset before growing a log that overflowed.)  Ids are widened to u64 to compare directly with the vector loops' ids.
+ * d_count and every column may be NULL.  Every engine, deep included; changes nothing but d_cursor and the outputs.
+ * Refused with BB_EINVAL for a NULL d_cursor, while host-queued instructions are pending, and on a handle with
+ * max_trades == 0.  Asynchronous on the handle's stream: one launch, no host synchronisation and no allocation, so the
+ * call may be recorded into a CUDA graph. */
+int bb_trades_device(bb_handle* h, uint32_t* d_cursor, uint32_t cap, uint32_t* d_count, uint64_t* d_t, uint8_t* d_side_is_bid,
+                     uint32_t* d_price, uint32_t* d_vol, uint64_t* d_active_id, uint64_t* d_passive_id);
 /* Device buffers for callers without a CUDA allocator of their own (numpy-only hosts); any device pointer works above.
  * bb_memcpy kind: 1 host to device, 2 device to host, 3 device to device; synchronous on the handle's stream. */
 int bb_device_alloc(bb_handle* h, uint64_t bytes, void** d_ptr);

@@ -12,8 +12,17 @@ every book — as RandomMarketAgents on every asset of every market (bb_run_agen
 VectorEnv(agents=c3_groups()) on the 8192 single-asset books (bb_run_agents_with_rows) — with the rows repriced into the
 agents' range as `bench.py --workload gym --bg-agents` does.
 
+--reads measures the device-resident order and trade reads (bb_orders_device / bb_trades_device) in the C3 loops of
+--bg-agents on the FAST engine, for 4096 single-asset envs (VectorEnv) and 2048 markets x 4 assets (MarketVectorEnv): the
+time per vector step without reads and with `trades(cap=64)` + `orders(k=8)` after every step (the difference is what the
+reads add to a step; plain and with-reads runs alternate, twice each), and the time per call of each read alone: CUDA
+events around 200 back-to-back calls on the books a window left behind, issued from Python and replayed from a CUDA graph
+(`time_calls`).  Those trades() calls find no new trades: they read the headers and write the padded windows.  The k = 8
+queried ids per env / market are fixed ids below 500 (every book has issued them after the warm-up steps).
+
     python scripts/bench_market_vector.py --steps 1000 --warmup 20
     python scripts/bench_market_vector.py --bg-agents --steps 1000 --warmup 20
+    python scripts/bench_market_vector.py --reads --steps 1000 --warmup 20
 """
 from __future__ import annotations
 
@@ -70,8 +79,9 @@ def windows(steps, warmup):
     return out
 
 
-def time_device(loop, d_blocks, steps, warmup):
-    """us per `loop.step` on a stream of its own: CUDA events around the timed steps of each window, summed."""
+def time_device(loop, d_blocks, steps, warmup, after_step=None):
+    """us per `loop.step` (followed by `after_step()` when given) on a stream of its own: CUDA events around the timed steps
+    of each window, summed."""
     import torch
     stream = torch.cuda.Stream()
     loop.env.set_stream(stream.cuda_stream)
@@ -85,6 +95,8 @@ def time_device(loop, d_blocks, steps, warmup):
         t0.record(stream)
         for s in range(pre, pre + timed):
             loop.step(d_blocks[s % n])
+            if after_step:
+                after_step()
         t1.record(stream)
         stream.synchronize()
         total += t0.elapsed_time(t1) * 1e3
@@ -93,17 +105,108 @@ def time_device(loop, d_blocks, steps, warmup):
     return total / steps, errors
 
 
+def c3_market_agents():
+    """The C3 population as RandomMarketAgents on every asset of a market."""
+    agents = []
+    for a in range(ASSETS):
+        for g in workloads.c3_groups():
+            agents.append(market.RandomMarketAgents(a, int(g["n_agents"]), (int(g["tick_lo"]), int(g["tick_hi"])),
+                                                    (int(g["vol_lo"]), int(g["vol_hi"])), int(g["tick_size"]), float(g["rate"])))
+    return agents
+
+
+def time_calls(loop, call, reps=200):
+    """us per `call()` on the loop's stream, two ways: CUDA events around `reps` back-to-back calls from Python (bounded by
+    the host's enqueue rate when the kernels are short), and around one replay of a CUDA graph holding `reps` calls (the
+    device's time per call, launch gaps included).  One untimed call first allocates the outputs."""
+    import torch
+    stream = torch.cuda.Stream()
+    loop.env.set_stream(stream.cuda_stream)
+    call()
+    stream.synchronize()
+    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    t0.record(stream)
+    for _ in range(reps):
+        call()
+    t1.record(stream)
+    stream.synchronize()
+    eager = t0.elapsed_time(t1) * 1e3 / reps
+    g = torch.cuda.CUDAGraph()
+    with torch.cuda.graph(g, stream=stream):
+        for _ in range(reps):
+            call()
+    g.replay()   # (untimed)
+    torch.cuda.synchronize()
+    t0.record(stream)
+    with torch.cuda.stream(stream):
+        g.replay()
+    t1.record(stream)
+    stream.synchronize()
+    loop.env.set_stream(0)
+    return eager, t0.elapsed_time(t1) * 1e3 / reps
+
+
+def bench_reads(args, name, power):
+    """--reads: see the module docstring."""
+    import torch
+    k, cap, n_envs = 8, 64, N_BOOKS // 2
+    res = {"card": name, "power_limit": power, "engine": "fast", "agents": "C3 (50 + 50 RandomAgents) on every book",
+           "orders_k": k, "trades_cap": cap, "steps": args.steps, "warmup": args.warmup, "rows_per_book": ROWS_PER_BOOK,
+           "us_per_step": {}, "us_per_call": {}, "errors": {}}
+    rng = np.random.default_rng(9)
+    c3 = workloads.c3_groups()
+    for label, units in (("vector_env_4096", n_envs), ("market_vector_2048x4", N_MARKETS)):
+        books = units if label.startswith("vector") else N_BOOKS
+        blocks = gym_action_blocks(args.blocks, books, ROWS_PER_BOOK, seed=5)
+        blocks["price"] = np.where((blocks["op_flags"] & abi.F_MARKET) != 0, blocks["price"], 2 * (40 + blocks["price"] % 21))
+        if label.startswith("vector"):
+            loop = gym.VectorEnv(n_envs, ROWS_PER_BOOK, 0, 0, 1, 1_000_000, agents=c3, agent_seed=5, **BG_KW)
+            d_blocks = [torch.from_numpy(x.view(np.uint8).reshape(n_envs, -1)).cuda() for x in blocks]
+            q_assets = None
+        else:
+            loop = gym.MarketVectorEnv(N_MARKETS, ROWS, 0, 0, [1] * ASSETS, 1_000_000, agents=c3_market_agents(), agent_seed=5, **BG_KW)
+            d_blocks = [torch.from_numpy(x.view(np.uint8).reshape(N_MARKETS, -1)).cuda() for x in market_blocks(blocks)]
+            q_assets = torch.from_numpy(np.tile(np.arange(k, dtype=np.int32) % ASSETS, (units, 1))).cuda()
+        q_ids = torch.from_numpy(rng.integers(0, 500, (units, k))).cuda()
+        torch.cuda.synchronize()
+
+        def orders():
+            return loop.orders(q_ids) if q_assets is None else loop.orders(q_ids, q_assets)
+
+        def reads():
+            loop.trades(cap)
+            orders()
+
+        for _ in range(2):   # plain and with reads, twice each, alternated
+            for tag, fn in (("plain", None), ("with_reads", reads)):
+                us, err = time_device(loop, d_blocks, args.steps, args.warmup, fn)
+                res["us_per_step"].setdefault(f"{label}_{tag}", []).append(us)
+                res["errors"][f"{label}_{tag}"] = res["errors"].get(f"{label}_{tag}", 0) | err
+        for tag, fn in (("orders", orders), ("trades", lambda: loop.trades(cap))):
+            eager, graph = time_calls(loop, fn)
+            res["us_per_call"][f"{label}_{tag}_eager"], res["us_per_call"][f"{label}_{tag}_graph"] = eager, graph
+        plain, with_reads = (min(res["us_per_step"][f"{label}_{t}"]) for t in ("plain", "with_reads"))
+        res["us_per_step"][f"{label}_added_by_reads"] = with_reads - plain
+        res["errors"][f"{label}_after_reads"] = int(np.bitwise_or.reduce(loop.env.env_errors()))
+        loop.close()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=1000)
     ap.add_argument("--warmup", type=int, default=20, help="untimed steps after each reset")
     ap.add_argument("--blocks", type=int, default=64, help="distinct action blocks, cycled")
     ap.add_argument("--bg-agents", action="store_true", help="the C3 population trades in every book (see the module docstring)")
+    ap.add_argument("--reads", action="store_true", help="time orders() / trades() in the C3 loops (see the module docstring)")
     args = ap.parse_args()
     import torch
 
     name, power = card()
     print(f"card: {name}, power limit: {power}", flush=True)
+    if args.reads:
+        print(json.dumps(bench_reads(args, name, power)), flush=True)
+        return
     blocks = gym_action_blocks(args.blocks, N_BOOKS, ROWS_PER_BOOK, seed=5)
     if args.bg_agents:   # limit prices into the agents' range, as bench.py run_gym does
         blocks["price"] = np.where((blocks["op_flags"] & abi.F_MARKET) != 0, blocks["price"], 2 * (40 + blocks["price"] % 21))
@@ -119,11 +222,7 @@ def main():
     if args.bg_agents:
         c3 = workloads.c3_groups()
         res["agents"] = "C3 (50 + 50 RandomAgents) on every book"
-        agents = []
-        for a in range(ASSETS):
-            for g in c3:
-                agents.append(market.RandomMarketAgents(a, int(g["n_agents"]), (int(g["tick_lo"]), int(g["tick_hi"])),
-                                                        (int(g["vol_lo"]), int(g["vol_hi"])), int(g["tick_size"]), float(g["rate"])))
+        agents = c3_market_agents()
         for eng, ekw in BG_ENGINES.items():
             v = gym.MarketVectorEnv(N_MARKETS, ROWS, 0, 0, [1] * ASSETS, 1_000_000, agents=agents, agent_seed=5, **BG_KW, **ekw)
             res["us_per_step"][f"market_vector_bg_{eng}"], res["errors"][f"market_vector_bg_{eng}"] = time_device(v, d_mkt, args.steps, args.warmup)
