@@ -397,7 +397,8 @@ int ensure_instr_capacity(bb_handle* h, size_t n) {
     return BB_OK;
 }
 
-// bb_step_device*: the kernel keeps the ids between assignment and execution; without a caller buffer it uses the handle's
+// device rows: the kernel writes every row's id (k_apply also reads them back at execution); without a caller buffer it uses
+// the handle's
 int id_buffer(bb_handle* h, uint64_t n_rows, u64** d_out_ids) {
     if (*d_out_ids) return BB_OK;
     if (n_rows + 1 > h->d_ids_cap) {
@@ -409,6 +410,54 @@ int id_buffer(bb_handle* h, uint64_t n_rows, u64** d_out_ids) {
     }
     *d_out_ids = h->d_ids;
     return BB_OK;
+}
+
+// calls that read or change the books on the device would run ahead of instructions bb_submit queued on the host
+int refuse_pending_queue(bb_handle* h) {
+    for (auto& q : h->queue)
+        if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
+    return BB_OK;
+}
+
+bool stream_capturing(bb_handle* h) {
+    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
+    cudaStreamIsCapturing(h->stream, &cap);
+    return cap != cudaStreamCaptureStatusNone;
+}
+
+// what bb_step_device(_market) and bb_run_agents_with_rows(_market) refuse before their launch; `wrong_handle` is the
+// message for a handle of the other kind (multi-asset for a single-asset call and the reverse)
+int check_device_rows(bb_handle* h, const bb_instr* d_instrs, const u64* d_offsets, u64 n_rows, bool market, const char* wrong_handle) {
+    if (!d_offsets || (n_rows && !d_instrs)) return fail(h, BB_EINVAL, "null argument");
+    if (market != (h->assets > 1)) return fail(h, BB_EINVAL, wrong_handle);
+    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine replays instruction streams only");
+    if (market && (u64)h->assets * h->cfg.max_queue > 65535) return fail(h, BB_EINVAL, "assets * max_queue must stay below 65536");
+    return refuse_pending_queue(h);
+}
+
+// the compiled variant of k_apply / k_sim a launch runs; grid_for sizes the grid for the same pointer
+typedef void (*Kernel)(KParams);
+template <int M> Kernel apply_kernel_for(int eng, bool all_resident) {
+    if (eng == ENG_DENSE) return k_apply<M, ENG_DENSE>;
+    if (eng == ENG_DENSE_L) return k_apply<M, ENG_DENSE_L>;
+    if (eng == ENG_FAST) return k_apply<M, ENG_FAST>;
+    return all_resident ? k_apply<M, ENG_PAGED_RES> : k_apply<M, ENG_PAGED>;
+}
+Kernel apply_kernel(int mode, int eng, bool all_resident) {
+    if (mode == MODE_REPLAY) return apply_kernel_for<MODE_REPLAY>(eng, all_resident);
+    return mode == MODE_ENV_MKT ? apply_kernel_for<MODE_ENV_MKT>(eng, all_resident) : apply_kernel_for<MODE_ENV>(eng, all_resident);
+}
+// external rows run on the MOM variants (they carry no slot hints)
+template <int E> Kernel sim_kernel_for(bool mom, bool mkt, bool ext) {
+    if (ext) return mkt ? k_sim<E, true, true, true> : k_sim<E, true, false, true>;
+    if (mkt) return mom ? k_sim<E, true, true> : k_sim<E, false, true>;
+    return mom ? k_sim<E, true, false> : k_sim<E, false, false>;
+}
+Kernel sim_kernel(int eng, bool mom, bool mkt, bool ext) {
+    if (eng == ENG_FAST) return sim_kernel_for<ENG_FAST>(mom, mkt, ext);
+    if (eng == ENG_DENSE) return sim_kernel_for<ENG_DENSE>(mom, mkt, ext);
+    if (eng == ENG_DENSE_L) return sim_kernel_for<ENG_DENSE_L>(mom, mkt, ext);
+    return sim_kernel_for<ENG_PAGED>(mom, mkt, ext);
 }
 
 int launch_apply(bb_handle* h, int mode, const bb_instr* d_instrs, const u64* d_offsets, u32 n_steps, bool host_order = false,
@@ -440,38 +489,13 @@ int launch_apply(bb_handle* h, int mode, const bb_instr* d_instrs, const u64* d_
     }
     int grid = 0, rc;
     const u32 wpb = wpb_for(lay.warp_bytes);
-    const size_t smem = (size_t)lay.warp_bytes * wpb;
-#define LAUNCH_APPLY(M, E)                                                                            \
-    do {                                                                                              \
-        if ((rc = grid_for(h, k_apply<M, E>, lay, h->cfg.n_envs, &grid, wpb))) return rc;             \
-        k_apply<M, E><<<grid, wpb * 32, smem, h->stream>>>(p);                                        \
-    } while (0)
-    if (mode == MODE_REPLAY) {
-        if (h->eng == ENG_DENSE) LAUNCH_APPLY(MODE_REPLAY, ENG_DENSE);
-        else if (h->eng == ENG_DENSE_L) LAUNCH_APPLY(MODE_REPLAY, ENG_DENSE_L);
-        else if (h->eng == ENG_FAST) LAUNCH_APPLY(MODE_REPLAY, ENG_FAST);
-        else if (h->all_resident) LAUNCH_APPLY(MODE_REPLAY, ENG_PAGED_RES);
-        else LAUNCH_APPLY(MODE_REPLAY, ENG_PAGED);
-    } else if (mode == MODE_ENV_MKT) {
-        if (h->eng == ENG_DENSE) LAUNCH_APPLY(MODE_ENV_MKT, ENG_DENSE);
-        else if (h->eng == ENG_DENSE_L) LAUNCH_APPLY(MODE_ENV_MKT, ENG_DENSE_L);
-        else if (h->eng == ENG_FAST) LAUNCH_APPLY(MODE_ENV_MKT, ENG_FAST);
-        else if (h->all_resident) LAUNCH_APPLY(MODE_ENV_MKT, ENG_PAGED_RES);
-        else LAUNCH_APPLY(MODE_ENV_MKT, ENG_PAGED);
-    } else {
-        if (h->eng == ENG_DENSE) LAUNCH_APPLY(MODE_ENV, ENG_DENSE);
-        else if (h->eng == ENG_DENSE_L) LAUNCH_APPLY(MODE_ENV, ENG_DENSE_L);
-        else if (h->eng == ENG_FAST) LAUNCH_APPLY(MODE_ENV, ENG_FAST);
-        else if (h->all_resident) LAUNCH_APPLY(MODE_ENV, ENG_PAGED_RES);
-        else LAUNCH_APPLY(MODE_ENV, ENG_PAGED);
-    }
-#undef LAUNCH_APPLY
+    const Kernel k = apply_kernel(mode, h->eng, h->all_resident);
+    if ((rc = grid_for(h, k, lay, h->cfg.n_envs, &grid, wpb))) return rc;
+    k<<<grid, wpb * 32, (size_t)lay.warp_bytes * wpb, h->stream>>>(p);
     CUDA_TRY(h, cudaGetLastError());
     // a launch recorded into a CUDA graph (bb_step_device inside a captured RL loop) will run any number of times:
     // the host-side record count is unknown from here on and is re-read from the device when next needed
-    cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-    cudaStreamIsCapturing(h->stream, &cap);
-    if (mode != MODE_REPLAY && h->recorded_host >= 0 && cap == cudaStreamCaptureStatusNone) h->recorded_host += n_steps;
+    if (mode != MODE_REPLAY && h->recorded_host >= 0 && !stream_capturing(h)) h->recorded_host += n_steps;
     else h->recorded_host = -1;
     return BB_OK;
 }
@@ -486,17 +510,9 @@ int snapshot(bb_handle* h, u32 first_env, u32 n, u32* d45, u32* d8, u32 words = 
     }
     int grid = 0, rc;
     const u32 wpb = wpb_for(h->lay_snap.warp_bytes);
-    const size_t smem = (size_t)h->lay_snap.warp_bytes * wpb;
-    if (h->eng == ENG_DENSE) {
-        if ((rc = grid_for(h, k_snapshot<ENG_DENSE>, h->lay_snap, n, &grid, wpb))) return rc;
-        k_snapshot<ENG_DENSE><<<grid, wpb * 32, smem, h->stream>>>(p, d45, d8, first_env, n, words);
-    } else if (h->eng == ENG_DENSE_L) {
-        if ((rc = grid_for(h, k_snapshot<ENG_DENSE_L>, h->lay_snap, n, &grid, wpb))) return rc;
-        k_snapshot<ENG_DENSE_L><<<grid, wpb * 32, smem, h->stream>>>(p, d45, d8, first_env, n, words);
-    } else {
-        if ((rc = grid_for(h, k_snapshot<ENG_PAGED>, h->lay_snap, n, &grid, wpb))) return rc;
-        k_snapshot<ENG_PAGED><<<grid, wpb * 32, smem, h->stream>>>(p, d45, d8, first_env, n, words);
-    }
+    const auto k = h->eng == ENG_DENSE ? k_snapshot<ENG_DENSE> : h->eng == ENG_DENSE_L ? k_snapshot<ENG_DENSE_L> : k_snapshot<ENG_PAGED>;
+    if ((rc = grid_for(h, k, h->lay_snap, n, &grid, wpb))) return rc;
+    k<<<grid, wpb * 32, (size_t)h->lay_snap.warp_bytes * wpb, h->stream>>>(p, d45, d8, first_env, n, words);
     CUDA_TRY(h, cudaGetLastError());
     return BB_OK;
 }
@@ -964,14 +980,11 @@ static int set_agents_impl(bb_handle* h, const bb_agent_group* groups, const uin
 int bb_step_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_env_offsets, uint64_t n_rows, uint64_t* d_out_ids,
                    uint32_t* d_obs_out) {
     CHECK_H(h);
-    if (!d_env_offsets || (n_rows && !d_instrs)) return fail(h, BB_EINVAL, "null argument");
-    if (h->assets > 1) return fail(h, BB_EINVAL, "bb_step_device drives single-asset envs (multi-asset queues are ordered on the host)");
-    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine replays instruction streams only");
-    for (auto& q : h->queue)
-        if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
-    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    int rc = id_buffer(h, n_rows, &d_out_ids);
+    int rc = check_device_rows(h, d_instrs, d_env_offsets, n_rows, false,
+                               "bb_step_device drives single-asset envs (multi-asset queues are ordered on the host)");
     if (rc) return rc;
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    if ((rc = id_buffer(h, n_rows, &d_out_ids))) return rc;
     h->mirror_dirty = true;  // ids were handed out on the device
     return launch_apply(h, MODE_ENV, d_instrs, d_env_offsets, 1, false, d_out_ids, d_obs_out);
 }
@@ -979,26 +992,19 @@ int bb_step_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_env
 int bb_step_device_market(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_market_offsets, uint64_t n_rows,
                           uint64_t* d_out_ids, uint32_t* d_obs_out) {
     CHECK_H(h);
-    if (!d_market_offsets || (n_rows && !d_instrs)) return fail(h, BB_EINVAL, "null argument");
-    if (h->assets < 2) return fail(h, BB_EINVAL, "bb_step_device_market drives multi-asset markets (single-asset envs: bb_step_device)");
-    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine replays instruction streams only");
-    if ((u64)h->assets * h->cfg.max_queue > 65535) return fail(h, BB_EINVAL, "assets * max_queue must stay below 65536");
-    for (auto& q : h->queue)
-        if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
+    int rc = check_device_rows(h, d_instrs, d_market_offsets, n_rows, true,
+                               "bb_step_device_market drives multi-asset markets (single-asset envs: bb_step_device)");
+    if (rc) return rc;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     if (h->market_rng_at == bb_handle::RNG_HOST_AHEAD) {
         // bb_step shuffled on the host since the books' copies of the streams were last written: bring them up to date, but
         // never inside a stream capture (the graph would replay a copy of the streams as they are now)
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        cudaStreamIsCapturing(h->stream, &cap);
-        if (cap != cudaStreamCaptureStatusNone)
+        if (stream_capturing(h))
             return fail(h, BB_EINVAL, "bb_step_device_market: the markets' shuffle streams last advanced in bb_step; call "
                                       "bb_step_device_market once outside the capture (or bb_reset) before capturing it");
-        int rc = market_rng_to_device(h);
-        if (rc) return rc;
+        if ((rc = market_rng_to_device(h))) return rc;
     }
-    int rc = id_buffer(h, n_rows, &d_out_ids);
-    if (rc) return rc;
+    if ((rc = id_buffer(h, n_rows, &d_out_ids))) return rc;
     h->mirror_dirty = true;  // ids were handed out on the device
     if ((rc = launch_apply(h, MODE_ENV_MKT, d_instrs, d_market_offsets, 1, false, d_out_ids, d_obs_out))) return rc;
     h->market_rng_at = bb_handle::RNG_DEVICE_AHEAD;
@@ -1026,8 +1032,7 @@ int bb_orders_device(bb_handle* h, const uint64_t* d_ids, const uint32_t* d_asse
     if (!d_ids) return fail(h, BB_EINVAL, "null argument");
     if (h->assets > 1 && !d_assets) return fail(h, BB_EINVAL, "bb_orders_device: d_assets is required on a multi-asset handle");
     if (h->assets == 1 && d_assets) return fail(h, BB_EINVAL, "bb_orders_device: d_assets must be NULL on a single-asset handle");
-    for (auto& q : h->queue)
-        if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
+    if (int rc = refuse_pending_queue(h)) return rc;
     const u64 units = h->cfg.n_envs / h->assets, max_queries = 256ull * 0x7FFFFFFFull;  // (one launch: grid.x < 2^31)
     if (n_per_unit > max_queries / units) return fail(h, BB_EINVAL, "bb_orders_device: too many queries for one launch");
     const u64 n_queries = units * n_per_unit;
@@ -1045,8 +1050,7 @@ int bb_trades_device(bb_handle* h, uint32_t* d_cursor, uint32_t cap, uint32_t* d
     CHECK_H(h);
     if (!d_cursor) return fail(h, BB_EINVAL, "null argument");
     if (h->cfg.max_trades == 0) return fail(h, BB_EINVAL, "bb_trades_device: the trade log is disabled (max_trades == 0)");
-    for (auto& q : h->queue)
-        if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
+    if (int rc = refuse_pending_queue(h)) return rc;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     k_trades_window<<<(h->cfg.n_envs + 7) / 8, 256, 0, h->stream>>>(h->blobs, h->blob_stride, h->tr, h->cfg.max_trades, h->cfg.n_envs,
                                                                      d_cursor, cap, d_count, d_t, d_side_is_bid, d_price, d_vol,
@@ -1167,6 +1171,7 @@ namespace {
 struct ExtRows {  // bb_run_agents_with_rows(_market): the caller's device-resident rows for the launch's first step
     const bb_instr* d_instrs;
     const u64* d_offsets;
+    u64 n_rows;
     u64* d_out_ids;
     u32* d_obs_out;
 };
@@ -1178,19 +1183,19 @@ int bb_run_agents(bb_handle* h, uint64_t seed, uint32_t n_steps) { return run_ag
 int bb_run_agents_with_rows(bb_handle* h, uint64_t seed, const bb_instr* d_instrs, const uint64_t* d_env_offsets, uint64_t n_rows,
                             uint64_t* d_out_ids, uint32_t* d_obs_out) {
     CHECK_H(h);
-    if (!d_env_offsets || (n_rows && !d_instrs)) return fail(h, BB_EINVAL, "null argument");
-    if (h->assets > 1) return fail(h, BB_EINVAL, "bb_run_agents_with_rows drives single-asset envs");
-    const ExtRows ext{d_instrs, d_env_offsets, d_out_ids, d_obs_out};
+    if (int rc = check_device_rows(h, d_instrs, d_env_offsets, n_rows, false, "bb_run_agents_with_rows drives single-asset envs")) return rc;
+    const ExtRows ext{d_instrs, d_env_offsets, n_rows, d_out_ids, d_obs_out};
     return run_agents_impl(h, seed, 1, &ext);
 }
 
 int bb_run_agents_with_rows_market(bb_handle* h, uint64_t seed, const bb_instr* d_instrs, const uint64_t* d_market_offsets,
                                    uint64_t n_rows, uint64_t* d_out_ids, uint32_t* d_obs_out) {
     CHECK_H(h);
-    if (!d_market_offsets || (n_rows && !d_instrs)) return fail(h, BB_EINVAL, "null argument");
-    if (h->assets < 2) return fail(h, BB_EINVAL, "bb_run_agents_with_rows_market drives multi-asset markets (single-asset envs: use bb_run_agents_with_rows)");
+    if (int rc = check_device_rows(h, d_instrs, d_market_offsets, n_rows, true,
+                                   "bb_run_agents_with_rows_market drives multi-asset markets (single-asset envs: use bb_run_agents_with_rows)"))
+        return rc;
     if (h->group_asset.empty()) return fail(h, BB_EINVAL, "bb_set_agents_market has not been called");
-    const ExtRows ext{d_instrs, d_market_offsets, d_out_ids, d_obs_out};
+    const ExtRows ext{d_instrs, d_market_offsets, n_rows, d_out_ids, d_obs_out};
     return run_agents_impl(h, seed, 1, &ext);
 }
 
@@ -1204,14 +1209,10 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
         return fail(h, BB_EINVAL, "single-asset agents on a multi-asset handle: use bb_set_agents_market");
     if (n_steps == 0) return BB_OK;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
-    for (auto& q : h->queue)
-        if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
-    {   // k_sim stages its records without per-step capacity checks, so the count must be known on the host: no graph capture
-        cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
-        cudaStreamIsCapturing(h->stream, &cap);
-        if (cap != cudaStreamCaptureStatusNone)
-            return fail(h, BB_EINVAL, "agent launches cannot be captured into a CUDA graph (bb_step_device can)");
-    }
+    int rc;
+    if (!ext && (rc = refuse_pending_queue(h))) return rc;  // (the device-row calls checked it with their arguments)
+    // k_sim stages its records without per-step capacity checks, so the count must be known on the host: no graph capture
+    if (stream_capturing(h)) return fail(h, BB_EINVAL, "agent launches cannot be captured into a CUDA graph (bb_step_device can)");
     // history capacity is validated up front so the kernel can stage records without per-step checks
     if (h->recorded_host < 0) {  // after a replay the number of emitted records is only known to the device
         CUDA_TRY(h, cudaMemcpy2DAsync(h->h_offsets, 8, h->blobs + offsetof(BookHdr, n_steps), h->blob_stride, 4, 1,
@@ -1243,24 +1244,16 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
         p.offsets = ext->d_offsets;
         p.out_ids = ext->d_out_ids;
         p.obs_out = ext->d_obs_out;
+        if ((rc = id_buffer(h, ext->n_rows, &p.out_ids))) return rc;
     }
-    int grid = 0, rc;
+    int grid = 0;
     // external rows carry no slot hints: they run on the variants that also serve MomentumAgent / NoiseAgent events.  So
     // does a RandomAgents group that can draw off its book's tick: only those variants check the queued prices
     const bool mom = h->mom_groups != 0 || ext != nullptr || h->rand_tick_mask != 0;
     // markets: the A books of a market are A consecutive warps of one CTA (a CTA holds as many whole markets as fit in 4 warps)
     const u32 wpb = mkt ? (WPB / h->assets) * h->assets : wpb_for(lay.warp_bytes);
-    const size_t sim_smem = (size_t)lay.warp_bytes * wpb;
-#define SIM_CASE(E, M)                                                                                     \
-    if (h->eng == E && mom == M) {                                                                         \
-        if (mkt && ext) { if ((rc = grid_for(h, k_sim<E, true, true, true>, lay, h->cfg.n_envs, &grid, wpb))) return rc; } \
-        else if (mkt) { if ((rc = grid_for(h, k_sim<E, M, true>, lay, h->cfg.n_envs, &grid, wpb))) return rc; } \
-        else if (ext) { if ((rc = grid_for(h, k_sim<E, true, false, true>, lay, h->cfg.n_envs, &grid, wpb))) return rc; } \
-        else if ((rc = grid_for(h, k_sim<E, M, false>, lay, h->cfg.n_envs, &grid, wpb))) return rc;  \
-    }
-    SIM_CASE(ENG_FAST, false) SIM_CASE(ENG_FAST, true) SIM_CASE(ENG_PAGED, false) SIM_CASE(ENG_PAGED, true)
-    SIM_CASE(ENG_DENSE, false) SIM_CASE(ENG_DENSE, true) SIM_CASE(ENG_DENSE_L, false) SIM_CASE(ENG_DENSE_L, true)
-#undef SIM_CASE
+    const Kernel k = sim_kernel(h->eng, mom, mkt, ext != nullptr);
+    if ((rc = grid_for(h, k, lay, h->cfg.n_envs, &grid, wpb))) return rc;
     const size_t warps = (size_t)grid * wpb;
     if (h->eng < ENG_DENSE && warps > h->scratch_warps) {
         cudaFree(h->scratch);
@@ -1269,16 +1262,7 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
         h->scratch_warps = warps;
     }
     p.scratch = h->scratch;
-#define SIM_LAUNCH(E, M)                                                                       \
-    if (h->eng == E && mom == M) {                                                             \
-        if (mkt && ext) k_sim<E, true, true, true><<<grid, wpb * 32, sim_smem, h->stream>>>(p); \
-        else if (mkt) k_sim<E, M, true><<<grid, wpb * 32, sim_smem, h->stream>>>(p);           \
-        else if (ext) k_sim<E, true, false, true><<<grid, wpb * 32, sim_smem, h->stream>>>(p); \
-        else k_sim<E, M, false><<<grid, wpb * 32, sim_smem, h->stream>>>(p);                   \
-    }
-    SIM_LAUNCH(ENG_FAST, false) SIM_LAUNCH(ENG_FAST, true) SIM_LAUNCH(ENG_PAGED, false) SIM_LAUNCH(ENG_PAGED, true)
-    SIM_LAUNCH(ENG_DENSE, false) SIM_LAUNCH(ENG_DENSE, true) SIM_LAUNCH(ENG_DENSE_L, false) SIM_LAUNCH(ENG_DENSE_L, true)
-#undef SIM_LAUNCH
+    k<<<grid, wpb * 32, (size_t)lay.warp_bytes * wpb, h->stream>>>(p);
     CUDA_TRY(h, cudaGetLastError());
     h->mirror_dirty = true;
     h->status_valid = false;
@@ -1511,8 +1495,7 @@ static_assert(sizeof(bb_order_rec) == sizeof(OrderRec) && sizeof(bb_trade_rec) =
 int bb_orders_all(bb_handle* h, uint32_t cap_per_env, bb_order_rec* out, uint32_t* counts) {
     CHECK_H(h);
     if (!out || !counts) return fail(h, BB_EINVAL, "null argument");
-    for (auto& q : h->queue)
-        if (!q.empty()) return fail(h, BB_EINVAL, "host-queued instructions pending: call bb_step first");
+    if (int rc = refuse_pending_queue(h)) return rc;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     const u32 cap = std::min(cap_per_env, h->cfg.max_orders);
     CUDA_TRY(h, cudaMemcpy2DAsync(counts, 4, h->blobs + offsetof(BookHdr, n_orders), h->blob_stride, 4, h->cfg.n_envs,

@@ -212,6 +212,70 @@ template <bool CT, class G> __device__ __forceinline__ void apply_instr(const G&
     }
 }
 
+// Submission of a caller's device-resident rows: what Env / MarketEnv::place_order, cancel_order and modify_order do
+// (env.rs:173, market_env.rs:163-219), warp-wide in row order over the slice p.instrs[off, off + m), for book `b`.  Only
+// the first n_acc rows are submitted; the others create, queue and flag nothing (each kernel keeps its own queue-capacity
+// policy).  A NEW row takes the next id of its book; a limit price off the tick of the row's book is create_order's
+// PriceError (orderbook.rs:367-383): nothing is created or queued and the book is flagged ERR_PRICE.  Every row gets its id,
+// or BB_NO_ID, in out_ids from the book it belongs to.
+//   MKT   the slice is a market's and bb_instr::aux the row's asset; b is asset mk_a of the market.  Every book walks the
+//         whole slice.  Rows naming no asset of the market queue nothing and flag book 0, which writes their ids.
+//   SIMQ  k_sim's queue carries NEW and CANCEL only: a MODIFY row, or a NEW whose trader id does not fit 19 bits, is dropped
+//         with ERR_ROW_OP.  A cancel of an id its book has not issued by the end of submission is the reference's panic
+//         (orderbook.rs:642): ERR_BAD_ID.  Without SIMQ (k_apply) MODIFY rows are queued and each new id's order record is
+//         published with status New, as create_order does at submission.
+// c.next is the book's next id, c.n counts this book's queued rows, c.n_mkt (MKT) the market's.  Every queued row is handed
+// to sink(j, x, y, mine, is_new, id, pos, pos_mkt): the row's two 16-byte halves, whether it is this book's, whether it took
+// id `id` of this book, and its positions among this book's and the market's queued rows.
+struct RowCount {
+    u32 next, n, n_mkt;
+};
+template <bool MKT, bool SIMQ, class G, class Sink>
+__device__ __forceinline__ void submit_rows(const G& g, const KParams& p, Book& b, u64 off, u32 m, u32 n_acc, u32 mk_a, RowCount& c,
+                                            Sink sink) {
+    const bb_instr* ins = p.instrs + off;
+    const u32 book0 = b.env - mk_a, tick = MKT ? 0u : __ldg(g.ticks + book0), below = (1u << b.lane) - 1u;
+    u32 max_cancel = 0;  // SIMQ: 1 + the largest id a cancel row of this book names
+    for (u32 j0 = 0; j0 < n_acc; j0 += 32) {
+        const u32 j = j0 + b.lane;
+        // x: (t), op_flags, order_id; y: price, vol, trader, aux — loaded field by field, so that a caller that needs only
+        // some of them (k_apply: op_flags, price, aux) loads only those
+        uint4 x = make_uint4(0u, 0u, 0u, 0u), y = x;
+        if (j < n_acc) {
+            x.z = ins[j].op_flags;
+            x.w = ins[j].order_id;
+            y = make_uint4(ins[j].price, ins[j].vol, ins[j].trader, ins[j].aux);
+        }
+        const u32 op = x.z & BB_OP_MASK, asset = MKT ? y.w : 0u;
+        const bool ok = !MKT || asset < p.assets;  // (a lane past the slice holds a no-op row)
+        const bool own = !MKT || (ok ? asset == mk_a : mk_a == 0u);
+        const bool bad_tick = ok && op == BB_OP_NEW && !(x.z & BB_F_MARKET) && (y.x % (MKT ? __ldg(g.ticks + book0 + asset) : tick) != 0u);
+        const bool bad_op = SIMQ && ok && (op == BB_OP_MODIFY || (op == BB_OP_NEW && y.z >= (1u << 19)));
+        const bool is_new = ok && op == BB_OP_NEW && !bad_tick && !bad_op;
+        const bool queued = is_new || (ok && (op == BB_OP_CANCEL || (!SIMQ && op == BB_OP_MODIFY)));
+        const u32 nm = __ballot_sync(BB_FULL, is_new && own), om = __ballot_sync(BB_FULL, queued && own);
+        const u32 qm = MKT ? __ballot_sync(BB_FULL, queued) : om;
+        const u32 id = c.next + __popc(nm & below), pos = c.n + __popc(om & below);
+        if (j < n_acc && own) {
+            p.out_ids[off + j] = is_new ? (u64)id : BB_NO_ID;
+            if (!SIMQ && is_new && id < g.max_orders) stg32(b.oh + (u64)id * ORD_STRIDE + OH_META, ST_NEW | ((x.z & BB_F_BID) ? META_BID : 0u));
+        }
+        if (queued) sink(j, x, y, own, is_new && own, id, pos, MKT ? c.n_mkt + __popc(qm & below) : pos);
+        if (SIMQ && own && ok && op == BB_OP_CANCEL) max_cancel = max(max_cancel, x.w == 0xFFFFFFFFu ? x.w : x.w + 1u);
+        if (__any_sync(BB_FULL, bad_tick && own)) b.err |= ERR_PRICE;
+        if ((MKT || SIMQ) && __any_sync(BB_FULL, (bad_op && own) || (MKT && !ok && mk_a == 0u))) b.err |= ERR_ROW_OP;
+        c.next += __popc(nm);
+        c.n += __popc(om);
+        if (MKT) c.n_mkt += __popc(qm);
+    }
+    if (SIMQ && __reduce_max_sync(BB_FULL, max_cancel) > c.next) b.err |= ERR_BAD_ID;
+#pragma unroll 1
+    for (u32 j = n_acc + b.lane; j < m; j += 32) {  // (kept rolled: it runs only for a slice over the cap)
+        const u32 asset = MKT ? ins[j].aux : 0u;
+        if (!MKT || (asset < p.assets ? asset == mk_a : mk_a == 0u)) p.out_ids[off + j] = BB_NO_ID;
+    }
+}
+
 // the generic paged geometry is shared-memory limited to <= 5 CTAs per SM anyway: give it the registers
 template <int MODE, int ENG> __global__ void __launch_bounds__(128, (ENG == ENG_PAGED || ENG == ENG_PAGED_RES) ? 5 : 7) k_apply(const __grid_constant__ KParams p) {
     typedef GeoT<ENG> G;
@@ -295,95 +359,34 @@ template <int MODE, int ENG> __global__ void __launch_bounds__(128, (ENG == ENG_
                 b.trade_vol = 0;  // env.rs:117-118
                 const u32 m = (s == 0) ? n : 0u;
                 u32 nv;  // transactions in the queue
+                // device-submitted rows (bb_step_device, bb_step_device_market): the queue is a permutation of row indices
+                // (a market's: every book keeps the whole market's queue)
+                auto to_perm = [&](u32 j, uint4, uint4, bool, bool, u32, u32, u32 pos_mkt) { sts16(perm + 2u * pos_mkt, j); };
                 if constexpr (MK) {
-                    // device-submitted market rows: every book of the market walks the whole slice and does, in row order,
-                    // what MarketEnv::place_order / cancel_order / modify_order (market_env.rs:163-219) would have done for
-                    // the rows of its own asset (bb_instr::aux): NEW rows take the next ids of that asset's book
-                    // (market.rs:270-280), an off-tick limit price creates and queues nothing and flags that book.  Rows
-                    // naming no asset of the market queue nothing and flag book 0.  Each book writes the ids of its own
-                    // rows only (book 0 also those of the asset-less rows), and keeps the market-wide queue in `perm`
                     const bool drop = m > p.assets * p.max_queue;  // the whole market's queue must fit the permutation
                     if (drop) b.err |= ERR_CAP_QUEUE;
-                    const u32 book0 = env - mk_a;
-                    u32 next = b.n_orders, n_mine = 0;
-                    nv = 0;
-                    for (u32 j0 = 0; j0 < m; j0 += 32) {
-                        const u32 j = j0 + lane;
-                        u32 of = 0, price = 0, asset = 0;
-                        if (j < m) {
-                            const uint4 y = reinterpret_cast<const uint4*>(ins + j)[1];
-                            of = ins[j].op_flags;
-                            price = y.x;
-                            asset = y.w;
-                        }
-                        const u32 op = of & BB_OP_MASK;
-                        const bool row_ok = j < m && !drop && asset < p.assets;
-                        const bool bad_tick = row_ok && op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % __ldg(g.ticks + book0 + asset) != 0u);
-                        const bool is_new = row_ok && op == BB_OP_NEW && !bad_tick;
-                        const bool queued = is_new || (row_ok && (op == BB_OP_CANCEL || op == BB_OP_MODIFY));
-                        const bool own = j < m && (asset < p.assets ? asset == mk_a : mk_a == 0u);
-                        const bool my_new = is_new && asset == mk_a;
-                        const u32 below = (1u << lane) - 1u;
-                        const u32 nm = __ballot_sync(BB_FULL, my_new), qm = __ballot_sync(BB_FULL, queued);
-                        const u32 id = next + __popc(nm & below);
-                        if (own) {
-                            p.out_ids[off + j] = my_new ? (u64)id : ~0ULL;
-                            if (my_new && id < g.max_orders)
-                                stg32(b.oh + (u64)id * ORD_STRIDE + OH_META, ST_NEW | ((of & BB_F_BID) ? META_BID : 0u));
-                        }
-                        if (queued) sts16(perm + 2u * (nv + __popc(qm & below)), j);
-                        if (__any_sync(BB_FULL, bad_tick && asset == mk_a)) b.err |= ERR_PRICE;
-                        if (__any_sync(BB_FULL, j < m && !drop && asset >= p.assets) && mk_a == 0u) b.err |= ERR_ROW_OP;
-                        next += __popc(nm);
-                        nv += __popc(qm);
-                        n_mine += __popc(__ballot_sync(BB_FULL, queued && asset == mk_a));
-                    }
-                    b.n_orders = next;
+                    RowCount c{b.n_orders, 0u, 0u};
+                    submit_rows<true, false>(g, p, b, off, m, drop ? 0u : m, mk_a, c, to_perm);
+                    b.n_orders = c.next;
+                    nv = c.n_mkt;
                     // the host-ordered path's rule, over this book's share of the queue
                     if constexpr (G::DENSE) {
-                        if (n_mine > p.step_size || (start <= b.max_key_time && (b.flags & (FL_HAS_ASK | FL_HAS_BID)))) b.err |= ERR_TIME_ORDER;
+                        if (c.n > p.step_size || (start <= b.max_key_time && (b.flags & (FL_HAS_ASK | FL_HAS_BID)))) b.err |= ERR_TIME_ORDER;
                     }
                 } else {
                     if (m > p.max_queue) b.err |= ERR_CAP_QUEUE;
                     if constexpr (G::DENSE) {  // the dense engine relies on t = start + i being new, increasing key times
                         if (m > p.step_size || (start <= b.max_key_time && (b.flags & (FL_HAS_ASK | FL_HAS_BID)))) b.err |= ERR_TIME_ORDER;
                     }
-                    const u32 mm = min(m, p.max_queue);
-                    // (a) create_order happened at submission (env.rs:173): publish status New for the new ids
+                    const u32 mm = min(m, p.max_queue);  // the first max_queue rows run
                     nv = mm;
                     if (p.assign_ids) {
-                        // device-submitted rows: what Env::place_order / cancel_order / modify_order would have done at
-                        // submission happens here, in row order — NEW rows take the next ids; a limit price off the tick grid
-                        // is create_order's PriceError (orderbook.rs:367-383): nothing is created or queued, the env is flagged
-                        u32 next = b.n_orders;
-                        nv = 0;
-                        const u32 tick = __ldg(g.ticks + env);
-                        for (u32 j0 = 0; j0 < mm; j0 += 32) {
-                            const u32 j = j0 + lane;
-                            u32 of = 0, price = 0;
-                            if (j < mm) {
-                                of = ins[j].op_flags;
-                                price = ins[j].price;
-                            }
-                            const u32 op = of & BB_OP_MASK;
-                            const bool bad_tick = op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % tick != 0u);
-                            const bool is_new = op == BB_OP_NEW && !bad_tick;
-                            const bool queued = is_new || op == BB_OP_CANCEL || op == BB_OP_MODIFY;
-                            const u32 below = (1u << lane) - 1u;
-                            const u32 nm = __ballot_sync(BB_FULL, is_new), qm = __ballot_sync(BB_FULL, queued);
-                            const u32 id = next + __popc(nm & below);
-                            if (j < mm) {
-                                p.out_ids[off + j] = is_new ? (u64)id : ~0ULL;
-                                if (is_new && id < g.max_orders)
-                                    stg32(b.oh + (u64)id * ORD_STRIDE + OH_META, ST_NEW | ((of & BB_F_BID) ? META_BID : 0u));
-                            }
-                            if (queued) sts16(perm + 2u * (nv + __popc(qm & below)), j);
-                            if (__any_sync(BB_FULL, bad_tick)) b.err |= ERR_PRICE;
-                            next += __popc(nm);
-                            nv += __popc(qm);
-                        }
-                        b.n_orders = next;
+                        RowCount c{b.n_orders, 0u, 0u};
+                        submit_rows<false, false>(g, p, b, off, m, mm, 0u, c, to_perm);
+                        b.n_orders = c.next;
+                        nv = c.n;
                     } else {
+                        // (a) create_order happened at submission (env.rs:173): publish status New for the new ids
                         u32 max_id = 0;
                         for (u32 j = lane; j < mm; j += 32) {
                             const u32 of = ins[j].op_flags, id = ins[j].order_id;
@@ -844,114 +847,49 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                 if (mine) chip_base += ag.n_agents;
             }
             u32 mk_nr = 0;  // MKT + EXT: the market's queued rows (every book of the market counts the same)
-            if constexpr (EXT && !MKT) {
-                const u64 off = p.offsets[env];
-                const u32 m = s == 0 ? (u32)(p.offsets[env + 1] - off) : 0u;  // the rows belong to the launch's first step
-                const bb_instr* ins = p.instrs + off;
-                u32 max_cancel = 0;  // 1 + largest id a cancel row names
-                const u32 tick = __ldg(g.ticks + env);
-                for (u32 j0 = 0; j0 < m; j0 += 32) {
-                    const u32 j = j0 + lane;
-                    u32 of = 0, price = 0, vol = 0, trader = 0, oid = 0;
-                    if (j < m) {
-                        const uint4 x = reinterpret_cast<const uint4*>(ins + j)[0], y = reinterpret_cast<const uint4*>(ins + j)[1];
-                        of = x.z; oid = x.w; price = y.x; vol = y.y; trader = y.z;
-                    }
-                    const u32 op = of & BB_OP_MASK;
-                    const bool bid = (of & BB_F_BID) != 0u;
-                    // create_order's tick check (orderbook.rs:367-383): the row is dropped like the Err return
-                    const bool bad_tick = op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % tick != 0u);
-                    const bool is_new = op == BB_OP_NEW && !bad_tick, is_cancel = op == BB_OP_CANCEL;
-                    const bool queued = is_new || is_cancel;
-                    const u32 below = (1u << lane) - 1u;
-                    const u32 nm = __ballot_sync(BB_FULL, is_new), qm = __ballot_sync(BB_FULL, queued);
-                    const u32 id = e.next_id + __popc(nm & below), pos = e.n + __popc(qm & below);
-                    if (of & BB_F_MARKET) price = bid ? 0xFFFFFFFFu : 0u;  // types.rs:160-172, 213-225
-                    if (j < m && p.out_ids) p.out_ids[off + j] = is_new ? (u64)id : ~0ULL;
-                    if (queued && pos < p.max_queue) {
-                        // the in-kernel queue format: bit 0 NEW, bit 1 bid, no hint, trader id above bit 13
-                        const uint4 ev = make_uint4(is_new ? (1u | (bid ? 2u : 0u) | (trader << 13)) : 0u, is_new ? id : oid, price, vol);
+            if constexpr (EXT) {
+                // the caller's rows belong to the launch's first step; markets: the market's slice, every book walks it all
+                const u32 unit = MKT ? env / p.assets : env;
+                const u64 off = p.offsets[unit];
+                const u32 m = s == 0 ? (u32)(p.offsets[unit + 1] - off) : 0u;
+                const u32 cap = p.assets * p.max_queue;  // MKT: queued rows beyond it drop the market's step (below)
+                const u32 nw = MKT ? min((m + 31u) >> 5, mk_words) : 0u;  // mask words the slice can touch
+                if constexpr (MKT) {
+                    for (u32 w = lane; w < nw; w += 32) sts(mk_rm + 4u * w, 0u);
+                    __syncwarp();
+                }
+                // this book's rows join its queue as in-kernel events: bit 0 NEW, bit 1 bid, no hint, trader id above bit 13;
+                // markets also mark each one's index among the market's queued rows in the mask
+                auto to_queue = [&](u32, uint4 x, uint4 y, bool mine, bool is_new, u32 id, u32 pos, u32 pos_mkt) {
+                    if (!mine) return;
+                    const bool bid = (x.z & BB_F_BID) != 0u;
+                    if (pos < p.max_queue) {
+                        const u32 price = (x.z & BB_F_MARKET) ? (bid ? 0xFFFFFFFFu : 0u) : y.x;  // types.rs:160-172, 213-225
+                        const uint4 ev = make_uint4(is_new ? (1u | (bid ? 2u : 0u) | (y.z << 13)) : 0u, is_new ? id : x.w, price, y.y);
                         if constexpr (G::DENSE) sts128(qs + 16u * pos, ev);
                         else q[pos] = ev;
                     }
-                    if (is_cancel) max_cancel = max(max_cancel, oid == 0xFFFFFFFFu ? oid : oid + 1u);
-                    // the queue carries NEW and CANCEL only: a MODIFY row, or a trader id beyond 19 bits, is refused
-                    if (__any_sync(BB_FULL, bad_tick)) b.err |= ERR_PRICE;
-                    if (__any_sync(BB_FULL, op == BB_OP_MODIFY || (is_new && trader >= (1u << 19)))) b.err |= ERR_ROW_OP;
-                    e.next_id += __popc(nm);
-                    e.n += __popc(qm);
-                }
-                // a cancel of an id that does not exist by the end of submission is the reference's panic (orderbook.rs:642)
-                if (__reduce_max_sync(BB_FULL, max_cancel) > e.next_id) b.err |= ERR_BAD_ID;
+                    if (MKT && pos_mkt < cap) asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(mk_rm + 4u * (pos_mkt >> 5)), "r"(1u << (pos_mkt & 31u)) : "memory");
+                };
+                RowCount rows{e.next_id, e.n, 0u};
+                submit_rows<MKT, true>(g, p, b, off, m, m, mk_a, rows, to_queue);
+                e.next_id = rows.next;
+                e.n = rows.n;
+                mk_nr = rows.n_mkt;
                 __syncwarp();
-            }
-            if constexpr (EXT && MKT) {
-                // MarketEnv::place_order / cancel_order (market_env.rs:163-219) for the market's rows in row order: every
-                // book walks the whole slice; NEW rows take the next ids of their asset's book, rows naming no asset of the
-                // market queue nothing and flag book 0, each row's id is written by its asset's book (book 0: asset-less rows)
-                const u64 off = p.offsets[env / p.assets];
-                const u32 m = s == 0 ? (u32)(p.offsets[env / p.assets + 1] - off) : 0u;
-                const bb_instr* ins = p.instrs + off;
-                const u32 book0 = env - mk_a;
-                const u32 cap = p.assets * p.max_queue;  // queued rows beyond it drop the market's step (below)
-                const u32 nw = min((m + 31u) >> 5, mk_words);  // mask words the slice can touch
-                for (u32 w = lane; w < nw; w += 32) sts(mk_rm + 4u * w, 0u);
-                __syncwarp();
-                u32 max_cancel = 0;  // 1 + largest id a cancel row of this book names
-                for (u32 j0 = 0; j0 < m; j0 += 32) {
-                    const u32 j = j0 + lane;
-                    u32 of = 0, price = 0, vol = 0, trader = 0, oid = 0, asset = 0;
-                    if (j < m) {
-                        const uint4 x = reinterpret_cast<const uint4*>(ins + j)[0], y = reinterpret_cast<const uint4*>(ins + j)[1];
-                        of = x.z; oid = x.w; price = y.x; vol = y.y; trader = y.z; asset = y.w;
+                if constexpr (MKT) {
+                    // prefix counts: own queued rows in the words before each mask word
+                    u32 run = 0;
+                    for (u32 w0 = 0; w0 < nw; w0 += 32) {
+                        const u32 w = w0 + lane;
+                        u32 tot;
+                        const u32 c = w < nw ? __popc(lds(mk_rm + 4u * w)) : 0u;
+                        const u32 ex = warp_excl_scan(c, lane, &tot);
+                        if (w < nw) sts(mk_rm + 4u * (mk_words + w), run + ex);
+                        run += tot;
                     }
-                    const u32 op = of & BB_OP_MASK;
-                    const bool bid = (of & BB_F_BID) != 0u;
-                    const bool in_mkt = j < m && asset < p.assets;
-                    // create_order's tick check against the row's own asset (orderbook.rs:367-383); the in-kernel queue
-                    // carries NEW and CANCEL only, so a MODIFY row or a trader id beyond 19 bits is dropped and flagged
-                    const bool bad_tick = in_mkt && op == BB_OP_NEW && !(of & BB_F_MARKET) && (price % __ldg(g.ticks + book0 + asset) != 0u);
-                    const bool bad_op = in_mkt && (op == BB_OP_MODIFY || (op == BB_OP_NEW && trader >= (1u << 19)));
-                    const bool is_new = in_mkt && op == BB_OP_NEW && !bad_tick && !bad_op;
-                    const bool is_cancel = in_mkt && op == BB_OP_CANCEL;
-                    const bool queued = is_new || is_cancel, mine = queued && asset == mk_a;
-                    const u32 below = (1u << lane) - 1u;
-                    const u32 nm = __ballot_sync(BB_FULL, is_new && asset == mk_a), qm = __ballot_sync(BB_FULL, queued);
-                    const u32 om = __ballot_sync(BB_FULL, mine);
-                    const u32 id = e.next_id + __popc(nm & below), pos = e.n + __popc(om & below);
-                    const u32 xq = mk_nr + __popc(qm & below);  // the row's index among the market's queued rows
-                    if (of & BB_F_MARKET) price = bid ? 0xFFFFFFFFu : 0u;  // types.rs:160-172, 213-225
-                    if (p.out_ids && (in_mkt ? asset == mk_a : (j < m && mk_a == 0u)))
-                        p.out_ids[off + j] = is_new ? (u64)id : ~0ULL;
-                    if (mine) {
-                        if (pos < p.max_queue) {
-                            const uint4 ev = make_uint4(is_new ? (1u | (bid ? 2u : 0u) | (trader << 13)) : 0u, is_new ? id : oid, price, vol);
-                            if constexpr (G::DENSE) sts128(qs + 16u * pos, ev);
-                            else q[pos] = ev;
-                        }
-                        if (xq < cap) asm volatile("red.shared.or.b32 [%0], %1;" ::"r"(mk_rm + 4u * (xq >> 5)), "r"(1u << (xq & 31u)) : "memory");
-                    }
-                    if (is_cancel && asset == mk_a) max_cancel = max(max_cancel, oid == 0xFFFFFFFFu ? oid : oid + 1u);
-                    if (__any_sync(BB_FULL, bad_tick && asset == mk_a)) b.err |= ERR_PRICE;
-                    if (__any_sync(BB_FULL, bad_op && asset == mk_a)) b.err |= ERR_ROW_OP;
-                    if (__any_sync(BB_FULL, j < m && asset >= p.assets) && mk_a == 0u) b.err |= ERR_ROW_OP;
-                    e.next_id += __popc(nm);
-                    e.n += __popc(om);
-                    mk_nr += __popc(qm);
+                    __syncwarp();
                 }
-                if (__reduce_max_sync(BB_FULL, max_cancel) > e.next_id) b.err |= ERR_BAD_ID;
-                __syncwarp();
-                // prefix counts: own queued rows in the words before each mask word
-                u32 run = 0;
-                for (u32 w0 = 0; w0 < nw; w0 += 32) {
-                    const u32 w = w0 + lane;
-                    u32 tot;
-                    const u32 c = w < nw ? __popc(lds(mk_rm + 4u * w)) : 0u;
-                    const u32 ex = warp_excl_scan(c, lane, &tot);
-                    if (w < nw) sts(mk_rm + 4u * (mk_words + w), run + ex);
-                    run += tot;
-                }
-                __syncwarp();
             }
             if (e.n > p.max_queue) b.err |= ERR_CAP_QUEUE;
             u32 n = min(e.n, p.max_queue);

@@ -139,22 +139,19 @@ class DeviceArray:
             self.ptr = 0
 
 
-def _device_ptr(x, nbytes: int) -> typing.Optional[int]:
+def _device_array(x) -> typing.Optional[typing.Tuple[int, typing.Tuple[int, ...], np.dtype, typing.Any]]:
+    """(device address, shape, dtype, keep-alive object) of a C-contiguous CUDA array (CUDA array interface or DLPack), or
+    None for a host array.  The keep-alive object must outlive the launch that reads the array."""
     cai = getattr(x, "__cuda_array_interface__", None)
-    if cai is None:
-        if hasattr(x, "__dlpack__") and not isinstance(x, np.ndarray):   # DLPack-only producers
-            ptr, n, keep, _, _ = _dlpack_import(x)
-            if n != nbytes:
-                raise ValueError(f"device array holds {n} bytes, expected {nbytes}")
-            _device_ptr.keep = keep   # alive until the next call: the launch that reads it is already enqueued by then
-            return ptr
-        return None
-    if cai.get("strides") is not None:
-        raise ValueError("device arrays must be C-contiguous")
-    n = int(np.prod(cai["shape"])) * np.dtype(cai["typestr"]).itemsize
-    if n != nbytes:
-        raise ValueError(f"device array holds {n} bytes, expected {nbytes}")
-    return int(cai["data"][0])
+    if cai is not None:
+        if cai.get("strides") is not None:
+            raise ValueError("device arrays must be C-contiguous")
+        return int(cai["data"][0]), tuple(cai["shape"]), np.dtype(cai["typestr"]), x
+    if hasattr(x, "__dlpack__") and not isinstance(x, np.ndarray):   # DLPack-only producers
+        ptr, _, keep, shape, (code, bits) = _dlpack_import(x)
+        kind = "i" if code == KDL_INT else "u" if code == KDL_UINT else "V"
+        return ptr, shape, np.dtype(f"{kind}{bits // 8}"), keep
+    return None
 
 
 def pack_actions(op, bid=None, vol=None, trader=None, price=None, order_id=None, market=None, has_price=None, has_vol=None,
@@ -243,17 +240,11 @@ class _DeviceLoop:
         """(device address, k) of a [units, k] query block: the caller's device array (CUDA array interface or DLPack, any
         integer type of `dtype`'s size), or a staging copy of a host array."""
         dtype, units = np.dtype(dtype), self._units
-        cai = getattr(x, "__cuda_array_interface__", None)
-        if cai is not None:
-            shape, typ = tuple(cai["shape"]), np.dtype(cai["typestr"])
+        dev = _device_array(x)
+        if dev is not None:
+            ptr, shape, typ, self._keep = dev   # alive until the next call: the launch that reads it is already enqueued by then
             if len(shape) != 2 or shape[0] != units or typ.kind not in "iu" or typ.itemsize != dtype.itemsize:
                 raise ValueError(f"{name} must be a [{units}, k] array of {dtype.itemsize}-byte integers")
-            return _device_ptr(x, units * shape[1] * dtype.itemsize), int(shape[1])
-        if hasattr(x, "__dlpack__") and not isinstance(x, np.ndarray):
-            ptr, _, keep, shape, (code, bits) = _dlpack_import(x)
-            if len(shape) != 2 or shape[0] != units or code not in (KDL_INT, KDL_UINT) or bits != 8 * dtype.itemsize:
-                raise ValueError(f"{name} must be a [{units}, k] array of {dtype.itemsize}-byte integers")
-            _device_ptr.keep = keep   # alive until the next call: the launch that reads it is already enqueued by then
             return ptr, int(shape[1])
         a = np.ascontiguousarray(x, dtype=dtype)
         if a.ndim != 2 or a.shape[0] != units:
@@ -291,9 +282,14 @@ class _DeviceLoop:
 
     def _action_ptr(self, actions) -> int:
         """Device address of the step's action block: the caller's device array, or the staging copy of a host array."""
-        shape = self._actions.shape
-        ptr = _device_ptr(actions, self._actions.nbytes)
-        if ptr is None:  # host array: one H2D copy
+        shape, nbytes = self._actions.shape, self._actions.nbytes
+        dev = _device_array(actions)
+        if dev is not None:
+            ptr, dshape, typ, self._keep = dev   # alive until the next call: the launch that reads it is already enqueued by then
+            n = int(np.prod(dshape)) * typ.itemsize
+            if n != nbytes:
+                raise ValueError(f"device array holds {n} bytes, expected {nbytes}")
+        else:  # host array: one H2D copy
             a = np.ascontiguousarray(actions, dtype=ACTION_DTYPE)
             if a.shape != shape:
                 raise ValueError(f"actions must have shape {shape}")

@@ -238,7 +238,8 @@ int bb_step(bb_handle* h, uint32_t n_steps);
  * next order ids (d_out_ids[row], BB_NO_ID for every other row; may be NULL), BB_OP_CANCEL / BB_OP_MODIFY rows are queued,
  * BB_OP_NOOP and unknown codes queue nothing; then ONE Env::step.  A NEW row whose limit price is off the tick grid is
  * dropped, as when create_order returns PriceError, and flags the env with BB_ERR_PRICE (the next synchronous call
- * reports BB_EPRICE).  d_obs_out (device, [n_envs][obs_words], may be NULL) receives every env's end-of-step
+ * reports BB_EPRICE).  Only the first max_queue rows of an env's slice are submitted: the rows past them create and queue
+ * nothing (BB_NO_ID) and the env is flagged BB_ERR_CAP_QUEUE.  d_obs_out (device, [n_envs][obs_words], may be NULL) receives every env's end-of-step
  * observation record from the same launch — what StepEnvNumpy.level_1_data / level_2_data would return next.
  * Asynchronous on the handle's stream: one kernel launch and no host synchronisation, so the call may be recorded into a
  * CUDA graph together with the caller's own kernels (stream capture on the stream given to bb_set_stream). */
@@ -362,7 +363,8 @@ int bb_run_agents(bb_handle* h, uint64_t seed, uint32_t n_steps);
 /* ONE env-step of { agents.update(env); <the caller's rows>; env.step() } with the rows already in DEVICE memory: the loop of a
  * learning agent trading against the built-in background agents (SURVEY.md 8f rank 4).  Rows are laid out as for
  * bb_step_device and submitted after the agents' updates, in row order: BB_OP_NEW (ids in d_out_ids, BB_NO_ID elsewhere;
- * may be NULL) and BB_OP_CANCEL; no-op rows queue nothing; BB_OP_MODIFY rows are refused (BB_ERR_ROW_OP).  Everything
+ * may be NULL) and BB_OP_CANCEL; no-op rows queue nothing; BB_OP_MODIFY rows, and BB_OP_NEW rows whose trader id is >= 2^19,
+ * are dropped (BB_NO_ID, no id taken) and flag the env BB_ERR_ROW_OP.  Everything
  * takes part in the step's one Philox-keyed shuffle.  d_obs_out ([n_envs][obs_words], may be NULL) receives the
  * end-of-step records from the same launch.  Asynchronous on the handle's stream. */
 int bb_run_agents_with_rows(bb_handle* h, uint64_t seed, const bb_instr* d_instrs, const uint64_t* d_env_offsets, uint64_t n_rows,

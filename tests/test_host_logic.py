@@ -1,5 +1,7 @@
 """CPU suite for host-side logic that needs no GPU: action packing of the vectorised loop (bourse_b200.gym), the agent-group
 records built by the Rust-named constructors (bourse_b200.market / core), shard ranges, and the bench's synthetic policy."""
+import types
+
 import numpy as np
 import pytest
 
@@ -29,16 +31,18 @@ def test_pack_actions_broadcasts_to_blocks():
     assert a.nbytes == 4 * 3 * 2 * 32
 
 
-def test_device_pointer_extraction():
+def test_device_array_import():
     class Fake:
         def __init__(self, shape, typestr, strides=None):
             self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (0xABC000, False), "version": 3, "strides": strides}
-    assert gym._device_ptr(Fake((4, 2, 32), "|u1"), 256) == 0xABC000
-    assert gym._device_ptr(np.zeros(4), 32) is None           # host arrays take the copy path
-    with pytest.raises(ValueError, match="bytes"):
-        gym._device_ptr(Fake((4, 2), "<u4"), 256)
+    ptr, shape, dtype, _ = gym._device_array(Fake((4, 2, 32), "|u1"))
+    assert (ptr, shape, dtype) == (0xABC000, (4, 2, 32), np.dtype(np.uint8))
+    assert gym._device_array(np.zeros(4)) is None             # host arrays take the copy path
+    loop = types.SimpleNamespace(_actions=types.SimpleNamespace(shape=(4, 2), nbytes=256))
+    with pytest.raises(ValueError, match="bytes"):            # the action block's size is checked against the env's
+        gym._DeviceLoop._action_ptr(loop, Fake((4, 2), "<u4"))
     with pytest.raises(ValueError, match="contiguous"):
-        gym._device_ptr(Fake((4, 2, 32), "|u1", strides=(128, 64, 2)), 256)
+        gym._device_array(Fake((4, 2, 32), "|u1", strides=(128, 64, 2)))
 
 
 def test_market_agent_constructors_follow_the_rust_argument_order():
