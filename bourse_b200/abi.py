@@ -62,7 +62,7 @@ EXPORTS = [
     "bb_n_orders", "bb_n_trades", "bb_orders", "bb_trades", "bb_order_status", "bb_time", "bb_set_time",
     "bb_set_trading", "bb_env_errors", "bb_stats", "bb_history_device", "bb_order_keys", "bb_load_book",
     "bb_set_agents_market", "bb_step_device", "bb_level2_device", "bb_level1_device", "bb_device_alloc", "bb_device_free", "bb_memcpy", "bb_run_agents_with_rows", "bb_reserve", "bb_reserve_queue", "bb_clear_history", "bb_clear_errors",
-    "bb_orders_all", "bb_trades_all", "bb_set_tick_sizes", "bb_step_device_market", "bb_run_agents_with_rows_market", "bb_orders_device", "bb_trades_device", "bb_comm_unique_id", "bb_comm_init_rank", "bb_comm_init_all", "bb_comm_n_ranks", "bb_comm_destroy", "bb_comm_last_error", "bb_gather_stats",
+    "bb_orders_all", "bb_trades_all", "bb_set_tick_sizes", "bb_step_device_market", "bb_run_agents_with_rows_market", "bb_orders_device", "bb_trades_device", "bb_reset_device", "bb_comm_unique_id", "bb_comm_init_rank", "bb_comm_init_all", "bb_comm_n_ranks", "bb_comm_destroy", "bb_comm_last_error", "bb_gather_stats",
 ]
 
 _lib = None
@@ -113,6 +113,7 @@ def load() -> C.CDLL:
     sig("bb_step_device_market", i32, vp, vp, vp, u64, vp, vp)
     sig("bb_orders_device", i32, vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, vp)
     sig("bb_trades_device", i32, vp, vp, u32, vp, vp, vp, vp, vp, vp, vp)
+    sig("bb_reset_device", i32, vp, vp, vp, vp, vp)
     sig("bb_level2_device", i32, vp, vp)
     sig("bb_level1_device", i32, vp, vp)
     sig("bb_device_alloc", i32, vp, u64, P(vp))

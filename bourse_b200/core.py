@@ -262,6 +262,14 @@ class BatchedEnv:
         self._ck(self._lib.bb_trades_device(self._h, p(d_cursor_ptr), cap, p(count), p(t), p(side_is_bid), p(price), p(vol),
                                             p(active_id), p(passive_id)))
 
+    def reset_device(self, mask_ptr: int, seeds_ptr: int = 0, obs_ptr: int = 0, cursor_ptr: int = 0):
+        """Reset the units (envs, or markets on a multi-asset handle) whose u8 entry of the device mask `mask_ptr` is
+        non-zero (bb_reset_device); asynchronous.  `seeds_ptr`: u64 [units] re-seeding them, or 0 to continue their random
+        streams.  `obs_ptr` [n_envs, obs_words] receives the fresh records of reset books, `cursor_ptr` (u32 [n_envs], a
+        trades_device cursor) has their entries zeroed."""
+        p = C.c_void_p
+        self._ck(self._lib.bb_reset_device(self._h, p(mask_ptr), p(seeds_ptr or None), p(obs_ptr or None), p(cursor_ptr or None)))
+
     def level_2_data_device(self, d_out_ptr: int): self._ck(self._lib.bb_level2_device(self._h, C.c_void_p(d_out_ptr)))
     def level_1_data_device(self, d_out_ptr: int): self._ck(self._lib.bb_level1_device(self._h, C.c_void_p(d_out_ptr)))
 

@@ -296,13 +296,25 @@ int upload_seeds(bb_handle* h) {
     return BB_OK;
 }
 
-// asynchronous on the handle's stream: one small kernel rewrites every book header and page directory
-int init_books(bb_handle* h) {
+// one small kernel rewrites the header and page directory (or window) of every book, or of the units r.mask selects
+int launch_init(bb_handle* h, const ResetArgs& r) {
     const bb_config& c = h->cfg;
-    if (h->eng == ENG_DEEP) {
+    if (h->eng == ENG_DEEP)
         k_init_deep<<<c.n_envs, 128, 0, h->stream>>>(h->blobs, h->blob_stride, c.n_envs, c.start_time, c.trading ? 1u : 0u, h->d_seeds,
-                                                     h->dp.bm, h->dp.lht - h->dp.bm);  // bitmaps, summaries, level volumes and order counts start at zero
-        CUDA_TRY(h, cudaGetLastError());
+                                                     h->dp.bm, h->dp.lht - h->dp.bm, r);  // bitmaps, summaries, level volumes and order counts start at zero
+    else
+        k_init<<<c.n_envs, 64, 0, h->stream>>>(h->blobs, h->blob_stride, c.n_envs, h->p_total, c.start_time, c.trading ? 1u : 0u,
+                                               h->d_seeds, h->rslot, h->agents_per_env, h->mom, h->mom_groups, h->mom_stride, h->dgeo,
+                                               h->dense_lp, h->dense_nwmax, r);
+    CUDA_TRY(h, cudaGetLastError());
+    return BB_OK;
+}
+
+// asynchronous on the handle's stream
+int init_books(bb_handle* h) {
+    int rc = launch_init(h, ResetArgs{nullptr, nullptr, 1u, nullptr, 0u, nullptr});
+    if (rc) return rc;
+    if (h->eng == ENG_DEEP) {
         CUDA_TRY(h, cudaMemsetAsync(h->err_flag, 0, 4, h->stream));
         h->status_valid = false;
         for (auto& q : h->queue) q.clear();
@@ -311,9 +323,6 @@ int init_books(bb_handle* h) {
         h->recorded_host = 0;
         return BB_OK;
     }
-    k_init<<<c.n_envs, 64, 0, h->stream>>>(h->blobs, h->blob_stride, c.n_envs, h->p_total, c.start_time, c.trading ? 1u : 0u,
-                                           h->d_seeds, h->rslot, h->agents_per_env, h->mom, h->mom_groups, h->mom_stride, h->dgeo, h->dense_lp, h->dense_nwmax);
-    CUDA_TRY(h, cudaGetLastError());
     CUDA_TRY(h, cudaMemsetAsync(h->err_flag, 0, 4, h->stream));
     h->status_valid = false;
     for (auto& q : h->queue) q.clear();
@@ -672,6 +681,30 @@ int bb_reset(bb_handle* h) {
     CHECK_H(h);
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     return init_books(h);
+}
+
+int bb_reset_device(bb_handle* h, const uint8_t* d_mask, const uint64_t* d_seeds, uint32_t* d_obs_out, uint32_t* d_cursor) {
+    CHECK_H(h);
+    if (!d_mask) return fail(h, BB_EINVAL, "null argument");
+    int rc = refuse_pending_queue(h);
+    if (rc) return rc;
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    const bool market_seeds = h->assets > 1 && d_seeds;
+    if (market_seeds && h->market_rng_at == bb_handle::RNG_HOST_AHEAD) {
+        // the markets that are not reset keep their streams, whose current copy is the host's: bring the books' copies up to
+        // date first, never inside a stream capture (the graph would replay a copy of the streams as they are now)
+        if (stream_capturing(h))
+            return fail(h, BB_EINVAL, "bb_reset_device: the markets' shuffle streams last advanced in bb_step; call "
+                                      "bb_step_device_market or a seeded bb_reset_device once outside the capture (or bb_reset) "
+                                      "before capturing it");
+        if ((rc = market_rng_to_device(h))) return rc;
+    }
+    if ((rc = launch_init(h, ResetArgs{d_mask, d_seeds, h->assets, d_obs_out, h->cfg.obs_words, d_cursor}))) return rc;
+    h->mirror_dirty = true;  // reset books hold no orders now
+    h->status_valid = false;
+    // (recorded_host is left as it is: reset books' record counts only fall, so it still bounds every env's count)
+    if (market_seeds) h->market_rng_at = bb_handle::RNG_DEVICE_AHEAD;
+    return BB_OK;
 }
 
 // KParams::rand_tick_mask: bit gi for a RandomAgents group that trades some book whose tick does not divide its tick_size.
@@ -1215,10 +1248,12 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
     if (stream_capturing(h)) return fail(h, BB_EINVAL, "agent launches cannot be captured into a CUDA graph (bb_step_device can)");
     // history capacity is validated up front so the kernel can stage records without per-step checks
     if (h->recorded_host < 0) {  // after a replay the number of emitted records is only known to the device
-        CUDA_TRY(h, cudaMemcpy2DAsync(h->h_offsets, 8, h->blobs + offsetof(BookHdr, n_steps), h->blob_stride, 4, 1,
+        // the largest count of any env: after bb_reset_device the envs' counts differ
+        std::vector<u32> n(h->cfg.n_envs);
+        CUDA_TRY(h, cudaMemcpy2DAsync(n.data(), 4, h->blobs + offsetof(BookHdr, n_steps), h->blob_stride, 4, h->cfg.n_envs,
                                       cudaMemcpyDeviceToHost, h->stream));
         CUDA_TRY(h, cudaStreamSynchronize(h->stream));
-        h->recorded_host = *(u32*)h->h_offsets;
+        h->recorded_host = *std::max_element(n.begin(), n.end());
     }
     if ((u64)h->recorded_host + n_steps > h->max_steps_padded) return fail(h, BB_ECAP, "max_steps exceeded");
     // agents plus market rows: the market variants' layout with the row mask behind the permutation (only that variant has it)

@@ -1675,23 +1675,72 @@ template <int ENG> __global__ void __launch_bounds__(128) k_snapshot(const __gri
     }
 }
 
-// fresh-book initialisation (OrderBook::new orderbook.rs:158-171 + Env::new env.rs:84-95)
-__global__ void k_init(unsigned char* blobs, u64 blob_stride, u32 n_envs, u32 p_total, u64 start_time, u32 trading,
-                       const u64* rng_seeds, u32* rslot, u32 agents_per_env, MomState* mom, u32 mom_per_env, u32 mom_stride, Geo dense,
-                       u32 dense_lp, u32 dense_nwmax) {
-    const u32 env = blockIdx.x;
-    if (env >= n_envs) return;
-    unsigned char* b = blobs + (size_t)env * blob_stride;
-    if (threadIdx.x == 0) {
-        BookHdr h;
-        memset(&h, 0, sizeof(h));
-        h.t = start_time;
-        h.trading = trading;
+// bb_reset_device: which units k_init / k_init_deep reset and what else the launch writes.  mask == nullptr: every book,
+// from the handle's creation seeds (bb_create, bb_reset).  A unit is an env, or a market of `assets` books.
+struct ResetArgs {
+    const uint8_t* mask;  // [units]; 0 leaves the unit's books untouched
+    const u64* seeds;     // [units] or nullptr: re-seed the unit's shuffle stream and restart its step counter, or keep both
+    u32 assets;
+    u32* obs;             // [n_envs][obs_words] or nullptr: the fresh book's record (bb_level1_device / bb_level2_device)
+    u32 obs_words;
+    u32* cursor;          // [n_envs] or nullptr: a bb_trades_device cursor, zeroed for reset books
+};
+
+// thread 0 of a book's CTA: the fresh header (OrderBook::new orderbook.rs:158-171 + Env::new env.rs:84-95) with its random
+// streams.  A masked reset reads the old header's stream and step counter before the caller overwrites it.
+__device__ __forceinline__ BookHdr fresh_hdr(const unsigned char* b, u32 env, u64 start_time, u32 trading, const u64* rng_seeds,
+                                             const ResetArgs& r) {
+    BookHdr h;
+    memset(&h, 0, sizeof(h));
+    h.t = start_time;
+    h.trading = trading;
+    if (!r.mask) {
         h.rng_s0 = rng_seeds[2 * env];
         h.rng_s1 = rng_seeds[2 * env + 1];
+    } else if (r.seeds) {  // Xoroshiro128StarStar::seed_from_u64: two SplitMix64 outputs (as upload_seeds on the host)
+        u64 x = r.seeds[env / r.assets];
+        u64 z[2];
+        for (int i = 0; i < 2; ++i) {
+            x += 0x9e3779b97f4a7c15ULL;
+            u64 y = x;
+            y = (y ^ (y >> 30)) * 0xbf58476d1ce4e5b9ULL;
+            y = (y ^ (y >> 27)) * 0x94d049bb133111ebULL;
+            z[i] = y ^ (y >> 31);
+        }
+        h.rng_s0 = z[0];
+        h.rng_s1 = z[1];
+    } else {
+        const BookHdr* old = reinterpret_cast<const BookHdr*>(b);
+        h.rng_s0 = old->rng_s0;
+        h.rng_s1 = old->rng_s1;
+        h.step_counter = old->step_counter;
+    }
+    return h;
+}
+
+// what a reset book's CTA writes besides its blob: the fresh record (an empty book: ask = 0xFFFFFFFF, every other word 0)
+// and its trade cursor
+__device__ __forceinline__ void reset_outputs(u32 env, const ResetArgs& r) {
+    if (r.obs)
+        for (u32 i = threadIdx.x; i < r.obs_words; i += blockDim.x) r.obs[(size_t)env * r.obs_words + i] = i == 2u ? 0xFFFFFFFFu : 0u;
+    if (r.cursor && threadIdx.x == 0) r.cursor[env] = 0u;
+}
+
+// fresh-book initialisation (OrderBook::new orderbook.rs:158-171 + Env::new env.rs:84-95), of every book or of the units
+// r.mask selects
+__global__ void k_init(unsigned char* blobs, u64 blob_stride, u32 n_envs, u32 p_total, u64 start_time, u32 trading,
+                       const u64* rng_seeds, u32* rslot, u32 agents_per_env, MomState* mom, u32 mom_per_env, u32 mom_stride, Geo dense,
+                       u32 dense_lp, u32 dense_nwmax, ResetArgs r) {
+    const u32 env = blockIdx.x;
+    if (env >= n_envs) return;
+    if (r.mask && !r.mask[env / r.assets]) return;
+    unsigned char* b = blobs + (size_t)env * blob_stride;
+    if (threadIdx.x == 0) {
+        BookHdr h = fresh_hdr(b, env, start_time, trading, rng_seeds, r);
         h.free_top = dense.d_live;
         *reinterpret_cast<BookHdr*>(b) = h;
     }
+    reset_outputs(env, r);
     if (dense_lp) {  // dense engine (DenseLayout<dense_lp, dense_nwmax>): empty bitmaps, every slot free
         const u32 off_fs = 128u + 12u * dense_lp, off_bm = off_fs + dense_lp;
         u32* bm = reinterpret_cast<u32*>(b + off_bm);
@@ -1720,18 +1769,14 @@ __global__ void k_init(unsigned char* blobs, u64 blob_stride, u32 n_envs, u32 p_
 
 // fresh deep book (deep.cuh image): header, empty bitmaps, chunk 0 reserved as a sink
 __global__ void k_init_deep(unsigned char* blobs, u64 blob_stride, u32 n_envs, u64 start_time, u32 trading, const u64* rng_seeds,
-                            u32 off_bm, u32 bm_bytes) {
+                            u32 off_bm, u32 bm_bytes, ResetArgs r) {
     const u32 env = blockIdx.x;
     if (env >= n_envs) return;
+    if (r.mask && !r.mask[env / r.assets]) return;
     unsigned char* b = blobs + (size_t)env * blob_stride;
+    reset_outputs(env, r);
     if (threadIdx.x == 0) {
-        BookHdr h;
-        memset(&h, 0, sizeof(h));
-        h.t = start_time;
-        h.trading = trading;
-        h.rng_s0 = rng_seeds[2 * env];
-        h.rng_s1 = rng_seeds[2 * env + 1];
-        *reinterpret_cast<BookHdr*>(b) = h;
+        *reinterpret_cast<BookHdr*>(b) = fresh_hdr(b, env, start_time, trading, rng_seeds, r);
         *reinterpret_cast<u32*>(b + DP_OFF_BUMP) = 1u;
         *reinterpret_cast<u32*>(b + DP_OFF_NFREE) = 0u;
     }

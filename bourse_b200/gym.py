@@ -31,7 +31,7 @@ from . import abi
 from .core import BatchedEnv
 
 # ---- DLPack (dlpack.h, v0.8 ABI: DLManagedTensor in a PyCapsule named "dltensor"), pure ctypes ---------------------------
-KDL_CUDA, KDL_INT, KDL_UINT = 2, 0, 1
+KDL_CUDA, KDL_INT, KDL_UINT, KDL_BOOL = 2, 0, 1, 6
 
 
 class _DLDevice(C.Structure):
@@ -149,7 +149,7 @@ def _device_array(x) -> typing.Optional[typing.Tuple[int, typing.Tuple[int, ...]
         return int(cai["data"][0]), tuple(cai["shape"]), np.dtype(cai["typestr"]), x
     if hasattr(x, "__dlpack__") and not isinstance(x, np.ndarray):   # DLPack-only producers
         ptr, _, keep, shape, (code, bits) = _dlpack_import(x)
-        kind = "i" if code == KDL_INT else "u" if code == KDL_UINT else "V"
+        kind = "i" if code == KDL_INT else "u" if code == KDL_UINT else "b" if code == KDL_BOOL and bits == 8 else "V"
         return ptr, shape, np.dtype(f"{kind}{bits // 8}"), keep
     return None
 
@@ -220,11 +220,55 @@ class _DeviceLoop:
         (self.env.level_1_data_device if self.obs_words == abi.OBS_L1 else self.env.level_2_data_device)(self.obs.ptr)
         return self.obs
 
-    def reset(self) -> DeviceArray:
-        self._n_steps = 0
-        self.env.reset()   # (the agent population survives a reset; its state is cleared with the books)
-        self._cursor.copy_from_host(np.zeros(self.env.n_envs, np.uint32))
-        return self._observe()
+    def reset(self, mask=None, seeds=None) -> DeviceArray:
+        """Without `mask`: every env back to its freshly created state (`bb_reset`), the trade cursor zeroed.
+
+        With `mask`, a `[units]` array (`units` = `n_envs`, or `n_markets` for `MarketVectorEnv`), only the units whose entry
+        is non-zero are reset — gymnasium's per-env autoreset (bb_reset_device): their books are emptied, their history,
+        order table, trade log and error bits restart at 0, their agents' state is cleared; every other unit is untouched.
+        `mask` is a device array (CUDA array interface or DLPack: a torch `bool` / `uint8` tensor) or a numpy `bool` /
+        `uint8` array (copied into a staging buffer).  `seeds` (same shape, 8-byte integers, device or numpy) re-seeds
+        the reset units' shuffle streams as `StepEnvNumpy(seed, ...)` / `MarketEnv` construction does and restarts their
+        step counters, so a unit reset with its creation seed (`seed + e`) replays episode 1 under the same actions; without
+        `seeds` the streams continue (the next episode draws what the unit would have drawn without the reset, agent draws
+        included).  One launch writes the reset units' rows of `self.obs` (the fresh record) and zeroes their entries of
+        the `trades` cursor; returns `self.obs`.
+
+        Order ids the learner holds for a reset env are void: a CANCEL of one flags `BB_ERR_BAD_ID` as any unknown id does.
+        `self.obs` is overwritten for reset units: copy the final observation first if it is needed.  With device arrays
+        for `mask` and `seeds` the call has no host synchronisation and can be captured into a CUDA graph together with
+        `step` (a seeded `MarketVectorEnv` reset right after host-side `bb_step` shuffles refuses capture)."""
+        if mask is None:
+            if seeds is not None:
+                raise ValueError("seeds re-seed the units a mask selects: pass a mask")
+            self._n_steps = 0
+            self.env.reset()   # (the agent population survives a reset; its state is cleared with the books)
+            self._cursor.copy_from_host(np.zeros(self.env.n_envs, np.uint32))
+            return self._observe()
+        mask_ptr, keep_mask = self._unit_array(mask, np.uint8, "mask")
+        seeds_ptr, keep_seeds = self._unit_array(seeds, np.uint64, "seeds") if seeds is not None else (0, None)
+        self._keep = (keep_mask, keep_seeds)   # alive until the next call, as in _action_ptr
+        self.env.reset_device(mask_ptr, seeds_ptr, self.obs.ptr, self._cursor.ptr)
+        return self.obs
+
+    def _unit_array(self, x, dtype, name) -> typing.Tuple[int, typing.Any]:
+        """(device address, keep-alive object) of a [units] mask (bool / 1-byte integers) or seed array (8-byte integers):
+        the caller's device array, or a staging copy of a host array."""
+        dtype, units = np.dtype(dtype), self._units
+        kinds = "biu" if dtype.itemsize == 1 else "iu"
+        what = f"{name} must be a [{units}] array of " + ("bool or 1-byte integers" if dtype.itemsize == 1 else "8-byte integers")
+        dev = _device_array(x)
+        if dev is not None:
+            ptr, shape, typ, keep = dev
+            if shape != (units,) or typ.kind not in kinds or typ.itemsize != dtype.itemsize:
+                raise ValueError(what)
+            return ptr, keep
+        a = np.asarray(x)
+        if a.shape != (units,) or a.dtype.kind not in kinds or (dtype.itemsize == 1 and a.dtype.itemsize != 1):
+            raise ValueError(what)
+        buf = self._buffer((name,), (units,), dtype)
+        buf.copy_from_host(a.astype(dtype))
+        return buf.ptr, None
 
     def _buffer(self, key, shape, dtype) -> DeviceArray:
         if key not in self._reads:

@@ -328,6 +328,39 @@ int bb_orders_device(bb_handle* h, const uint64_t* d_ids, const uint32_t* d_asse
  * call may be recorded into a CUDA graph. */
 int bb_trades_device(bb_handle* h, uint32_t* d_cursor, uint32_t cap, uint32_t* d_count, uint64_t* d_t, uint8_t* d_side_is_bid,
                      uint32_t* d_price, uint32_t* d_vol, uint64_t* d_active_id, uint64_t* d_passive_id);
+/* Per-unit reset for the device-resident loops: end the episodes of some envs (a unit is an env on a single-asset handle and
+ * a market of `assets` books on a multi-asset one, as in bb_orders_device) while the others keep running — gymnasium's
+ * per-env autoreset, with the done mask computed on the device.  All pointers are device pointers.
+ *   d_mask [units] (required): a non-zero entry resets the unit.  Every book of a reset unit returns to what bb_reset makes
+ *     it: an empty book at start_time with the config's trading flag; order count, trade log and history count at 0; sticky
+ *     error word and header counters zeroed; its in-kernel agents' state cleared (RandomAgents held ids, MomentumAgent /
+ *     NoiseAgent state and live lists).  It keeps its tick size, the agent groups and all else bb_reset keeps.  So a
+ *     book's order table and trade log start again from slot 0: each env recycles max_orders / max_trades at its own
+ *     episode boundary.  Books of units whose entry is 0 are not touched.
+ *   d_seeds [units] or NULL: the unit's random streams.  NULL: they continue — the Xoroshiro128** shuffle state and the
+ *     step counter (the `step` word of every agent's Philox draw) keep their values, so the next episode draws the shuffles
+ *     and agent draws the unit would have drawn without the reset.  Non-NULL: the unit's shuffle stream becomes
+ *     Xoroshiro128StarStar::seed_from_u64(d_seeds[u]) (every book of a market gets the market's stream) and its step
+ *     counter restarts at 0.  A unit re-seeded with its creation seed (seed + env_id_base + e; markets
+ *     seed + env_id_base / assets + m) is therefore bit-identical from then on to that unit of a freshly created handle.
+ *     The agents' Philox key is (launch seed, global env / market id, step): a seeded reset replays the creation-time agent
+ *     draws as well, fresh agent draws come from an unseeded reset (or a new launch seed).
+ *   d_obs_out [n_envs][obs_words] or NULL: the rows of reset books receive the fresh book's record, what bb_level1_device /
+ *     bb_level2_device return for them right after the reset; other rows are not written.
+ *   d_cursor [n_envs] or NULL: a bb_trades_device cursor array; the entries of reset books are zeroed, so the next read
+ *     reports the new episode's trades from log index 0.
+ * Order ids a caller holds for a reset book are void: a later CANCEL of one flags BB_ERR_BAD_ID as any unknown id does.
+ * bb_stats counts from the reset on for reset books (their counters restart at 0); its env_steps is the sum of the step
+ * counters, so it keeps an unseeded unit's steps and drops a seeded unit's.  bb_n_steps of a reset book is 0, so the envs'
+ * history counts differ afterwards: bb_run_agents_to_host, which streams every env's records from one common index, needs
+ * a bb_clear_history first.
+ * On a multi-asset handle right after a bb_step that shuffled, a seeded reset first copies the host's streams of the
+ * markets to the books (synchronous); inside a stream capture that case is refused with BB_EINVAL.  An unseeded reset
+ * leaves every market's stream where it is.  Every engine: paged, dense and deep (the deep engine has no shuffle or agents:
+ * only d_mask, d_obs_out and d_cursor matter there).  Refused with BB_EINVAL, the handle unchanged, for a NULL handle or
+ * d_mask, while host-queued instructions are pending, and in the capture case above.  Asynchronous on the handle's stream:
+ * one launch, no host synchronisation and no allocation, so the call may be recorded into a CUDA graph with the steps. */
+int bb_reset_device(bb_handle* h, const uint8_t* d_mask, const uint64_t* d_seeds, uint32_t* d_obs_out, uint32_t* d_cursor);
 /* Device buffers for callers without a CUDA allocator of their own (numpy-only hosts); any device pointer works above.
  * bb_memcpy kind: 1 host to device, 2 device to host, 3 device to device; synchronous on the handle's stream. */
 int bb_device_alloc(bb_handle* h, uint64_t bytes, void** d_ptr);

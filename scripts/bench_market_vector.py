@@ -20,9 +20,16 @@ events around 200 back-to-back calls on the books a window left behind, issued f
 (`time_calls`).  Those trades() calls find no new trades: they read the headers and write the padded windows.  The k = 8
 queried ids per env / market are fixed ids below 500 (every book has issued them after the warm-up steps).
 
+--resets measures the per-unit reset (bb_reset_device, `reset(mask)`) in the rows-only loops on the FAST engine, for 4096
+single-asset envs (VectorEnv) and 2048 markets x 4 assets (MarketVectorEnv): the time per step of the step alone and of
+the step followed by `reset(mask)` with 0 %, 1 % and 100 % of the units selected (fixed device masks).  Each variant is
+captured once as a CUDA graph of 100 steps and replayed from reset books, timed with CUDA events; the plain and with-reset
+passes alternate, --passes times each, and the best pass of each counts.
+
     python scripts/bench_market_vector.py --steps 1000 --warmup 20
     python scripts/bench_market_vector.py --bg-agents --steps 1000 --warmup 20
     python scripts/bench_market_vector.py --reads --steps 1000 --warmup 20
+    python scripts/bench_market_vector.py --resets --passes 3
 """
 from __future__ import annotations
 
@@ -192,6 +199,61 @@ def bench_reads(args, name, power):
     return res
 
 
+def bench_resets(args, name, power):
+    """--resets: see the module docstring."""
+    import torch
+    K, n_envs = 100, N_BOOKS // 2
+    res = {"card": name, "power_limit": power, "engine": "fast", "agents": None, "steps_per_graph": K, "passes": args.passes,
+           "rows_per_book": ROWS_PER_BOOK, "us_per_step": {}, "errors": {}}
+    fractions = (("reset_0pct", 0.0), ("reset_1pct", 0.01), ("reset_100pct", 1.0))
+    for label, units in (("vector_env_4096", n_envs), ("market_vector_2048x4", N_MARKETS)):
+        books = units if label.startswith("vector") else N_BOOKS
+        blocks = gym_action_blocks(min(args.blocks, K), books, ROWS_PER_BOOK, seed=5)
+        if label.startswith("vector"):
+            loop = gym.VectorEnv(n_envs, ROWS_PER_BOOK, 0, 0, 1, 1000, **KW)
+        else:
+            loop = gym.MarketVectorEnv(N_MARKETS, ROWS, 0, 0, [1] * ASSETS, 1000, **KW)
+            blocks = market_blocks(blocks)
+        d_blocks = [torch.from_numpy(x.view(np.uint8).reshape(units, -1)).cuda() for x in blocks]
+        rng = np.random.default_rng(3)
+        masks = {tag: torch.from_numpy(rng.permutation(units) < round(f * units)).cuda() for tag, f in fractions}
+        stream = torch.cuda.Stream()
+        loop.env.set_stream(stream.cuda_stream)
+        torch.cuda.synchronize()
+        with torch.cuda.stream(stream):   # the first launches query kernel attributes: outside any capture
+            loop.step(d_blocks[0])
+            loop.reset(masks["reset_1pct"])
+        graphs = {}
+        for tag in ("plain",) + tuple(t for t, _ in fractions):
+            loop.reset()   # (also restarts the history ring of VectorEnv.step, so no clear is captured)
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g, stream=stream):
+                for s in range(K):
+                    loop.step(d_blocks[s % len(d_blocks)])
+                    if tag != "plain":
+                        loop.reset(masks[tag])
+            graphs[tag] = g
+        for _ in range(args.passes):   # plain and with-reset graphs alternate
+            for tag, g in graphs.items():
+                loop.reset()
+                stream.synchronize()
+                t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                t0.record(stream)
+                with torch.cuda.stream(stream):
+                    g.replay()
+                t1.record(stream)
+                stream.synchronize()
+                res["us_per_step"].setdefault(f"{label}_{tag}", []).append(t0.elapsed_time(t1) * 1e3 / K)
+                res["errors"][f"{label}_{tag}"] = res["errors"].get(f"{label}_{tag}", 0) | int(np.bitwise_or.reduce(loop.env.env_errors()))
+        plain = min(res["us_per_step"][f"{label}_plain"])
+        for tag, _ in fractions:
+            res["us_per_step"][f"{label}_added_by_{tag}"] = min(res["us_per_step"][f"{label}_{tag}"]) - plain
+        del graphs
+        loop.env.set_stream(0)
+        loop.close()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=1000)
@@ -199,6 +261,8 @@ def main():
     ap.add_argument("--blocks", type=int, default=64, help="distinct action blocks, cycled")
     ap.add_argument("--bg-agents", action="store_true", help="the C3 population trades in every book (see the module docstring)")
     ap.add_argument("--reads", action="store_true", help="time orders() / trades() in the C3 loops (see the module docstring)")
+    ap.add_argument("--resets", action="store_true", help="time reset(mask) in the rows-only loops (see the module docstring)")
+    ap.add_argument("--passes", type=int, default=3, help="--resets: timed passes of each variant")
     args = ap.parse_args()
     import torch
 
@@ -206,6 +270,9 @@ def main():
     print(f"card: {name}, power limit: {power}", flush=True)
     if args.reads:
         print(json.dumps(bench_reads(args, name, power)), flush=True)
+        return
+    if args.resets:
+        print(json.dumps(bench_resets(args, name, power)), flush=True)
         return
     blocks = gym_action_blocks(args.blocks, N_BOOKS, ROWS_PER_BOOK, seed=5)
     if args.bg_agents:   # limit prices into the agents' range, as bench.py run_gym does
