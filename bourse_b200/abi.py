@@ -19,6 +19,7 @@ OBS_L1, OBS_L2 = 9, 45
 NO_ID = 2**64 - 1
 STATUS_NONE = 0xFF   # bb_orders_device: status of a query that names no order
 ALL_ENVS = 0xFFFFFFFF
+NO_SLOT = 0xFFFFFFFF   # bb_save_device / bb_restore_device: leave this slot / unit as it is
 OP_NOOP, OP_NEW, OP_CANCEL, OP_MODIFY, OP_SET_TRADING, OP_RESTORE = 0, 1, 2, 3, 4, 5
 F_BID, F_MARKET, F_HAS_PRICE, F_HAS_VOL, F_EMIT = 1 << 8, 1 << 9, 1 << 10, 1 << 11, 1 << 12
 ACT_NOOP, ACT_NEW, ACT_CANCEL, ACT_MODIFY = 0, 1, 2, 3
@@ -62,7 +63,7 @@ EXPORTS = [
     "bb_n_orders", "bb_n_trades", "bb_orders", "bb_trades", "bb_order_status", "bb_time", "bb_set_time",
     "bb_set_trading", "bb_env_errors", "bb_stats", "bb_history_device", "bb_order_keys", "bb_load_book",
     "bb_set_agents_market", "bb_step_device", "bb_level2_device", "bb_level1_device", "bb_device_alloc", "bb_device_free", "bb_memcpy", "bb_run_agents_with_rows", "bb_reserve", "bb_reserve_queue", "bb_clear_history", "bb_clear_errors",
-    "bb_orders_all", "bb_trades_all", "bb_set_tick_sizes", "bb_step_device_market", "bb_run_agents_with_rows_market", "bb_orders_device", "bb_trades_device", "bb_reset_device", "bb_comm_unique_id", "bb_comm_init_rank", "bb_comm_init_all", "bb_comm_n_ranks", "bb_comm_destroy", "bb_comm_last_error", "bb_gather_stats",
+    "bb_orders_all", "bb_trades_all", "bb_set_tick_sizes", "bb_step_device_market", "bb_run_agents_with_rows_market", "bb_orders_device", "bb_trades_device", "bb_reset_device", "bb_store_create", "bb_store_destroy", "bb_save_device", "bb_restore_device", "bb_comm_unique_id", "bb_comm_init_rank", "bb_comm_init_all", "bb_comm_n_ranks", "bb_comm_destroy", "bb_comm_last_error", "bb_gather_stats",
 ]
 
 _lib = None
@@ -114,6 +115,10 @@ def load() -> C.CDLL:
     sig("bb_orders_device", i32, vp, vp, vp, u64, vp, vp, vp, vp, vp, vp, vp, vp)
     sig("bb_trades_device", i32, vp, vp, u32, vp, vp, vp, vp, vp, vp, vp)
     sig("bb_reset_device", i32, vp, vp, vp, vp, vp)
+    sig("bb_store_create", i32, vp, u32, P(vp), P(u64))
+    sig("bb_store_destroy", i32, vp)
+    sig("bb_save_device", i32, vp, vp, vp)
+    sig("bb_restore_device", i32, vp, vp, vp, vp, vp, vp)
     sig("bb_level2_device", i32, vp, vp)
     sig("bb_level1_device", i32, vp, vp)
     sig("bb_device_alloc", i32, vp, u64, P(vp))

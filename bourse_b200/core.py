@@ -270,6 +270,30 @@ class BatchedEnv:
         p = C.c_void_p
         self._ck(self._lib.bb_reset_device(self._h, p(mask_ptr), p(seeds_ptr or None), p(obs_ptr or None), p(cursor_ptr or None)))
 
+    def store_create(self, n_slots: int, allocate: bool = True) -> typing.Tuple[int, int]:
+        """(store handle, bytes) of a device store of `n_slots` unit snapshots (bb_store_create), sized from the current
+        capacities; with `allocate=False` only the size is computed and the handle is 0.  Free it with `store_destroy`
+        (the env's `close` frees every store left)."""
+        s, nbytes = C.c_void_p(), C.c_uint64()
+        self._ck(self._lib.bb_store_create(self._h, n_slots, C.byref(s) if allocate else None, C.byref(nbytes)))
+        return (s.value or 0), nbytes.value
+
+    def store_destroy(self, store: int): self._ck(self._lib.bb_store_destroy(C.c_void_p(store)))
+
+    def save_device(self, store: int, units_ptr: int):
+        """Slot k of `store` receives unit u32 [n_slots] `units_ptr`[k] (bb_save_device; NO_SLOT keeps the slot, a unit
+        index >= units empties it); asynchronous."""
+        self._ck(self._lib.bb_save_device(self._h, C.c_void_p(store), C.c_void_p(units_ptr)))
+
+    def restore_device(self, store: int, slots_ptr: int, seeds_ptr: int = 0, obs_ptr: int = 0, cursor_ptr: int = 0):
+        """Unit u takes the state saved in slot u32 [units] `slots_ptr`[u] of `store` (bb_restore_device; NO_SLOT leaves it);
+        `seeds_ptr` u64 [units] re-seeds the restored units' shuffle streams, 0 takes the slot's.  `obs_ptr` [n_envs,
+        obs_words] receives the restored books' records, `cursor_ptr` (a trades_device cursor) their logged trade counts;
+        asynchronous."""
+        p = C.c_void_p
+        self._ck(self._lib.bb_restore_device(self._h, p(store), p(slots_ptr), p(seeds_ptr or None), p(obs_ptr or None),
+                                             p(cursor_ptr or None)))
+
     def level_2_data_device(self, d_out_ptr: int): self._ck(self._lib.bb_level2_device(self._h, C.c_void_p(d_out_ptr)))
     def level_1_data_device(self, d_out_ptr: int): self._ck(self._lib.bb_level1_device(self._h, C.c_void_p(d_out_ptr)))
 

@@ -110,6 +110,19 @@ struct bb_handle {
     struct OccEntry { const void* fn; size_t smem; u32 wpb; int per_sm; };
     std::vector<OccEntry> occ_cache;  // resident CTAs per SM of the kernels launched so far (grid_for)
     std::string err;
+    // bb_store_create: the handle's stores, freed by bb_destroy, and the generation they must match: bumped by every call
+    // that changes what a slot holds or how it is sized (bb_reserve growing a capacity, bb_set_agents(_market),
+    // bb_set_tick_sizes)
+    std::vector<bb_store*> stores;
+    u64 store_gen = 0;
+};
+
+struct bb_store {
+    bb_handle* owner;
+    u64 gen;
+    u32 n_slots;
+    unsigned char* mem;  // one allocation: slot records, then meta, then the restored-book mask
+    StoreCopy c;         // the launch arguments, less the handle's current pointers
 };
 
 namespace {
@@ -509,11 +522,11 @@ int launch_apply(bb_handle* h, int mode, const bb_instr* d_instrs, const u64* d_
     return BB_OK;
 }
 
-int snapshot(bb_handle* h, u32 first_env, u32 n, u32* d45, u32* d8, u32 words = 45u) {
+int snapshot(bb_handle* h, u32 first_env, u32 n, u32* d45, u32* d8, u32 words = 45u, const uint8_t* only = nullptr) {
     KParams p;
     fill_params(h, h->lay_snap, p);
     if (h->eng == ENG_DEEP) {
-        k_snapshot_deep<<<(n + 3) / 4, 128, 0, h->stream>>>(p, d45, d8, first_env, n, words);
+        k_snapshot_deep<<<(n + 3) / 4, 128, 0, h->stream>>>(p, d45, d8, first_env, n, words, only);
         CUDA_TRY(h, cudaGetLastError());
         return BB_OK;
     }
@@ -521,7 +534,7 @@ int snapshot(bb_handle* h, u32 first_env, u32 n, u32* d45, u32* d8, u32 words = 
     const u32 wpb = wpb_for(h->lay_snap.warp_bytes);
     const auto k = h->eng == ENG_DENSE ? k_snapshot<ENG_DENSE> : h->eng == ENG_DENSE_L ? k_snapshot<ENG_DENSE_L> : k_snapshot<ENG_PAGED>;
     if ((rc = grid_for(h, k, h->lay_snap, n, &grid, wpb))) return rc;
-    k<<<grid, wpb * 32, (size_t)h->lay_snap.warp_bytes * wpb, h->stream>>>(p, d45, d8, first_env, n, words);
+    k<<<grid, wpb * 32, (size_t)h->lay_snap.warp_bytes * wpb, h->stream>>>(p, d45, d8, first_env, n, words, only);
     CUDA_TRY(h, cudaGetLastError());
     return BB_OK;
 }
@@ -664,6 +677,10 @@ int bb_destroy(bb_handle* h) {
     cudaSetDevice(h->cfg.device);
     if (h->stream) cudaStreamSynchronize(h->stream);
     if (h->copy_stream) cudaStreamSynchronize(h->copy_stream);
+    for (bb_store* s : h->stores) {
+        cudaFree(s->mem);
+        delete s;
+    }
     cudaFree(h->blobs); cudaFree(h->ord); cudaFree(h->tr); cudaFree(h->hist); cudaFree(h->err_flag);
     cudaFree(h->d_offsets); cudaFree(h->d_seeds); cudaFree(h->d_instrs); cudaFree(h->d_snap); cudaFree(h->d_stats); cudaFree(h->d_tick);
     cudaFree(h->rslot); cudaFree(h->mom); cudaFree(h->scratch); cudaFree(h->d_ids); cudaFree(h->dp_pool);
@@ -707,6 +724,129 @@ int bb_reset_device(bb_handle* h, const uint8_t* d_mask, const uint64_t* d_seeds
     return BB_OK;
 }
 
+namespace {
+// the sizes of a slot book's sections at the handle's current capacities (StoreCopy's layout fields)
+StoreCopy store_layout(const bb_handle* h) {
+    StoreCopy c{};
+    auto a16 = [](u64 x) { return (x + 15u) / 16u * 16u; };
+    c.rslot_bytes = h->rslot ? 4u * h->agents_per_env : 0u;
+    c.mom_bytes = h->mom ? h->mom_groups * h->mom_stride : 0u;
+    c.pool_chunks = h->eng == ENG_DEEP ? h->dp_chunks : 0u;
+    c.off_ord = h->blob_stride;
+    c.off_tr = c.off_ord + (u64)h->cfg.max_orders * sizeof(OrderRec);
+    c.off_rslot = c.off_tr + (u64)h->cfg.max_trades * sizeof(TradeRec);
+    c.off_mom = c.off_rslot + a16(c.rslot_bytes);
+    c.off_pool = c.off_mom + a16(c.mom_bytes);
+    c.book_bytes = c.off_pool + (u64)c.pool_chunks * DP_CHUNK_BYTES;
+    c.max_orders = h->cfg.max_orders;
+    c.max_trades = h->cfg.max_trades;
+    c.assets = h->assets;
+    c.n_units = h->cfg.n_envs / h->assets;
+    return c;
+}
+
+// what bb_save_device and bb_restore_device refuse, and the markets' shuffle streams brought to the books first
+int store_precheck(bb_handle* h, bb_store* s, const void* d_sel, const char* who) {
+    if (!s || !d_sel) return fail(h, BB_EINVAL, "null argument");
+    if (s->owner != h) return fail(h, BB_EINVAL, std::string(who) + ": the store was created by another handle");
+    if (s->gen != h->store_gen)
+        return fail(h, BB_EINVAL, std::string(who) + ": the store predates a bb_reserve that grew a capacity, or a bb_set_agents / "
+                                                     "bb_set_agents_market / bb_set_tick_sizes call: create a new one");
+    if (int rc = refuse_pending_queue(h)) return rc;
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    if (h->assets > 1 && h->market_rng_at == bb_handle::RNG_HOST_AHEAD) {
+        // the books' copies of the markets' streams are behind the host's: bring them up to date, never inside a stream
+        // capture (the graph would replay a copy of the streams as they are now)
+        if (stream_capturing(h))
+            return fail(h, BB_EINVAL, std::string(who) + ": the markets' shuffle streams last advanced in bb_step; call "
+                                                         "bb_step_device_market once outside the capture (or bb_reset) before capturing it");
+        return market_rng_to_device(h);
+    }
+    return BB_OK;
+}
+
+int launch_store_copy(bb_handle* h, bb_store* s, bool restore, const u32* d_sel, const u64* d_seeds, u32* d_cursor) {
+    StoreCopy c = s->c;
+    c.blobs = h->blobs;
+    c.blob_stride = h->blob_stride;
+    c.ord = h->ord;
+    c.tr = h->tr;
+    c.rslot = h->rslot;
+    c.mom = reinterpret_cast<unsigned char*>(h->mom);
+    c.pool = h->dp_pool;
+    c.tick = h->d_tick;
+    // a part per 256 KB of a slot book at capacity (at most 16), and about 8 CTAs of 256 threads per SM in all
+    const u32 n_books = restore ? h->cfg.n_envs : s->n_slots * h->assets;
+    const u32 parts = (u32)std::min<u64>(16, (c.book_bytes + (256u << 10) - 1) / (256u << 10));
+    const dim3 grid(std::max(1u, std::min(n_books, 8u * (u32)h->sm_count / parts)), parts);
+    if (restore) k_store_copy<true><<<grid, 256, 0, h->stream>>>(c, n_books, d_sel, d_seeds, d_cursor);
+    else k_store_copy<false><<<grid, 256, 0, h->stream>>>(c, n_books, d_sel, nullptr, nullptr);
+    CUDA_TRY(h, cudaGetLastError());
+    return BB_OK;
+}
+}  // namespace
+
+int bb_store_create(bb_handle* h, uint32_t n_slots, bb_store** out, uint64_t* out_bytes) {
+    CHECK_H(h);
+    if (!out && !out_bytes) return fail(h, BB_EINVAL, "null argument");
+    if (out) *out = nullptr;
+    if (n_slots == 0) return fail(h, BB_EINVAL, "bb_store_create: n_slots must be > 0");
+    StoreCopy c = store_layout(h);
+    const u64 books = (u64)n_slots * h->assets;
+    const u64 off_meta = books * c.book_bytes, off_restored = off_meta + books * 16u, bytes = off_restored + h->cfg.n_envs;
+    if (out_bytes) *out_bytes = bytes;
+    if (!out) return BB_OK;  // a size query
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    unsigned char* mem = nullptr;
+    if (cudaMalloc(&mem, bytes) != cudaSuccess) {
+        cudaGetLastError();
+        return fail(h, BB_ECUDA, "bb_store_create: cannot allocate " + std::to_string(bytes) + " bytes for " + std::to_string(n_slots) +
+                                     " slots of " + std::to_string(h->assets * c.book_bytes) + " bytes");
+    }
+    if (cudaMemsetAsync(mem + off_meta, 0, books * 16u, h->stream) != cudaSuccess) {  // every slot starts empty
+        cudaFree(mem);
+        return fail(h, BB_ECUDA, "bb_store_create: cudaMemsetAsync failed");
+    }
+    c.data = mem;
+    c.meta = reinterpret_cast<uint4*>(mem + off_meta);
+    c.restored = mem + off_restored;
+    c.n_slots = n_slots;
+    bb_store* s = new bb_store{h, h->store_gen, n_slots, mem, c};
+    h->stores.push_back(s);
+    *out = s;
+    return BB_OK;
+}
+
+int bb_store_destroy(bb_store* s) {
+    if (!s) return BB_OK;
+    bb_handle* h = s->owner;
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    h->stores.erase(std::find(h->stores.begin(), h->stores.end(), s));
+    cudaFree(s->mem);
+    delete s;
+    return BB_OK;
+}
+
+int bb_save_device(bb_handle* h, bb_store* s, const uint32_t* d_units) {
+    CHECK_H(h);
+    if (int rc = store_precheck(h, s, d_units, "bb_save_device")) return rc;
+    return launch_store_copy(h, s, false, d_units, nullptr, nullptr);
+}
+
+int bb_restore_device(bb_handle* h, bb_store* s, const uint32_t* d_slots, const uint64_t* d_seeds, uint32_t* d_obs_out, uint32_t* d_cursor) {
+    CHECK_H(h);
+    int rc = store_precheck(h, s, d_slots, "bb_restore_device");
+    if (rc) return rc;
+    if ((rc = launch_store_copy(h, s, true, d_slots, d_seeds, d_cursor))) return rc;
+    h->mirror_dirty = true;  // restored books hold the slot's orders
+    h->status_valid = false;
+    // (recorded_host is left as it is: restored books' record counts are 0, so it still bounds every env's count)
+    if (h->assets > 1) h->market_rng_at = bb_handle::RNG_DEVICE_AHEAD;
+    if (d_obs_out) return snapshot(h, 0, h->cfg.n_envs, d_obs_out, nullptr, h->cfg.obs_words, s->c.restored);
+    return BB_OK;
+}
+
 // KParams::rand_tick_mask: bit gi for a RandomAgents group that trades some book whose tick does not divide its tick_size.
 // Only such groups can draw an off-tick limit price: a population with one runs on the k_sim variants that check the
 // queued prices (run_agents_impl), on-grid populations keep the RandomAgents-only kernels, which carry no check.
@@ -746,6 +886,7 @@ int bb_set_tick_sizes(bb_handle* h, const uint32_t* ticks, uint32_t n) {
             return fail(h, BB_EINVAL, "bb_set_tick_sizes: env " + std::to_string(e) + " has orders or queued transactions (bb_reset first)");
     std::vector<u32> t(ne);
     for (u32 e = 0; e < ne; ++e) t[e] = ticks[n == ne ? e : e % h->assets];  // market m's book a = env m * assets + a
+    ++h->store_gen;
     CUDA_TRY(h, cudaMemcpyAsync(h->d_tick, t.data(), (size_t)ne * 4, cudaMemcpyHostToDevice, h->stream));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     h->tick.swap(t);
@@ -974,6 +1115,7 @@ static int set_agents_impl(bb_handle* h, const bb_agent_group* groups, const uin
     // agent state is (re)allocated only when the population's shape changes: cudaFree / cudaMalloc synchronise the
     // whole device and cost ~100 ms next to tens of GB of slabs, which used to dominate the end-to-end pass
     const size_t ne = h->cfg.n_envs;
+    ++h->store_gen;  // (slots hold the agents' state)
     mom_cap = (mom_cap + 1u) & ~1u;  // (records stay 8-byte aligned)
     if (total != h->agents_per_env || mom != h->mom_groups || mom_cap != h->mom_cap || (total && !h->rslot) || (mom && !h->mom)) {
         CUDA_TRY(h, cudaStreamSynchronize(h->stream));
@@ -1134,6 +1276,7 @@ int bb_reserve(bb_handle* h, uint32_t max_orders, uint32_t max_trades, uint32_t 
     const size_t ne = h->cfg.n_envs;
     // one slab at a time: allocate the larger one, copy every env's rows across (2-D copy, old pitch -> new pitch), swap
     auto grow = [&](void** slab, size_t old_row, size_t new_row) -> int {
+        ++h->store_gen;  // (slots are sized by the capacities)
         void* fresh = nullptr;
         CUDA_TRY(h, cudaMalloc(&fresh, ne * new_row));
         if (*slab && old_row)

@@ -1635,8 +1635,10 @@ __global__ void __launch_bounds__(128, ROOMY ? 2 : 4) k_deepw(const __grid_const
 // ---------------------------------------------------------------------------------------------------
 // Live market data of every book: out45[env][45] (level_2_data layout) and out8[env][8] =
 // OrderBook::level_1_data field order (orderbook.rs:287-301, touch by the `volumes` map).
+// `only` [n_books] or nullptr: write the rows of the books whose entry is non-zero (bb_restore_device's restored books)
 template <int ENG> __global__ void __launch_bounds__(128) k_snapshot(const __grid_constant__ KParams p, u32* out45, u32* out8,
-                                                                     u32 first_env, u32 n_out, u32 words = 45u) {
+                                                                     u32 first_env, u32 n_out, u32 words = 45u,
+                                                                     const uint8_t* only = nullptr) {
     extern __shared__ __align__(128) unsigned char smem[];
     const u32 lane = keep32(threadIdx.x & 31u), warp = threadIdx.x >> 5, wpb = blockDim.x >> 5;
     const u32 sb = keep32(smem_u32(smem) + warp * p.warp_smem_bytes);
@@ -1652,6 +1654,7 @@ template <int ENG> __global__ void __launch_bounds__(128) k_snapshot(const __gri
     pcache_init(g, sb, lane);
     for (u32 i = blockIdx.x * wpb + warp; i < n_out; i += gridDim.x * wpb) {
         const u32 env = first_env + i;
+        if (only && !only[env]) continue;
         Book b;
         make_book(b, p, sb, env, lane);
         if (!blob_load(p, sb, env, bar, ph, lane)) return;
@@ -1686,6 +1689,20 @@ struct ResetArgs {
     u32* cursor;          // [n_envs] or nullptr: a bb_trades_device cursor, zeroed for reset books
 };
 
+// Xoroshiro128StarStar::seed_from_u64: two SplitMix64 outputs (as upload_seeds on the host)
+__device__ __forceinline__ void seed_stream(BookHdr& h, u64 x) {
+    u64 z[2];
+    for (int i = 0; i < 2; ++i) {
+        x += 0x9e3779b97f4a7c15ULL;
+        u64 y = x;
+        y = (y ^ (y >> 30)) * 0xbf58476d1ce4e5b9ULL;
+        y = (y ^ (y >> 27)) * 0x94d049bb133111ebULL;
+        z[i] = y ^ (y >> 31);
+    }
+    h.rng_s0 = z[0];
+    h.rng_s1 = z[1];
+}
+
 // thread 0 of a book's CTA: the fresh header (OrderBook::new orderbook.rs:158-171 + Env::new env.rs:84-95) with its random
 // streams.  A masked reset reads the old header's stream and step counter before the caller overwrites it.
 __device__ __forceinline__ BookHdr fresh_hdr(const unsigned char* b, u32 env, u64 start_time, u32 trading, const u64* rng_seeds,
@@ -1697,18 +1714,8 @@ __device__ __forceinline__ BookHdr fresh_hdr(const unsigned char* b, u32 env, u6
     if (!r.mask) {
         h.rng_s0 = rng_seeds[2 * env];
         h.rng_s1 = rng_seeds[2 * env + 1];
-    } else if (r.seeds) {  // Xoroshiro128StarStar::seed_from_u64: two SplitMix64 outputs (as upload_seeds on the host)
-        u64 x = r.seeds[env / r.assets];
-        u64 z[2];
-        for (int i = 0; i < 2; ++i) {
-            x += 0x9e3779b97f4a7c15ULL;
-            u64 y = x;
-            y = (y ^ (y >> 30)) * 0xbf58476d1ce4e5b9ULL;
-            y = (y ^ (y >> 27)) * 0x94d049bb133111ebULL;
-            z[i] = y ^ (y >> 31);
-        }
-        h.rng_s0 = z[0];
-        h.rng_s1 = z[1];
+    } else if (r.seeds) {
+        seed_stream(h, r.seeds[env / r.assets]);
     } else {
         const BookHdr* old = reinterpret_cast<const BookHdr*>(b);
         h.rng_s0 = old->rng_s0;
@@ -1786,10 +1793,11 @@ __global__ void k_init_deep(unsigned char* blobs, u64 blob_stride, u32 n_envs, u
 
 // live market data of deep books, read straight from the blobs in HBM (same outputs as k_snapshot)
 __global__ void __launch_bounds__(128) k_snapshot_deep(const __grid_constant__ KParams p, u32* out45, u32* out8, u32 first_env, u32 n_out,
-                                                       u32 words) {
+                                                       u32 words, const uint8_t* only = nullptr) {
     const u32 lane = threadIdx.x & 31u, i = blockIdx.x * 4u + (threadIdx.x >> 5);
     if (i >= n_out) return;
     const u32 env = first_env + i;
+    if (only && !only[env]) return;
     const unsigned char* b = p.blobs + (size_t)env * p.blob_stride;
     const BookHdr* h = reinterpret_cast<const BookHdr*>(b);
     const u32 W = p.geo.d_levels, nw = W >> 5, lo = p.geo.d_win_lo;
@@ -1917,6 +1925,120 @@ __global__ void __launch_bounds__(256) k_trades_window(const unsigned char* blob
         if (count) count[book] = avail;
         if (n) cursor[book] = c + n;
     }
+}
+
+// bb_save_device / bb_restore_device.  A slot holds one unit (an env, or a market of `assets` books); slot book k =
+// slot * assets + a sits at data + k * book_bytes: the blob, the order table, the trade log, the agents' rslot slice, their
+// MomState slice and (deep engine) the chunk pool, each section at its capacity, and meta[k] = {valid, tick, 0, 0}.
+#define ERR_SLOT 0x1000u  // == BB_ERR_SLOT
+struct StoreCopy {
+    unsigned char* blobs;
+    u64 blob_stride;
+    OrderRec* ord;
+    TradeRec* tr;
+    u32* rslot;
+    unsigned char* mom;
+    unsigned char* pool;
+    const u32* tick;
+    unsigned char* data;  // the store
+    uint4* meta;
+    uint8_t* restored;    // [n_envs]: 1 for the books a restore rewrote (the mask of its observation launch), else 0
+    u64 book_bytes, off_ord, off_tr, off_rslot, off_mom, off_pool;
+    u32 max_orders, max_trades, rslot_bytes, mom_bytes, pool_chunks /* 0: not the deep engine */, assets, n_units, n_slots;
+};
+
+// part `part` of `parts` of a CTA-strided copy: 16 bytes a thread and iteration where both ends and the length allow it (the
+// blob, order and trade sections), 4 bytes otherwise (the agent slices, whose per-env offsets are multiples of 4 or 8)
+__device__ __forceinline__ void store_copy_part(unsigned char* dst, const unsigned char* src, u64 bytes, u32 part, u32 parts) {
+    const u64 i0 = (u64)part * blockDim.x + threadIdx.x, step = (u64)parts * blockDim.x;
+    if (((reinterpret_cast<uintptr_t>(dst) | reinterpret_cast<uintptr_t>(src) | bytes) & 15u) == 0) {
+        uint4* d = reinterpret_cast<uint4*>(dst);
+        const uint4* s = reinterpret_cast<const uint4*>(src);
+        for (u64 i = i0; i < bytes / 16u; i += step) d[i] = s[i];
+    } else {
+        u32* d = reinterpret_cast<u32*>(dst);
+        const u32* s = reinterpret_cast<const u32*>(src);
+        for (u64 i = i0; i < bytes / 4u; i += step) d[i] = s[i];
+    }
+}
+
+// One book of k_store_copy, part `part` of `parts`.  Save: book = slot book k, sel[slot] the unit to save (BB_NO_SLOT: slot
+// untouched; >= n_units: slot marked empty).  Restore: book = the handle's book, sel[unit] the slot to restore from
+// (BB_NO_SLOT: unit untouched); a slot out of range, empty, or saved at another tick than any book of the unit flags every
+// book of the unit ERR_SLOT and changes nothing else.  Every CTA reads the prefix lengths from the source header, which no
+// CTA of the launch writes, and evaluates the slot's validity the same way.  Part 0 writes the header: on restore the
+// slot's, with the history count at 0 and, given seeds, the unit's shuffle stream re-seeded (the step counter stays the
+// slot's).
+template <bool RESTORE>
+__device__ __forceinline__ void store_copy_book(const StoreCopy& c, u32 book, u32 part, u32 parts, const u32* sel, const u64* seeds,
+                                                u32* cursor) {
+    const u32 A = c.assets, unit = book / A, a = book % A;
+    const bool lead = part == 0 && threadIdx.x == 0;
+    u64 live, stored;  // book indices into the handle's arrays and the store
+    if (RESTORE) {
+        const u32 slot = sel[unit];
+        if (slot == BB_NO_SLOT) {
+            if (lead) c.restored[book] = 0u;
+            return;
+        }
+        bool ok = slot < c.n_slots;
+        for (u32 j = 0; ok && j < A; ++j) {
+            const uint4 m = c.meta[(u64)slot * A + j];
+            ok = m.x != 0u && m.y == c.tick[(u64)unit * A + j];
+        }
+        if (lead) c.restored[book] = ok ? 1u : 0u;
+        if (!ok) {
+            if (lead) atomicOr(&reinterpret_cast<BookHdr*>(c.blobs + (u64)book * c.blob_stride)->err, ERR_SLOT);
+            return;
+        }
+        live = book;
+        stored = (u64)slot * A + a;
+    } else {
+        const u32 u = sel[unit];
+        if (u == BB_NO_SLOT) return;
+        if (u >= c.n_units) {
+            if (lead) c.meta[book] = make_uint4(0u, 0u, 0u, 0u);
+            return;
+        }
+        live = (u64)u * A + a;
+        stored = book;
+    }
+    unsigned char* rec = c.data + stored * c.book_bytes;
+    unsigned char* blob = c.blobs + live * c.blob_stride;
+    const BookHdr* src_hdr = reinterpret_cast<const BookHdr*>(RESTORE ? rec : blob);
+    const u64 n_ord = min(src_hdr->n_orders, c.max_orders), n_tr = min(src_hdr->n_trades, c.max_trades);
+    const u64 n_chunks = c.pool_chunks ? min(*reinterpret_cast<const u32*>((RESTORE ? rec : blob) + DP_OFF_BUMP), c.pool_chunks) : 0u;
+    auto copy = [&](unsigned char* live_p, unsigned char* stored_p, u64 bytes) {
+        if (RESTORE) store_copy_part(live_p, stored_p, bytes, part, parts);
+        else store_copy_part(stored_p, live_p, bytes, part, parts);
+    };
+    copy(blob + sizeof(BookHdr), rec + sizeof(BookHdr), c.blob_stride - sizeof(BookHdr));
+    copy(reinterpret_cast<unsigned char*>(c.ord + live * c.max_orders), rec + c.off_ord, n_ord * sizeof(OrderRec));
+    if (c.max_trades) copy(reinterpret_cast<unsigned char*>(c.tr + live * c.max_trades), rec + c.off_tr, n_tr * sizeof(TradeRec));
+    if (c.rslot_bytes) copy(reinterpret_cast<unsigned char*>(c.rslot) + live * c.rslot_bytes, rec + c.off_rslot, c.rslot_bytes);
+    if (c.mom_bytes) copy(c.mom + live * c.mom_bytes, rec + c.off_mom, c.mom_bytes);
+    if (n_chunks) copy(c.pool + live * c.pool_chunks * DP_CHUNK_BYTES, rec + c.off_pool, n_chunks * DP_CHUNK_BYTES);
+    if (!lead) return;
+    BookHdr h = *src_hdr;
+    if (RESTORE) {
+        h.n_steps = 0u;
+        if (seeds && !c.pool_chunks) seed_stream(h, seeds[unit]);  // (the deep engine has no shuffle)
+        *reinterpret_cast<BookHdr*>(blob) = h;
+        if (cursor) cursor[book] = (u32)n_tr;
+    } else {
+        *reinterpret_cast<BookHdr*>(rec) = h;
+        c.meta[book] = make_uint4(1u, c.tick[live], 0u, 0u);
+    }
+}
+
+// bb_save_device (n_books = slot books) / bb_restore_device (n_books = the handle's books).  Grid (x, part): part y of every
+// book is copied by the CTAs of row y, which stride over the books, so a book with a long prefix is copied by gridDim.y
+// CTAs and a launch that selects few units costs a read of `sel` per unselected book.
+template <bool RESTORE>
+__global__ void __launch_bounds__(256) k_store_copy(const __grid_constant__ StoreCopy c, u32 n_books, const u32* sel, const u64* seeds,
+                                                    u32* cursor) {
+    for (u32 book = blockIdx.x; book < n_books; book += gridDim.x)
+        store_copy_book<RESTORE>(c, book, blockIdx.y, gridDim.y, sel, seeds, cursor);
 }
 
 // reduction of per-env counters for bb_stats

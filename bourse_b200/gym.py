@@ -188,6 +188,24 @@ TRADE_COLUMNS = (("t", np.uint64), ("side_is_bid", np.uint8), ("price", np.uint3
                  ("passive_id", np.uint64))
 
 
+NO_SLOT = abi.NO_SLOT
+
+
+class Store:
+    """A device store of `n_slots` unit snapshots made by `VectorEnv` / `MarketVectorEnv.snapshots` (bb_store_create).  A slot
+    holds one unit's full state — books, order tables, trade logs, agent state and random streams — but not its history.
+    `nbytes` is its size on the device.  It belongs to its env: `close()` frees it, and so does the env's `close()`."""
+
+    def __init__(self, env: BatchedEnv, n_slots: int):
+        self.env, self.n_slots = env, int(n_slots)
+        self.ptr, self.nbytes = env.store_create(self.n_slots)
+
+    def close(self):
+        if self.ptr:
+            self.env.store_destroy(self.ptr)
+            self.ptr = 0
+
+
 class _DeviceLoop:
     """What `VectorEnv` and `MarketVectorEnv` share: the handle, the device buffers, host-action staging, the history ring and
     the order / trade reads."""
@@ -207,8 +225,11 @@ class _DeviceLoop:
         self._cursor = DeviceArray(self.env, (self.env.n_envs,), np.uint32)  # trades(): each book's next unread trade
         self._cursor.copy_from_host(np.zeros(self.env.n_envs, np.uint32))
         self._reads: dict = {}   # orders() / trades() outputs and query staging, by kind and size: allocated once, then reused
+        self._stores: typing.List[Store] = []
 
     def close(self):
+        for st in self._stores:
+            st.close()
         for a in (self.obs, self.ids, self._actions, self._offsets, self._cursor):
             a.free()
         for bufs in self._reads.values():
@@ -251,12 +272,49 @@ class _DeviceLoop:
         self.env.reset_device(mask_ptr, seeds_ptr, self.obs.ptr, self._cursor.ptr)
         return self.obs
 
-    def _unit_array(self, x, dtype, name) -> typing.Tuple[int, typing.Any]:
-        """(device address, keep-alive object) of a [units] mask (bool / 1-byte integers) or seed array (8-byte integers):
-        the caller's device array, or a staging copy of a host array."""
-        dtype, units = np.dtype(dtype), self._units
+    def snapshots(self, n_slots: int) -> Store:
+        """A device store of `n_slots` slots for `save` / `restore`, sized from the env's current capacities (every slot
+        empty).  Growing a capacity (`env.reserve`), new agents or new tick sizes make it unusable: create another."""
+        st = Store(self.env, n_slots)
+        self._stores.append(st)
+        return st
+
+    def save(self, store: Store, units=None):
+        """Save units into the slots of `store` (bb_save_device): slot k receives unit `units[k]`.  `units` is an
+        `[n_slots]` array of 4-byte integers, device (CUDA array interface or DLPack) or numpy; `None` saves unit k into
+        slot k.  `NO_SLOT` leaves a slot as it is, an index >= units empties it.  The env is not changed.  One launch on
+        the env's stream with no host synchronisation (device `units`), so it can be captured into a CUDA graph."""
+        if units is None:
+            units = np.arange(store.n_slots, dtype=np.uint32)
+        ptr, keep = self._unit_array(units, np.uint32, "units", store.n_slots)
+        self._keep = keep   # alive until the next call, as in _action_ptr
+        self.env.save_device(store.ptr, ptr)
+
+    def restore(self, store: Store, slots, seeds=None) -> DeviceArray:
+        """Restore units from the slots of `store` (bb_restore_device): unit u takes the state saved in slot `slots[u]`
+        (`NO_SLOT`: untouched), several units may name one slot.  `slots` is a `[units]` array of 4-byte integers, device
+        or numpy.  A restored unit is the saved one — books, order tables, trade logs, time, error bits, agent state —
+        with its history count at 0.  Without `seeds` it takes the slot's shuffle stream and step counter, so a unit
+        restored from its own snapshot continues bit-identically under the same actions (background agents draw by
+        env / market id, so another unit restored from that slot draws other agent instructions).  `seeds` (`[units]`,
+        8-byte integers) re-seeds the restored units' shuffle streams as `reset(mask, seeds)` does; the step counter stays
+        the slot's.  A slot out of range, empty, or saved at another tick flags the unit (`BB_ERR_SLOT`, `check_errors`
+        raises) and leaves it untouched.  The rows of restored units in `self.obs` receive their records, their `trades`
+        cursors the restored logs' counts; returns `self.obs`.  Launches on the env's stream with no host synchronisation
+        (device arrays), so it can be captured into a CUDA graph with `step`."""
+        slots_ptr, keep_slots = self._unit_array(slots, np.uint32, "slots")
+        seeds_ptr, keep_seeds = self._unit_array(seeds, np.uint64, "seeds") if seeds is not None else (0, None)
+        self._keep = (keep_slots, keep_seeds)
+        self.env.restore_device(store.ptr, slots_ptr, seeds_ptr, self.obs.ptr, self._cursor.ptr)
+        return self.obs
+
+    def _unit_array(self, x, dtype, name, n=None) -> typing.Tuple[int, typing.Any]:
+        """(device address, keep-alive object) of an [n] (default: [units]) mask (bool / 1-byte integers), unit or slot
+        array (4-byte integers) or seed array (8-byte integers): the caller's device array, or a staging copy of a host
+        array."""
+        dtype, units = np.dtype(dtype), self._units if n is None else n
         kinds = "biu" if dtype.itemsize == 1 else "iu"
-        what = f"{name} must be a [{units}] array of " + ("bool or 1-byte integers" if dtype.itemsize == 1 else "8-byte integers")
+        what = f"{name} must be a [{units}] array of " + ("bool or 1-byte integers" if dtype.itemsize == 1 else f"{dtype.itemsize}-byte integers")
         dev = _device_array(x)
         if dev is not None:
             ptr, shape, typ, keep = dev
@@ -266,7 +324,9 @@ class _DeviceLoop:
         a = np.asarray(x)
         if a.shape != (units,) or a.dtype.kind not in kinds or (dtype.itemsize == 1 and a.dtype.itemsize != 1):
             raise ValueError(what)
-        buf = self._buffer((name,), (units,), dtype)
+        if dtype.itemsize == 4 and a.size and (int(a.min()) < 0 or int(a.max()) > 0xFFFFFFFF):
+            raise ValueError(what + " in [0, 2^32)")
+        buf = self._buffer((name, units), (units,), dtype)
         buf.copy_from_host(a.astype(dtype))
         return buf.ptr, None
 

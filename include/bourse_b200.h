@@ -25,6 +25,7 @@ extern "C" {
 #define BB_ABI_VERSION 1
 
 typedef struct bb_handle bb_handle;
+typedef struct bb_store bb_store; /* device-resident book snapshots of a handle (bb_store_create) */
 
 typedef enum {
     BB_OK = 0,
@@ -49,6 +50,7 @@ typedef enum {
 #define BB_ERR_PRICE 0x200u      /* bb_step_device: a NEW row's limit price was not a multiple of its env's tick (row dropped) */
 #define BB_ERR_ROW_OP 0x400u     /* bb_run_agents_with_rows(_market): a MODIFY row or a trader id >= 2^19 (row dropped); markets: a row's aux names no asset */
 #define BB_ERR_LOCKED 0x800u     /* deep engine: both sides would rest at one price level (trading disabled) */
+#define BB_ERR_SLOT 0x1000u      /* bb_restore_device: the slot was empty, out of range, or saved from a book of another tick */
 
 #define BB_OBS_L1 9u   /* StepEnvNumpy.level_1_data layout, rust/src/step_sim_numpy.rs:300-318 */
 #define BB_OBS_L2 45u  /* StepEnvNumpy.level_2_data layout, rust/src/step_sim_numpy.rs:351-368 */
@@ -361,6 +363,53 @@ int bb_trades_device(bb_handle* h, uint32_t* d_cursor, uint32_t cap, uint32_t* d
  * d_mask, while host-queued instructions are pending, and in the capture case above.  Asynchronous on the handle's stream:
  * one launch, no host synchronisation and no allocation, so the call may be recorded into a CUDA graph with the steps. */
 int bb_reset_device(bb_handle* h, const uint8_t* d_mask, const uint64_t* d_seeds, uint32_t* d_obs_out, uint32_t* d_cursor);
+/* Device-resident book snapshots for the vector loops: save the full state of some units into the slots of a device store,
+ * and restore any units from any slots (one slot into many units included) — episodes that start from a warm book,
+ * branching rollouts, replays from a midpoint.  A unit is an env, or a market of `assets` books on a multi-asset handle, as
+ * in bb_reset_device; a slot holds one unit.
+ *
+ * bb_store_create: a store of n_slots slots, sized from the handle's current capacities; every slot starts empty.
+ *   *out_bytes (may be NULL) receives its size in bytes; with out == NULL the call only reports that size and allocates
+ *   nothing.  An allocation failure returns BB_ECUDA with the size in the message.  The store belongs to the handle:
+ *   bb_destroy frees every store not yet destroyed (its pointer is then invalid).
+ * bb_store_destroy: frees a store (synchronises the handle's stream).  NULL is a no-op.
+ *
+ * What a slot holds, per book: the blob (header, page directory and pages; the dense window; or the deep image), the order
+ * table prefix [0, min(n_orders, max_orders)), the trade log prefix [0, min(n_trades, max_trades)), the in-kernel agents'
+ * state of the book (RandomAgents held ids, MomentumAgent / NoiseAgent state and live lists), on the deep engine the chunk
+ * pool prefix up to its allocator's bump, and the book's tick.  The per-step history is not saved.
+ *
+ * bb_save_device: d_units [n_slots] (device): slot k receives unit d_units[k]; BB_NO_SLOT leaves slot k as it is, and a
+ *   unit index >= units marks slot k empty.  The handle is not changed.
+ * bb_restore_device: d_slots [units] (device): unit u takes the state of slot d_slots[u]; BB_NO_SLOT leaves the unit
+ *   untouched; many units may name one slot.  A restored book is the saved book — book, order table, trade log, time,
+ *   trading flag, sticky error word, header counters and agent state — with a history count (bb_n_steps) of 0.
+ *   d_seeds [units] or NULL: NULL gives the book the slot's Xoroshiro128** shuffle state and Philox step counter, so a unit
+ *   restored from its own saved state continues bit-identically under the same actions (agent draws are keyed by the global
+ *   env / market id as well: another unit restored from that slot draws other agent instructions; rows-only units restored
+ *   from one slot continue identically).  Non-NULL: the unit's shuffle stream becomes
+ *   Xoroshiro128StarStar::seed_from_u64(d_seeds[u]), as bb_reset_device seeds it; the step counter is the slot's.
+ *   d_obs_out [n_envs][obs_words] or NULL: the rows of restored books receive what bb_level1_device / bb_level2_device
+ *   return for them right after the restore (a second launch); other rows are not written.
+ *   d_cursor [n_envs] or NULL: a bb_trades_device cursor; the entries of restored books are set to the restored log's
+ *   logged count, so the next read reports only trades made after the restore.
+ *   A unit that names a slot >= n_slots, an empty slot, or a slot whose saved tick differs from that of the book it would
+ *   restore (checked per book, so per-env ticks work) is left untouched and each of its books is flagged BB_ERR_SLOT; all
+ *   books of a market share the outcome.  Order ids a caller holds for a restored book now name the slot's orders.
+ *
+ * Both calls work on every engine; on the deep engine a unit is a book and d_seeds has no effect.  On a multi-asset handle
+ * right after a bb_step that shuffled, both first copy the host's streams of the markets to the books (synchronous), which
+ * is refused inside a stream capture.  Refused with BB_EINVAL, the handle and the store unchanged, for NULL arguments, a
+ * store created by another handle, a store created before a later bb_reserve that grew a capacity or a later
+ * bb_set_agents / bb_set_agents_market / bb_set_tick_sizes, while host-queued instructions are pending, and in the
+ * capture case above.  Asynchronous on the handle's stream, with no host synchronisation and no allocation, so both may be
+ * recorded into a CUDA graph with the steps. */
+#define BB_NO_SLOT 0xFFFFFFFFu
+int bb_store_create(bb_handle* h, uint32_t n_slots, bb_store** out, uint64_t* out_bytes);
+int bb_store_destroy(bb_store* s);
+int bb_save_device(bb_handle* h, bb_store* s, const uint32_t* d_units);
+int bb_restore_device(bb_handle* h, bb_store* s, const uint32_t* d_slots, const uint64_t* d_seeds, uint32_t* d_obs_out,
+                      uint32_t* d_cursor);
 /* Device buffers for callers without a CUDA allocator of their own (numpy-only hosts); any device pointer works above.
  * bb_memcpy kind: 1 host to device, 2 device to host, 3 device to device; synchronous on the handle's stream. */
 int bb_device_alloc(bb_handle* h, uint64_t bytes, void** d_ptr);

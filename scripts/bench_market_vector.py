@@ -26,10 +26,19 @@ the step followed by `reset(mask)` with 0 %, 1 % and 100 % of the units selected
 captured once as a CUDA graph of 100 steps and replayed from reset books, timed with CUDA events; the plain and with-reset
 passes alternate, --passes times each, and the best pass of each counts.
 
+--snapshots measures bb_save_device / bb_restore_device (`save` / `restore`) on warmed C3 books on the FAST engine, for
+4096 single-asset envs (VectorEnv) and 2048 markets x 4 assets (MarketVectorEnv): after --warmup-steps steps of the C3
+population, a store with one slot per unit; each call saves 1 % or 100 % of the units into their own slots, or restores
+them from those slots (with the observation rows and trade cursors), replayed 50 times from a CUDA graph and timed with CUDA
+events, --passes times, best pass.  The bytes a call copies come from the prefix lengths of the selected books (blob,
+orders and trades logged, agent state); bytes/s is that over the time per call (a save reads and writes each byte once, as
+does a restore, so the DRAM traffic is twice it).
+
     python scripts/bench_market_vector.py --steps 1000 --warmup 20
     python scripts/bench_market_vector.py --bg-agents --steps 1000 --warmup 20
     python scripts/bench_market_vector.py --reads --steps 1000 --warmup 20
     python scripts/bench_market_vector.py --resets --passes 3
+    python scripts/bench_market_vector.py --snapshots --passes 3
 """
 from __future__ import annotations
 
@@ -56,6 +65,8 @@ WINDOW = 100
 # background agents: the C3 population's prices are 20..178 (bench.py --workload gym --bg-agents)
 BG_ENGINES = {"fast": dict(), "dense": dict(price_window=(20, 180), live_cap=254)}
 BG_KW = dict(max_orders=8192, max_trades=16384, max_steps=256, max_queue=128)
+# --snapshots: room for the orders and trades of 300 warm-up steps of C3 (about 13,500 and 6,500 per book)
+SNAP_KW = dict(max_orders=16384, max_trades=16384, max_steps=256, max_queue=128)
 
 
 def card():
@@ -254,6 +265,80 @@ def bench_resets(args, name, power):
     return res
 
 
+def bench_snapshots(args, name, power):
+    """--snapshots: see the module docstring."""
+    import torch
+    R, n_envs = 50, N_BOOKS // 2
+    c3 = workloads.c3_groups()
+    agents_per_book = sum(int(g["n_agents"]) for g in c3)
+    blob = 128 + (12 + 512) * 32   # the FAST engine's book blob: header, 32-entry page directory, 32 pages
+    res = {"card": name, "power_limit": power, "engine": "fast", "agents": "C3 (50 + 50 RandomAgents) on every book",
+           "warmup_steps": args.warmup_steps, "calls_per_graph": R, "passes": args.passes, "us_per_call": {}, "bytes_per_call": {},
+           "GB_per_s": {}, "errors": {}}
+    for label, units in (("vector_env_4096", n_envs), ("market_vector_2048x4", N_MARKETS)):
+        books = units if label.startswith("vector") else N_BOOKS
+        A = books // units
+        blocks = gym_action_blocks(args.blocks, books, ROWS_PER_BOOK, seed=5)
+        blocks["price"] = np.where((blocks["op_flags"] & abi.F_MARKET) != 0, blocks["price"], 2 * (40 + blocks["price"] % 21))
+        if label.startswith("vector"):
+            loop = gym.VectorEnv(n_envs, ROWS_PER_BOOK, 0, 0, 1, 1_000_000, agents=c3, agent_seed=5, **SNAP_KW)
+        else:
+            loop = gym.MarketVectorEnv(N_MARKETS, ROWS, 0, 0, [1] * ASSETS, 1_000_000, agents=c3_market_agents(), agent_seed=5, **SNAP_KW)
+            blocks = market_blocks(blocks)
+        d_blocks = [torch.from_numpy(x.view(np.uint8).reshape(units, -1)).cuda() for x in blocks]
+        loop.reset()
+        for s in range(args.warmup_steps):
+            loop.step(d_blocks[s % len(d_blocks)])
+        store = loop.snapshots(units)
+        res[f"{label}_store_bytes"] = store.nbytes
+        n_ord = np.array([loop.env.n_orders(b) for b in range(books)], np.int64)
+        n_tr = np.array([loop.env.n_trades(b) for b in range(books)], np.int64)
+        per_book = blob + 64 * np.minimum(n_ord, SNAP_KW["max_orders"]) + 32 * np.minimum(n_tr, SNAP_KW["max_trades"]) + 4 * agents_per_book
+        per_unit = per_book.reshape(units, A).sum(axis=1)
+        res[f"{label}_mean_orders_logged"], res[f"{label}_mean_trades_logged"] = float(n_ord.mean()), float(n_tr.mean())
+        rng = np.random.default_rng(3)
+        stream = torch.cuda.Stream()
+        loop.env.set_stream(stream.cuda_stream)
+        calls = {}
+        for tag, f in (("1pct", 0.01), ("100pct", 1.0)):
+            sel = rng.permutation(units) < round(f * units)
+            own = np.where(sel, np.arange(units), gym.NO_SLOT).astype(np.uint32)   # unit u <-> slot u
+            d_sel = torch.from_numpy(own.view(np.int32)).cuda()
+            calls[f"save_{tag}"] = (lambda d=d_sel: loop.save(store, d), int(per_unit[sel].sum()))
+            calls[f"restore_{tag}"] = (lambda d=d_sel: loop.restore(store, d), int(per_unit[sel].sum()))
+        torch.cuda.synchronize()
+        with torch.cuda.stream(stream):   # every slot filled, and the first launches (attribute queries) outside any capture
+            loop.save(store)
+            for fn, _ in calls.values():
+                fn()
+        stream.synchronize()
+        graphs = {}
+        for tag, (fn, nbytes) in calls.items():
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g, stream=stream):
+                for _ in range(R):
+                    fn()
+            graphs[tag] = g
+            res["bytes_per_call"][f"{label}_{tag}"] = nbytes
+        for _ in range(args.passes):
+            for tag, g in graphs.items():
+                t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+                t0.record(stream)
+                with torch.cuda.stream(stream):
+                    g.replay()
+                t1.record(stream)
+                stream.synchronize()
+                res["us_per_call"].setdefault(f"{label}_{tag}", []).append(t0.elapsed_time(t1) * 1e3 / R)
+        for tag in graphs:
+            best = min(res["us_per_call"][f"{label}_{tag}"])
+            res["GB_per_s"][f"{label}_{tag}"] = res["bytes_per_call"][f"{label}_{tag}"] / best / 1e3
+        res["errors"][label] = int(np.bitwise_or.reduce(loop.env.env_errors()))
+        del graphs
+        loop.env.set_stream(0)
+        loop.close()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=1000)
@@ -262,7 +347,9 @@ def main():
     ap.add_argument("--bg-agents", action="store_true", help="the C3 population trades in every book (see the module docstring)")
     ap.add_argument("--reads", action="store_true", help="time orders() / trades() in the C3 loops (see the module docstring)")
     ap.add_argument("--resets", action="store_true", help="time reset(mask) in the rows-only loops (see the module docstring)")
-    ap.add_argument("--passes", type=int, default=3, help="--resets: timed passes of each variant")
+    ap.add_argument("--snapshots", action="store_true", help="time save / restore on warmed C3 books (see the module docstring)")
+    ap.add_argument("--warmup-steps", type=int, default=300, help="--snapshots: C3 steps before the store is filled")
+    ap.add_argument("--passes", type=int, default=3, help="--resets / --snapshots: timed passes of each variant")
     args = ap.parse_args()
     import torch
 
@@ -273,6 +360,9 @@ def main():
         return
     if args.resets:
         print(json.dumps(bench_resets(args, name, power)), flush=True)
+        return
+    if args.snapshots:
+        print(json.dumps(bench_snapshots(args, name, power)), flush=True)
         return
     blocks = gym_action_blocks(args.blocks, N_BOOKS, ROWS_PER_BOOK, seed=5)
     if args.bg_agents:   # limit prices into the agents' range, as bench.py run_gym does
