@@ -270,6 +270,14 @@ class BatchedEnv:
         p = C.c_void_p
         self._ck(self._lib.bb_reset_device(self._h, p(mask_ptr), p(seeds_ptr or None), p(obs_ptr or None), p(cursor_ptr or None)))
 
+    def set_agent_params_device(self, params_ptr: int, keys_ptr: int = 0, mask_ptr: int = 0):
+        """Per-unit agent parameters and Philox keys (bb_set_agent_params_device): the units (envs, or markets) whose u8
+        entry of the device mask `mask_ptr` is non-zero (0: every unit) take their row of the device records `params_ptr`
+        ([units][n_groups] bb_agent_group, 0 keeps the records) and their u64 key of `keys_ptr` (0 keeps the keys).  A unit
+        with a record outside the declared population is flagged BB_ERR_PARAMS and keeps what it had; asynchronous."""
+        p = C.c_void_p
+        self._ck(self._lib.bb_set_agent_params_device(self._h, p(params_ptr or None), p(keys_ptr or None), p(mask_ptr or None)))
+
     def store_create(self, n_slots: int, allocate: bool = True) -> typing.Tuple[int, int]:
         """(store handle, bytes) of a device store of `n_slots` unit snapshots (bb_store_create), sized from the current
         capacities; with `allocate=False` only the size is computed and the handle is 0.  Free it with `store_destroy`

@@ -91,6 +91,10 @@ struct bb_handle {
     std::vector<u32> group_asset;  // bb_set_agents_market: asset each group trades (empty: single-asset agents)
     u32 agents_per_env = 0, mom_groups = 0;
     u32 chip_agents = 0;  // on-chip agent table capacity of the dense engine (markets: the largest per-asset agent count)
+    // bb_set_agent_params_device: per-unit group records [units][groups] and Philox keys [units], allocated by its first call
+    // and dropped by bb_set_agents(_market); while they exist every agent launch runs the k_sim<.., PU> variants
+    bb_agent_group* d_unit_groups = nullptr;
+    u64* d_unit_keys = nullptr;
     // host mirrors for Env mode
     std::vector<std::vector<bb_instr>> queue;
     std::vector<u64> n_orders_host;  // ids handed out so far (includes queued NEW)
@@ -395,7 +399,8 @@ int check_device_errors(bb_handle* h) {
         CUDA_TRY(h, cudaMemsetAsync(h->err_flag, 0, 4, h->stream));
         char buf[256];
         snprintf(buf, sizeof buf, "device flagged env errors 0x%x (0x1 orders 0x2 trades 0x4 pages/window 0x8 queue 0x10 bad id "
-                                  "0x20 granule 0x40 steps 0x80 live slots 0x100 time order 0x200 tick size 0x400 unsupported row); see bb_env_errors", flag);
+                                  "0x20 granule 0x40 steps 0x80 live slots 0x100 time order 0x200 tick size 0x400 unsupported row 0x2000 agent "
+                                  "parameters); see bb_env_errors", flag);
         return fail(h, (flag & ERR_BAD_ID) ? BB_EBADID : (flag & 0x80000000u) ? BB_ECUDA : (flag & ERR_PRICE) ? BB_EPRICE : (flag & ERR_ROW_OP) ? BB_EINVAL : BB_ECAP, buf);
     }
     return BB_OK;
@@ -469,17 +474,21 @@ Kernel apply_kernel(int mode, int eng, bool all_resident) {
     if (mode == MODE_REPLAY) return apply_kernel_for<MODE_REPLAY>(eng, all_resident);
     return mode == MODE_ENV_MKT ? apply_kernel_for<MODE_ENV_MKT>(eng, all_resident) : apply_kernel_for<MODE_ENV>(eng, all_resident);
 }
-// external rows run on the MOM variants (they carry no slot hints)
-template <int E> Kernel sim_kernel_for(bool mom, bool mkt, bool ext) {
+// external rows and per-unit parameters run on the MOM variants (they carry no slot hints)
+template <int E> Kernel sim_kernel_for(bool mom, bool mkt, bool ext, bool pu) {
+    if (pu) {
+        if (ext) return mkt ? k_sim<E, true, true, true, true> : k_sim<E, true, false, true, true>;
+        return mkt ? k_sim<E, true, true, false, true> : k_sim<E, true, false, false, true>;
+    }
     if (ext) return mkt ? k_sim<E, true, true, true> : k_sim<E, true, false, true>;
     if (mkt) return mom ? k_sim<E, true, true> : k_sim<E, false, true>;
     return mom ? k_sim<E, true, false> : k_sim<E, false, false>;
 }
-Kernel sim_kernel(int eng, bool mom, bool mkt, bool ext) {
-    if (eng == ENG_FAST) return sim_kernel_for<ENG_FAST>(mom, mkt, ext);
-    if (eng == ENG_DENSE) return sim_kernel_for<ENG_DENSE>(mom, mkt, ext);
-    if (eng == ENG_DENSE_L) return sim_kernel_for<ENG_DENSE_L>(mom, mkt, ext);
-    return sim_kernel_for<ENG_PAGED>(mom, mkt, ext);
+Kernel sim_kernel(int eng, bool mom, bool mkt, bool ext, bool pu) {
+    if (eng == ENG_FAST) return sim_kernel_for<ENG_FAST>(mom, mkt, ext, pu);
+    if (eng == ENG_DENSE) return sim_kernel_for<ENG_DENSE>(mom, mkt, ext, pu);
+    if (eng == ENG_DENSE_L) return sim_kernel_for<ENG_DENSE_L>(mom, mkt, ext, pu);
+    return sim_kernel_for<ENG_PAGED>(mom, mkt, ext, pu);
 }
 
 int launch_apply(bb_handle* h, int mode, const bb_instr* d_instrs, const u64* d_offsets, u32 n_steps, bool host_order = false,
@@ -684,6 +693,7 @@ int bb_destroy(bb_handle* h) {
     cudaFree(h->blobs); cudaFree(h->ord); cudaFree(h->tr); cudaFree(h->hist); cudaFree(h->err_flag);
     cudaFree(h->d_offsets); cudaFree(h->d_seeds); cudaFree(h->d_instrs); cudaFree(h->d_snap); cudaFree(h->d_stats); cudaFree(h->d_tick);
     cudaFree(h->rslot); cudaFree(h->mom); cudaFree(h->scratch); cudaFree(h->d_ids); cudaFree(h->dp_pool);
+    cudaFree(h->d_unit_groups); cudaFree(h->d_unit_keys);
     if (h->h_instrs) cudaFreeHost(h->h_instrs);
     if (h->h_offsets) cudaFreeHost(h->h_offsets);
     if (h->h_snap) cudaFreeHost(h->h_snap);
@@ -1116,6 +1126,9 @@ static int set_agents_impl(bb_handle* h, const bb_agent_group* groups, const uin
     // whole device and cost ~100 ms next to tens of GB of slabs, which used to dominate the end-to-end pass
     const size_t ne = h->cfg.n_envs;
     ++h->store_gen;  // (slots hold the agents' state)
+    // a new population takes its parameters from `groups` again, with zero keys (cudaFree waits for launches that read them)
+    cudaFree(h->d_unit_groups); h->d_unit_groups = nullptr;
+    cudaFree(h->d_unit_keys); h->d_unit_keys = nullptr;
     mom_cap = (mom_cap + 1u) & ~1u;  // (records stay 8-byte aligned)
     if (total != h->agents_per_env || mom != h->mom_groups || mom_cap != h->mom_cap || (total && !h->rslot) || (mom && !h->mom)) {
         CUDA_TRY(h, cudaStreamSynchronize(h->stream));
@@ -1343,6 +1356,51 @@ int bb_set_agents_market(bb_handle* h, const bb_agent_group* groups, const uint3
     return set_agents_impl(h, groups, asset, n_groups);
 }
 
+int bb_set_agent_params_device(bb_handle* h, const bb_agent_group* d_params, const uint64_t* d_keys, const uint8_t* d_mask) {
+    CHECK_H(h);
+    if (h->groups.empty())  // (the deep engine has no population)
+        return fail(h, BB_EINVAL, "bb_set_agent_params_device: bb_set_agents / bb_set_agents_market has not been called");
+    if (!d_params && !d_keys) return fail(h, BB_EINVAL, "bb_set_agent_params_device: d_params and d_keys are both NULL");
+    CUDA_TRY(h, cudaSetDevice(h->cfg.device));
+    const u32 units = h->cfg.n_envs / h->assets, ng = (u32)h->groups.size();
+    if (!h->d_unit_groups) {  // first call: every unit starts from the declared groups and key 0
+        std::vector<bb_agent_group> rows((size_t)units * ng);
+        for (u32 u = 0; u < units; ++u) std::copy(h->groups.begin(), h->groups.end(), rows.begin() + (size_t)u * ng);
+        bb_agent_group* g = nullptr;
+        u64* k = nullptr;
+        if (cudaMalloc(&g, rows.size() * sizeof(bb_agent_group)) != cudaSuccess || cudaMalloc(&k, (size_t)units * 8) != cudaSuccess) {
+            cudaGetLastError();
+            cudaFree(g);
+            return fail(h, BB_ECUDA, "bb_set_agent_params_device: cannot allocate the per-unit tables");
+        }
+        // (pageable source: the call returns once `rows` has been staged)
+        if (cudaMemcpyAsync(g, rows.data(), rows.size() * sizeof(bb_agent_group), cudaMemcpyHostToDevice, h->stream) != cudaSuccess ||
+            cudaMemsetAsync(k, 0, (size_t)units * 8, h->stream) != cudaSuccess) {
+            cudaStreamSynchronize(h->stream);
+            cudaFree(g);
+            cudaFree(k);
+            return fail(h, BB_ECUDA, "bb_set_agent_params_device: cannot fill the per-unit tables");
+        }
+        h->d_unit_groups = g;
+        h->d_unit_keys = k;
+    }
+    AgentParamsArgs a{};
+    std::copy(h->groups.begin(), h->groups.end(), a.decl);
+    a.src = d_params;
+    a.src_keys = d_keys;
+    a.mask = d_mask;
+    a.dst = h->d_unit_groups;
+    a.dst_keys = h->d_unit_keys;
+    a.blobs = h->blobs;
+    a.blob_stride = h->blob_stride;
+    a.n_groups = ng;
+    a.units = units;
+    a.assets = h->assets;
+    k_agent_params<<<(units + 7) / 8, 256, 0, h->stream>>>(a);
+    CUDA_TRY(h, cudaGetLastError());
+    return BB_OK;
+}
+
 namespace {
 struct ExtRows {  // bb_run_agents_with_rows(_market): the caller's device-resident rows for the launch's first step
     const bb_instr* d_instrs;
@@ -1417,6 +1475,9 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
     for (size_t i = 0; i < h->groups.size(); ++i) p.groups[i] = h->groups[i];
     p.rand_tick_mask = h->rand_tick_mask;
     for (size_t i = 0; i < h->group_asset.size(); ++i) p.group_asset[i] = h->group_asset[i];
+    p.unit_groups = h->d_unit_groups;
+    p.unit_keys = h->d_unit_keys;
+    const bool pu = h->d_unit_groups != nullptr;
     if (ext) {
         p.instrs = ext->d_instrs;
         p.offsets = ext->d_offsets;
@@ -1426,11 +1487,12 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
     }
     int grid = 0;
     // external rows carry no slot hints: they run on the variants that also serve MomentumAgent / NoiseAgent events.  So
-    // does a RandomAgents group that can draw off its book's tick: only those variants check the queued prices
-    const bool mom = h->mom_groups != 0 || ext != nullptr || h->rand_tick_mask != 0;
+    // does a RandomAgents group that can draw off its book's tick: only those variants check the queued prices.  Per-unit
+    // parameters too: the RandomAgents-only kernels get no per-unit twin (DESIGN.md §8)
+    const bool mom = h->mom_groups != 0 || ext != nullptr || h->rand_tick_mask != 0 || pu;
     // markets: the A books of a market are A consecutive warps of one CTA (a CTA holds as many whole markets as fit in 4 warps)
     const u32 wpb = mkt ? (WPB / h->assets) * h->assets : wpb_for(lay.warp_bytes);
-    const Kernel k = sim_kernel(h->eng, mom, mkt, ext != nullptr);
+    const Kernel k = sim_kernel(h->eng, mom, mkt, ext != nullptr, pu);
     if ((rc = grid_for(h, k, lay, h->cfg.n_envs, &grid, wpb))) return rc;
     const size_t warps = (size_t)grid * wpb;
     if (h->eng < ENG_DENSE && warps > h->scratch_warps) {

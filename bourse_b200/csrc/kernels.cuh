@@ -85,6 +85,11 @@ struct KParams {
     // prices are checked against the book's tick (the host derives it from the groups and the tick table).  Last, so that
     // the other kernels' parameter offsets stay where they were
     u32 rand_tick_mask;
+    // k_sim<.., PU = true> (bb_set_agent_params_device): each unit's own group records, [units][n_groups], read in place of
+    // `groups`, and its Philox key, [units], XORed into (seed_lo, seed_hi) for every draw of the unit.  After
+    // rand_tick_mask for the same reason
+    const bb_agent_group* unit_groups;
+    const u64* unit_keys;
 };
 
 // Values the optimiser would otherwise rematerialise at every use (S2R for the lane id, cvta + multiply
@@ -491,13 +496,31 @@ __device__ __forceinline__ bool order_is_active(const Geo& g, const Book& b, u32
     return id < g.max_orders && (ldg32(b.oh + (u64)id * ORD_STRIDE + OH_META) & META_STATUS_MASK) == ST_ACTIVE;
 }
 
+// the Philox key halves of an agent draw: the unit's effective key (k_sim<.., PU>: seed ^ unit key, in key_l / key_h), else the
+// launch's seed read where it is used, so that the other variants compile as they did before per-unit keys existed
+template <bool PU> __device__ __forceinline__ u32 key_lo(const KParams& p, u32 key_l) {
+    if constexpr (PU) return key_l;
+    else return p.seed_lo;
+}
+template <bool PU> __device__ __forceinline__ u32 key_hi(const KParams& p, u32 key_h) {
+    if constexpr (PU) return key_h;
+    else return p.seed_hi;
+}
+// k_sim<.., PU>: the key halves of unit `unit`, the launch's seed XOR the unit's key
+__device__ __forceinline__ void unit_key(const KParams& p, u32 unit, u32& key_l, u32& key_h) {
+    const u64 key = __ldg(p.unit_keys + unit);
+    key_l = p.seed_lo ^ (u32)key;
+    key_h = p.seed_hi ^ (u32)(key >> 32);
+}
+
 // RandomAgents::update (crates/step_sim/src/agents/random_agent.rs:85-119), one lane per agent
+template <bool PU>
 __device__ __forceinline__ void random_agents_update(const KParams& p, const bb_agent_group& ag, const Book& b, uint4* q,
-                                                     Emit& e, u32* slots, u32 env_g, u32 step, u32 slot_base) {
+                                                     Emit& e, u32* slots, u32 env_g, u32 step, u32 slot_base, u32 key_l, u32 key_h) {
     for (u32 a0 = 0; a0 < ag.n_agents; a0 += 32) {
         const u32 a = a0 + b.lane;
         const bool valid = a < ag.n_agents;
-        const uint4 r = philox4x32_10(env_g, step, slot_base + a, 0, p.seed_lo, p.seed_hi);
+        const uint4 r = philox4x32_10(env_g, step, slot_base + a, 0, key_lo<PU>(p, key_l), key_hi<PU>(p, key_h));
         const bool active = valid && (u32_to_f32_unit(r.x) < ag.rate);
         u32 held = BB_NIL;
         if (valid) held = slots[slot_base + a];
@@ -523,14 +546,15 @@ __device__ __forceinline__ void random_agents_update(const KParams& p, const bb_
 // emitted instructions carry the hints described at d_apply (dense.cuh).
 // `chip_base`: index of the group's first agent in the on-chip tables (== slot_base except in markets, whose books keep
 // only their own groups' agents on chip).
-template <class G>
+template <class G, bool PU>
 __device__ __forceinline__ void random_agents_update_dense(const KParams& p, const bb_agent_group& ag, const Book& b, u32 qs, Emit& e,
-                                                           u32 agh, u32 env_g, u32 step, u32 slot_base, u32 chip_base) {
+                                                           u32 agh, u32 env_g, u32 step, u32 slot_base, u32 chip_base, u32 key_l,
+                                                           u32 key_h) {
     for (u32 a0 = 0; a0 < ag.n_agents; a0 += 32) {
         const u32 a = a0 + b.lane;
         const bool valid = a < ag.n_agents;
         const u32 ai = valid ? chip_base + a : 0u;
-        const uint4 r = philox4x32_10(env_g, step, slot_base + a, 0, p.seed_lo, p.seed_hi);
+        const uint4 r = philox4x32_10(env_g, step, slot_base + a, 0, key_lo<PU>(p, key_l), key_hi<PU>(p, key_h));
         const bool active = valid && (u32_to_f32_unit(r.x) < ag.rate);
         const u32 held = lds(agh + 4u * ai);
         const u32 hs = lds8(b.ags + 1u + ai);
@@ -596,12 +620,16 @@ __device__ __forceinline__ u32 round_price(double x, double tick, bool up) {
 struct MomOut {
     u32 n, next_id, err;
 };
+template <bool PU>
 __device__ __noinline__ MomOut momentum_agent_update(const KParams& p, const bb_agent_group& ag, u64 oh, u32 book_tick, u32 bid,
                                                      u32 ask, uint4* q, u32 e_n, u32 e_next_id, MomState* ms, u32 env_g,
                                                      u32 step, u32 gi, u32 slot_base) {
     // (`book_tick`, the tick of the book the group trades, takes the argument slot of the lane id, which is recomputed here:
-    // one more argument costs the momentum k_sim variants spill traffic)
+    // one more argument costs the momentum k_sim variants spill traffic; for the same reason PU reads the unit's key here:
+    // env_g is the unit's id plus the launch's first, and env_id_base is a multiple of assets)
     const u32 lane = threadIdx.x & 31u;
+    u32 key_l = 0, key_h = 0;
+    if constexpr (PU) unit_key(p, env_g - p.env_id_base / p.assets, key_l, key_h);
     Emit e;
     e.n = e_n;
     e.next_id = e_next_id;
@@ -618,7 +646,7 @@ __device__ __noinline__ MomOut momentum_agent_update(const KParams& p, const bb_
             id = ms->live[k];
             active = id < p.geo.max_orders && (ldg32(oh + (u64)id * ORD_STRIDE + OH_META) & META_STATUS_MASK) == ST_ACTIVE;
         }
-        const uint4 r = philox4x32_10(env_g, step, PHILOX_SLOT_CANCEL | gi, k >> 2, p.seed_lo, p.seed_hi);
+        const uint4 r = philox4x32_10(env_g, step, PHILOX_SLOT_CANCEL | gi, k >> 2, key_lo<PU>(p, key_l), key_hi<PU>(p, key_h));
         const u32 word = (k & 3u) == 0 ? r.x : (k & 3u) == 1 ? r.y : (k & 3u) == 2 ? r.z : r.w;
         const bool keep = active && (u32_to_f32_unit(word) > ag.rate);
         const bool cancel = active && !keep;
@@ -644,8 +672,8 @@ __device__ __noinline__ MomOut momentum_agent_update(const KParams& p, const bb_
     for (u32 j0 = 0; j0 < ag.n_agents; j0 += 32) {
         const u32 j = j0 + lane;
         const bool valid = j < ag.n_agents;
-        const uint4 ra = philox4x32_10(env_g, step, slot_base + j, 0, p.seed_lo, p.seed_hi);
-        const uint4 rb = philox4x32_10(env_g, step, slot_base + j, 1, p.seed_lo, p.seed_hi);
+        const uint4 ra = philox4x32_10(env_g, step, slot_base + j, 0, key_lo<PU>(p, key_l), key_hi<PU>(p, key_h));
+        const uint4 rb = philox4x32_10(env_g, step, slot_base + j, 1, key_lo<PU>(p, key_l), key_hi<PU>(p, key_h));
         const bool dir = (m > 0.0) || (m < 0.0);
         bool do_limit = valid && dir && (u64_to_f64_unit(ra.x, ra.y) < p_limit);
         bool do_market = valid && dir && (u64_to_f64_unit(ra.z, ra.w) < p_market);
@@ -732,9 +760,14 @@ __device__ __forceinline__ void market_bar_sync(u32 id, u32 n_threads) {
 // those rows are its own: the queued rows follow all groups' instructions in the market's queue, and each book appends
 // its own after its agents' events.  A per-warp bitmask over the market's queued rows (with per-word prefix counts) maps a
 // shuffled position back to the book's own list; it sits behind jarr, in a layout only this variant uses.
-template <int ENG, bool MOM, bool MKT = false, bool EXT = false>
+// PU (bb_set_agent_params_device; always with MOM): every unit (env, or market) draws with its own group records and Philox
+// key, p.unit_groups / p.unit_keys, instead of the launch's p.groups and (seed_lo, seed_hi).  The records stay inside the
+// declared population (bb_set_agents sized everything from p.groups: n_agents, agent ids, live-list capacities, the dense
+// window), so only the draws' parameters and key differ; n_agents is still read from p.groups.
+template <int ENG, bool MOM, bool MKT = false, bool EXT = false, bool PU = false>
 __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __grid_constant__ KParams p) {
     static_assert(!EXT || MOM, "external rows ride on the unhinted (MOM) variants");
+    static_assert(!PU || MOM, "per-unit parameters ride on the unhinted (MOM) variants");
     typedef GeoT<ENG> G;
     extern __shared__ __align__(128) unsigned char smem[];
     const u32 lane = keep32(threadIdx.x & 31u), warp = threadIdx.x >> 5, wpb = blockDim.x >> 5;
@@ -779,6 +812,14 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
         book_from_header(g, b);
         // the RNG unit: the env, or the whole market (agent slots and the shuffle are market-wide)
         const u32 env_g = MKT ? (p.env_id_base + env) / p.assets : p.env_id_base + env;
+        // PU: the unit's Philox key halves and group records
+        u32 key_l = 0, key_h = 0;
+        const bb_agent_group* urow = nullptr;
+        if constexpr (PU) {
+            const u32 unit = MKT ? env / p.assets : env;
+            unit_key(p, unit, key_l, key_h);
+            urow = p.unit_groups + (size_t)unit * p.n_groups;
+        }
         u32* slots = p.rslot + (size_t)env * p.agents_per_env;
         const u32 agh = sb + p.off_ag;  // dense engine: held order id per agent, u32 [agents_per_env]
         if constexpr (G::DENSE) {
@@ -823,17 +864,17 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
             u32 slot_base = 0, chip_base = 0, mi = 0;
             u32 mk_cnt = 0;  // markets: lane gi holds the number of instructions group gi queued (own groups only)
             for (u32 gi = 0; gi < p.n_groups; ++gi) {
-                const bb_agent_group& ag = p.groups[gi];
+                const bb_agent_group& ag = PU ? urow[gi] : p.groups[gi];  // PU: the unit's row in global memory, read through L1
                 const bool mine = !MKT || p.group_asset[gi] == mk_a;
                 const u32 n_before = e.n;
                 if (!MOM || ag.kind == BB_GROUP_RANDOM) {
                     if (mine) {
-                        if constexpr (G::DENSE) random_agents_update_dense<G>(p, ag, b, qs, e, agh, env_g, step, slot_base, chip_base);
-                        else random_agents_update(p, ag, b, q, e, slots, env_g, step, slot_base);
+                        if constexpr (G::DENSE) random_agents_update_dense<G, PU>(p, ag, b, qs, e, agh, env_g, step, slot_base, chip_base, key_l, key_h);
+                        else random_agents_update<PU>(p, ag, b, q, e, slots, env_g, step, slot_base, key_l, key_h);
                     }
                 } else {
                     if (mine) {
-                        const MomOut mo = momentum_agent_update(p, ag, b.oh, __ldg(g.ticks + env), best_price(g, b, 1), best_price(g, b, 0), q, e.n,
+                        const MomOut mo = momentum_agent_update<PU>(p, ag, b.oh, __ldg(g.ticks + env), best_price(g, b, 1), best_price(g, b, 0), q, e.n,
                                                                 e.next_id, (MomState*)((char*)p.mom + ((size_t)env * p.mom_groups_per_env + mi) * p.mom_stride), env_g,
                                                                 step, gi, slot_base);
                         e.n = mo.n;
@@ -952,7 +993,7 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
             for (u32 b0 = 0; b0 * 4u < nq; b0 += 32) {
                 const u32 blk = b0 + lane;
                 if (blk * 4u < nq) {
-                    const uint4 r = philox4x32_10(env_g, step, PHILOX_SLOT_SHUFFLE, blk, p.seed_lo, p.seed_hi);
+                    const uint4 r = philox4x32_10(env_g, step, PHILOX_SLOT_SHUFFLE, blk, key_lo<PU>(p, key_l), key_hi<PU>(p, key_h));
                     const u32 i = blk * 4u;
                     // 4 consecutive u16 slots are always in bounds: the array is padded to a multiple of 8 bytes
                     const u32 j0 = mulhi_range(r.x, i + 1), j1 = mulhi_range(r.y, i + 2);
@@ -2039,6 +2080,45 @@ __global__ void __launch_bounds__(256) k_store_copy(const __grid_constant__ Stor
                                                     u32* cursor) {
     for (u32 book = blockIdx.x; book < n_books; book += gridDim.x)
         store_copy_book<RESTORE>(c, book, blockIdx.y, gridDim.y, sel, seeds, cursor);
+}
+
+// bb_set_agent_params_device: one warp per unit, lane gi checks the unit's record for group gi against the declared one
+// (the envelope rule of include/bourse_b200.h).  The unit's verdict is the warp's ballot: a unit with any
+// record outside the declared population keeps its records and key and every book of it is flagged ERR_PARAMS; a valid
+// unit takes its row and / or key.  Units the mask leaves out are not read.
+#define ERR_PARAMS 0x2000u  // == BB_ERR_PARAMS
+struct AgentParamsArgs {
+    bb_agent_group decl[MAX_GROUPS];  // the declared population (bb_set_agents / bb_set_agents_market)
+    const bb_agent_group* src;        // [units][n_groups] or null: records stay
+    const u64* src_keys;              // [units] or null: keys stay
+    const uint8_t* mask;              // [units] or null: every unit
+    bb_agent_group* dst;              // the handle's tables
+    u64* dst_keys;
+    unsigned char* blobs;
+    u64 blob_stride;
+    u32 n_groups, units, assets;
+};
+
+__device__ __forceinline__ bool agent_record_fits(const bb_agent_group& r, const bb_agent_group& d) {
+    if (r.kind != d.kind || r.n_agents != d.n_agents || r.tick_size != d.tick_size) return false;
+    if (d.kind == BB_GROUP_RANDOM)
+        return d.tick_lo <= r.tick_lo && r.tick_lo < r.tick_hi && r.tick_hi <= d.tick_hi && d.vol_lo <= r.vol_lo && r.vol_lo < r.vol_hi &&
+               r.vol_hi <= d.vol_hi;
+    return r.tick_lo == d.tick_lo && r.vol_hi == d.vol_hi;  // agent_id_start, live-list capacity
+}
+
+__global__ void __launch_bounds__(256) k_agent_params(const __grid_constant__ AgentParamsArgs a) {
+    const u32 lane = threadIdx.x & 31u, unit = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (unit >= a.units || (a.mask && !a.mask[unit])) return;  // (whole warps leave together)
+    const bool mine = a.src && lane < a.n_groups;
+    bb_agent_group r;
+    if (mine) r = a.src[(size_t)unit * a.n_groups + lane];
+    if (!__all_sync(BB_FULL, !mine || agent_record_fits(r, a.decl[lane]))) {
+        if (lane < a.assets) atomicOr(&reinterpret_cast<BookHdr*>(a.blobs + ((u64)unit * a.assets + lane) * a.blob_stride)->err, ERR_PARAMS);
+        return;
+    }
+    if (mine) a.dst[(size_t)unit * a.n_groups + lane] = r;
+    if (a.src_keys && lane == 0) a.dst_keys[unit] = a.src_keys[unit];
 }
 
 // reduction of per-env counters for bb_stats

@@ -214,6 +214,7 @@ class _DeviceLoop:
     obs: DeviceArray
     ids: DeviceArray
     _what = "env"
+    _groups: typing.Optional[np.ndarray] = None   # the declared background population, abi.GROUP_DTYPE [n_groups]
 
     def _buffers(self, obs_shape, rows_shape):
         self.obs = DeviceArray(self.env, obs_shape, np.uint32)
@@ -307,6 +308,54 @@ class _DeviceLoop:
         self._keep = (keep_slots, keep_seeds)
         self.env.restore_device(store.ptr, slots_ptr, seeds_ptr, self.obs.ptr, self._cursor.ptr)
         return self.obs
+
+    def agent_params(self) -> np.ndarray:
+        """A host `abi.GROUP_DTYPE` array `[units, n_groups]` filled with the declared background groups: the template for
+        `set_agent_params` (edit it, e.g. `p["rate"][:, 0] = rates`, and pass it back)."""
+        if self._groups is None:
+            raise ValueError("the env has no background agents")
+        return np.tile(self._groups, (self._units, 1))
+
+    def set_agent_params(self, params=None, *, keys=None, mask=None):
+        """Per-unit background-agent parameters and Philox keys (bb_set_agent_params_device); a unit is an env, or a market
+        for `MarketVectorEnv`.  Every unit `mask` selects (default: all) takes its row of `params` and / or its entry of
+        `keys`; every later `step` runs group gi of unit u with `params[u, gi]` and draws with the agent seed XOR `keys[u]`
+        (agent draws and the step's shuffle).  Keys start at 0, the parameters at the declared groups.
+
+        `params`: the `[units, n_groups]` array `agent_params()` returns, edited, or any C-contiguous device array (CUDA
+        array interface / DLPack) of exactly `units * n_groups * 80` bytes in that layout; `None` keeps the parameters.
+        `keys`: `[units]` 8-byte integers; `mask`: `[units]` bool / 1-byte integers; each a device array or numpy.  Rows
+        must stay inside the declared population: same kind, agent count and tick size; RandomAgents tick and volume
+        ranges inside the declared ones; Momentum / Noise agent id start and live-list capacity (`tick_lo`, `vol_hi`)
+        unchanged.  A unit with any other row keeps its parameters and key and is flagged (`BB_ERR_PARAMS`,
+        `check_errors` raises).  `reset` and `restore` keep parameters and keys.  One launch with no host
+        synchronisation (device arrays)."""
+        if params is None and keys is None:
+            raise ValueError("pass params, keys or both")
+        if self._groups is None:
+            raise ValueError("the env has no background agents")
+        units, ng = self._units, len(self._groups)
+        nbytes = units * ng * abi.GROUP_DTYPE.itemsize
+        params_ptr, keep_params, host_params = 0, None, None
+        if params is not None:
+            dev = _device_array(params)
+            if dev is not None:
+                params_ptr, shape, typ, keep_params = dev
+                n = int(np.prod(shape)) * typ.itemsize
+                if n != nbytes:
+                    raise ValueError(f"params: device array holds {n} bytes, expected {nbytes} ([{units}, {ng}] records of 80 bytes)")
+            else:
+                host_params = np.asarray(params)
+                if host_params.dtype != abi.GROUP_DTYPE or host_params.shape != (units, ng):
+                    raise ValueError(f"params must be a [{units}, {ng}] abi.GROUP_DTYPE array (agent_params())")
+        keys_ptr, keep_keys = self._unit_array(keys, np.uint64, "keys") if keys is not None else (0, None)
+        mask_ptr, keep_mask = self._unit_array(mask, np.uint8, "mask") if mask is not None else (0, None)
+        if host_params is not None:
+            buf = self._buffer(("params", units, ng), (nbytes,), np.uint8)
+            buf.copy_from_host(np.ascontiguousarray(host_params).view(np.uint8).reshape(-1))
+            params_ptr = buf.ptr
+        self._keep = (keep_params, keep_keys, keep_mask)   # alive until the next call, as in _action_ptr
+        self.env.set_agent_params_device(params_ptr, keys_ptr, mask_ptr)
 
     def _unit_array(self, x, dtype, name, n=None) -> typing.Tuple[int, typing.Any]:
         """(device address, keep-alive object) of an [n] (default: [units]) mask (bool / 1-byte integers), unit or slot
@@ -407,11 +456,13 @@ class _DeviceLoop:
         return ptr
 
     def check_errors(self):
-        """Raise if any env flagged an error (capacity, bad order id, off-tick price); synchronises."""
+        """Raise if any env flagged an error (capacity, bad order id, off-tick price, a refused `set_agent_params` row);
+        synchronises."""
         e = self.env.env_errors()
         if e.any():
             bad = np.flatnonzero(e)
-            raise RuntimeError(f"{len(bad)} {self._what}(s) flagged errors, first {self._what} {bad[0]}: 0x{int(e[bad[0]]):x}")
+            params = " (0x2000: a set_agent_params row outside the declared population)" if (e & abi.ERR_PARAMS).any() else ""
+            raise RuntimeError(f"{len(bad)} {self._what}(s) flagged errors, first {self._what} {bad[0]}: 0x{int(e[bad[0]]):x}{params}")
 
 
 class VectorEnv(_DeviceLoop):
@@ -434,7 +485,11 @@ class VectorEnv(_DeviceLoop):
     synchronisation, so a loop of policy + `step` can be captured into a CUDA graph and replayed (tests/test_gpu_gym.py);
     steps that include the built-in agents refuse capture (their history staging is validated on the host).  The library's
     per-step history is a scratch ring for this class: `step` clears it (`bb_clear_history`) whenever `max_steps` records
-    have accumulated; a caller replaying a captured step must do the same every `max_steps` replays."""
+    have accumulated; a caller replaying a captured step must do the same every `max_steps` replays.
+
+    With background agents, `set_agent_params` gives each env its own group parameters (a market regime per env) and its own
+    agent key.  Reproducible but distinct episodes: `reset(mask, seeds)` with the envs' creation seeds replays the same agent
+    draws, and `set_agent_params(keys=new_keys, mask=mask)` before it makes them new ones; the same key replays them."""
 
     def __init__(self, n_envs: int, rows_per_env: int, seed: int, start_time: int, tick_size: typing.Union[int, typing.Sequence[int]], step_size: int,
                  trading: bool = True, *, level_1: bool = False, agents=None, agent_seed: int = 0, **kw):
@@ -449,6 +504,7 @@ class VectorEnv(_DeviceLoop):
         if rows_per_env > kw["max_queue"]:
             raise ValueError("rows_per_env exceeds max_queue")
         self._agents, self._agent_seed = agents, agent_seed
+        self._groups = np.array(list(agents), dtype=abi.GROUP_DTYPE) if agents else None
         self._n_steps = 0
         self.n_envs, self.rows = n_envs, rows_per_env
         self.env = BatchedEnv(n_envs, seed, start_time, tick_size, step_size, trading, obs_words=abi.OBS_L1 if level_1 else abi.OBS_L2, **kw)
@@ -502,7 +558,11 @@ class MarketVectorEnv(_DeviceLoop):
 
     Which class: this one for an RL-style loop over many markets, alone (no `agents`) or against built-in agents in the
     same shuffled queue (`agents=`); `market.MarketEnv` (`place_order` / `submit` + `step` on the host) for scripted,
-    order-by-order use, and its `run_agents` for markets of built-in agents with no learner."""
+    order-by-order use, and its `run_agents` for markets of built-in agents with no learner.
+
+    With `agents`, `set_agent_params` gives each market its own group parameters (group gi applies to its asset's book) and
+    its own agent key; `reset(mask, seeds)` plus `set_agent_params(keys=..., mask=...)` gives reproducible but distinct
+    episodes, as for `VectorEnv`."""
 
     _what = "book"
 
@@ -536,6 +596,7 @@ class MarketVectorEnv(_DeviceLoop):
         if A * kw["max_queue"] > 65535:
             raise ValueError("assets * max_queue must stay below 65536")
         self._agents, self._agent_seed = agents, agent_seed
+        self._groups = np.array([a.group for a in agents], dtype=abi.GROUP_DTYPE) if agents else None
         self._n_steps = 0
         self.n_markets, self.rows, self.n_assets, self.tick_sizes = n_markets, rows_per_market, A, ticks
         self.obs_words = abi.OBS_L1 if level_1 else abi.OBS_L2

@@ -51,6 +51,7 @@ typedef enum {
 #define BB_ERR_ROW_OP 0x400u     /* bb_run_agents_with_rows(_market): a MODIFY row or a trader id >= 2^19 (row dropped); markets: a row's aux names no asset */
 #define BB_ERR_LOCKED 0x800u     /* deep engine: both sides would rest at one price level (trading disabled) */
 #define BB_ERR_SLOT 0x1000u      /* bb_restore_device: the slot was empty, out of range, or saved from a book of another tick */
+#define BB_ERR_PARAMS 0x2000u    /* bb_set_agent_params_device: a unit's parameter row broke the declared population (row not applied) */
 
 #define BB_OBS_L1 9u   /* StepEnvNumpy.level_1_data layout, rust/src/step_sim_numpy.rs:300-318 */
 #define BB_OBS_L2 45u  /* StepEnvNumpy.level_2_data layout, rust/src/step_sim_numpy.rs:351-368 */
@@ -438,6 +439,29 @@ int bb_set_agents(bb_handle* h, const bb_agent_group* groups, uint32_t n_groups)
  * whole and event i executes at start + i on its asset's book (market_env.rs:108-121).  The RNG unit is the market:
  * Philox key (seed; global market id = (env_id_base + env) / assets, step, agent slot counted over all groups). */
 int bb_set_agents_market(bb_handle* h, const bb_agent_group* groups, const uint32_t* asset, uint32_t n_groups);
+/* Per-unit agent parameters and Philox keys for the population bb_set_agents / bb_set_agents_market declared.  A unit is an
+ * env, or a market on a multi-asset handle.  Every unit whose d_mask byte is non-zero (d_mask NULL: every unit) takes its row
+ * d_params[u][0 .. n_groups) and / or its key d_keys[u]; d_params NULL keeps the units' records, d_keys NULL their keys.
+ * From then on every agent launch of the handle (bb_run_agents, bb_run_agents_to_host, bb_run_agents_with_rows(_market))
+ * runs group gi of unit u with record d_params[u][gi], and draws with key seed ^ key[u] (a 64-bit XOR): every RandomAgents,
+ * MomentumAgent and NoiseAgent draw and the step's shuffle.  Unit u with key k draws what it would draw with seed ^ k;
+ * keys start at 0.  The shuffle streams that bb_reset_device re-seeds (device-row steps, bb_step) are not affected.
+ *   The declared population is the envelope: what bb_set_agents sized from the groups (agent state, trader ids, live
+ * lists, the dense window) stays valid.  A record r for group gi, declared as d, is valid only if r.kind, r.n_agents and
+ * r.tick_size equal d's and
+ *   - RandomAgents: d.tick_lo <= r.tick_lo < r.tick_hi <= d.tick_hi and d.vol_lo <= r.vol_lo < r.vol_hi <= d.vol_hi; rate free;
+ *   - MomentumAgent / NoiseAgent: r.tick_lo == d.tick_lo (agent_id_start) and r.vol_hi == d.vol_hi (live-list capacity);
+ *     rate, vol_lo (trade_vol), decay, demand, scale, order_ratio, mu and sigma free.
+ * Validation happens on the device: a unit with any invalid record changes nothing, its key included, and every book of it
+ * is flagged BB_ERR_PARAMS; the other units are applied.
+ *   Lifetime: the first call allocates [units][n_groups] records and [units] keys, filled from the declared groups and zero
+ * keys, then applies the call.  bb_set_agents(_market) drops both (shared parameters and zero keys again); bb_reset,
+ * bb_reset_device and bb_restore_device keep them (they are configuration, not state: store slots do not hold them);
+ * bb_destroy frees them.  With the tables, agent launches run variants that read each unit's row from memory.
+ *   One launch on the handle's stream, no host synchronisation (the first call also allocates).  BB_EINVAL, handle
+ * unchanged: no population (which covers the deep engine), or d_params and d_keys both NULL. */
+int bb_set_agent_params_device(bb_handle* h, const bb_agent_group* d_params /* [units][n_groups] or NULL */,
+                               const uint64_t* d_keys /* [units] or NULL */, const uint8_t* d_mask /* [units] or NULL = all */);
 /* n_steps of { agents.update(env); env.step() } for every env inside one persistent kernel.
  * Draws are Philox4x32-10 keyed (seed; global env id, step, agent) — DESIGN.md "RNG contract".
  * Asynchronous on the handle's stream; pair with bb_synchronize or any read call. */

@@ -39,6 +39,15 @@ does a restore, so the DRAM traffic is twice it).
     python scripts/bench_market_vector.py --reads --steps 1000 --warmup 20
     python scripts/bench_market_vector.py --resets --passes 3
     python scripts/bench_market_vector.py --snapshots --passes 3
+    python scripts/bench_market_vector.py --agent-params --steps 1000 --warmup 20 --passes 3
+
+--agent-params measures per-unit agent parameters (bb_set_agent_params_device, `set_agent_params`): the step time of
+VectorEnv(4096 envs, agents=c3_groups()) on FAST and dense and of c4_groups() on FAST, and of MarketVectorEnv(2048 markets x
+4 assets) with the C3 population on every asset on FAST and dense, each with shared parameters and with per-unit rows and
+keys (the per-unit variants of k_sim), 2 rows per book; shared and per-unit runs alternate, --passes times each, best pass.
+The per-unit rows are the declared groups with each unit's rates drawn from [0.1, 0.9), so the books stay as busy as with
+the shared ones.  Then the time of one `set_agent_params` call (device rows, keys and mask) selecting 1 % and 100 % of the
+units: CUDA events around 200 calls replayed from a CUDA graph.
 """
 from __future__ import annotations
 
@@ -339,6 +348,63 @@ def bench_snapshots(args, name, power):
     return res
 
 
+def bench_agent_params(args, name, power):
+    """--agent-params: see the module docstring."""
+    import torch
+    n_envs = N_BOOKS // 2
+    res = {"card": name, "power_limit": power, "steps": args.steps, "warmup": args.warmup, "passes": args.passes,
+           "rows_per_book": ROWS_PER_BOOK, "us_per_step": {}, "us_per_call": {}, "errors": {}}
+    blocks = gym_action_blocks(args.blocks, n_envs, ROWS_PER_BOOK, seed=5)
+    blocks["price"] = np.where((blocks["op_flags"] & abi.F_MARKET) != 0, blocks["price"], 2 * (40 + blocks["price"] % 21))
+    mblocks = blocks.reshape(len(blocks), N_MARKETS, ROWS).copy()
+    mblocks["aux"] = np.repeat(np.arange(ASSETS, dtype=np.uint32), ROWS_PER_BOOK)
+
+    def as_device(b):
+        return [torch.from_numpy(x.view(np.uint8).reshape(x.shape[0], -1)).cuda() for x in b]
+
+    d_env, d_mkt = as_device(blocks), as_device(mblocks)
+    rng = np.random.default_rng(9)
+
+    def per_unit(loop):
+        p = loop.agent_params()
+        p["rate"] = rng.uniform(0.1, 0.9, p.shape).astype(np.float32)
+        loop.set_agent_params(p, keys=rng.integers(0, 2**63, p.shape[0], dtype=np.uint64))
+
+    cases = [("vector_c3_fast", lambda: gym.VectorEnv(n_envs, ROWS_PER_BOOK, 0, 0, 1, 1_000_000, agents=workloads.c3_groups(),
+                                                       agent_seed=5, **BG_KW), d_env),
+             ("vector_c3_dense", lambda: gym.VectorEnv(n_envs, ROWS_PER_BOOK, 0, 0, 1, 1_000_000, agents=workloads.c3_groups(),
+                                                        agent_seed=5, **BG_KW, **BG_ENGINES["dense"]), d_env),
+             ("vector_c4_fast", lambda: gym.VectorEnv(n_envs, ROWS_PER_BOOK, 0, 0, 1, 1_000_000, agents=workloads.c4_groups(),
+                                                       agent_seed=5, **BG_KW), d_env),
+             ("market_c3_fast", lambda: gym.MarketVectorEnv(N_MARKETS, ROWS, 0, 0, [1] * ASSETS, 1_000_000, agents=c3_market_agents(),
+                                                             agent_seed=5, **BG_KW), d_mkt),
+             ("market_c3_dense", lambda: gym.MarketVectorEnv(N_MARKETS, ROWS, 0, 0, [1] * ASSETS, 1_000_000, agents=c3_market_agents(),
+                                                              agent_seed=5, **BG_KW, **BG_ENGINES["dense"]), d_mkt)]
+    for case, make, d in cases:
+        shared, pu = make(), make()
+        per_unit(pu)
+        best = {"shared": float("inf"), "per_unit": float("inf")}
+        for _ in range(args.passes):   # shared and per-unit runs alternate
+            for kind, loop in (("shared", shared), ("per_unit", pu)):
+                us, err = time_device(loop, d, args.steps, args.warmup)
+                best[kind] = min(best[kind], us)
+                res["errors"][f"{case}_{kind}"] = res["errors"].get(f"{case}_{kind}", 0) | err
+        for kind in best:
+            res["us_per_step"][f"{case}_{kind}"] = best[kind]
+        # one set_agent_params call with device rows, keys and a mask selecting 1 % / 100 % of the units
+        units = pu._units
+        rows = torch.from_numpy(pu.agent_params().view(np.uint8).reshape(units, -1).copy()).cuda()
+        keys = torch.arange(units, device="cuda", dtype=torch.int64)
+        for frac in (0.01, 1.0):
+            mask = torch.zeros(units, device="cuda", dtype=torch.uint8)
+            mask[: max(1, int(units * frac))] = 1
+            _, graph_us = time_calls(pu, lambda: pu.set_agent_params(rows, keys=keys, mask=mask))
+            res["us_per_call"][f"{case}_set_agent_params_{int(frac * 100)}pct"] = graph_us
+        shared.close()
+        pu.close()
+    return res
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=1000)
@@ -348,8 +414,9 @@ def main():
     ap.add_argument("--reads", action="store_true", help="time orders() / trades() in the C3 loops (see the module docstring)")
     ap.add_argument("--resets", action="store_true", help="time reset(mask) in the rows-only loops (see the module docstring)")
     ap.add_argument("--snapshots", action="store_true", help="time save / restore on warmed C3 books (see the module docstring)")
+    ap.add_argument("--agent-params", action="store_true", help="per-unit agent parameters (see the module docstring)")
     ap.add_argument("--warmup-steps", type=int, default=300, help="--snapshots: C3 steps before the store is filled")
-    ap.add_argument("--passes", type=int, default=3, help="--resets / --snapshots: timed passes of each variant")
+    ap.add_argument("--passes", type=int, default=3, help="--resets / --snapshots / --agent-params: timed passes of each variant")
     args = ap.parse_args()
     import torch
 
@@ -363,6 +430,9 @@ def main():
         return
     if args.snapshots:
         print(json.dumps(bench_snapshots(args, name, power)), flush=True)
+        return
+    if args.agent_params:
+        print(json.dumps(bench_agent_params(args, name, power)), flush=True)
         return
     blocks = gym_action_blocks(args.blocks, N_BOOKS, ROWS_PER_BOOK, seed=5)
     if args.bg_agents:   # limit prices into the agents' range, as bench.py run_gym does
