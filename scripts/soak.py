@@ -121,7 +121,7 @@ while time.time() < t_end and (not only or rounds < len(only)):
                 for a in range(A):
                     assert np.array_equal(e.history(m * A + a), o.history(a)) and e.get_trades(m * A + a) == o.get_trades(a) and e.get_orders(m * A + a) == o.get_orders(a), (m, a)
         else:
-            n_envs = int(rng.integers(1, 64)); rows = int(rng.integers(1, 7))
+            n_envs = int(rng.integers(1, 64)); rows = int(rng.integers(1, 71))  # up to 70: rounds cross the 32-row passes of submit_rows
             v = gym.VectorEnv(n_envs, rows, 0, 0, 1, 1_000_000, agents=build(core, gs), agent_seed=rs, max_orders=16384, max_trades=32768, max_steps=64, max_queue=512, **kw)
             last_env = v.env
             os_ = [orc.StepEnv(0, 0, 1, 1_000_000) for _ in range(n_envs)]
