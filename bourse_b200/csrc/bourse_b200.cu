@@ -84,6 +84,10 @@ struct bb_handle {
     unsigned char* dp_pool = nullptr;
     u32 dp_chunks = 0;
     bool deep_attr_set = false;
+    // bb_step_device on the deep engine: the staged replay slices, bb_instr [n_envs][max_queue + 1], and their bounds
+    // u64 [n_envs][2] (k_env_deep_stage -> k_deepw<.., ENV>); allocated at creation, regrown by bb_reserve_queue
+    bb_instr* d_stage = nullptr;
+    u64* d_stage_off = nullptr;
     bool deep_serial = false;  // developer switch (BOURSE_B200_DEEP=serial): every event through k_deepw's serial path
     // agents
     std::vector<bb_agent_group> groups;
@@ -279,6 +283,19 @@ DeepOff deep_layout(u32 W, u32 roomy /* filter size multiplier: 1, 4, 8 */) {
     return o;
 }
 
+// k_env_deep_stage's dynamic shared memory: the step's permutation, u16 [max_queue]
+size_t stage_smem(u32 max_queue) { return align_up(2u * max_queue, 16); }
+
+// the deep engine's staging stream for bb_step_device, sized for max_queue (synchronous: the old one may be in use)
+int alloc_stage(bb_handle* h, u32 max_queue) {
+    CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+    cudaFree(h->d_stage);
+    h->d_stage = nullptr;
+    CUDA_TRY(h, cudaMalloc(&h->d_stage, (size_t)h->cfg.n_envs * (max_queue + 1u) * sizeof(bb_instr)));
+    if (!h->d_stage_off) CUDA_TRY(h, cudaMalloc(&h->d_stage_off, (size_t)h->cfg.n_envs * 16u));
+    return BB_OK;
+}
+
 template <class K> int grid_for(bb_handle* h, K kernel, const SmemLayout& l, u32 n_items, int* grid_out, u32 wpb = WPB) {
     const size_t smem = (size_t)l.warp_bytes * wpb;
     // the attribute / occupancy queries cost several microseconds of host time: a per-step caller (bb_step_device in an
@@ -457,7 +474,6 @@ bool stream_capturing(bb_handle* h) {
 int check_device_rows(bb_handle* h, const bb_instr* d_instrs, const u64* d_offsets, u64 n_rows, bool market, const char* wrong_handle) {
     if (!d_offsets || (n_rows && !d_instrs)) return fail(h, BB_EINVAL, "null argument");
     if (market != (h->assets > 1)) return fail(h, BB_EINVAL, wrong_handle);
-    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine replays instruction streams only");
     if (market && (u64)h->assets * h->cfg.max_queue > 65535) return fail(h, BB_EINVAL, "assets * max_queue must stay below 65536");
     return refuse_pending_queue(h);
 }
@@ -491,6 +507,46 @@ Kernel sim_kernel(int eng, bool mom, bool mkt, bool ext, bool pu) {
     return sim_kernel_for<ENG_PAGED>(mom, mkt, ext, pu);
 }
 
+int deep_attrs(bb_handle* h) {
+    if (h->deep_attr_set) return BB_OK;
+    CUDA_TRY(h, cudaFuncSetAttribute(k_deepw<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 1024));
+    CUDA_TRY(h, cudaFuncSetAttribute(k_deepw<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 1024));
+    CUDA_TRY(h, cudaFuncSetAttribute(k_deepw<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 1024));
+    CUDA_TRY(h, cudaFuncSetAttribute(k_deepw<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 1024));
+    CUDA_TRY(h, cudaFuncSetAttribute(k_env_deep_stage, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stage_smem(65535u)));
+    h->deep_attr_set = true;
+    return BB_OK;
+}
+
+// one k_deepw launch over the slices p.instrs / p.offsets describe (ENV: the staged ones, {begin, end} per book)
+template <bool ENV> int launch_deepw(bb_handle* h, KParams& p) {
+    if (int rc = deep_attrs(h)) return rc;
+    p.dp_fast = h->deep_serial ? 0u : 1u;
+    if (h->dp.dirty_n > DW_DIRTY) k_deepw<true, ENV><<<h->cfg.n_envs, 128, h->dp.total, h->stream>>>(p);
+    else k_deepw<false, ENV><<<h->cfg.n_envs, 128, h->dp.total, h->stream>>>(p);
+    CUDA_TRY(h, cudaGetLastError());
+    h->recorded_host = -1;  // (re-read from the device when needed)
+    return BB_OK;
+}
+
+// bb_step_device on the deep engine: submission and shuffle into the staging stream, then the staged slices through k_deepw
+int step_deep(bb_handle* h, const bb_instr* d_instrs, const u64* d_offsets, u64* d_out_ids, u32* d_obs_out) {
+    if (int rc = deep_attrs(h)) return rc;
+    KParams p;
+    fill_params(h, h->lay_apply, p);
+    p.instrs = d_instrs;
+    p.offsets = d_offsets;
+    p.assign_ids = 1u;
+    p.out_ids = d_out_ids;
+    p.obs_out = d_obs_out;
+    h->status_valid = false;
+    k_env_deep_stage<<<h->cfg.n_envs, 32, stage_smem(h->cfg.max_queue), h->stream>>>(p, h->d_stage, h->d_stage_off);
+    CUDA_TRY(h, cudaGetLastError());
+    p.instrs = h->d_stage;
+    p.offsets = h->d_stage_off;
+    return launch_deepw<true>(h, p);
+}
+
 int launch_apply(bb_handle* h, int mode, const bb_instr* d_instrs, const u64* d_offsets, u32 n_steps, bool host_order = false,
                  u64* d_out_ids = nullptr, u32* d_obs_out = nullptr) {
     KParams p;
@@ -506,17 +562,7 @@ int launch_apply(bb_handle* h, int mode, const bb_instr* d_instrs, const u64* d_
     p.obs_out = d_obs_out;
     if (h->eng == ENG_DEEP) {
         if (mode != MODE_REPLAY || d_out_ids || d_obs_out) return fail(h, BB_EINVAL, "the deep-book engine replays instruction streams only");
-        if (!h->deep_attr_set) {
-            CUDA_TRY(h, cudaFuncSetAttribute(k_deepw<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 1024));
-            CUDA_TRY(h, cudaFuncSetAttribute(k_deepw<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 1024));
-            h->deep_attr_set = true;
-        }
-        p.dp_fast = h->deep_serial ? 0u : 1u;
-        if (h->dp.dirty_n > DW_DIRTY) k_deepw<true><<<h->cfg.n_envs, 128, h->dp.total, h->stream>>>(p);
-        else k_deepw<false><<<h->cfg.n_envs, 128, h->dp.total, h->stream>>>(p);
-        CUDA_TRY(h, cudaGetLastError());
-        h->recorded_host = -1;
-        return BB_OK;
+        return launch_deepw<false>(h, p);
     }
     int grid = 0, rc;
     const u32 wpb = wpb_for(lay.warp_bytes);
@@ -676,6 +722,7 @@ int bb_create(const bb_config* cfg, bb_handle** out) {
     int rc = upload_seeds(h);
     if (!rc) rc = init_books(h);
     if (!rc && cudaStreamSynchronize(h->stream) != cudaSuccess) rc = fail(nullptr, BB_ECUDA, "init kernel failed");
+    if (!rc && h->eng == ENG_DEEP) rc = alloc_stage(h, cfg->max_queue);
     if (rc) return bail(rc);
     *out = h;
     return BB_OK;
@@ -693,7 +740,7 @@ int bb_destroy(bb_handle* h) {
     cudaFree(h->blobs); cudaFree(h->ord); cudaFree(h->tr); cudaFree(h->hist); cudaFree(h->err_flag);
     cudaFree(h->d_offsets); cudaFree(h->d_seeds); cudaFree(h->d_instrs); cudaFree(h->d_snap); cudaFree(h->d_stats); cudaFree(h->d_tick);
     cudaFree(h->rslot); cudaFree(h->mom); cudaFree(h->scratch); cudaFree(h->d_ids); cudaFree(h->dp_pool);
-    cudaFree(h->d_unit_groups); cudaFree(h->d_unit_keys);
+    cudaFree(h->d_unit_groups); cudaFree(h->d_unit_keys); cudaFree(h->d_stage); cudaFree(h->d_stage_off);
     if (h->h_instrs) cudaFreeHost(h->h_instrs);
     if (h->h_offsets) cudaFreeHost(h->h_offsets);
     if (h->h_snap) cudaFreeHost(h->h_snap);
@@ -978,7 +1025,7 @@ int bb_submit(bb_handle* h, uint64_t n, const uint32_t* env, const uint32_t* act
 
 int bb_step(bb_handle* h, uint32_t n_steps) {
     CHECK_H(h);
-    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine replays instruction streams only (bb_replay / bb_replay_device)");
+    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine has no host-queued Env steps: use bb_step_device, bb_replay or bb_replay_device");
     if (n_steps == 0) return BB_OK;
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     const u32 ne = h->cfg.n_envs;
@@ -1092,7 +1139,7 @@ int bb_replay_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_e
 
 static int set_agents_impl(bb_handle* h, const bb_agent_group* groups, const uint32_t* asset, uint32_t n_groups) {
     CHECK_H(h);
-    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine replays instruction streams only (no in-kernel agents)");
+    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine has no in-kernel agents");
     if (n_groups > MAX_GROUPS) return fail(h, BB_EINVAL, "at most 8 agent groups");
     if (n_groups && !groups) return fail(h, BB_EINVAL, "null groups");
     if (asset) {
@@ -1174,6 +1221,7 @@ int bb_step_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_env
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     if ((rc = id_buffer(h, n_rows, &d_out_ids))) return rc;
     h->mirror_dirty = true;  // ids were handed out on the device
+    if (h->eng == ENG_DEEP) return step_deep(h, d_instrs, d_env_offsets, d_out_ids, d_obs_out);
     return launch_apply(h, MODE_ENV, d_instrs, d_env_offsets, 1, false, d_out_ids, d_obs_out);
 }
 
@@ -1321,12 +1369,17 @@ int bb_reserve(bb_handle* h, uint32_t max_orders, uint32_t max_trades, uint32_t 
 
 int bb_reserve_queue(bb_handle* h, uint32_t max_queue) {
     CHECK_H(h);
-    if (max_queue <= h->cfg.max_queue || h->eng == ENG_DEEP) return BB_OK;  // (the deep-book engine has no Env-step queue)
+    if (max_queue <= h->cfg.max_queue) return BB_OK;
     if (max_queue > 65535 || (h->assets > 1 && (u64)h->assets * max_queue > 65535))
         return fail(h, BB_EINVAL, "max_queue (times assets, for markets) must stay below 65536");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
     CUDA_TRY(h, cudaStreamSynchronize(h->stream));
     if (h->copy_stream) CUDA_TRY(h, cudaStreamSynchronize(h->copy_stream));
+    if (h->eng == ENG_DEEP) {  // the step's permutation is k_env_deep_stage's alone (it always fits); the staging stream grows
+        if (int rc = alloc_stage(h, max_queue)) return rc;
+        h->cfg.max_queue = max_queue;
+        return BB_OK;
+    }
     // the step's permutation (and, for the dense engine's in-kernel agents, the queue itself) lives in shared memory: the
     // layouts are rebuilt for the new capacity, and the request is refused while the Env-step kernel could not run one book
     // per CTA with it (k_sim's fit is checked at its launch, like at creation)
@@ -1436,7 +1489,7 @@ int bb_run_agents_with_rows_market(bb_handle* h, uint64_t seed, const bb_instr* 
 namespace {
 int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows* ext) {
     CHECK_H(h);
-    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine replays instruction streams only");
+    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine has no in-kernel agents");
     if (h->groups.empty()) return fail(h, BB_EINVAL, "bb_set_agents has not been called");
     const bool mkt = !h->group_asset.empty();
     if (h->assets > 1 && !mkt)

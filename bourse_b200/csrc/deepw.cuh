@@ -370,6 +370,8 @@ __device__ __forceinline__ void bk_obs(const BkReg& r, u32 tick, u32 lane, u32 t
 // One event through the whole reference algorithm, warp-uniformly (x, y: the pre-decoded instruction; a, c: the prefetched
 // order record of a cancel / modify).  `ev_done`: events complete once this one is; `rf`: events whose record writes were
 // in HBM when the record was fetched.  Returns false when a bounded wait ran out.
+// ENV (bb_step_device): a NEW carries the id submission gave it, and the order count is already the post-submission one.
+template <bool ENV = false>
 __device__ __forceinline__ bool bk_serial(const BkReg& r, BkSt& s, u32 lane, uint4 x, uint4 y, uint4 a, uint4 c, u32 ev_done, u32 rf, u32& lane_err) {
     s.t = ((u64)x.y << 32) | x.x;
     const u32 op = x.z & BB_OP_MASK;
@@ -382,7 +384,7 @@ __device__ __forceinline__ bool bk_serial(const BkReg& r, BkSt& s, u32 lane, uin
             s.err |= ERR_CAP_ORDERS;
         } else {
             id = x.w;
-            s.n_orders = id + 1u;
+            if (!ENV) s.n_orders = id + 1u;
             kind = RK_NEW;
             side = (x.z >> 8) & 1u;  // BB_F_BID
             price = y.x;
@@ -1005,7 +1007,9 @@ __device__ __forceinline__ bool bk_chain_place(const BkReg& r, BkSt& s, u32 co, 
 // The events of one batch still to do (`pending`: a contiguous run of lanes; lane i holds event i: x, y pre-decoded
 // instruction, a, c prefetched record).  `ev0`: events complete before this batch.  Comes back early (obs_lane < 32) after an
 // event that asks for a market-data record.  Returns false when a bounded wait ran out.
-template <bool COMPACT>
+// ENV (bb_step_device): every id the step's rows created is below s.n_orders from the start, so a cancel / modify is checked
+// against that count alone and a NEW does not add to it.
+template <bool COMPACT, bool ENV = false>
 __device__ __forceinline__ bool bk_batch(const BkReg& r, BkSt& s, u32 lane, u32& pending, uint4 x, uint4 y, uint4 a, uint4 c, u32 ev0, u32 rf,
                                          u32 fast, u32& lane_err, u32& obs_lane) {
     constexpr bool compact = COMPACT;
@@ -1039,7 +1043,7 @@ __device__ __forceinline__ bool bk_batch(const BkReg& r, BkSt& s, u32 lane, u32&
                 pvol = y.y;
             } else if (is_cm) {
                 ef = EF_INSTR;
-                if (id >= s.n_orders + __popc(newm & lt) || id >= r.max_orders) {
+                if (id >= s.n_orders + (ENV ? 0u : __popc(newm & lt)) || id >= r.max_orders) {
                     cx = true;  // unknown id
                 } else {
                     if (lds(r.dirty + 4u * (id & r.dirty_mask)) > rfl) { cx = true; why = CXR_DOUBT; }
@@ -1235,7 +1239,7 @@ __device__ __forceinline__ bool bk_batch(const BkReg& r, BkSt& s, u32 lane, u32&
                 const bool mine = ((clean >> lane) & 1u) && lane < e;
                 s.d_instr += __popc(__ballot_sync(BB_FULL, mine && (ef & EF_INSTR)));
                 s.d_applied += __popc(__ballot_sync(BB_FULL, mine && (ef & (EF_PLACE | EF_REM | EF_RED))));
-                s.n_orders += __popc(__ballot_sync(BB_FULL, mine && (ef & EF_NEW)));
+                if (!ENV) s.n_orders += __popc(__ballot_sync(BB_FULL, mine && (ef & EF_NEW)));
                 if (e > first) s.t = ((u64)__shfl_sync(BB_FULL, t_hi, e - 1u) << 32) | __shfl_sync(BB_FULL, t_lo, e - 1u);
             }
             pending &= ~(clean & (e >= 32u ? BB_FULL : ((1u << e) - 1u)));
@@ -1272,7 +1276,7 @@ __device__ __forceinline__ bool bk_batch(const BkReg& r, BkSt& s, u32 lane, u32&
             kc.x = __shfl_sync(BB_FULL, c.x, k); kc.y = __shfl_sync(BB_FULL, c.y, k); kc.z = __shfl_sync(BB_FULL, c.z, k); kc.w = __shfl_sync(BB_FULL, c.w, k);
             // the replay warp parks; the whole reference algorithm for this event runs here, on the queues as they are
             if (!bk_borrow(r, s, lane)) return false;
-            const bool sok = bk_serial(r, s, lane, kx, ky, ka, kc, ev0 + k + 1u, rf, lane_err);
+            const bool sok = bk_serial<ENV>(r, s, lane, kx, ky, ka, kc, ev0 + k + 1u, rf, lane_err);
             pending &= ~(1u << k);
             if (sok && (kx.z & BB_F_EMIT)) {  // the caller writes the market-data record, gives the queues back and returns for the rest
                 obs_lane = k;

@@ -1276,7 +1276,8 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
 #define DPF_MARKET (1u << 16)      // the order takes the market path: BB_F_MARKET, or a limit price equal to the sentinel (N3)
 #define DPF_CAP_ORDERS (1u << 17)  // a NEW row whose id would not fit the order table
 
-template <u32 RB, bool NAP = false>
+// ENV (bb_step_device): a NEW row carries the id submission gave it (k_env_deep_stage) instead of taking the next one.
+template <u32 RB, bool NAP = false, bool ENV = false>
 __device__ __forceinline__ void dp_fetch_warp(const KParams& p, const DeepOff& o, u32 sb, u32 lane, const bb_instr* ins, u32 n, u64 oh,
                                               u32 next_id) {
     const u32 ctl = sb + o.ctl;
@@ -1315,7 +1316,7 @@ __device__ __forceinline__ void dp_fetch_warp(const KParams& p, const DeepOff& o
         // sentinel price (types.rs:160-172, 213-225), and the write-once half of their record goes straight to HBM
         const u32 new_mask = __ballot_sync(BB_FULL, op == BB_OP_NEW);
         if (op == BB_OP_NEW) {
-            const u32 id = next_id + __popc(new_mask & ((1u << lane) - 1u));
+            const u32 id = ENV ? x.w : next_id + __popc(new_mask & ((1u << lane) - 1u));
             const u32 side = (x.z >> 8) & 1u;
             const u32 price = (x.z & BB_F_MARKET) ? (side ? 0xFFFFFFFFu : 0u) : y.x;
             const bool market = side ? (price == 0xFFFFFFFFu) : (price == 0u);
@@ -1465,7 +1466,9 @@ namespace bb {
 // each), warp 1 = fetch, warp 2 = retire.  Same blob image, chunk pool, order records and trade log as k_deep.
 // ROOMY: at most two books per SM — the staleness filters take their (larger) sizes from the launch; otherwise they are
 // compile-time constants and the kernel is the compact one the four-books-per-SM case needs (its instruction cache is the limiter).
-template <bool ROOMY>
+// ENV: the second launch of bb_step_device — the slices k_env_deep_stage staged (p.offsets holds {begin, end} per book), NEW
+// rows with their ids, trade_vol from 0 (env.rs:117-118), and the closing record also written to p.obs_out.
+template <bool ROOMY, bool ENV = false>
 __global__ void __launch_bounds__(128, ROOMY ? 2 : 4) k_deepw(const __grid_constant__ KParams p) {
     extern __shared__ __align__(128) unsigned char smem[];
     // The four roles rotate with the wave a CTA belongs to (CTAs go round the 148 SMs of a B200, so the up-to-four CTAs that
@@ -1478,8 +1481,8 @@ __global__ void __launch_bounds__(128, ROOMY ? 2 : 4) k_deepw(const __grid_const
     if (env >= p.n_envs) return;
     const u64 oh = (u64)(p.ord + (size_t)env * p.geo.max_orders);
     const u64 tr = (u64)(p.tr + (size_t)env * p.geo.max_trades);
-    const u64 off = p.offsets[env];
-    const u32 n = (u32)(p.offsets[env + 1] - off);
+    const u64 off = p.offsets[ENV ? 2u * env : env];
+    const u32 n = (u32)(p.offsets[ENV ? 2u * env + 1u : env + 1u] - off);
     const bb_instr* ins = p.instrs + off;
     // ---- set-up: barriers, control words, cache tags, filter; then the book image (one bulk copy)
     if (threadIdx.x == 0) {
@@ -1532,7 +1535,7 @@ __global__ void __launch_bounds__(128, ROOMY ? 2 : 4) k_deepw(const __grid_const
     }
     __syncthreads();
     if (warp == 1u) {
-        dp_fetch_warp<DW_RB, true>(p, o, sb, lane, ins, n, oh, lds(sb + HDR_NORDERS));
+        dp_fetch_warp<DW_RB, true, ENV>(p, o, sb, lane, ins, n, oh, lds(sb + HDR_NORDERS));
     } else if (warp == 2u) {
         dp_retire_warp<DW_RCAP, false, true>(p, o, sb, lane, oh, tr, n_tr0);
     } else if (warp == 3u) {
@@ -1544,7 +1547,7 @@ __global__ void __launch_bounds__(128, ROOMY ? 2 : 4) k_deepw(const __grid_const
         s.t = lds64(sb + HDR_T);
         s.max_key_time = lds64(sb + HDR_MAXKT);
         s.n_orders = lds(sb + HDR_NORDERS);
-        s.trade_vol = lds(sb + HDR_TRADEVOL);
+        s.trade_vol = ENV ? 0u : lds(sb + HDR_TRADEVOL);
         s.vol_ask = lds(sb + HDR_SIDEVOL);
         s.vol_bid = lds(sb + HDR_SIDEVOL + 4u);
         s.bq_ask = lds(sb + HDR_BESTQ);
@@ -1583,13 +1586,18 @@ __global__ void __launch_bounds__(128, ROOMY ? 2 : 4) k_deepw(const __grid_const
             u32 pending = cnt >= 32u ? BB_FULL : ((1u << cnt) - 1u);
             while (pending) {
                 u32 obs_lane = 32u;
-                if (!bk_batch<!ROOMY>(r, s, lane, pending, x, y, a, c, 32u * b, rf, fast, lane_err, obs_lane)) { aborted = true; break; }
+                if (!bk_batch<!ROOMY, ENV>(r, s, lane, pending, x, y, a, c, 32u * b, rf, fast, lane_err, obs_lane)) { aborted = true; break; }
                 if (obs_lane < 32u) {  // Level2DataRecords::append_record (data.rs:44-56) for a row flagged BB_F_EMIT
                     const u32 bid = (s.flags & FL_HAS_BID) ? r.win_lo + s.bq_bid : 0u;
                     const u32 ask = (s.flags & FL_HAS_ASK) ? r.win_lo + s.bq_ask : 0xFFFFFFFFu;
                     u32 w0, w1;
                     bk_obs(r, lds(r.ctl + CT_TICK), lane, s.trade_vol, bid, ask, s.vol_ask, s.vol_bid, &w0, &w1);
                     // (a level-1 record is the first 9 words of the level-2 one: words 5..8 are the touch level of each side)
+                    if (ENV && p.obs_out) {  // the step's observation (bb_step_device's d_obs_out)
+                        u32* ob = p.obs_out + (size_t)env * p.obs_words;
+                        if (lane < p.obs_words) ob[lane] = w0;
+                        if (lane + 32u < p.obs_words) ob[lane + 32u] = w1;
+                    }
                     const u32 nrec = lds(sb + HDR_NSTEPS);
                     __syncwarp();
                     if (nrec < p.max_steps) {
@@ -1670,6 +1678,74 @@ __global__ void __launch_bounds__(128, ROOMY ? 2 : 4) k_deepw(const __grid_const
         bulk_s2g_a(p.blobs + (size_t)env * p.blob_stride, sb, o.smem_image);
         bulk_commit();
         bulk_wait_all<0>();
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------
+// bb_step_device on the deep engine, first of its two launches (the second is k_deepw<.., ENV>): Env::step up to the
+// processing of its events (env.rs:116-127), one warp per book.  The rows are submitted as on the other engines
+// (submit_rows: ids in row order, status New published, off-tick prices and rows past max_queue flagged), the queue is
+// shuffled with the book's Xoroshiro stream (Fisher-Yates from the back, as k_apply), and the result is written as a replay
+// slice into the staging stream: row stage[book][i] is event i at start + i (a NEW with its id), then a no-op at
+// start + step_size flagged BB_F_EMIT that appends the step's record.  stage_off[2 book], [2 book + 1]: the slice's bounds.
+// The header takes the new order count, stream state and step counter.  Dynamic shared memory: the permutation, u16
+// [max_queue].
+__global__ void __launch_bounds__(32) k_env_deep_stage(const __grid_constant__ KParams p, bb_instr* stage, u64* stage_off) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    const u32 lane = threadIdx.x, env = blockIdx.x, perm = smem_u32(smem);
+    BookHdr* hdr = reinterpret_cast<BookHdr*>(p.blobs + (size_t)env * p.blob_stride);
+    Book b;
+    b.env = env;
+    b.lane = lane;
+    b.err = 0u;
+    b.oh = (u64)(p.ord + (size_t)env * p.geo.max_orders);
+    const u64 off = p.offsets[env];
+    const u32 m = (u32)(p.offsets[env + 1] - off), mm = min(m, p.max_queue);  // the first max_queue rows run
+    if (m > p.max_queue) b.err |= ERR_CAP_QUEUE;
+    const u32 n0 = hdr->n_orders;
+    const u64 start = hdr->t;
+    RowCount c{n0, 0u, 0u};
+    submit_rows<false, false>(p.geo, p, b, off, m, mm, 0u, c, [&](u32 j, uint4, uint4, bool, bool, u32, u32 pos, u32) { sts16(perm + 2u * pos, j); });
+    __syncwarp();
+    if (lane == 0u) {  // transactions.shuffle(rng) (env.rs:121)
+        u64 s0 = hdr->rng_s0, s1 = hdr->rng_s1;
+        for (u32 i = c.n; i > 1; --i) {
+            const u32 j = xoroshiro_range(s0, s1, i);
+            const u32 x = lds16(perm + 2u * (i - 1)), y = lds16(perm + 2u * j);
+            sts16(perm + 2u * (i - 1), y);
+            sts16(perm + 2u * j, x);
+        }
+        hdr->rng_s0 = s0;
+        hdr->rng_s1 = s1;
+        hdr->n_orders = c.next;
+        hdr->n_created += c.next - n0;
+        hdr->step_counter += 1u;
+        if (b.err) {
+            hdr->err |= b.err;
+            atomicOr(p.err_flag, b.err);
+        }
+    }
+    __syncwarp();
+    const u64 base = (u64)env * (p.max_queue + 1u);
+    uint4* dst = reinterpret_cast<uint4*>(stage + base);
+    for (u32 i = lane; i < c.n; i += 32u) {
+        const u32 j = lds16(perm + 2u * i);
+        const uint4* src = reinterpret_cast<const uint4*>(p.instrs + off + j);
+        uint4 x = src[0];
+        const u64 t = start + i;
+        x.x = (u32)t;
+        x.y = (u32)(t >> 32);
+        x.z &= ~BB_F_EMIT;
+        if ((x.z & BB_OP_MASK) == BB_OP_NEW) x.w = (u32)p.out_ids[off + j];
+        dst[2u * i] = x;
+        dst[2u * i + 1u] = src[1];
+    }
+    if (lane == 0u) {
+        const u64 t = start + p.step_size;  // env.rs:129-134
+        dst[2u * c.n] = make_uint4((u32)t, (u32)(t >> 32), BB_OP_NOOP | BB_F_EMIT, 0u);
+        dst[2u * c.n + 1u] = make_uint4(0u, 0u, 0u, 0u);
+        stage_off[2u * env] = base;
+        stage_off[2u * env + 1u] = base + c.n + 1u;
     }
 }
 
@@ -2009,7 +2085,7 @@ __device__ __forceinline__ void store_copy_part(unsigned char* dst, const unsign
 // book of the unit ERR_SLOT and changes nothing else.  Every CTA reads the prefix lengths from the source header, which no
 // CTA of the launch writes, and evaluates the slot's validity the same way.  Part 0 writes the header: on restore the
 // slot's, with the history count at 0 and, given seeds, the unit's shuffle stream re-seeded (the step counter stays the
-// slot's).
+// slot's; deep books included: their Env steps shuffle with the same stream).
 template <bool RESTORE>
 __device__ __forceinline__ void store_copy_book(const StoreCopy& c, u32 book, u32 part, u32 parts, const u32* sel, const u64* seeds,
                                                 u32* cursor) {
@@ -2063,7 +2139,7 @@ __device__ __forceinline__ void store_copy_book(const StoreCopy& c, u32 book, u3
     BookHdr h = *src_hdr;
     if (RESTORE) {
         h.n_steps = 0u;
-        if (seeds && !c.pool_chunks) seed_stream(h, seeds[unit]);  // (the deep engine has no shuffle)
+        if (seeds) seed_stream(h, seeds[unit]);
         *reinterpret_cast<BookHdr*>(blob) = h;
         if (cursor) cursor[book] = (u32)n_tr;
     } else {

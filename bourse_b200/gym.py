@@ -489,7 +489,15 @@ class VectorEnv(_DeviceLoop):
 
     With background agents, `set_agent_params` gives each env its own group parameters (a market regime per env) and its own
     agent key.  Reproducible but distinct episodes: `reset(mask, seeds)` with the envs' creation seeds replays the same agent
-    draws, and `set_agent_params(keys=new_keys, mask=mask)` before it makes them new ones; the same key replays them."""
+    draws, and `set_agent_params(keys=new_keys, mask=mask)` before it makes them new ones; the same key replays them.
+
+    Deep books: `price_window=(lo, hi)` with `deep_chunks=N` (see `core.BatchedEnv`) runs every env on the deep-book engine,
+    for books with thousands to millions of resting orders.  Preload them with `self.env.replay(...)` (or a saved book), copy
+    them into many envs with `save` / `restore`, then `step` as above: same semantics, two kernel launches per step and still
+    no host synchronisation, so the step can be captured into a CUDA graph.  Every limit price that rests must lie inside the
+    window, and `step_size` must be at least `max_queue` (the engine needs strictly increasing times between resting orders;
+    otherwise the env is flagged `BB_ERR_TIME_ORDER`).  For the same reason a preload stream should end with a no-op one
+    nanosecond after its last event: a step's first event runs at the book's time.  No background agents on deep books."""
 
     def __init__(self, n_envs: int, rows_per_env: int, seed: int, start_time: int, tick_size: typing.Union[int, typing.Sequence[int]], step_size: int,
                  trading: bool = True, *, level_1: bool = False, agents=None, agent_seed: int = 0, **kw):
@@ -499,6 +507,8 @@ class VectorEnv(_DeviceLoop):
         `agent_seed`).  Action rows may then be NEW, CANCEL or no-op (MODIFY is refused).  At one step per launch the
         general engine (no `price_window`) is the faster choice here: 92 us against 117 us per 4096-env step on the dense
         engine, whose per-launch agent-table rebuild only pays off inside the persistent multi-step kernel."""
+        if agents and kw.get("deep_chunks"):
+            raise ValueError("background agents do not run on the deep-book engine (deep_chunks): drop agents= or deep_chunks=")
         n_bg = sum(int(g["n_agents"]) for g in agents) if agents else 0
         kw.setdefault("max_queue", max(rows_per_env + 2 * n_bg, 16))
         if rows_per_env > kw["max_queue"]:

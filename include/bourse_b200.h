@@ -107,8 +107,9 @@ typedef struct {
      * price_granule == 1; deep_chunks = 256-byte queue chunks per book (31 entries each; one per resting order in the
      * worst case, ~ resting orders / 31 + win_levels + entries appended during a launch / 31 in practice).  Preconditions
      * beyond the window: strictly increasing time between resting inserts (BB_ERR_TIME_ORDER) and one side per price
-     * level (BB_ERR_LOCKED: only reachable while trading is disabled).  Env mode and in-kernel agents are
-     * not available on a deep handle (BB_EINVAL). */
+     * level (BB_ERR_LOCKED: only reachable while trading is disabled).  Env steps run through bb_step_device (device
+     * rows; step_size >= max_queue keeps the time precondition, since event i of a step runs at start + i); the host-queued
+     * Env calls (bb_submit / bb_step) and in-kernel agents are not available on a deep handle (BB_EINVAL). */
     uint32_t deep_chunks;
 } bb_config;
 
@@ -197,7 +198,8 @@ int bb_reserve(bb_handle* h, uint32_t max_orders, uint32_t max_trades, uint32_t 
  * Env::transactions is an unbounded Vec (crates/step_sim/src/env.rs:93-96, 121); here a step's queue is shuffled in shared
  * memory, so it is bounded by what fits there next to the book image (BB_ECAP beyond that, nothing changed).  bb_step refuses
  * a step whose queue exceeds max_queue with BB_ECAP BEFORE applying anything (the transactions stay queued), so a host can
- * call this and step again; the Python StepEnv / StepEnvNumpy classes reserve ahead of need.  Synchronous. */
+ * call this and step again; the Python StepEnv / StepEnvNumpy classes reserve ahead of need.  On a deep-book handle it
+ * regrows the staging stream of bb_step_device (n_envs x (max_queue + 1) instructions), which always fits.  Synchronous. */
 int bb_reserve_queue(bb_handle* h, uint32_t max_queue);
 /* Forget the per-step records (Level2DataRecords, data.rs:9-57) of every env: the history restarts at record 0, the books,
  * order tables and trade logs are untouched.  For open-ended loops that consume each step's observation as it is produced
@@ -245,7 +247,12 @@ int bb_step(bb_handle* h, uint32_t n_steps);
  * nothing (BB_NO_ID) and the env is flagged BB_ERR_CAP_QUEUE.  d_obs_out (device, [n_envs][obs_words], may be NULL) receives every env's end-of-step
  * observation record from the same launch — what StepEnvNumpy.level_1_data / level_2_data would return next.
  * Asynchronous on the handle's stream: one kernel launch and no host synchronisation, so the call may be recorded into a
- * CUDA graph together with the caller's own kernels (stream capture on the stream given to bb_set_stream). */
+ * CUDA graph together with the caller's own kernels (stream capture on the stream given to bb_set_stream).
+ * Deep-book handles (bb_config.deep_chunks) take the same rows with the same results, in two launches and with no
+ * allocation: the first submits and shuffles each env's rows into a staging stream sized by max_queue, the second
+ * replays it through the deep engine.  Its preconditions apply: a resting limit price outside the window flags
+ * BB_ERR_CAP_PAGES, and BB_ERR_TIME_ORDER is flagged where resting orders of one step would reuse key times of an earlier
+ * one, which step_size >= max_queue rules out. */
 int bb_step_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_env_offsets, uint64_t n_rows, uint64_t* d_out_ids,
                    uint32_t* d_obs_out);
 /* The same device-resident loop for multi-asset markets (bb_config.assets >= 2; no upper limit on assets here).  One call
@@ -398,7 +405,8 @@ int bb_reset_device(bb_handle* h, const uint8_t* d_mask, const uint64_t* d_seeds
  *   restore (checked per book, so per-env ticks work) is left untouched and each of its books is flagged BB_ERR_SLOT; all
  *   books of a market share the outcome.  Order ids a caller holds for a restored book now name the slot's orders.
  *
- * Both calls work on every engine; on the deep engine a unit is a book and d_seeds has no effect.  On a multi-asset handle
+ * Both calls work on every engine; on the deep engine a unit is a book, and d_seeds re-seeds the stream its
+ * bb_step_device steps shuffle with.  On a multi-asset handle
  * right after a bb_step that shuffled, both first copy the host's streams of the markets to the books (synchronous), which
  * is refused inside a stream capture.  Refused with BB_EINVAL, the handle and the store unchanged, for NULL arguments, a
  * store created by another handle, a store created before a later bb_reserve that grew a capacity or a later
