@@ -57,8 +57,9 @@ class BatchedEnv:
     `deep_chunks=N` (with `price_window`, up to 8192 levels) selects the deep-book engine: one CTA per book (fetch / chain /
     replay / retire warps, csrc/deepw.cuh) and chunked array queues in HBM (N 256-byte chunks of 31 queue entries per book)
     — for books with ~10^6 resting orders, driven by replayed streams (`replay`, `replay_device`) or by device-resident Env
-    steps (`step_device`, `gym.VectorEnv`; rows as on the other engines, `step_size >= max_queue`).  The host-queued Env
-    calls (`submit`, `step`) and in-kernel agents raise.
+    steps (`step_device`, `gym.VectorEnv`; rows as on the other engines, `step_size >= max_queue`), with or without in-kernel
+    agents (`set_agents`: RandomAgents price ranges inside the window; `run_agents`, `run_agents_with_rows`).  The
+    host-queued Env calls (`submit`, `step`) raise.
 
     `assets=A` (> 1) groups consecutive books into multi-asset markets with MarketEnv semantics
     (crates/step_sim/src/market_env.rs:108-121); see `bourse_b200.market`.

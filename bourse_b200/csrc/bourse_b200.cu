@@ -285,6 +285,8 @@ DeepOff deep_layout(u32 W, u32 roomy /* filter size multiplier: 1, 4, 8 */) {
 
 // k_env_deep_stage's dynamic shared memory: the step's permutation, u16 [max_queue]
 size_t stage_smem(u32 max_queue) { return align_up(2u * max_queue, 16); }
+// k_env_agents_stage's: the permutation and the shuffle's swap targets
+size_t agent_stage_smem(u32 max_queue) { return 2u * stage_smem(max_queue); }
 
 // the deep engine's staging stream for bb_step_device, sized for max_queue (synchronous: the old one may be in use)
 int alloc_stage(bb_handle* h, u32 max_queue) {
@@ -335,7 +337,8 @@ int launch_init(bb_handle* h, const ResetArgs& r) {
     const bb_config& c = h->cfg;
     if (h->eng == ENG_DEEP)
         k_init_deep<<<c.n_envs, 128, 0, h->stream>>>(h->blobs, h->blob_stride, c.n_envs, c.start_time, c.trading ? 1u : 0u, h->d_seeds,
-                                                     h->dp.bm, h->dp.lht - h->dp.bm, r);  // bitmaps, summaries, level volumes and order counts start at zero
+                                                     h->dp.bm, h->dp.lht - h->dp.bm,  // bitmaps, summaries, level volumes and order counts start at zero
+                                                     h->rslot, h->agents_per_env, h->mom, h->mom_groups, h->mom_stride, r);
     else
         k_init<<<c.n_envs, 64, 0, h->stream>>>(h->blobs, h->blob_stride, c.n_envs, h->p_total, c.start_time, c.trading ? 1u : 0u,
                                                h->d_seeds, h->rslot, h->agents_per_env, h->mom, h->mom_groups, h->mom_stride, h->dgeo,
@@ -514,6 +517,10 @@ int deep_attrs(bb_handle* h) {
     CUDA_TRY(h, cudaFuncSetAttribute(k_deepw<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 1024));
     CUDA_TRY(h, cudaFuncSetAttribute(k_deepw<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, 232448 - 1024));
     CUDA_TRY(h, cudaFuncSetAttribute(k_env_deep_stage, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)stage_smem(65535u)));
+    // (the largest max_queue, 65535, does not fit the agents' staging: run_agents_deep refuses what would not)
+    const int agent_smem = (int)std::min<size_t>(agent_stage_smem(65535u), 232448u - 1024u);
+    CUDA_TRY(h, cudaFuncSetAttribute(k_env_agents_stage<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, agent_smem));
+    CUDA_TRY(h, cudaFuncSetAttribute(k_env_agents_stage<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, agent_smem));
     h->deep_attr_set = true;
     return BB_OK;
 }
@@ -1139,7 +1146,6 @@ int bb_replay_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_e
 
 static int set_agents_impl(bb_handle* h, const bb_agent_group* groups, const uint32_t* asset, uint32_t n_groups) {
     CHECK_H(h);
-    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine has no in-kernel agents");
     if (n_groups > MAX_GROUPS) return fail(h, BB_EINVAL, "at most 8 agent groups");
     if (n_groups && !groups) return fail(h, BB_EINVAL, "null groups");
     if (asset) {
@@ -1167,8 +1173,20 @@ static int set_agents_impl(bb_handle* h, const bb_agent_group* groups, const uin
         }
         total += g.n_agents;
     }
+    // a deep book's resting prices must lie in its window: a RandomAgents group's whole price range is known up front (Momentum /
+    // Noise quotes follow the book and are flagged BB_ERR_CAP_PAGES at run time, as out-of-window rows are)
+    if (h->eng == ENG_DEEP)
+        for (u32 i = 0; i < n_groups; ++i) {
+            const bb_agent_group& g = groups[i];
+            const u64 lo = (u64)g.tick_lo * g.tick_size, hi = (u64)(g.tick_hi - 1u) * g.tick_size;
+            const u64 wlo = h->cfg.win_lo, whi = wlo + h->cfg.win_levels;
+            if (g.kind == BB_GROUP_RANDOM && (lo < wlo || hi >= whi))
+                return fail(h, BB_EINVAL, "RandomAgents group " + std::to_string(i) + " quotes prices " + std::to_string(lo) + ".." +
+                                              std::to_string(hi) + ", outside the deep-book engine's price window [" + std::to_string(wlo) +
+                                              ", " + std::to_string(whi) + ")");
+        }
     // every check happens before any allocation is touched: a refused population leaves the previous one intact
-    if (h->eng >= ENG_DENSE && total > 2046) return fail(h, BB_EINVAL, "the dense engine supports at most 2046 agents per env");
+    if ((h->eng == ENG_DENSE || h->eng == ENG_DENSE_L) && total > 2046) return fail(h, BB_EINVAL, "the dense engine supports at most 2046 agents per env");
     // agent state is (re)allocated only when the population's shape changes: cudaFree / cudaMalloc synchronise the
     // whole device and cost ~100 ms next to tens of GB of slabs, which used to dominate the end-to-end pass
     const size_t ne = h->cfg.n_envs;
@@ -1378,6 +1396,9 @@ int bb_reserve_queue(bb_handle* h, uint32_t max_queue) {
     if (h->eng == ENG_DEEP) {  // the step's permutation is k_env_deep_stage's alone (it always fits); the staging stream grows
         if (int rc = alloc_stage(h, max_queue)) return rc;
         h->cfg.max_queue = max_queue;
+        cudaFree(h->scratch);  // the agents' queues: reallocated at the next agent launch
+        h->scratch = nullptr;
+        h->scratch_warps = 0;
         return BB_OK;
     }
     // the step's permutation (and, for the dense engine's in-kernel agents, the queue itself) lives in shared memory: the
@@ -1411,7 +1432,7 @@ int bb_set_agents_market(bb_handle* h, const bb_agent_group* groups, const uint3
 
 int bb_set_agent_params_device(bb_handle* h, const bb_agent_group* d_params, const uint64_t* d_keys, const uint8_t* d_mask) {
     CHECK_H(h);
-    if (h->groups.empty())  // (the deep engine has no population)
+    if (h->groups.empty())
         return fail(h, BB_EINVAL, "bb_set_agent_params_device: bb_set_agents / bb_set_agents_market has not been called");
     if (!d_params && !d_keys) return fail(h, BB_EINVAL, "bb_set_agent_params_device: d_params and d_keys are both NULL");
     CUDA_TRY(h, cudaSetDevice(h->cfg.device));
@@ -1487,9 +1508,37 @@ int bb_run_agents_with_rows_market(bb_handle* h, uint64_t seed, const bb_instr* 
 }
 
 namespace {
+// bb_run_agents(_with_rows) on the deep engine: per step, k_env_agents_stage (the agents' updates, on the first step the
+// caller's rows, the shuffle) into the staging stream, then k_deepw<.., ENV> over the staged slices.  `p` is the step's
+// parameter block as k_sim would take it.
+int run_agents_deep(bb_handle* h, KParams& p, u32 n_steps) {
+    const size_t smem = agent_stage_smem(h->cfg.max_queue);
+    if (smem > 232448u - 1024u) return fail(h, BB_ECAP, "agents on the deep-book engine: max_queue above 57856 does not fit in shared memory");
+    if (int rc = deep_attrs(h)) return rc;
+    const u32 ne = h->cfg.n_envs;
+    if (h->scratch_warps < ne) {  // one queue per book
+        cudaFree(h->scratch);
+        h->scratch = nullptr;
+        h->scratch_warps = 0;
+        CUDA_TRY(h, cudaMalloc(&h->scratch, (size_t)ne * h->cfg.max_queue * sizeof(uint4)));
+        h->scratch_warps = ne;
+    }
+    p.scratch = h->scratch;
+    KParams pd = p;
+    pd.instrs = h->d_stage;
+    pd.offsets = h->d_stage_off;
+    const auto k = h->d_unit_groups ? k_env_agents_stage<true> : k_env_agents_stage<false>;
+    for (u32 s = 0; s < n_steps; ++s) {
+        if (s == 1) p.offsets = nullptr;  // the rows belong to the first step
+        k<<<ne, 32, smem, h->stream>>>(p, h->d_stage, h->d_stage_off);
+        CUDA_TRY(h, cudaGetLastError());
+        if (int rc = launch_deepw<true>(h, pd)) return rc;
+    }
+    return BB_OK;
+}
+
 int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows* ext) {
     CHECK_H(h);
-    if (h->eng == ENG_DEEP) return fail(h, BB_EINVAL, "the deep-book engine has no in-kernel agents");
     if (h->groups.empty()) return fail(h, BB_EINVAL, "bb_set_agents has not been called");
     const bool mkt = !h->group_asset.empty();
     if (h->assets > 1 && !mkt)
@@ -1537,6 +1586,14 @@ int run_agents_impl(bb_handle* h, uint64_t seed, uint32_t n_steps, const ExtRows
         p.out_ids = ext->d_out_ids;
         p.obs_out = ext->d_obs_out;
         if ((rc = id_buffer(h, ext->n_rows, &p.out_ids))) return rc;
+    }
+    if (h->eng == ENG_DEEP) {
+        const long long rec = h->recorded_host;  // (launch_deepw forgets the count; every env gains n_steps records here)
+        if ((rc = run_agents_deep(h, p, n_steps))) return rc;
+        h->mirror_dirty = true;
+        h->status_valid = false;
+        h->recorded_host = rec + n_steps;
+        return BB_OK;
     }
     int grid = 0;
     // external rows carry no slot hints: they run on the variants that also serve MomentumAgent / NoiseAgent events.  So

@@ -735,6 +735,56 @@ __device__ __noinline__ MomOut momentum_agent_update(const KParams& p, const bb_
     return out;
 }
 
+// The step's shuffle (k_sim, k_env_agents_stage): Fisher-Yates from the back over the nq queued events, one Philox word per
+// position (counter (env_g, step, PHILOX_SLOT_SHUFFLE, block of 4)), the draws made lane-parallel into jarr (u16 [nq]).
+// The swaps are one serial chain: lane 0 applies them alone (32 lanes storing the same 16 bytes are 4 L1 wavefronts
+// instead of 1, and the tools rightly flag unsynchronised same-address traffic between lanes).  The chain permutes perm
+// (u16 [nq], built here from the identity) or, with QSWAP (the dense engine's on-chip queue at qs), the 16-byte events.
+template <bool PU, bool QSWAP>
+__device__ __forceinline__ void shuffle_queue(const KParams& p, u32 perm, u32 jarr, u32 qs, u32 nq, u32 env_g, u32 step, u32 key_l,
+                                              u32 key_h, u32 lane) {
+    if constexpr (!QSWAP)
+        for (u32 i = lane; i < nq; i += 32) sts16(perm + 2u * i, i);
+    for (u32 b0 = 0; b0 * 4u < nq; b0 += 32) {
+        const u32 blk = b0 + lane;
+        if (blk * 4u < nq) {
+            const uint4 r = philox4x32_10(env_g, step, PHILOX_SLOT_SHUFFLE, blk, key_lo<PU>(p, key_l), key_hi<PU>(p, key_h));
+            const u32 i = blk * 4u;
+            // 4 consecutive u16 slots are always in bounds: the array is padded to a multiple of 8 bytes
+            const u32 j0 = mulhi_range(r.x, i + 1), j1 = mulhi_range(r.y, i + 2);
+            const u32 j2 = mulhi_range(r.z, i + 3), j3 = mulhi_range(r.w, i + 4);
+            sts(jarr + 2u * i, j0 | (j1 << 16));
+            sts(jarr + 2u * i + 4u, j2 | (j3 << 16));
+        }
+    }
+    __syncwarp();
+    if (lane != 0u) {
+    } else if constexpr (QSWAP) {  // the queue is on chip: swap the 16-byte instructions themselves
+        for (u32 i = nq; i > 1; --i) {
+            const u32 j = lds16(jarr + 2u * (i - 1));
+            const uint4 x = lds128(qs + 16u * (i - 1)), y = lds128(qs + 16u * j);
+            sts128(qs + 16u * (i - 1), y);
+            sts128(qs + 16u * j, x);
+        }
+    } else {
+        for (u32 i = nq; i > 1; --i) {
+            const u32 j = lds16(jarr + 2u * (i - 1));
+            const u32 x = lds16(perm + 2u * (i - 1)), y = lds16(perm + 2u * j);
+            sts16(perm + 2u * (i - 1), y);
+            sts16(perm + 2u * j, x);
+        }
+    }
+    __syncwarp();
+}
+
+// A caller's queued row as an event of the agents' queue (k_sim<.., EXT>, k_env_agents_stage): bit 0 NEW, bit 1 bid, no
+// hint, trader id above bit 13; a market order carries the sentinel price (types.rs:160-172, 213-225)
+__device__ __forceinline__ uint4 row_event(uint4 x, uint4 y, bool is_new, u32 id) {
+    const bool bid = (x.z & BB_F_BID) != 0u;
+    const u32 price = (x.z & BB_F_MARKET) ? (bid ? 0xFFFFFFFFu : 0u) : y.x;
+    return make_uint4(is_new ? (1u | (bid ? 2u : 0u) | (y.z << 13)) : 0u, is_new ? id : x.w, price, y.y);
+}
+
 // named barrier over the warps of one market (bar.sync with an explicit thread count)
 // Barrier ids are immediates (a CTA holds at most two markets): with a register id ptxas reserves all 16 hardware
 // barriers for the CTA, which caps residency at 4 CTAs per SM.
@@ -774,8 +824,10 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
     const u32 sb = keep32(smem_u32(smem) + warp * p.warp_smem_bytes);
     const u32 bar = sb + p.off_bar;
     const u32 perm = sb + p.off_perm;          // u16 [max_queue]
-    // u16 [max_queue] (the dense engine has no perm array); markets: perm and jarr hold the whole market's queue
-    const u32 jarr = perm + (MKT ? 2u * ((p.assets * p.max_queue + 7u) & ~7u) : G::DENSE ? 0u : 2u * p.max_queue);
+    // u16 [max_queue] (the dense engine has no perm array); markets: perm and jarr hold the whole market's queue.  jarr
+    // starts 8-byte aligned (the shuffle stores its draws as u32 pairs; an odd max_queue would misalign them), inside the
+    // 16 bytes of slack make_layout reserves behind the two arrays
+    const u32 jarr = perm + (MKT ? 2u * ((p.assets * p.max_queue + 7u) & ~7u) : G::DENSE ? 0u : 2u * ((p.max_queue + 3u) & ~3u));
     const u32 stage = sb + p.off_obs;          // u32 [2][OBS_STAGE_STEPS * obs_words]
     const u32 mk_a = MKT ? warp % p.assets : 0u;                           // the asset this warp's book is
     const u32 mk_sb = MKT ? sb - mk_a * p.warp_smem_bytes + p.off_mkt : 0u;  // u32 [2][MAX_GROUPS] in the market's first warp
@@ -899,14 +951,12 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                     for (u32 w = lane; w < nw; w += 32) sts(mk_rm + 4u * w, 0u);
                     __syncwarp();
                 }
-                // this book's rows join its queue as in-kernel events: bit 0 NEW, bit 1 bid, no hint, trader id above bit 13;
-                // markets also mark each one's index among the market's queued rows in the mask
+                // this book's rows join its queue as in-kernel events (row_event); markets also mark each one's index among
+                // the market's queued rows in the mask
                 auto to_queue = [&](u32, uint4 x, uint4 y, bool mine, bool is_new, u32 id, u32 pos, u32 pos_mkt) {
                     if (!mine) return;
-                    const bool bid = (x.z & BB_F_BID) != 0u;
                     if (pos < p.max_queue) {
-                        const u32 price = (x.z & BB_F_MARKET) ? (bid ? 0xFFFFFFFFu : 0u) : y.x;  // types.rs:160-172, 213-225
-                        const uint4 ev = make_uint4(is_new ? (1u | (bid ? 2u : 0u) | (y.z << 13)) : 0u, is_new ? id : x.w, price, y.y);
+                        const uint4 ev = row_event(x, y, is_new, id);
                         if constexpr (G::DENSE) sts128(qs + 16u * pos, ev);
                         else q[pos] = ev;
                     }
@@ -987,41 +1037,7 @@ __global__ void __launch_bounds__(128, ENG == ENG_PAGED ? 5 : 7) k_sim(const __g
                     if (nq > p.step_size) b.err |= ERR_TIME_ORDER;
                 }
             }
-            // shuffle: Fisher-Yates from the back, one Philox word per position, draws made lane-parallel
-            if constexpr (MKT || !G::DENSE)
-                for (u32 i = lane; i < nq; i += 32) sts16(perm + 2u * i, i);
-            for (u32 b0 = 0; b0 * 4u < nq; b0 += 32) {
-                const u32 blk = b0 + lane;
-                if (blk * 4u < nq) {
-                    const uint4 r = philox4x32_10(env_g, step, PHILOX_SLOT_SHUFFLE, blk, key_lo<PU>(p, key_l), key_hi<PU>(p, key_h));
-                    const u32 i = blk * 4u;
-                    // 4 consecutive u16 slots are always in bounds: the array is padded to a multiple of 8 bytes
-                    const u32 j0 = mulhi_range(r.x, i + 1), j1 = mulhi_range(r.y, i + 2);
-                    const u32 j2 = mulhi_range(r.z, i + 3), j3 = mulhi_range(r.w, i + 4);
-                    sts(jarr + 2u * i, j0 | (j1 << 16));
-                    sts(jarr + 2u * i + 4u, j2 | (j3 << 16));
-                }
-            }
-            __syncwarp();
-            // the swaps are one serial chain: lane 0 applies them alone (32 lanes storing the same 16 bytes are 4 L1
-            // wavefronts instead of 1, and the tools rightly flag unsynchronised same-address traffic between lanes)
-            if (lane != 0u) {
-            } else if constexpr (G::DENSE && !MKT) {  // the queue is on chip: swap the 16-byte instructions themselves
-                for (u32 i = n; i > 1; --i) {
-                    const u32 j = lds16(jarr + 2u * (i - 1));
-                    const uint4 x = lds128(qs + 16u * (i - 1)), y = lds128(qs + 16u * j);
-                    sts128(qs + 16u * (i - 1), y);
-                    sts128(qs + 16u * j, x);
-                }
-            } else {
-                for (u32 i = nq; i > 1; --i) {
-                    const u32 j = lds16(jarr + 2u * (i - 1));
-                    const u32 x = lds16(perm + 2u * (i - 1)), y = lds16(perm + 2u * j);
-                    sts16(perm + 2u * (i - 1), y);
-                    sts16(perm + 2u * j, x);
-                }
-            }
-            __syncwarp();
+            shuffle_queue<PU, G::DENSE && !MKT>(p, perm, jarr, qs, nq, env_g, step, key_l, key_h, lane);
             if constexpr (MKT) {
                 // pull this book's events out of the market-wide permutation, in queue order: (index in the book's own
                 // list, position in the shuffled queue = time offset), one u32 each, over the consumed draw array
@@ -1750,6 +1766,101 @@ __global__ void __launch_bounds__(32) k_env_deep_stage(const __grid_constant__ K
 }
 
 // ---------------------------------------------------------------------------------------------------
+// bb_run_agents(_with_rows) on the deep engine, first of the two launches of each step (the second is k_deepw<.., ENV>): one
+// k_sim<.., MOM, EXT> step up to the processing of its events, one warp per book.  The groups update in declaration order
+// exactly as in k_sim (held ids in p.rslot, Momentum / Noise state in p.mom, the touch from the header's has_best / best_q)
+// into the book's queue in global scratch, p.scratch [n_envs][max_queue]; a launch given rows (p.offsets) submits them next
+// (submit_rows: NEW and CANCEL only).  Past max_queue events the queue is truncated and flagged ERR_CAP_QUEUE; it is checked
+// against the book's tick when rand_tick_mask is set, shuffled with k_sim's Philox draws (shuffle_queue), and written as a
+// replay slice in k_env_deep_stage's layout: event i at start + i (a NEW with its id, trader and price; a market order keeps
+// its sentinel price, which k_deepw routes to the market path), then the BB_F_EMIT no-op at start + step_size.  Every staged
+// NEW's record is published with status New, as create_order does at submission.  The header takes the new order count
+// and step counter; the Xoroshiro stream is not used.  Dynamic shared memory: the permutation, then the swap targets, u16
+// [max_queue] each, 16-byte aligned.
+template <bool PU>
+__global__ void __launch_bounds__(32) k_env_agents_stage(const __grid_constant__ KParams p, bb_instr* stage, u64* stage_off) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    const u32 lane = threadIdx.x, env = blockIdx.x, perm = smem_u32(smem), jarr = perm + ((2u * p.max_queue + 15u) & ~15u);
+    BookHdr* hdr = reinterpret_cast<BookHdr*>(p.blobs + (size_t)env * p.blob_stride);
+    Book b;
+    b.env = env;
+    b.lane = lane;
+    b.err = 0u;
+    b.oh = (u64)(p.ord + (size_t)env * p.geo.max_orders);
+    uint4* q = p.scratch + (size_t)env * p.max_queue;
+    const u32 env_g = p.env_id_base + env, step = hdr->step_counter, n0 = hdr->n_orders, tick = __ldg(p.geo.ticks + env);
+    const u64 start = hdr->t;
+    const u32 bid = hdr->has_best[1] ? p.geo.d_win_lo + hdr->best_q[1] : 0u;
+    const u32 ask = hdr->has_best[0] ? p.geo.d_win_lo + hdr->best_q[0] : 0xFFFFFFFFu;
+    u32 key_l = 0, key_h = 0;
+    const bb_agent_group* urow = nullptr;
+    if constexpr (PU) {
+        unit_key(p, env, key_l, key_h);
+        urow = p.unit_groups + (size_t)env * p.n_groups;
+    }
+    u32* slots = p.rslot + (size_t)env * p.agents_per_env;
+    // ---- agents.update(env, rng) in declaration order (crates/macros/src/lib.rs:57-72)
+    Emit e;
+    e.n = 0;
+    e.next_id = n0;
+    u32 slot_base = 0, mi = 0;
+    for (u32 gi = 0; gi < p.n_groups; ++gi) {
+        const bb_agent_group& ag = PU ? urow[gi] : p.groups[gi];
+        if (ag.kind == BB_GROUP_RANDOM) {
+            random_agents_update<PU>(p, ag, b, q, e, slots, env_g, step, slot_base, key_l, key_h);
+        } else {
+            const MomOut mo = momentum_agent_update<PU>(p, ag, b.oh, tick, bid, ask, q, e.n, e.next_id,
+                                                        (MomState*)((char*)p.mom + ((size_t)env * p.mom_groups_per_env + mi) * p.mom_stride),
+                                                        env_g, step, gi, slot_base);
+            e.n = mo.n;
+            e.next_id = mo.next_id;
+            b.err |= mo.err;
+            ++mi;
+        }
+        slot_base += ag.n_agents;
+    }
+    if (p.offsets) {  // the caller's rows, after the agents' instructions
+        const u64 off = p.offsets[env];
+        const u32 m = (u32)(p.offsets[env + 1] - off);
+        RowCount rows{e.next_id, e.n, 0u};
+        submit_rows<false, true>(p.geo, p, b, off, m, m, 0u, rows, [&](u32, uint4 x, uint4 y, bool, bool is_new, u32 id, u32 pos, u32) {
+            if (pos < p.max_queue) q[pos] = row_event(x, y, is_new, id);
+        });
+        e.next_id = rows.next;
+        e.n = rows.n;
+    }
+    if (e.n > p.max_queue) b.err |= ERR_CAP_QUEUE;
+    const u32 n = min(e.n, p.max_queue);
+    if (p.rand_tick_mask) agent_tick_check<false>(q, 0u, tick, n, lane, b.err);
+    __syncwarp();
+    shuffle_queue<PU, false>(p, perm, jarr, 0u, n, env_g, step, key_l, key_h, lane);
+    const u64 base = (u64)env * (p.max_queue + 1u);
+    uint4* dst = reinterpret_cast<uint4*>(stage + base);
+    for (u32 i = lane; i < n; i += 32u) {
+        const uint4 ev = q[lds16(perm + 2u * i)];
+        const bool is_new = (ev.x & 1u) != 0u, side_bid = (ev.x & 2u) != 0u;
+        if (is_new && ev.y < p.geo.max_orders) stg32(b.oh + (u64)ev.y * ORD_STRIDE + OH_META, ST_NEW | (side_bid ? META_BID : 0u));
+        const u64 t = start + i;
+        dst[2u * i] = make_uint4((u32)t, (u32)(t >> 32), is_new ? (BB_OP_NEW | (side_bid ? BB_F_BID : 0u)) : BB_OP_CANCEL, ev.y);
+        dst[2u * i + 1u] = make_uint4(ev.z, ev.w, is_new ? ev.x >> 13 : 0u, 0u);
+    }
+    if (lane == 0u) {
+        const u64 t = start + p.step_size;  // env.rs:129-134
+        dst[2u * n] = make_uint4((u32)t, (u32)(t >> 32), BB_OP_NOOP | BB_F_EMIT, 0u);
+        dst[2u * n + 1u] = make_uint4(0u, 0u, 0u, 0u);
+        stage_off[2u * env] = base;
+        stage_off[2u * env + 1u] = base + n + 1u;
+        hdr->n_orders = e.next_id;  // create_order at submission (env.rs:173)
+        hdr->n_created += e.next_id - n0;
+        hdr->step_counter = step + 1u;
+        if (b.err) {
+            hdr->err |= b.err;
+            atomicOr(p.err_flag, b.err);
+        }
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------
 // Live market data of every book: out45[env][45] (level_2_data layout) and out8[env][8] =
 // OrderBook::level_1_data field order (orderbook.rs:287-301, touch by the `volumes` map).
 // `only` [n_books] or nullptr: write the rows of the books whose entry is non-zero (bb_restore_device's restored books)
@@ -1850,6 +1961,17 @@ __device__ __forceinline__ void reset_outputs(u32 env, const ResetArgs& r) {
     if (r.cursor && threadIdx.x == 0) r.cursor[env] = 0u;
 }
 
+// the agents' state of a fresh book (k_init, k_init_deep): no held orders, no momentum history, empty live-order lists
+__device__ __forceinline__ void reset_agents(u32 env, u32* rslot, u32 agents_per_env, MomState* mom, u32 mom_per_env, u32 mom_stride) {
+    if (rslot)
+        for (u32 i = threadIdx.x; i < agents_per_env; i += blockDim.x) rslot[(size_t)env * agents_per_env + i] = BB_NIL;
+    if (mom)
+        for (u32 i = threadIdx.x; i < mom_per_env; i += blockDim.x) {
+            MomState* m = (MomState*)((char*)mom + ((size_t)env * mom_per_env + i) * mom_stride);
+            m->momentum = 0.0; m->last_price = 0.0; m->has_last = 0; m->n_live = 0;
+        }
+}
+
 // fresh-book initialisation (OrderBook::new orderbook.rs:158-171 + Env::new env.rs:84-95), of every book or of the units
 // r.mask selects
 __global__ void k_init(unsigned char* blobs, u64 blob_stride, u32 n_envs, u32 p_total, u64 start_time, u32 trading,
@@ -1882,18 +2004,13 @@ __global__ void k_init(unsigned char* blobs, u64 blob_stride, u32 n_envs, u32 p_
             tag[2 * p_total + i] = 0;
         }
     }
-    if (rslot)
-        for (u32 i = threadIdx.x; i < agents_per_env; i += blockDim.x) rslot[(size_t)env * agents_per_env + i] = BB_NIL;
-    if (mom)
-        for (u32 i = threadIdx.x; i < mom_per_env; i += blockDim.x) {
-            MomState* m = (MomState*)((char*)mom + ((size_t)env * mom_per_env + i) * mom_stride);
-            m->momentum = 0.0; m->last_price = 0.0; m->has_last = 0; m->n_live = 0;
-        }
+    reset_agents(env, rslot, agents_per_env, mom, mom_per_env, mom_stride);
 }
 
-// fresh deep book (deep.cuh image): header, empty bitmaps, chunk 0 reserved as a sink
+// fresh deep book (deep.cuh image): header, empty bitmaps, chunk 0 reserved as a sink; its agents' state as k_init's
 __global__ void k_init_deep(unsigned char* blobs, u64 blob_stride, u32 n_envs, u64 start_time, u32 trading, const u64* rng_seeds,
-                            u32 off_bm, u32 bm_bytes, ResetArgs r) {
+                            u32 off_bm, u32 bm_bytes, u32* rslot, u32 agents_per_env, MomState* mom, u32 mom_per_env, u32 mom_stride,
+                            ResetArgs r) {
     const u32 env = blockIdx.x;
     if (env >= n_envs) return;
     if (r.mask && !r.mask[env / r.assets]) return;
@@ -1906,6 +2023,7 @@ __global__ void k_init_deep(unsigned char* blobs, u64 blob_stride, u32 n_envs, u
     }
     u32* bm = reinterpret_cast<u32*>(b + off_bm);
     for (u32 i = threadIdx.x; i < bm_bytes / 4u; i += blockDim.x) bm[i] = 0u;
+    reset_agents(env, rslot, agents_per_env, mom, mom_per_env, mom_stride);
 }
 
 // live market data of deep books, read straight from the blobs in HBM (same outputs as k_snapshot)

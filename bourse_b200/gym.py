@@ -497,7 +497,9 @@ class VectorEnv(_DeviceLoop):
     no host synchronisation, so the step can be captured into a CUDA graph.  Every limit price that rests must lie inside the
     window, and `step_size` must be at least `max_queue` (the engine needs strictly increasing times between resting orders;
     otherwise the env is flagged `BB_ERR_TIME_ORDER`).  For the same reason a preload stream should end with a no-op one
-    nanosecond after its last event: a step's first event runs at the book's time.  No background agents on deep books."""
+    nanosecond after its last event: a step's first event runs at the book's time.  Background agents (`agents=`) run on
+    deep books too, two launches per step as well: every RandomAgents price range must lie inside the window (the
+    library refuses the population otherwise), and Momentum / Noise quotes that leave it flag `BB_ERR_CAP_PAGES`."""
 
     def __init__(self, n_envs: int, rows_per_env: int, seed: int, start_time: int, tick_size: typing.Union[int, typing.Sequence[int]], step_size: int,
                  trading: bool = True, *, level_1: bool = False, agents=None, agent_seed: int = 0, **kw):
@@ -507,8 +509,6 @@ class VectorEnv(_DeviceLoop):
         `agent_seed`).  Action rows may then be NEW, CANCEL or no-op (MODIFY is refused).  At one step per launch the
         general engine (no `price_window`) is the faster choice here: 92 us against 117 us per 4096-env step on the dense
         engine, whose per-launch agent-table rebuild only pays off inside the persistent multi-step kernel."""
-        if agents and kw.get("deep_chunks"):
-            raise ValueError("background agents do not run on the deep-book engine (deep_chunks): drop agents= or deep_chunks=")
         n_bg = sum(int(g["n_agents"]) for g in agents) if agents else 0
         kw.setdefault("max_queue", max(rows_per_env + 2 * n_bg, 16))
         if rows_per_env > kw["max_queue"]:
@@ -519,9 +519,13 @@ class VectorEnv(_DeviceLoop):
         self.n_envs, self.rows = n_envs, rows_per_env
         self.env = BatchedEnv(n_envs, seed, start_time, tick_size, step_size, trading, obs_words=abi.OBS_L1 if level_1 else abi.OBS_L2, **kw)
         self.obs_words = abi.OBS_L1 if level_1 else abi.OBS_L2
-        self._buffers((n_envs, self.obs_words), (n_envs, rows_per_env))
-        if agents:
-            self.env.set_agents(agents)
+        try:
+            self._buffers((n_envs, self.obs_words), (n_envs, rows_per_env))
+            if agents:
+                self.env.set_agents(agents)
+        except Exception:
+            self.env.close()
+            raise
 
     def step(self, actions) -> typing.Tuple[DeviceArray, DeviceArray]:
         ptr = self._action_ptr(actions)

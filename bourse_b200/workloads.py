@@ -74,6 +74,13 @@ def c3_groups():
     return [random_group(50, (40, 60), (10, 20), 2, 0.8), random_group(50, (10, 90), (50, 70), 2, 0.2)]
 
 
+def c3_groups_around(mid: int):
+    """C3's two RandomAgents groups (same widths, volumes, rates and tick size 2) re-centred on the price `mid`: for a deep
+    book's window, e.g. ticks (4990, 5010) and (4960, 5040) around the C5 mid of 10,000."""
+    c = mid // 2
+    return [random_group(50, (c - 10, c + 10), (10, 20), 2, 0.8), random_group(50, (c - 40, c + 40), (50, 70), 2, 0.2)]
+
+
 def c4_groups():
     """SURVEY.md 8d config C4: 40 + 40 RandomAgents and a 20-trader MomentumAgent."""
     return [random_group(40, (40, 60), (10, 20), 2, 0.8), random_group(40, (10, 90), (50, 70), 2, 0.2),

@@ -108,8 +108,9 @@ typedef struct {
      * worst case, ~ resting orders / 31 + win_levels + entries appended during a launch / 31 in practice).  Preconditions
      * beyond the window: strictly increasing time between resting inserts (BB_ERR_TIME_ORDER) and one side per price
      * level (BB_ERR_LOCKED: only reachable while trading is disabled).  Env steps run through bb_step_device (device
-     * rows; step_size >= max_queue keeps the time precondition, since event i of a step runs at start + i); the host-queued
-     * Env calls (bb_submit / bb_step) and in-kernel agents are not available on a deep handle (BB_EINVAL). */
+     * rows; step_size >= max_queue keeps the time precondition, since event i of a step runs at start + i), and so do
+     * in-kernel agents (bb_set_agents, bb_run_agents(_with_rows): every RandomAgents price must lie in the window); the
+     * host-queued Env calls (bb_submit / bb_step) are not available on a deep handle (BB_EINVAL). */
     uint32_t deep_chunks;
 } bb_config;
 
@@ -437,7 +438,10 @@ int bb_replay(bb_handle* h, const bb_instr* instrs, const uint64_t* env_offsets)
 int bb_replay_device(bb_handle* h, const bb_instr* d_instrs, const uint64_t* d_env_offsets);
 
 /* ---- built-in agents: sim_runner (crates/step_sim/src/runner.rs:46-69) ------------------------ */
-/* Defines the agent set (resets agent state).  Groups run in array order. */
+/* Defines the agent set (resets agent state).  Groups run in array order.  On a deep-book handle (bb_config.deep_chunks) the
+ * prices of every RandomAgents group, [tick_lo * tick_size, (tick_hi - 1) * tick_size], must lie in the window
+ * [win_lo, win_lo + win_levels): otherwise BB_EINVAL and the previous population stays.  MomentumAgent / NoiseAgent quotes
+ * follow the book and cannot be bounded up front; one that would rest outside the window flags BB_ERR_CAP_PAGES. */
 int bb_set_agents(bb_handle* h, const bb_agent_group* groups, uint32_t n_groups);
 /* Multi-asset handles (bb_config.assets = 2..4): the *Market twins of the built-in agents — RandomMarketAgents
  * (crates/step_sim/src/agents/random_agent.rs:165-247), MomentumMarketAgent (momentum_agent.rs:282-409),
@@ -467,12 +471,16 @@ int bb_set_agents_market(bb_handle* h, const bb_agent_group* groups, const uint3
  * bb_reset_device and bb_restore_device keep them (they are configuration, not state: store slots do not hold them);
  * bb_destroy frees them.  With the tables, agent launches run variants that read each unit's row from memory.
  *   One launch on the handle's stream, no host synchronisation (the first call also allocates).  BB_EINVAL, handle
- * unchanged: no population (which covers the deep engine), or d_params and d_keys both NULL. */
+ * unchanged: no population, or d_params and d_keys both NULL. */
 int bb_set_agent_params_device(bb_handle* h, const bb_agent_group* d_params /* [units][n_groups] or NULL */,
                                const uint64_t* d_keys /* [units] or NULL */, const uint8_t* d_mask /* [units] or NULL = all */);
 /* n_steps of { agents.update(env); env.step() } for every env inside one persistent kernel.
  * Draws are Philox4x32-10 keyed (seed; global env id, step, agent) — DESIGN.md "RNG contract".
- * Asynchronous on the handle's stream; pair with bb_synchronize or any read call. */
+ * Asynchronous on the handle's stream; pair with bb_synchronize or any read call.
+ * Deep-book handles run the same steps with the same results in two launches per step: the first runs the agents'
+ * updates, submits the rows (bb_run_agents_with_rows) and shuffles each book's queue into the staging stream, the second
+ * replays it through the deep engine.  Their preconditions apply as for bb_step_device (step_size >= max_queue; a resting
+ * price outside the window flags BB_ERR_CAP_PAGES), and max_queue is limited to 57856 there (BB_ECAP). */
 int bb_run_agents(bb_handle* h, uint64_t seed, uint32_t n_steps);
 /* ONE env-step of { agents.update(env); <the caller's rows>; env.step() } with the rows already in DEVICE memory: the loop of a
  * learning agent trading against the built-in background agents (SURVEY.md 8f rank 4).  Rows are laid out as for

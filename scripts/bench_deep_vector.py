@@ -17,9 +17,17 @@ Bytes moved between HBM and shared memory per book and launch come from deep_lay
 the book image up to the level counts in at its start and out at its end (`smem_image` bytes each way); k_env_deep_stage
 keeps only the step's permutation (2 bytes per queued row) in shared memory and copies nothing in or out.
 
+--bg-agents times the same books with background agents instead: workloads.c3_groups_around(MID) (C3's two RandomAgents
+groups re-centred on the C5 mid) through VectorEnv(agents=...), whose steps (bb_run_agents_with_rows: k_env_agents_stage +
+k_deepw<.., ENV>) refuse CUDA-graph capture, so every loop here is issued eagerly: per (books, rows) the deep step with the
+agents, the deep step with the rows only, and the FAST engine running the same population and rows on shallow books that
+start empty (their cancels name the agents' first ids).  The action block has no MODIFY rows (agent steps drop them);
+--rows defaults to 1,8 there.
+
 Prints the card and its power limit, then one JSON line; --out writes the JSON there too.
 
     python scripts/bench_deep_vector.py --steps 200 --warmup 20 --graph-steps 50 --out deep_vector.json
+    python scripts/bench_deep_vector.py --bg-agents --steps 200 --warmup 20 --out deep_agents.json
 """
 from __future__ import annotations
 
@@ -62,7 +70,7 @@ def smem_image_bytes(window) -> int:
     return lvol + 4 * W                # = lcnt
 
 
-def action_block(rng, n_books, rows):
+def action_block(rng, n_books, rows, modify=True):
     a = np.zeros((n_books, rows), dtype=gym.ACTION_DTYPE)
     u = rng.random((n_books, rows))
     new = u < 0.7
@@ -74,7 +82,69 @@ def action_block(rng, n_books, rows):
     a["vol"] = rng.integers(1, 51, (n_books, rows))
     a["trader"] = rng.integers(0, 1000, (n_books, rows))
     a["order_id"] = np.where(new, 0, rng.integers(0, N_REST, (n_books, rows)))
+    if not modify:
+        a["op_flags"] = np.where(u < 0.85, a["op_flags"], abi.OP_NOOP)
     return a
+
+
+def timed_eager(v, acts, st, steps, warmup):
+    """us per step of `steps` VectorEnv steps issued from Python after `warmup` steps (CUDA events on the env's stream)."""
+    import torch
+    with torch.cuda.stream(st):
+        for _ in range(warmup):
+            v.step(acts)
+    st.synchronize()
+    e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+    e0.record(st)
+    with torch.cuda.stream(st):
+        for _ in range(steps):
+            v.step(acts)
+    e1.record(st)
+    e1.synchronize()
+    return round(e0.elapsed_time(e1) * 1e3 / steps, 2)
+
+
+def bg_agents_cases(args, res, streams, books_list, rows_list):
+    import torch
+    groups = workloads.c3_groups_around(MID)
+    n_pre = len(streams[0])
+    n_steps_max = args.warmup + args.steps + 8
+    per_step = sum(int(g["n_agents"]) for g in groups) + max(rows_list)   # a bound on the ids a step can take
+    res["engine"] = "deep with background agents (k_env_agents_stage + k_deepw<.., ENV>), against deep rows-only and FAST with agents"
+    res["agents"] = "workloads.c3_groups_around(10000): 50 + 50 RandomAgents, tick size 2, ticks (4990, 5010) and (4960, 5040)"
+    rng = np.random.default_rng(0)
+    for n_books in books_list:
+        for rows in rows_list:
+            blk = action_block(rng, n_books, rows, modify=False)
+            acts = torch.from_numpy(blk.view(np.uint8).reshape(n_books, rows, 32)).cuda()
+            # the shallow books start empty: their cancels name the agents' first ids instead of preloaded ones
+            shallow = blk.copy()
+            shallow["order_id"] %= 16
+            acts_shallow = torch.from_numpy(shallow.view(np.uint8).reshape(n_books, rows, 32)).cuda()
+            case = {"books": n_books, "rows_per_env": rows}
+            for key, kw in (("deep_agents_us_per_step", dict(agents=groups, price_window=C5_WINDOW, deep_chunks=C5_CHUNKS)),
+                            ("deep_rows_only_us_per_step", dict(price_window=C5_WINDOW, deep_chunks=C5_CHUNKS)),
+                            ("fast_agents_us_per_step", dict(agents=groups))):
+                deep = "deep_chunks" in kw
+                v = gym.VectorEnv(n_books, rows, 0, 0, 1, STEP, agent_seed=7, max_orders=(n_pre if deep else 0) + per_step * n_steps_max + 64,
+                                  max_trades=1 << 18, max_steps=n_steps_max, **kw)
+                st = torch.cuda.Stream()
+                v.env.set_stream(st.cuda_stream)
+                v.reset()
+                if deep:   # C5 books: the distinct preloads saved and restored into every book
+                    v.env.replay(np.concatenate(streams), np.array([n_pre * min(i, N_DISTINCT) for i in range(n_books + 1)], np.uint64))
+                    store = v.snapshots(N_DISTINCT)
+                    v.save(store, np.arange(N_DISTINCT, dtype=np.uint32))
+                    v.restore(store, torch.from_numpy((np.arange(n_books) % N_DISTINCT).astype(np.int32)).cuda())
+                v.env.synchronize()
+                torch.cuda.synchronize()
+                case[key] = timed_eager(v, acts if deep else acts_shallow, st, args.steps, args.warmup)
+                err = v.env.env_errors()
+                if err.any():
+                    raise SystemExit(f"deep vector bench: env errors {[hex(x) for x in np.unique(err)]} at {n_books} books, {rows} rows, {key}")
+                v.close()
+            res["cases"].append(case)
+            print(json.dumps(case), flush=True)
 
 
 def main():
@@ -86,6 +156,7 @@ def main():
     ap.add_argument("--graph-steps", type=int, default=50)
     ap.add_argument("--graph-reps", type=int, default=4)
     ap.add_argument("--out", default=None)
+    ap.add_argument("--bg-agents", action="store_true", help="background agents: deep with agents, deep rows-only, FAST with agents (eager)")
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
@@ -93,7 +164,7 @@ def main():
     name, power = card()
     print(f"card: {name}, power limit: {power}", flush=True)
     books_list = [int(x) for x in args.books.split(",")]
-    rows_list = [int(x) for x in args.rows.split(",")]
+    rows_list = [int(x) for x in ("1,8" if args.bg_agents and args.rows == "1,8,32" else args.rows).split(",")]
     streams = []
     for i in range(N_DISTINCT):
         s = workloads.c5_stream(N_REST, 1, PER_STEP, seed=100 + i)
@@ -112,7 +183,7 @@ def main():
                                               "k_env_deep_stage": "2 bytes per queued row (permutation, not copied in or out)"},
            "cases": []}
     rng = np.random.default_rng(0)
-    for n_books in books_list:
+    for n_books in [] if args.bg_agents else books_list:
         for rows in [0] + rows_list:   # rows 0: one no-op row per env (the fixed cost of a step)
             r_eff = max(rows, 1)
             v = gym.VectorEnv(n_books, r_eff, 0, 0, 1, STEP, max_orders=n_pre + r_eff * n_steps_max + 64, max_trades=1 << 18,
@@ -184,6 +255,8 @@ def main():
             v.close()
             res["cases"].append(case)
             print(json.dumps(case), flush=True)
+    if args.bg_agents:
+        bg_agents_cases(args, res, streams, books_list, rows_list)
     line = json.dumps(res)
     print(line)
     if args.out:

@@ -1,5 +1,5 @@
-"""Randomised soak of the CUDA paths against the oracle: every round draws an engine, a population (single-asset, market
-twins, or background agents + external rows), sizes and a launch split, runs it on the GPU and compares a sample of books
+"""Randomised soak of the CUDA paths against the oracle: every round draws an engine (deep books included for the
+single-asset and external-row rounds), a population (single-asset, market twins, or background agents + external rows), sizes and a launch split, runs it on the GPU and compares a sample of books
 bit for bit (level-2 history, trade log, order table).  python scripts/soak.py <seconds> [first_seed]"""
 import sys
 import time
@@ -98,6 +98,11 @@ while time.time() < t_end and (not only or rounds < len(only)):
     dense = rng.random() < 0.4
     kw = dict(price_window=(0, 256), live_cap=254) if dense else (dict() if rng.random() < 0.6 else dict(pages_smem=int(rng.integers(2, 12)), pages_total=64))
     gs = rand_groups(rng, dense)
+    if mode != "market" and rng.random() < 0.25:
+        # the deep-book engine: C3 centred inside its window (every RandomAgents price must rest there), the rows' prices too
+        dense, kw = False, dict(price_window=(0, 256), deep_chunks=16384 // 8 + 2 * 256 + 64)
+        gs = [("r", (int(g["n_agents"]), (int(g["tick_lo"]), int(g["tick_hi"])), (int(g["vol_lo"]), int(g["vol_hi"])), int(g["tick_size"]),
+                     float(g["rate"]))) for g in workloads.c3_groups_around(100)]
     n_steps = int(rng.integers(5, 60)); split = int(rng.integers(1, n_steps + 1)); rs = int(rng.integers(1 << 30))
     desc = f"seed {seed} {mode} {'dense' if dense else kw} groups {[k for k, _ in gs]} steps {n_steps}/{split}"
     try:
